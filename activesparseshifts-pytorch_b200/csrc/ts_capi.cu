@@ -188,6 +188,8 @@ int ts_set_tuning(const char* spec) {
         else if (!strcmp(key, "flat_stage_kb")) t.flat_stage_kb = val;
         else if (!strcmp(key, "flat_stages")) t.flat_stages = val;
         else if (!strcmp(key, "flat_warps")) t.flat_warps = val;
+        else if (!strcmp(key, "cl_ahead")) t.cl_ahead = val;
+        else if (!strcmp(key, "cl_rows")) t.cl_rows = val;
         else return TS_ERR_INVALID_ARGUMENT;
         p += n;
         while (*p == ',' || *p == ' ') ++p;
@@ -197,7 +199,8 @@ int ts_set_tuning(const char* spec) {
         t.tma_ctas_per_sm < 0 || t.tma_ctas_per_sm > 8 || t.tma_warps < 0 || t.tma_warps > 31 || t.tma_stage_kb < 0 ||
         t.tma_stage_kb > 220 || t.nhwc_variant < 0 || t.nhwc_variant > 3 || t.nhwc_ring_rows < 0 || t.nhwc_rows_warps < 0 || t.nhwc_rows_warps > 12 || t.halo < 0 || t.halo > 16 ||
         t.halo_stages < 0 || t.halo_stages > 32 || t.halo_warps < 0 || t.halo_warps > 15 || t.flat_ctas < 0 || t.flat_ctas > 8 ||
-        t.flat_stage_kb < 0 || t.flat_stage_kb > 100 || t.flat_stages < 0 || t.flat_stages > 16 || t.flat_warps < 0 || t.flat_warps > 15)
+        t.flat_stage_kb < 0 || t.flat_stage_kb > 100 || t.flat_stages < 0 || t.flat_stages > 16 || t.flat_warps < 0 || t.flat_warps > 15 ||
+        t.cl_ahead < 0 || t.cl_ahead > 4 || (t.cl_rows != 0 && t.cl_rows != 1 && t.cl_rows != 2 && t.cl_rows != 4 && t.cl_rows != 8))
         return TS_ERR_INVALID_ARGUMENT;
     tuning() = t;
     g_tuning_epoch.fetch_add(1);
@@ -458,6 +461,57 @@ int ts_shift_backward_allreduce(const ts_geometry* gin, int dtype, int padding, 
         if (!peers->bufs[p] || ((uintptr_t)peers->bufs[p] & 7)) return TS_ERR_INVALID_ARGUMENT;
     return backward_impl(gin, dtype, padding, active, grad, x, weights, grad_input, grad_weight, workspace, workspace_bytes, peers,
                          stream);
+}
+
+int ts_shift_forward_nhwc(const ts_geometry* gin, int dtype, int padding, int active, const void* x, const void* weights, void* y,
+                          void* stream) {
+    Geo g;
+    int rc = make_geo(gin, padding, &g);
+    if (rc != TS_OK) return rc;
+    if (!elem_size(dtype)) return TS_ERR_INVALID_ARGUMENT;
+    if (g_forced_path.load() != TS_PATH_NONE) return TS_ERR_UNSUPPORTED;      // a forced family: callers take the planar path
+    if (g.N * g.C == 0 || g.out_plane == 0) return TS_ERR_UNSUPPORTED;
+    if (!x || !weights || !y) return TS_ERR_INVALID_ARGUMENT;
+    int sms = 0;
+    if ((rc = sm_count(&sms)) != TS_OK) return rc;
+    rc = cl_forward(g, dtype, active, x, weights, y, sms, (cudaStream_t)stream);
+    if (rc == TS_OK) t_last_path = TS_PATH_NHWC;
+    return rc;
+}
+
+size_t ts_shift_backward_nhwc_workspace_bytes(const ts_geometry* gin, int dtype) {
+    Geo g;
+    if (make_geo(gin, 0, &g) != TS_OK) return 0;
+    int sms = 148;
+    sm_count(&sms);
+    return cl_backward_workspace_bytes(g, dtype, sms);
+}
+
+int ts_shift_backward_nhwc(const ts_geometry* gin, int dtype, int padding, int active, const void* grad, const void* x, const void* weights,
+                           void* grad_input, void* grad_weight, void* workspace, size_t workspace_bytes, const ts_peer_group* peers,
+                           void* stream) {
+    Geo g;
+    int rc = make_geo(gin, padding, &g);
+    if (rc != TS_OK) return rc;
+    if (!elem_size(dtype)) return TS_ERR_INVALID_ARGUMENT;
+    if (peers) {      // the checks of ts_shift_backward_allreduce
+        if (peers->world < 1 || peers->world > 8 || peers->rank < 0 || peers->rank >= peers->world || !peers->state)
+            return TS_ERR_INVALID_ARGUMENT;
+        if (dtype != TS_F32 && dtype != TS_F16 && dtype != TS_BF16) return TS_ERR_UNSUPPORTED;
+        if (gin->C * gin->dim > peers->capacity || peers->capacity > 4096 || gin->C == 0) return TS_ERR_INVALID_ARGUMENT;
+        for (int p = 0; p < peers->world; ++p)
+            if (!peers->bufs[p] || ((uintptr_t)peers->bufs[p] & 7)) return TS_ERR_INVALID_ARGUMENT;
+    }
+    if (g_forced_path.load() != TS_PATH_NONE) return TS_ERR_UNSUPPORTED;
+    if (g.N * g.C == 0 || g.in_plane == 0) return TS_ERR_UNSUPPORTED;        // empty shards: the planar path (zeros / exchange)
+    if (!grad || !x || !weights || !grad_input || !grad_weight) return TS_ERR_INVALID_ARGUMENT;
+    if (!workspace || ((uintptr_t)workspace & 15)) return TS_ERR_WORKSPACE;
+    int sms = 0;
+    if ((rc = sm_count(&sms)) != TS_OK) return rc;
+    rc = cl_backward(g, dtype, active, grad, x, weights, grad_input, grad_weight, (double*)workspace, workspace_bytes, peers, sms,
+                     (cudaStream_t)stream);
+    if (rc == TS_OK) t_last_path = TS_PATH_NHWC;
+    return rc;
 }
 
 int ts_qshift_forward(const ts_geometry* gin, int elem_bytes, int padding, int64_t zero_point, const void* xq,

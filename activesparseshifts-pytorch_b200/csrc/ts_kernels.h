@@ -64,6 +64,13 @@ int nhwc_gather(const Geo& g, const void* x, void* y, unsigned long long fill, i
 
 int nhwc_to_planar(const void* x, void* y, long long N, long long C, long long P, int esize, cudaStream_t s);
 
+// ---- channels-last float forward / backward (ts_nhwc_float.cu): 2-D, fp32 / fp16 / bf16, dense NHWC, C % 32 == 0 ----
+// TS_ERR_UNSUPPORTED (nothing launched) for what they do not serve.  partials: cl_backward_workspace_bytes().
+int cl_forward(const Geo& g, int dtype, int active, const void* x, const void* w, void* y, int sm_count, cudaStream_t s);
+size_t cl_backward_workspace_bytes(const Geo& g, int dtype, int sm_count);
+int cl_backward(const Geo& g, int dtype, int active, const void* grad, const void* x, const void* w, void* gi, void* gw, double* partials,
+                size_t workspace_bytes, const ts_peer_group* peers, int sm_count, cudaStream_t s);
+
 // ---- staged family (ts_staged.cu): bulk-async shared-memory staging ---------------------------
 struct Tuning {
     int stages;        // ring depth
@@ -93,6 +100,7 @@ struct Tuning {
     int use_flat;      // 0: the automatic path choice never picks the flat zero-padding gather
     int flat_variant;  // 0 auto (a warp owns whole planes when C <= 512), 1 item-per-thread with shuffled shifts
     int flat_ctas, flat_stage_kb, flat_stages, flat_warps;   // flat gather: CTAs per SM (0 = 2), stage KiB (0 = 24), ring depth (0 = 4), consumer warps (0 = auto)
+    int cl_ahead, cl_rows;   // channels-last float kernels: steps of copies in flight (0 = 2, at most 4), rows per step (0 = 2; 1, 2, 4, 8)
 };
 Tuning& tuning();
 

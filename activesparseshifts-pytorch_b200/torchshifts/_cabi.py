@@ -23,6 +23,7 @@ EXPORTED_SYMBOLS = (
     'ts_debug_remap_reduced', 'ts_debug_split_f32', 'ts_debug_split_f64', 'ts_shift_forward',
     'ts_shift_backward_workspace_bytes', 'ts_shift_backward', 'ts_qshift_forward', 'ts_shift_backward_allreduce',
     'ts_qshift_forward_nhwc', 'ts_debug_nhwc_emulate', 'ts_nhwc_to_nchw', 'ts_shift2d_avgpool2_forward', 'ts_shift2d_avgpool2_backward',
+    'ts_shift_forward_nhwc', 'ts_shift_backward_nhwc_workspace_bytes', 'ts_shift_backward_nhwc',
 )
 
 
@@ -83,6 +84,9 @@ class NativeLibrary:
             'ts_debug_nhwc_emulate': (i, [gp, i, i, i64, vp, vp, i, i64, vp, i, i, i, i]),
             'ts_nhwc_to_nchw': (i, [vp, vp, i64, i64, i64, i, vp]),
             'ts_shift_backward_allreduce': (i, [gp, i, i, i, vp, vp, vp, vp, vp, vp, sz, ct.POINTER(PeerGroup), vp]),
+            'ts_shift_forward_nhwc': (i, [gp, i, i, i, vp, vp, vp, vp]),
+            'ts_shift_backward_nhwc_workspace_bytes': (sz, [gp, i]),
+            'ts_shift_backward_nhwc': (i, [gp, i, i, i, vp, vp, vp, vp, vp, vp, sz, ct.POINTER(PeerGroup), vp]),
         }
         for name, (res, args) in sig.items():
             if not hasattr(lib, name) and os.environ.get('TORCHSHIFTS_B200_LIB'):

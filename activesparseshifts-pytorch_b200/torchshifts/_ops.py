@@ -9,6 +9,17 @@ Operator names and schemas are the reference's (csrc/torchshifts.cpp:35-40, csrc
     torchshifts::_shift{1,2,3}d_backward(Tensor grad, Tensor weights, Tensor input, Tensor borders,
                                          int padding_mode, bool active_flag) -> (Tensor, Tensor)
 
+Extension over the reference (the functional layer routes channels-last inputs here under
+``memory_format=torch.preserve_format``; the reference's float path always returns NCHW):
+
+    torchshifts::_shift{2,3}d_forward_cl(Tensor input, Tensor weights, Tensor borders, int[] new_size,
+                                         int padding_mode, bool active_flag) -> Tensor
+    torchshifts::_shift{2,3}d_backward_cl(Tensor grad, Tensor weights, Tensor input, Tensor borders,
+                                          int padding_mode, bool active_flag) -> (Tensor, Tensor)
+
+same arguments and values as ``_shiftNd_forward/_backward``, but the output and ``grad_input`` are dense
+channels-last (``channels_last`` / ``channels_last_3d``).
+
 Dispatch keys: ``shiftNd`` is CompositeImplicitAutograd (border validation, then ``_shiftNd_forward``);
 ``_shiftNd_forward/_backward`` carry the autograd wiring of csrc/ops/autograd/shifts_autograd.cpp
 (``torch.library.register_autograd``: saves input/weights/borders, double backward is an error),
@@ -165,14 +176,18 @@ def _workspace_bytes(geo, key, code, device):
 
 
 # ------------------------------------------------------------------------------------------ CUDA
-def _forward_cuda(dim, input, weights, borders, new_size, padding_mode, active_flag):
-    fn = f'shift{dim}d_forward'
+def _check_forward(fn, dim, input, weights, padding_mode):
     _check_mode(padding_mode)
     _same_device_and_type(fn, input, weights)
     if input.dim() != dim + 2:
         raise RuntimeError(f'{fn}: expected a {dim + 2}-D input, got {input.dim()}-D')
     if weights.dim() != 2 or weights.shape[0] != input.shape[1] or weights.shape[1] != dim:
         raise RuntimeError(f'{fn}: weights must be [{input.shape[1]}, {dim}], got {list(weights.shape)}')
+
+
+def _forward_cuda(dim, input, weights, borders, new_size, padding_mode, active_flag):
+    fn = f'shift{dim}d_forward'
+    _check_forward(fn, dim, input, weights, padding_mode)
     lb, rb = _borders_lists(borders, dim)
     out = torch.empty(list(new_size), dtype=input.dtype, device=input.device)
     w = weights.contiguous()
@@ -271,6 +286,20 @@ def _pool_backward_meta(grad_pooled, weights, input, borders, new_size, padding_
     return input.new_empty(input.shape), weights.new_empty(weights.shape)
 
 
+def _check_fused(fn, fused, dev, code, weight_numel):
+    # Taking part in the in-kernel exchange must never depend on rank-local data (an empty shard, a ragged last
+    # batch): a rank that skipped it would leave its peers waiting.  What cannot be served raises on EVERY rank
+    # (dtype, weight count and device are the same everywhere for replicated layers).
+    if fused.device != dev:
+        raise RuntimeError(f'{fn}: FusedGradWeightAllReduce was created for {fused.device} but the tensors live on {dev}')
+    if code == 1:
+        raise RuntimeError(f'{fn}: the fused grad_weight all-reduce carries fp32 contributions; float64 layers must use '
+                           'torchshifts.sharded.allreduce_grad_weights (disable() the fused mode around them)')
+    if weight_numel > fused.capacity:
+        raise RuntimeError(f'{fn}: {weight_numel} weight elements exceed the exchange capacity {fused.capacity} '
+                           '(FusedGradWeightAllReduce(capacity=...), at most 4096)')
+
+
 def _backward_cuda(dim, grad, weights, input, borders, padding_mode, active_flag):
     fn = f'shift{dim}d_backward'
     _check_mode(padding_mode)
@@ -288,17 +317,7 @@ def _backward_cuda(dim, grad, weights, input, borders, padding_mode, active_flag
     dev = input.device
     fused = _FUSED_ALLREDUCE
     if fused is not None:
-        # Taking part in the in-kernel exchange must never depend on rank-local data (an empty shard, a ragged last
-        # batch): a rank that skipped it would leave its peers waiting.  What cannot be served raises on EVERY rank
-        # (dtype, weight count and device are the same everywhere for replicated layers).
-        if fused.device != dev:
-            raise RuntimeError(f'{fn}: FusedGradWeightAllReduce was created for {fused.device} but the tensors live on {dev}')
-        if code == 1:
-            raise RuntimeError(f'{fn}: the fused grad_weight all-reduce carries fp32 contributions; float64 layers must use '
-                               'torchshifts.sharded.allreduce_grad_weights (disable() the fused mode around them)')
-        if w.numel() > fused.capacity:
-            raise RuntimeError(f'{fn}: {w.numel()} weight elements exceed the exchange capacity {fused.capacity} '
-                               '(FusedGradWeightAllReduce(capacity=...), at most 4096)')
+        _check_fused(fn, fused, dev, code, w.numel())
     with _guard(dev):
         for attempt in (0, 1):
             nbytes = _workspace_bytes(geo, key, code, dev)
@@ -315,6 +334,94 @@ def _backward_cuda(dim, grad, weights, input, borders, padding_mode, active_flag
     if st:
         _NATIVE.check(st, 'ts_shift_backward_allreduce' if fused is not None else 'ts_shift_backward')
     return out_grad, weights_grad
+
+
+# ------------------------------------------------------------------------------------------ CUDA, channels-last
+_CL_WS_CACHE = {}      # (geometry key, dtype code, device index) -> workspace bytes of ts_shift_backward_nhwc
+
+
+def _cl_workspace_bytes(geo, key, code, device):
+    wkey = (key, code, device.index)
+    n = _CL_WS_CACHE.get(wkey)
+    if n is None:
+        if len(_CL_WS_CACHE) > 256:
+            _CL_WS_CACHE.clear()
+        with _guard(device):
+            n = _CL_WS_CACHE[wkey] = int(_NATIVE.lib.ts_shift_backward_nhwc_workspace_bytes(ct.byref(geo), code))
+    return n
+
+
+def _forward_cl_cuda(dim, input, weights, borders, new_size, padding_mode, active_flag):
+    """``_shiftNd_forward`` with a dense channels-last output.  2-D dense channels-last fp32 / fp16 / bf16 inputs run the
+    native NHWC kernel (ts_shift_forward_nhwc: one read, one write, no layout pass); whatever it does not serve takes the
+    planar forward and converts its output -- the same values."""
+    fn = f'shift{dim}d_forward_cl'
+    fmt = _CL_FORMATS[dim + 2]
+    _check_forward(fn, dim, input, weights, padding_mode)
+    if dim == 2 and input.dtype != torch.float64 and input.shape[1] % 32 == 0 and input.is_contiguous(memory_format=fmt):
+        lb, rb = _borders_lists(borders, dim)
+        if list(new_size) != list(input.shape[:2]) + [rb[a] - lb[a] for a in range(dim)]:
+            raise RuntimeError(f'{fn}: new_size {list(new_size)} does not match the borders')
+        out = torch.empty(list(new_size), dtype=input.dtype, device=input.device, memory_format=fmt)
+        w = weights.contiguous()
+        geo, _ = _geometry(dim, input, lb, rb)
+        with _guard(input.device):
+            st = _NATIVE.lib.ts_shift_forward_nhwc(ct.byref(geo), _DTYPES[input.dtype], int(padding_mode), int(bool(active_flag)),
+                                                   input.data_ptr(), w.data_ptr(), out.data_ptr(), _stream(input.device))
+        if st == 0:
+            return out
+        if st != 2:        # TS_ERR_UNSUPPORTED: the planar path below
+            _NATIVE.check(st, 'ts_shift_forward_nhwc')
+    return _forward_cuda(dim, input, weights, borders, new_size, padding_mode, active_flag).contiguous(memory_format=fmt)
+
+
+def _backward_cl_cuda(dim, grad, weights, input, borders, padding_mode, active_flag):
+    """``_shiftNd_backward`` with a dense channels-last ``grad_input``.  ``grad`` may arrive in any layout (an expanded
+    tensor from ``.sum()``, say): the native kernel (ts_shift_backward_nhwc) reads it dense channels-last.  What the
+    kernel does not serve takes the planar backward and converts ``grad_input`` -- the same values."""
+    fn = f'shift{dim}d_backward_cl'
+    fmt = _CL_FORMATS[dim + 2]
+    _check_mode(padding_mode)
+    _same_device_and_type(fn, input, weights, grad)
+    code = _DTYPES[input.dtype]
+    dev = input.device
+    fused = _FUSED_ALLREDUCE
+    if fused is not None:
+        _check_fused(fn, fused, dev, code, weights.numel())
+    nbytes = 0
+    if dim == 2 and code != 1 and input.dim() == 4 and input.shape[1] % 32 == 0 and input.is_contiguous(memory_format=fmt):
+        lb, rb = _borders_lists(borders, dim)
+        geo, key = _geometry(dim, input, lb, rb)
+        nbytes = _cl_workspace_bytes(geo, key, code, dev)
+    # 16 bytes: the kernel does not serve this geometry -- decided before grad is converted to a layout the planar path
+    # would convert again
+    for attempt in (0, 1):
+        if nbytes <= 16:
+            break
+        if list(grad.shape[2:]) != [rb[a] - lb[a] for a in range(dim)] or list(grad.shape[:2]) != list(input.shape[:2]):
+            raise RuntimeError(f'{fn}: grad shape {list(grad.shape)} does not match the (cropped) output of input {list(input.shape)}')
+        grad_cl = grad.contiguous(memory_format=fmt)
+        w = weights.contiguous()
+        out_grad = torch.empty(input.shape, dtype=input.dtype, device=dev, memory_format=fmt)
+        weights_grad = torch.empty(w.shape, dtype=w.dtype, device=dev)
+        workspace = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+        with _guard(dev):
+            st = _NATIVE.lib.ts_shift_backward_nhwc(ct.byref(geo), code, int(padding_mode), int(bool(active_flag)), grad_cl.data_ptr(),
+                                                    input.data_ptr(), w.data_ptr(), out_grad.data_ptr(), weights_grad.data_ptr(),
+                                                    workspace.data_ptr(), nbytes,
+                                                    ct.byref(fused.peer_group()) if fused is not None else None, _stream(dev))
+        if st == 0:
+            return out_grad, weights_grad
+        if st == 2:        # TS_ERR_UNSUPPORTED (e.g. a misaligned view): the planar path below
+            break
+        if st != 3:
+            _NATIVE.check(st, 'ts_shift_backward_nhwc')
+        _CL_WS_CACHE.clear()      # TS_ERR_WORKSPACE (nothing was launched): the tuning knobs changed since the size was cached
+        nbytes = _cl_workspace_bytes(geo, key, code, dev)
+    else:
+        _NATIVE.check(st, 'ts_shift_backward_nhwc')
+    grad_input, grad_weight = _backward_cuda(dim, grad, weights, input, borders, padding_mode, active_flag)
+    return grad_input.contiguous(memory_format=fmt), grad_weight
 
 
 _QW_CACHE = {}         # id(quantized weight) -> (weakref, version, device, raw integer weights on that device)
@@ -391,6 +498,15 @@ def _backward_meta(dim, grad, weights, input, borders, padding_mode, active_flag
     return input.new_empty(input.shape), weights.new_empty(weights.shape)
 
 
+def _forward_cl_meta(dim, input, weights, borders, new_size, padding_mode, active_flag):
+    return torch.empty(list(new_size), dtype=input.dtype, device=input.device, memory_format=_CL_FORMATS[dim + 2])
+
+
+def _backward_cl_meta(dim, grad, weights, input, borders, padding_mode, active_flag):
+    return (torch.empty(input.shape, dtype=input.dtype, device=input.device, memory_format=_CL_FORMATS[dim + 2]),
+            weights.new_empty(weights.shape))
+
+
 # ------------------------------------------------------------------------------------------ Autograd
 # csrc/ops/autograd/shifts_autograd.cpp:15-47 (and the 2d/3d twins): forward saves input, weights and
 # borders; backward calls _shiftNd_backward and returns grads for input and weights only; the backward
@@ -404,10 +520,10 @@ def _setup_forward_context(ctx, inputs, output):
         _claim_planar(input)
 
 
-def _make_forward_backward(dim):
+def _make_forward_backward(dim, suffix=''):
     def backward(ctx, grad_output):
         input, weights, borders = ctx.saved_tensors
-        op = getattr(torch.ops.torchshifts, f'_shift{dim}d_backward')
+        op = getattr(torch.ops.torchshifts, f'_shift{dim}d_backward{suffix}')
         grad_input, grad_weight = op(grad_output, weights, input, borders, ctx.padding_mode, ctx.active_flag)
         return grad_input, grad_weight, None, None, None, None
     return backward
@@ -483,6 +599,18 @@ def register(native):
         for key in ('CPU', 'QuantizedCPU'):
             lib.impl(fwd, _no_cpu, key)
             lib.impl(bwd, _no_cpu, key)
+    for dim in (2, 3):
+        fwd, bwd = f'_shift{dim}d_forward_cl', f'_shift{dim}d_backward_cl'
+        lib.define(f'{fwd}(Tensor input, Tensor weights, Tensor borders, int[] new_size, int padding_mode, bool active_flag) -> Tensor')
+        lib.define(f'{bwd}(Tensor grad, Tensor weights, Tensor input, Tensor borders, int padding_mode, bool active_flag) -> (Tensor, Tensor)')
+        lib.impl(fwd, _bind(_forward_cl_cuda, dim), 'CUDA')
+        lib.impl(bwd, _bind(_backward_cl_cuda, dim), 'CUDA')
+        lib.impl(fwd, _no_cpu, 'CPU')
+        lib.impl(bwd, _no_cpu, 'CPU')
+        torch.library.register_fake(f'torchshifts::{fwd}', _bind(_forward_cl_meta, dim), lib=lib)
+        torch.library.register_fake(f'torchshifts::{bwd}', _bind(_backward_cl_meta, dim), lib=lib)
+        torch.library.register_autograd(f'torchshifts::{fwd}', _make_forward_backward(dim, '_cl'), setup_context=_setup_forward_context, lib=lib)
+        torch.library.register_autograd(f'torchshifts::{bwd}', _double_backward, setup_context=_setup_backward_context, lib=lib)
     # fused epilogue of the strided depth-wise-conv emulation (modules/shifts.py:85-89): shift + crop + avg_pool2d(2, 2, ceil)
     pool = '_shift2d_avgpool2_forward'
     lib.define(f'{pool}(Tensor input, Tensor weights, Tensor borders, int[] new_size, int padding_mode, bool active_flag) -> Tensor')

@@ -45,10 +45,47 @@ def _std_borders(vals):
     return torch.tensor(list(vals), dtype=torch.int32)
 
 
+_CL_FORMATS = {2: torch.channels_last, 3: torch.channels_last_3d}
+
+
+def _check_memory_format(memory_format) -> bool:
+    """-> True for ``torch.preserve_format``, False for ``torch.contiguous_format``; anything else raises."""
+    if memory_format is torch.contiguous_format:
+        return False
+    if memory_format is torch.preserve_format:
+        return True
+    raise ValueError(f'memory_format must be torch.contiguous_format or torch.preserve_format, got {memory_format!r}')
+
+
+def _keeps_channels_last(dim: int, input: Tensor) -> bool:
+    """Dense channels-last (not also NCHW-contiguous) float input of a 2-D / 3-D shift."""
+    fmt = _CL_FORMATS.get(dim)
+    return (fmt is not None and not input.is_quantized and input.is_contiguous(memory_format=fmt)
+            and not input.is_contiguous())
+
+
+def _shift_cl(dim: int, input: Tensor, weights: Tensor, padding_mode: int, active_flag: bool,
+              borders: Optional[Tensor], _border_ints) -> Tensor:
+    """The channels-last operator ``_shift{dim}d_forward_cl``: output (and grad_input) dense channels-last."""
+    from . import _ops
+    if borders is None:
+        cuts = [[0, 0]] * dim
+    else:
+        cuts = _border_ints if _border_ints is not None else [[int(v) for v in row] for row in borders.tolist()]
+    lb, rb = _resolve_borders(dim, input.shape[2:], cuts)
+    std = _std_borders((lb[0], rb[0], lb[1], rb[1], lb[2], rb[2]))
+    new_size = [input.shape[0], input.shape[1]] + [rb[a] - lb[a] for a in range(dim)]
+    out = getattr(torch.ops.torchshifts, f'_shift{dim}d_forward_cl')(input, weights, std, new_size, padding_mode, active_flag)
+    if not torch.compiler.is_compiling():
+        _ops._LAST_PLANAR[0] = None      # a planar copy of the fallback path nobody claimed (no autograd): drop it now
+    return out
+
+
 def _shift_func(dim: int, input: Tensor, weights: Tensor, padding_mode: int, active_flag: bool,
-                borders: Optional[Tensor], _border_ints=None) -> Tensor:
+                borders: Optional[Tensor], _border_ints=None, memory_format=torch.contiguous_format) -> Tensor:
     name = f'shift{dim}d_func()'
     _assert_has_ops()
+    preserve = _check_memory_format(memory_format)
     assert padding_mode in [0, 1, 2, 3, 4], f'{name} expected padding_mode can be {_MODES}'
     assert len(input.shape) == dim + 2, f'{name[:-2]}(): expected {dim + 2}D tensor as input, but it is shape is {input.shape}'
     assert weights.shape[-1] == dim, f'{name[:-2]}(): expected [n_channels,{dim}] tensor as weight, but it is shape is {weights.shape}'
@@ -58,6 +95,9 @@ def _shift_func(dim: int, input: Tensor, weights: Tensor, padding_mode: int, act
                                             f'but input is  on {input.device} and weights is on {weights.device}')
     if borders is not None:
         assert (len(borders.shape) == 2) and (borders.shape[1] == 2) and (borders.shape[0] == dim), f'borders must have shape [{dim}, 2]'
+    if preserve and _keeps_channels_last(dim, input):
+        return _shift_cl(dim, input, weights, padding_mode, active_flag, borders, _border_ints)
+    if borders is not None:
         if _border_ints is not None and torch.compiler.is_compiling():
             # torch.compile: resolve the crop from Python integers (constants of the trace) and call the inner
             # operator, which has a fake kernel and a registered autograd formula
@@ -72,29 +112,36 @@ def _shift_func(dim: int, input: Tensor, weights: Tensor, padding_mode: int, act
 
 
 def shift1d_func(input: Tensor, weights: Tensor, padding_mode: int, active_flag: bool,
-                 borders: Optional[Tensor] = None, _border_ints=None) -> Tensor:
+                 borders: Optional[Tensor] = None, _border_ints=None, *, memory_format=torch.contiguous_format) -> Tensor:
     """Shift every channel of ``input [N, C, H]`` along H by its own learnable amount.
 
     ``weights [C, 1]`` holds sign and magnitude of the per-channel shift; ``padding_mode`` selects
     what is read outside the tensor (0 zeros, 1 border, 2 periodic, 3 reflect, 4 symmetric);
     ``active_flag`` switches from the rounded (sparse) shift to linear interpolation (ignored for
     quantized inputs); ``borders [1, 2]`` = (left_cut, right_cut) crops the output.
+    ``memory_format`` (keyword only) is accepted for symmetry with the 2-D / 3-D layers and ignored: 3-D
+    tensors have no channels-last format.
     """
-    return _shift_func(1, input, weights, padding_mode, active_flag, borders, _border_ints)
+    return _shift_func(1, input, weights, padding_mode, active_flag, borders, _border_ints, memory_format)
 
 
 def shift2d_func(input: Tensor, weights: Tensor, padding_mode: int, active_flag: bool,
-                 borders: Optional[Tensor] = None, _border_ints=None) -> Tensor:
+                 borders: Optional[Tensor] = None, _border_ints=None, *, memory_format=torch.contiguous_format) -> Tensor:
     """2-D version: ``input [N, C, H, W]``, ``weights [C, 2]`` (H and W shifts), ``borders [2, 2]``;
-    the active shift is bilinear."""
-    return _shift_func(2, input, weights, padding_mode, active_flag, borders, _border_ints)
+    the active shift is bilinear.
+
+    ``memory_format`` (keyword only): ``torch.contiguous_format`` (default) returns NCHW outputs and NCHW
+    ``grad_input``, as the reference does; ``torch.preserve_format`` returns both dense ``channels_last`` when
+    ``input`` is dense channels-last (and not also NCHW-contiguous), with the same values.  Other layouts give
+    the default result.  This is an extension over the reference."""
+    return _shift_func(2, input, weights, padding_mode, active_flag, borders, _border_ints, memory_format)
 
 
 def shift3d_func(input: Tensor, weights: Tensor, padding_mode: int, active_flag: bool,
-                 borders: Optional[Tensor] = None, _border_ints=None) -> Tensor:
+                 borders: Optional[Tensor] = None, _border_ints=None, *, memory_format=torch.contiguous_format) -> Tensor:
     """3-D version: ``input [N, C, H, W, D]``, ``weights [C, 3]``, ``borders [3, 2]``; the active
-    shift is trilinear."""
-    return _shift_func(3, input, weights, padding_mode, active_flag, borders, _border_ints)
+    shift is trilinear.  ``memory_format`` as for :func:`shift2d_func`, with ``channels_last_3d``."""
+    return _shift_func(3, input, weights, padding_mode, active_flag, borders, _border_ints, memory_format)
 
 
 def shift2d_avgpool2_func(input: Tensor, weights: Tensor, padding_mode: int, active_flag: bool,

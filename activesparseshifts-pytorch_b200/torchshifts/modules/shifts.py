@@ -18,7 +18,8 @@ from functools import partial
 import torch
 from torch import nn
 
-from torchshifts.functional import shift1d_func, shift2d_avgpool2_func, shift2d_func, shift3d_func
+from torchshifts.functional import (_check_memory_format, _keeps_channels_last, shift1d_func, shift2d_avgpool2_func,
+                                    shift2d_func, shift3d_func)
 
 paddings_dict = {'zeros': 0, 'border': 1, 'periodic': 2, 'reflect': 3, 'symmetric': 4}
 _SHIFT_FUNCS = {1: shift1d_func, 2: shift2d_func, 3: shift3d_func}
@@ -84,6 +85,9 @@ class _Shiftnd(nn.Module):
         emulate_dw (dict): parameters of the depth-wise convolution being replaced
             (kernel_size, padding, stride); output shape and initialisation follow it.
         init_thumb_rule (int): 1: uniform(-init_shift, init_shift); 2: see the module docstring.
+        memory_format (torch.memory_format): ``torch.contiguous_format`` (default): NCHW outputs, as the
+            reference; ``torch.preserve_format``: a dense channels-last input gives a channels-last output and
+            ``grad_input`` (see :func:`torchshifts.functional.shift2d_func`).  Ignored by ``Shift1d``.
     """
 
     @staticmethod
@@ -105,8 +109,10 @@ class _Shiftnd(nn.Module):
         return size * torch.rand(shape) * (1 if random.random() < 0.5 else -1)
 
     def __init__(self, in_channels, padding='zeros', init_shift=1, sparsity_term=5e-4, active_flag=False,
-                 emulate_dw=None, init_thumb_rule=1):
+                 emulate_dw=None, init_thumb_rule=1, memory_format=torch.contiguous_format):
         super(_Shiftnd, self).__init__()
+        _check_memory_format(memory_format)
+        self.memory_format = memory_format
         assert padding.lower() in paddings_dict.keys(), f'incorrect padding option: {padding}'
         self.padding = paddings_dict[padding]
         self.sparsity_term = sparsity_term
@@ -161,7 +167,8 @@ class _Shiftnd(nn.Module):
         """The stride-2 average pooling of a 2-D depth-wise-conv emulation runs inside the shift kernel (one read, one
         quarter-size write) for float32 CUDA tensors; everything else takes the shift followed by ``_reduction_fn``."""
         return (self.dim == 2 and self._reduction_fn is not self._identity and input.is_cuda and input.dtype == torch.float32
-                and not input.is_quantized and self._stride_ints == [2, 2])
+                and not input.is_quantized and self._stride_ints == [2, 2]
+                and not (self.memory_format is torch.preserve_format and _keeps_channels_last(2, input)))
 
     def forward(self, input):
         loss = self._compute_weight_loss() if bool(self.sparsity_term) else None
@@ -170,10 +177,10 @@ class _Shiftnd(nn.Module):
                                         _border_ints=self._border_ints())
             return out, loss
         if self.cut_borders is None:
-            out = self._shift_func(input, self.weight, self.padding, self._active_flag, None)
+            out = self._shift_func(input, self.weight, self.padding, self._active_flag, None, memory_format=self.memory_format)
         else:
             out = self._shift_func(input, self.weight, self.padding, self._active_flag, self.cut_borders,
-                                   _border_ints=self._border_ints())
+                                   _border_ints=self._border_ints(), memory_format=self.memory_format)
         return self._reduction_fn(out), loss
 
     def extra_repr(self):
@@ -186,9 +193,9 @@ class _Shiftnd(nn.Module):
 def _make_shift_class(dim, what):
     class _Shift(_Shiftnd):
         def __init__(self, in_channels, padding='zeros', init_shift=1, sparsity_term=5e-4, active_flag=False,
-                     emulate_dw=None, init_thumb_rule=1):
+                     emulate_dw=None, init_thumb_rule=1, memory_format=torch.contiguous_format):
             self.dim = dim
-            super().__init__(in_channels, padding, init_shift, sparsity_term, active_flag, emulate_dw, init_thumb_rule)
+            super().__init__(in_channels, padding, init_shift, sparsity_term, active_flag, emulate_dw, init_thumb_rule, memory_format)
 
     _Shift.__name__ = _Shift.__qualname__ = f'Shift{dim}d'
     _Shift.__doc__ = (f'Per-channel learnable shift of a {dim + 2}-D tensor ({what}).\n\n'

@@ -68,7 +68,8 @@ typedef enum ts_kernel_path {      /* which kernel family served the last call (
     TS_PATH_GENERIC = 1,           /* stride-generic one-element-per-thread kernels               */
     TS_PATH_STAGED = 2,            /* bulk-async (cp.async.bulk + mbarrier) shared-memory staged  */
     TS_PATH_TMA = 3,               /* TMA tensor copies: the copy engine applies shift + zero pad  */
-    TS_PATH_NHWC = 4,              /* channels-last in, channels-last out (ts_qshift_forward_nhwc) */
+    TS_PATH_NHWC = 4,              /* channels-last in, channels-last out (ts_qshift_forward_nhwc,
+                                      ts_shift_forward_nhwc, ts_shift_backward_nhwc)                */
     TS_PATH_HALO = 5,              /* slabs staged with a padded halo (TMA tensor loads), all-interior
                                       arithmetic: fp32 active forward / backward, every padding, crops  */
     TS_PATH_FLAT = 6               /* zeros padding, no crop: linear shifted copy of each dense slab with
@@ -93,7 +94,8 @@ const char*  ts_last_cuda_error(void);         /* text of the last CUDA error se
 int          ts_last_kernel_path(void);        /* ts_kernel_path of this thread's last launch     */
 int          ts_set_kernel_path(int path);     /* 0 auto (default), 1 force generic, 2 force staged,
                                                   3 force TMA, 5 force halo, 6 force flat (calls fail with TS_ERR_UNSUPPORTED
-                                                  when the forced family does not apply); returns
+                                                  when the forced family does not apply; the channels-last
+                                                  float entry points always do); returns
                                                   the old value                                   */
 uint64_t     ts_launch_count(void);            /* kernels launched by this library so far         */
 int          ts_set_tuning(const char* spec);  /* "key=value,..." staged-path tuning knobs; see
@@ -193,6 +195,22 @@ int ts_qshift_forward(const ts_geometry* g, int elem_bytes, int padding, int64_t
 int ts_qshift_forward_nhwc(const ts_geometry* g, int elem_bytes, int padding, int64_t zero_point,
                            const void* xq, const void* qweights, int qweight_kind,
                            int64_t weight_zero_point, void* yq, void* stream);
+
+/* Channels-last float forward and backward: tensors keep the channel axis innermost, no layout pass on either side.
+ * x dense channels-last (read through g->x_stride, channel stride 1); y dense [N, O0, O1(, O2), C];
+ * grad dense [N, O0, O1(, O2), C]; grad_input dense [N, S0, S1(, S2), C]; grad_weight dense [C, dim] in dtype,
+ * fully overwritten (deterministic two-pass reduction).  TS_ERR_UNSUPPORTED for what the kernels do not serve
+ * (dim 3, fp64, C not a multiple of 32, rows too wide to stage, misaligned pointers, empty tensors, a forced kernel
+ * family: see ts_set_kernel_path); callers then run the planar entry points and convert the layout.
+ * peers: NULL, or the exchange of ts_shift_backward_allreduce (same rules).  workspace: 16-byte aligned, at least
+ * ts_shift_backward_nhwc_workspace_bytes(). */
+int    ts_shift_forward_nhwc(const ts_geometry* g, int dtype, int padding, int active,
+                             const void* x, const void* weights, void* y, void* stream);
+size_t ts_shift_backward_nhwc_workspace_bytes(const ts_geometry* g, int dtype);
+int    ts_shift_backward_nhwc(const ts_geometry* g, int dtype, int padding, int active,
+                              const void* grad, const void* x, const void* weights,
+                              void* grad_input, void* grad_weight, void* workspace, size_t workspace_bytes,
+                              const ts_peer_group* peers /* NULL: no exchange */, void* stream);
 
 /* Layout adapter of the float path: x dense channels-last ([N, P, C] in memory, P = product of the spatial
  * sizes) -> y dense planar ([N, C, P]).  The reference hands channels-last float inputs to its nhwdc bodies

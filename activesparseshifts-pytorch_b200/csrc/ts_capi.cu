@@ -449,16 +449,23 @@ int ts_shift_backward(const ts_geometry* gin, int dtype, int padding, int active
                          stream);
 }
 
-int ts_shift_backward_allreduce(const ts_geometry* gin, int dtype, int padding, int active, const void* grad, const void* x,
-                                const void* weights, void* grad_input, void* grad_weight, void* workspace, size_t workspace_bytes,
-                                const ts_peer_group* peers, void* stream) {
-    if (!peers || !gin) return TS_ERR_INVALID_ARGUMENT;
+// the peer group of a backward with the in-kernel grad_weight exchange (gin and peers non-null)
+static int check_peers(const ts_geometry* gin, int dtype, const ts_peer_group* peers) {
     if (peers->world < 1 || peers->world > 8 || peers->rank < 0 || peers->rank >= peers->world || !peers->state)
         return TS_ERR_INVALID_ARGUMENT;
     if (dtype != TS_F32 && dtype != TS_F16 && dtype != TS_BF16) return TS_ERR_UNSUPPORTED;   // contributions travel as fp32
     if (gin->C * gin->dim > peers->capacity || peers->capacity > 4096 || gin->C == 0) return TS_ERR_INVALID_ARGUMENT;
     for (int p = 0; p < peers->world; ++p)
         if (!peers->bufs[p] || ((uintptr_t)peers->bufs[p] & 7)) return TS_ERR_INVALID_ARGUMENT;
+    return TS_OK;
+}
+
+int ts_shift_backward_allreduce(const ts_geometry* gin, int dtype, int padding, int active, const void* grad, const void* x,
+                                const void* weights, void* grad_input, void* grad_weight, void* workspace, size_t workspace_bytes,
+                                const ts_peer_group* peers, void* stream) {
+    if (!peers || !gin) return TS_ERR_INVALID_ARGUMENT;
+    const int rc = check_peers(gin, dtype, peers);
+    if (rc != TS_OK) return rc;
     return backward_impl(gin, dtype, padding, active, grad, x, weights, grad_input, grad_weight, workspace, workspace_bytes, peers,
                          stream);
 }
@@ -494,14 +501,7 @@ int ts_shift_backward_nhwc(const ts_geometry* gin, int dtype, int padding, int a
     int rc = make_geo(gin, padding, &g);
     if (rc != TS_OK) return rc;
     if (!elem_size(dtype)) return TS_ERR_INVALID_ARGUMENT;
-    if (peers) {      // the checks of ts_shift_backward_allreduce
-        if (peers->world < 1 || peers->world > 8 || peers->rank < 0 || peers->rank >= peers->world || !peers->state)
-            return TS_ERR_INVALID_ARGUMENT;
-        if (dtype != TS_F32 && dtype != TS_F16 && dtype != TS_BF16) return TS_ERR_UNSUPPORTED;
-        if (gin->C * gin->dim > peers->capacity || peers->capacity > 4096 || gin->C == 0) return TS_ERR_INVALID_ARGUMENT;
-        for (int p = 0; p < peers->world; ++p)
-            if (!peers->bufs[p] || ((uintptr_t)peers->bufs[p] & 7)) return TS_ERR_INVALID_ARGUMENT;
-    }
+    if (peers && (rc = check_peers(gin, dtype, peers)) != TS_OK) return rc;
     if (g_forced_path.load() != TS_PATH_NONE) return TS_ERR_UNSUPPORTED;
     if (g.N * g.C == 0 || g.in_plane == 0) return TS_ERR_UNSUPPORTED;        // empty shards: the planar path (zeros / exchange)
     if (!grad || !x || !weights || !grad_input || !grad_weight) return TS_ERR_INVALID_ARGUMENT;
@@ -514,20 +514,29 @@ int ts_shift_backward_nhwc(const ts_geometry* gin, int dtype, int padding, int a
     return rc;
 }
 
-int ts_qshift_forward(const ts_geometry* gin, int elem_bytes, int padding, int64_t zero_point, const void* xq,
-                      const void* qweights, int qweight_kind, int64_t weight_zero_point, void* yq, void* stream) {
-    Geo g;
-    int rc = make_geo(gin, padding, &g);
+static int qshift_common(const ts_geometry* gin, int elem_bytes, int padding, int qweight_kind, Geo* g) {
+    const int rc = make_geo(gin, padding, g);
     if (rc != TS_OK) return rc;
     if (elem_bytes != 1 && elem_bytes != 4) return TS_ERR_UNSUPPORTED;
     if (qweight_kind < TS_QW_U8 || qweight_kind > TS_QW_I32) return TS_ERR_INVALID_ARGUMENT;
+    return TS_OK;
+}
+
+static unsigned long long qfill(int elem_bytes, int64_t zero_point) {
+    return elem_bytes == 1 ? (unsigned long long)((unsigned)zero_point & 0xffu) : (unsigned long long)(uint32_t)(int32_t)zero_point;
+}
+
+int ts_qshift_forward(const ts_geometry* gin, int elem_bytes, int padding, int64_t zero_point, const void* xq,
+                      const void* qweights, int qweight_kind, int64_t weight_zero_point, void* yq, void* stream) {
+    Geo g;
+    int rc = qshift_common(gin, elem_bytes, padding, qweight_kind, &g);
+    if (rc != TS_OK) return rc;
     if (g.N * g.C == 0 || g.out_plane == 0) return TS_OK;
     if (!xq || !qweights || !yq) return TS_ERR_INVALID_ARGUMENT;
     int sms = 0;
     if ((rc = sm_count(&sms)) != TS_OK) return rc;
     cudaStream_t s = (cudaStream_t)stream;
-    const unsigned long long fill = elem_bytes == 1 ? (unsigned long long)((unsigned)zero_point & 0xffu)
-                                                    : (unsigned long long)(uint32_t)(int32_t)zero_point;
+    const unsigned long long fill = qfill(elem_bytes, zero_point);
     const int forced = g_forced_path.load();
     if ((forced == TS_PATH_NONE && tuning().use_tma) || forced == TS_PATH_TMA) {
         const TmaPlan tp = plan_tma(g, 0, 0, elem_bytes, -1, x_is_dense(g), fill, xq, yq, nullptr, sms);
@@ -555,18 +564,6 @@ int ts_qshift_forward(const ts_geometry* gin, int elem_bytes, int padding, int64
     }
     t_last_path = TS_PATH_GENERIC;
     return generic_gather(g, WK_QUANT, xq, yq, fill, elem_bytes, qweights, qweight_kind, weight_zero_point, s);
-}
-
-static int qshift_common(const ts_geometry* gin, int elem_bytes, int padding, int qweight_kind, Geo* g) {
-    const int rc = make_geo(gin, padding, g);
-    if (rc != TS_OK) return rc;
-    if (elem_bytes != 1 && elem_bytes != 4) return TS_ERR_UNSUPPORTED;
-    if (qweight_kind < TS_QW_U8 || qweight_kind > TS_QW_I32) return TS_ERR_INVALID_ARGUMENT;
-    return TS_OK;
-}
-
-static unsigned long long qfill(int elem_bytes, int64_t zero_point) {
-    return elem_bytes == 1 ? (unsigned long long)((unsigned)zero_point & 0xffu) : (unsigned long long)(uint32_t)(int32_t)zero_point;
 }
 
 int ts_qshift_forward_nhwc(const ts_geometry* gin, int elem_bytes, int padding, int64_t zero_point, const void* xq,

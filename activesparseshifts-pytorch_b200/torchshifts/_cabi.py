@@ -9,22 +9,12 @@ from pathlib import Path
 
 LIB_NAME = 'libtorchshifts_b200.so'
 
-TS_OK = 0
+TS_OK, TS_ERR_UNSUPPORTED, TS_ERR_WORKSPACE, TS_ERR_TOO_LARGE = 0, 2, 3, 4
 ABI_VERSION = 2
 STATUS_NAMES = {0: 'TS_OK', 1: 'TS_ERR_INVALID_ARGUMENT', 2: 'TS_ERR_UNSUPPORTED', 3: 'TS_ERR_WORKSPACE',
                 4: 'TS_ERR_TOO_LARGE', 5: 'TS_ERR_BORDERS', 6: 'TS_ERR_CUDA', 7: 'TS_ERR_NO_DEVICE'}
 PATH_NONE, PATH_GENERIC, PATH_STAGED, PATH_TMA, PATH_NHWC, PATH_HALO, PATH_FLAT = 0, 1, 2, 3, 4, 5, 6
 QW_U8, QW_I8, QW_I32 = 0, 1, 2
-
-# every symbol include/torchshifts_b200.h declares (tests check the library exports all of them)
-EXPORTED_SYMBOLS = (
-    'ts_abi_version', 'ts_cuda_version', 'ts_error_string', 'ts_last_cuda_error', 'ts_last_kernel_path',
-    'ts_set_kernel_path', 'ts_launch_count', 'ts_set_tuning', 'ts_check_borders', 'ts_debug_remap',
-    'ts_debug_remap_reduced', 'ts_debug_split_f32', 'ts_debug_split_f64', 'ts_shift_forward',
-    'ts_shift_backward_workspace_bytes', 'ts_shift_backward', 'ts_qshift_forward', 'ts_shift_backward_allreduce',
-    'ts_qshift_forward_nhwc', 'ts_debug_nhwc_emulate', 'ts_nhwc_to_nchw', 'ts_shift2d_avgpool2_forward', 'ts_shift2d_avgpool2_backward',
-    'ts_shift_forward_nhwc', 'ts_shift_backward_nhwc_workspace_bytes', 'ts_shift_backward_nhwc',
-)
 
 
 class Geometry(ct.Structure):
@@ -37,6 +27,36 @@ class PeerGroup(ct.Structure):
     """struct ts_peer_group."""
     _fields_ = [('world', ct.c_int32), ('rank', ct.c_int32), ('capacity', ct.c_int32), ('reserved', ct.c_int32),
                 ('timeout_ns', ct.c_uint64), ('bufs', ct.c_void_p * 8), ('state', ct.c_void_p)]
+
+
+_vp, _i, _i64, _sz = ct.c_void_p, ct.c_int, ct.c_int64, ct.c_size_t
+_geo, _peers, _i64p = ct.POINTER(Geometry), ct.POINTER(PeerGroup), ct.POINTER(ct.c_int64)
+# restype and argtypes of every symbol include/torchshifts_b200.h declares
+SIGNATURES = {
+    'ts_abi_version': (_i, []), 'ts_cuda_version': (_i, []),
+    'ts_error_string': (ct.c_char_p, [_i]), 'ts_last_cuda_error': (ct.c_char_p, []),
+    'ts_last_kernel_path': (_i, []), 'ts_set_kernel_path': (_i, [_i]),
+    'ts_launch_count': (ct.c_uint64, []), 'ts_set_tuning': (_i, [ct.c_char_p]),
+    'ts_check_borders': (_i, [_i, _i64p, _i64p, _i64p, _i64p]),
+    'ts_debug_remap': (_i, [_i, _i, _i]), 'ts_debug_remap_reduced': (_i, [_i, _i, _i, _i64, _i]),
+    'ts_debug_split_f32': (None, [_i, _i, ct.c_float, _i64p, ct.POINTER(ct.c_float)]),
+    'ts_debug_split_f64': (None, [_i, _i, ct.c_double, _i64p, ct.POINTER(ct.c_double)]),
+    'ts_shift_forward': (_i, [_geo, _i, _i, _i, _vp, _vp, _vp, _vp]),
+    'ts_shift2d_avgpool2_forward': (_i, [_geo, _i, _i, _i, _vp, _vp, _vp, _vp]),
+    'ts_shift_backward_workspace_bytes': (_sz, [_geo, _i]),
+    'ts_shift_backward': (_i, [_geo, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    'ts_shift2d_avgpool2_backward': (_i, [_geo, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    'ts_qshift_forward': (_i, [_geo, _i, _i, _i64, _vp, _vp, _i, _i64, _vp, _vp]),
+    'ts_qshift_forward_nhwc': (_i, [_geo, _i, _i, _i64, _vp, _vp, _i, _i64, _vp, _vp]),
+    'ts_debug_nhwc_emulate': (_i, [_geo, _i, _i, _i64, _vp, _vp, _i, _i64, _vp, _i, _i, _i, _i]),
+    'ts_nhwc_to_nchw': (_i, [_vp, _vp, _i64, _i64, _i64, _i, _vp]),
+    'ts_shift_backward_allreduce': (_i, [_geo, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _peers, _vp]),
+    'ts_shift_forward_nhwc': (_i, [_geo, _i, _i, _i, _vp, _vp, _vp, _vp]),
+    'ts_shift_backward_nhwc_workspace_bytes': (_sz, [_geo, _i]),
+    'ts_shift_backward_nhwc': (_i, [_geo, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _peers, _vp]),
+}
+# tests check that the library exports all of them and that the header declares no others
+EXPORTED_SYMBOLS = tuple(SIGNATURES)
 
 
 def make_geometry(dim, shape, strides, lb, rb):
@@ -62,33 +82,7 @@ class NativeLibrary:
                               f'(nvcc -gencode arch=compute_100a,code=sm_100a)')
         lib = ct.CDLL(str(self.path))
         self.lib = lib
-        vp, i, i64, sz = ct.c_void_p, ct.c_int, ct.c_int64, ct.c_size_t
-        gp = ct.POINTER(Geometry)
-        i64p = ct.POINTER(ct.c_int64)
-        sig = {
-            'ts_abi_version': (i, []), 'ts_cuda_version': (i, []),
-            'ts_error_string': (ct.c_char_p, [i]), 'ts_last_cuda_error': (ct.c_char_p, []),
-            'ts_last_kernel_path': (i, []), 'ts_set_kernel_path': (i, [i]),
-            'ts_launch_count': (ct.c_uint64, []), 'ts_set_tuning': (i, [ct.c_char_p]),
-            'ts_check_borders': (i, [i, i64p, i64p, i64p, i64p]),
-            'ts_debug_remap': (i, [i, i, i]), 'ts_debug_remap_reduced': (i, [i, i, i, i64, i]),
-            'ts_debug_split_f32': (None, [i, i, ct.c_float, i64p, ct.POINTER(ct.c_float)]),
-            'ts_debug_split_f64': (None, [i, i, ct.c_double, i64p, ct.POINTER(ct.c_double)]),
-            'ts_shift_forward': (i, [gp, i, i, i, vp, vp, vp, vp]),
-            'ts_shift2d_avgpool2_forward': (i, [gp, i, i, i, vp, vp, vp, vp]),
-            'ts_shift_backward_workspace_bytes': (sz, [gp, i]),
-            'ts_shift_backward': (i, [gp, i, i, i, vp, vp, vp, vp, vp, vp, sz, vp]),
-            'ts_shift2d_avgpool2_backward': (i, [gp, i, i, i, vp, vp, vp, vp, vp, vp, sz, vp]),
-            'ts_qshift_forward': (i, [gp, i, i, i64, vp, vp, i, i64, vp, vp]),
-            'ts_qshift_forward_nhwc': (i, [gp, i, i, i64, vp, vp, i, i64, vp, vp]),
-            'ts_debug_nhwc_emulate': (i, [gp, i, i, i64, vp, vp, i, i64, vp, i, i, i, i]),
-            'ts_nhwc_to_nchw': (i, [vp, vp, i64, i64, i64, i, vp]),
-            'ts_shift_backward_allreduce': (i, [gp, i, i, i, vp, vp, vp, vp, vp, vp, sz, ct.POINTER(PeerGroup), vp]),
-            'ts_shift_forward_nhwc': (i, [gp, i, i, i, vp, vp, vp, vp]),
-            'ts_shift_backward_nhwc_workspace_bytes': (sz, [gp, i]),
-            'ts_shift_backward_nhwc': (i, [gp, i, i, i, vp, vp, vp, vp, vp, vp, sz, ct.POINTER(PeerGroup), vp]),
-        }
-        for name, (res, args) in sig.items():
+        for name, (res, args) in SIGNATURES.items():
             if not hasattr(lib, name) and os.environ.get('TORCHSHIFTS_B200_LIB'):
                 continue              # an older build under A/B measurement may lack the newest entry points
             fn = getattr(lib, name)

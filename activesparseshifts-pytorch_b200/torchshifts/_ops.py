@@ -33,7 +33,7 @@ import weakref
 
 import torch
 
-from ._cabi import QW_I8, QW_I32, QW_U8, make_geometry
+from ._cabi import QW_I8, QW_I32, QW_U8, TS_ERR_TOO_LARGE, TS_ERR_UNSUPPORTED, TS_ERR_WORKSPACE, TS_OK, make_geometry
 
 _LIB = None            # torch.library.Library handle (kept alive)
 _FUSED_ALLREDUCE = None   # torchshifts.sharded.FusedGradWeightAllReduce while enabled: grad_weight is summed over the ranks in-kernel
@@ -77,9 +77,18 @@ def _same_device_and_type(fn, input, weights, grad=None):
 
 
 _COPY_THRESHOLD = 1 << 16
+CL_FORMATS = {2: torch.channels_last, 3: torch.channels_last_3d}    # number of spatial dims -> channels-last format
+_FALLBACK = (TS_ERR_UNSUPPORTED,)
 
 
-_CL_FORMATS = {4: torch.channels_last, 5: torch.channels_last_3d}
+def _served(status, what, fallback=()):
+    """Reads a library status: True for TS_OK, False for a status in ``fallback`` (the kernel does not serve the call and
+    nothing was launched: the caller runs its fallback path); any other status raises."""
+    if status == TS_OK:
+        return True
+    if status in fallback:
+        return False
+    _NATIVE.check(status, what)
 
 
 _PLANAR = collections.OrderedDict()     # (data_ptr, shape, strides, version) -> planar copy made by the forward, for the backward
@@ -94,11 +103,11 @@ def _dense(input, keep=False, take=False):
     channels-last tensor goes through the library's own tiled transpose (``ts_nhwc_to_nchw``), anything
     else through ``.contiguous()``.
 
-    ``keep`` (forward): park the planar copy in ``_LAST_PLANAR``; when autograd records the call,
-    ``_setup_forward_context`` -- the one place that knows the call is differentiated: the CUDA kernel runs below the
-    Autograd key, with grad mode off -- moves it to ``_PLANAR``, otherwise the composite drops it when the operator
-    returns.  ``take`` (backward): reuse that copy instead of converting the saved input a second time (0.26 ms per step
-    for cfg3) -- at most ``_PLANAR_MAX`` copies are held."""
+    ``keep`` (forward): park the planar copy in ``_LAST_PLANAR``; when autograd records the call, the forward's
+    ``setup_context`` -- the one place that knows the call is differentiated: the CUDA kernel runs below the Autograd key,
+    with grad mode off -- moves it to ``_PLANAR``, otherwise ``drop_unclaimed_planar`` drops it when the operator returns.
+    ``take`` (backward): reuse that copy instead of converting the saved input a second time (0.26 ms per step for cfg3)
+    -- at most ``_PLANAR_MAX`` copies are held."""
     if input.numel() < _COPY_THRESHOLD or input.is_contiguous():
         return input
     key = _planar_key(input)
@@ -106,14 +115,14 @@ def _dense(input, keep=False, take=False):
         hit = _PLANAR.pop(key, None)
         if hit is not None:
             return hit
-    fmt = _CL_FORMATS.get(input.dim())
+    fmt = CL_FORMATS.get(input.dim() - 2)
     if fmt is not None and input.is_contiguous(memory_format=fmt) and input.element_size() in (2, 4, 8):
         out = torch.empty(input.shape, dtype=input.dtype, device=input.device)
         n, c = input.shape[0], input.shape[1]
         with _guard(input.device):
             st = _NATIVE.lib.ts_nhwc_to_nchw(input.data_ptr(), out.data_ptr(), n, c, input.numel() // max(n * c, 1),
                                              input.element_size(), _stream(input.device))
-        _NATIVE.check(st, 'ts_nhwc_to_nchw')
+        _served(st, 'ts_nhwc_to_nchw')
     else:
         out = input.contiguous()
     if keep:
@@ -136,6 +145,12 @@ def _claim_planar(input):
             _PLANAR.popitem(last=False)
 
 
+def drop_unclaimed_planar():
+    """Called when a shift operator returns to its caller: a planar copy no autograd record claimed is not needed."""
+    if not torch.compiler.is_compiling():
+        _LAST_PLANAR[0] = None
+
+
 def _stream(device):
     return ct.c_void_p(torch._C._cuda_getCurrentRawStream(device.index))
 
@@ -150,7 +165,7 @@ def _guard(device):
 
 
 _GEO_CACHE = {}        # (dim, shape, strides, lb, rb) -> ts_geometry; shift layers see the same few shapes every step
-_WS_CACHE = {}         # (geometry key, dtype code, device index) -> backward workspace bytes
+_WS_CACHE = {}         # (workspace query's name, geometry key, dtype code, device index) -> backward workspace bytes
 
 
 def _geometry(dim, input, lb, rb):
@@ -165,14 +180,44 @@ def _geometry(dim, input, lb, rb):
     return geo, key
 
 
-def _workspace_bytes(geo, key, code, device):
-    wkey = (key, code, device.index)
-    n = _WS_CACHE.get(wkey)
-    if n is None:
-        if len(_WS_CACHE) > 256:
+def _check_size(fn, name, size, dim, input, lb, rb):
+    """``size`` (a forward's ``new_size``, a backward's ``grad`` shape) must be input's N, C and the cropped extent."""
+    if list(size) != list(input.shape[:2]) + [rb[a] - lb[a] for a in range(dim)]:
+        raise RuntimeError(f'{fn}: {name} {list(size)} does not match the borders and input {list(input.shape)}')
+
+
+def _launch_backward(entry, query, geo, key, grad, input, weights, padding_mode, active_flag, peers=(),
+                     fmt=torch.contiguous_format, fallback=()):
+    """Runs the backward entry point ``entry`` -> (grad_input in ``fmt``, grad_weight).  ``query`` is its workspace-size
+    function, cached per geometry; ``peers``: the trailing peer-group argument of the entry points that take one.
+
+    With a ``fallback`` (statuses as for ``_served``) returns None when the kernel does not serve the call: the launch
+    returned such a status, or ``query`` answered 16 bytes (no partials), which is decided before ``grad`` is converted
+    to ``fmt`` -- a conversion the caller's fallback path would do again."""
+    code = _DTYPES[input.dtype]
+    dev = input.device
+    wkey = (query.__name__, key, code, dev.index)
+    with _guard(dev):
+        for attempt in (0, 1):
+            nbytes = _WS_CACHE.get(wkey)
+            if nbytes is None:
+                if len(_WS_CACHE) > 256:
+                    _WS_CACHE.clear()
+                nbytes = _WS_CACHE[wkey] = int(query(ct.byref(geo), code))
+            if fallback and nbytes <= 16:
+                return None
+            grad = grad.contiguous(memory_format=fmt)
+            w = weights.contiguous()
+            grad_input = torch.empty(input.shape, dtype=input.dtype, device=dev, memory_format=fmt)
+            grad_weight = torch.empty(w.shape, dtype=w.dtype, device=dev)
+            workspace = torch.empty(max(nbytes, 16), dtype=torch.uint8, device=dev)
+            st = entry(ct.byref(geo), code, int(padding_mode), int(bool(active_flag)), grad.data_ptr(), input.data_ptr(),
+                       w.data_ptr(), grad_input.data_ptr(), grad_weight.data_ptr(), workspace.data_ptr(), nbytes, *peers,
+                       _stream(dev))
+            if st != TS_ERR_WORKSPACE:      # (nothing was launched): the tuning knobs changed since the size was cached
+                break
             _WS_CACHE.clear()
-        n = _WS_CACHE[wkey] = int(_NATIVE.lib.ts_shift_backward_workspace_bytes(ct.byref(geo), code))
-    return n
+    return (grad_input, grad_weight) if _served(st, entry.__name__, fallback) else None
 
 
 # ------------------------------------------------------------------------------------------ CUDA
@@ -193,13 +238,11 @@ def _forward_cuda(dim, input, weights, borders, new_size, padding_mode, active_f
     w = weights.contiguous()
     input = _dense(input, keep=True)
     geo, _ = _geometry(dim, input, lb, rb)
-    if list(out.shape[2:]) != [rb[a] - lb[a] for a in range(dim)]:
-        raise RuntimeError(f'{fn}: new_size {list(new_size)} does not match the borders')
+    _check_size(fn, 'new_size', new_size, dim, input, lb, rb)
     with _guard(input.device):
         st = _NATIVE.lib.ts_shift_forward(ct.byref(geo), _DTYPES[input.dtype], int(padding_mode), int(bool(active_flag)),
                                           input.data_ptr(), w.data_ptr(), out.data_ptr(), _stream(input.device))
-    if st:
-        _NATIVE.check(st, 'ts_shift_forward')
+    _served(st, 'ts_shift_forward')
     return out
 
 
@@ -219,29 +262,14 @@ def _pool_forward_cuda(input, weights, borders, new_size, padding_mode, active_f
         with _guard(input.device):
             st = _NATIVE.lib.ts_shift2d_avgpool2_forward(ct.byref(geo), 0, int(padding_mode), int(bool(active_flag)), input.data_ptr(),
                                                          w.data_ptr(), out.data_ptr(), _stream(input.device))
-        if st == 0:
+        if _served(st, 'ts_shift2d_avgpool2_forward', _FALLBACK):
             return out
-        if st != 2:        # TS_ERR_UNSUPPORTED: fall through to the two-step path
-            _NATIVE.check(st, 'ts_shift2d_avgpool2_forward')
     y = _forward_cuda(2, input, weights, borders, new_size, padding_mode, active_flag)
     return torch.nn.functional.avg_pool2d(y, kernel_size=2, stride=2, ceil_mode=True)
 
 
 def _pool_forward_meta(input, weights, borders, new_size, padding_mode, active_flag):
     return input.new_empty([new_size[0], new_size[1], (new_size[2] + 1) // 2, (new_size[3] + 1) // 2])
-
-
-def _pool_setup_context(ctx, inputs, output):
-    input, weights, borders, new_size, padding_mode, active_flag = inputs
-    ctx.save_for_backward(input, weights, borders)
-    ctx.padding_mode, ctx.active_flag, ctx.new_size = padding_mode, active_flag, list(new_size)
-
-
-def _pool_backward(ctx, grad_pooled):
-    input, weights, borders = ctx.saved_tensors
-    op = torch.ops.torchshifts._shift2d_avgpool2_backward
-    grad_input, grad_weight = op(grad_pooled, weights, input, borders, ctx.new_size, ctx.padding_mode, ctx.active_flag)
-    return grad_input, grad_weight, None, None, None, None
 
 
 def _pool_backward_cuda(grad_pooled, weights, input, borders, new_size, padding_mode, active_flag):
@@ -257,26 +285,11 @@ def _pool_backward_cuda(grad_pooled, weights, input, borders, new_size, padding_
         raise RuntimeError(f'{fn}: grad has shape {list(grad_pooled.shape)}, the pooled output is '
                            f'{[input.shape[0], input.shape[1], (oh + 1) // 2, (ow + 1) // 2]}')
     if input.dtype == torch.float32 and input.is_contiguous() and ow % 8 == 0 and input.dim() == 4 and input.numel() > 0:
-        grad = grad_pooled.contiguous()
-        w = weights.contiguous()
-        out_grad = torch.empty(input.shape, dtype=input.dtype, device=input.device)
-        weights_grad = torch.empty(w.shape, dtype=w.dtype, device=w.device)
         geo, key = _geometry(2, input, lb, rb)
-        dev = input.device
-        with _guard(dev):
-            for attempt in (0, 1):
-                nbytes = _workspace_bytes(geo, key, 0, dev)
-                workspace = torch.empty(max(nbytes, 16), dtype=torch.uint8, device=dev)
-                st = _NATIVE.lib.ts_shift2d_avgpool2_backward(ct.byref(geo), 0, int(padding_mode), int(bool(active_flag)), grad.data_ptr(),
-                                                              input.data_ptr(), w.data_ptr(), out_grad.data_ptr(), weights_grad.data_ptr(),
-                                                              workspace.data_ptr(), nbytes, _stream(dev))
-                if st != 3:
-                    break
-                _WS_CACHE.clear()
-        if st == 0:
-            return out_grad, weights_grad
-        if st != 2:        # TS_ERR_UNSUPPORTED: fall through to the two-step path
-            _NATIVE.check(st, 'ts_shift2d_avgpool2_backward')
+        grads = _launch_backward(_NATIVE.lib.ts_shift2d_avgpool2_backward, _NATIVE.lib.ts_shift_backward_workspace_bytes, geo, key,
+                                 grad_pooled, input, weights, padding_mode, active_flag, fallback=_FALLBACK)
+        if grads is not None:
+            return grads
     like = torch.empty(list(new_size), dtype=grad_pooled.dtype, device=grad_pooled.device)
     grad_y = torch.ops.aten.avg_pool2d_backward(grad_pooled.contiguous(), like, [2, 2], [2, 2], [0, 0], True, True, None)
     return _backward_cuda(2, grad_y, weights, input, borders, padding_mode, active_flag)
@@ -305,73 +318,37 @@ def _backward_cuda(dim, grad, weights, input, borders, padding_mode, active_flag
     _check_mode(padding_mode)
     _same_device_and_type(fn, input, weights, grad)
     lb, rb = _borders_lists(borders, dim)
-    grad = grad.contiguous()
-    w = weights.contiguous()
-    out_grad = torch.empty(input.shape, dtype=input.dtype, device=input.device)
-    weights_grad = torch.empty(w.shape, dtype=w.dtype, device=w.device)
     input = _dense(input, take=True)
     geo, key = _geometry(dim, input, lb, rb)
-    if list(grad.shape[2:]) != [rb[a] - lb[a] for a in range(dim)] or list(grad.shape[:2]) != list(input.shape[:2]):
-        raise RuntimeError(f'{fn}: grad shape {list(grad.shape)} does not match the (cropped) output of input {list(input.shape)}')
-    code = _DTYPES[input.dtype]
-    dev = input.device
-    fused = _FUSED_ALLREDUCE
-    if fused is not None:
-        _check_fused(fn, fused, dev, code, w.numel())
-    with _guard(dev):
-        for attempt in (0, 1):
-            nbytes = _workspace_bytes(geo, key, code, dev)
-            workspace = torch.empty(max(nbytes, 16), dtype=torch.uint8, device=dev)
-            args = (ct.byref(geo), code, int(padding_mode), int(bool(active_flag)), grad.data_ptr(), input.data_ptr(), w.data_ptr(),
-                    out_grad.data_ptr(), weights_grad.data_ptr(), workspace.data_ptr(), nbytes)
-            if fused is not None:
-                st = _NATIVE.lib.ts_shift_backward_allreduce(*args, ct.byref(fused.peer_group()), _stream(dev))
-            else:
-                st = _NATIVE.lib.ts_shift_backward(*args, _stream(dev))
-            if st != 3:       # TS_ERR_WORKSPACE (nothing was launched): the tuning knobs changed since the size was cached
-                break
-            _WS_CACHE.clear()
-    if st:
-        _NATIVE.check(st, 'ts_shift_backward_allreduce' if fused is not None else 'ts_shift_backward')
-    return out_grad, weights_grad
+    _check_size(fn, 'grad shape', grad.shape, dim, input, lb, rb)
+    lib, fused = _NATIVE.lib, _FUSED_ALLREDUCE
+    if fused is None:
+        return _launch_backward(lib.ts_shift_backward, lib.ts_shift_backward_workspace_bytes, geo, key, grad, input, weights,
+                                padding_mode, active_flag)
+    _check_fused(fn, fused, input.device, _DTYPES[input.dtype], weights.numel())
+    return _launch_backward(lib.ts_shift_backward_allreduce, lib.ts_shift_backward_workspace_bytes, geo, key, grad, input, weights,
+                            padding_mode, active_flag, (ct.byref(fused.peer_group()),))
 
 
 # ------------------------------------------------------------------------------------------ CUDA, channels-last
-_CL_WS_CACHE = {}      # (geometry key, dtype code, device index) -> workspace bytes of ts_shift_backward_nhwc
-
-
-def _cl_workspace_bytes(geo, key, code, device):
-    wkey = (key, code, device.index)
-    n = _CL_WS_CACHE.get(wkey)
-    if n is None:
-        if len(_CL_WS_CACHE) > 256:
-            _CL_WS_CACHE.clear()
-        with _guard(device):
-            n = _CL_WS_CACHE[wkey] = int(_NATIVE.lib.ts_shift_backward_nhwc_workspace_bytes(ct.byref(geo), code))
-    return n
-
-
 def _forward_cl_cuda(dim, input, weights, borders, new_size, padding_mode, active_flag):
     """``_shiftNd_forward`` with a dense channels-last output.  2-D dense channels-last fp32 / fp16 / bf16 inputs run the
     native NHWC kernel (ts_shift_forward_nhwc: one read, one write, no layout pass); whatever it does not serve takes the
     planar forward and converts its output -- the same values."""
     fn = f'shift{dim}d_forward_cl'
-    fmt = _CL_FORMATS[dim + 2]
+    fmt = CL_FORMATS[dim]
     _check_forward(fn, dim, input, weights, padding_mode)
     if dim == 2 and input.dtype != torch.float64 and input.shape[1] % 32 == 0 and input.is_contiguous(memory_format=fmt):
         lb, rb = _borders_lists(borders, dim)
-        if list(new_size) != list(input.shape[:2]) + [rb[a] - lb[a] for a in range(dim)]:
-            raise RuntimeError(f'{fn}: new_size {list(new_size)} does not match the borders')
+        _check_size(fn, 'new_size', new_size, dim, input, lb, rb)
         out = torch.empty(list(new_size), dtype=input.dtype, device=input.device, memory_format=fmt)
         w = weights.contiguous()
         geo, _ = _geometry(dim, input, lb, rb)
         with _guard(input.device):
             st = _NATIVE.lib.ts_shift_forward_nhwc(ct.byref(geo), _DTYPES[input.dtype], int(padding_mode), int(bool(active_flag)),
                                                    input.data_ptr(), w.data_ptr(), out.data_ptr(), _stream(input.device))
-        if st == 0:
+        if _served(st, 'ts_shift_forward_nhwc', _FALLBACK):
             return out
-        if st != 2:        # TS_ERR_UNSUPPORTED: the planar path below
-            _NATIVE.check(st, 'ts_shift_forward_nhwc')
     return _forward_cuda(dim, input, weights, borders, new_size, padding_mode, active_flag).contiguous(memory_format=fmt)
 
 
@@ -380,46 +357,23 @@ def _backward_cl_cuda(dim, grad, weights, input, borders, padding_mode, active_f
     tensor from ``.sum()``, say): the native kernel (ts_shift_backward_nhwc) reads it dense channels-last.  What the
     kernel does not serve takes the planar backward and converts ``grad_input`` -- the same values."""
     fn = f'shift{dim}d_backward_cl'
-    fmt = _CL_FORMATS[dim + 2]
+    fmt = CL_FORMATS[dim]
     _check_mode(padding_mode)
     _same_device_and_type(fn, input, weights, grad)
-    code = _DTYPES[input.dtype]
-    dev = input.device
     fused = _FUSED_ALLREDUCE
     if fused is not None:
-        _check_fused(fn, fused, dev, code, weights.numel())
-    nbytes = 0
-    if dim == 2 and code != 1 and input.dim() == 4 and input.shape[1] % 32 == 0 and input.is_contiguous(memory_format=fmt):
+        _check_fused(fn, fused, input.device, _DTYPES[input.dtype], weights.numel())
+    if dim == 2 and input.dtype != torch.float64 and input.dim() == 4 and input.shape[1] % 32 == 0 \
+            and input.is_contiguous(memory_format=fmt):
         lb, rb = _borders_lists(borders, dim)
+        _check_size(fn, 'grad shape', grad.shape, dim, input, lb, rb)
         geo, key = _geometry(dim, input, lb, rb)
-        nbytes = _cl_workspace_bytes(geo, key, code, dev)
-    # 16 bytes: the kernel does not serve this geometry -- decided before grad is converted to a layout the planar path
-    # would convert again
-    for attempt in (0, 1):
-        if nbytes <= 16:
-            break
-        if list(grad.shape[2:]) != [rb[a] - lb[a] for a in range(dim)] or list(grad.shape[:2]) != list(input.shape[:2]):
-            raise RuntimeError(f'{fn}: grad shape {list(grad.shape)} does not match the (cropped) output of input {list(input.shape)}')
-        grad_cl = grad.contiguous(memory_format=fmt)
-        w = weights.contiguous()
-        out_grad = torch.empty(input.shape, dtype=input.dtype, device=dev, memory_format=fmt)
-        weights_grad = torch.empty(w.shape, dtype=w.dtype, device=dev)
-        workspace = torch.empty(nbytes, dtype=torch.uint8, device=dev)
-        with _guard(dev):
-            st = _NATIVE.lib.ts_shift_backward_nhwc(ct.byref(geo), code, int(padding_mode), int(bool(active_flag)), grad_cl.data_ptr(),
-                                                    input.data_ptr(), w.data_ptr(), out_grad.data_ptr(), weights_grad.data_ptr(),
-                                                    workspace.data_ptr(), nbytes,
-                                                    ct.byref(fused.peer_group()) if fused is not None else None, _stream(dev))
-        if st == 0:
-            return out_grad, weights_grad
-        if st == 2:        # TS_ERR_UNSUPPORTED (e.g. a misaligned view): the planar path below
-            break
-        if st != 3:
-            _NATIVE.check(st, 'ts_shift_backward_nhwc')
-        _CL_WS_CACHE.clear()      # TS_ERR_WORKSPACE (nothing was launched): the tuning knobs changed since the size was cached
-        nbytes = _cl_workspace_bytes(geo, key, code, dev)
-    else:
-        _NATIVE.check(st, 'ts_shift_backward_nhwc')
+        lib = _NATIVE.lib
+        grads = _launch_backward(lib.ts_shift_backward_nhwc, lib.ts_shift_backward_nhwc_workspace_bytes, geo, key, grad, input,
+                                 weights, padding_mode, active_flag, (ct.byref(fused.peer_group()) if fused is not None else None,),
+                                 fmt, _FALLBACK)
+        if grads is not None:
+            return grads
     grad_input, grad_weight = _backward_cuda(dim, grad, weights, input, borders, padding_mode, active_flag)
     return grad_input.contiguous(memory_format=fmt), grad_weight
 
@@ -450,15 +404,14 @@ def _forward_qcuda(dim, input, weights, borders, new_size, padding_mode, active_
     if input.dtype not in _QBYTES or weights.dtype not in _QKINDS:
         raise RuntimeError(f'{fn}: unsupported quantized dtype {input.dtype} / {weights.dtype}')
     lb, rb = _borders_lists(borders, dim)
-    if list(new_size[2:]) != [rb[a] - lb[a] for a in range(dim)] or list(new_size[:2]) != list(input.shape[:2]):
-        raise RuntimeError(f'{fn}: new_size {list(new_size)} does not match the borders')
+    _check_size(fn, 'new_size', new_size, dim, input, lb, rb)
     wq = _raw_qweights(weights, input.device)
     args = (_QBYTES[input.dtype], int(padding_mode), int(input.q_zero_point()))
     wargs = (wq.data_ptr(), _QKINDS[weights.dtype], int(weights.q_zero_point()))
     # the reference allocates the quantized output in the input's memory format
     # (quantized/shifts_quantized.cpp:119-122): channels-last in, channels-last out -- served by the
     # native NHWC kernel (one read + one write, no layout conversion on either side)
-    fmt = {2: torch.channels_last, 3: torch.channels_last_3d}.get(dim)
+    fmt = CL_FORMATS.get(dim)
     if fmt is not None and not input.is_contiguous() and input.is_contiguous(memory_format=fmt):
         to_cl = (0,) + tuple(range(2, dim + 2)) + (1,)
         to_nc = (0, dim + 1) + tuple(range(1, dim + 1))
@@ -468,8 +421,8 @@ def _forward_qcuda(dim, input, weights, borders, new_size, padding_mode, active_
         with _guard(input.device):
             st = _NATIVE.lib.ts_qshift_forward_nhwc(ct.byref(geo), *args, input.data_ptr(), *wargs, out_cl.data_ptr(),
                                                     _stream(input.device))
-        if st not in (2, 4):      # TS_ERR_UNSUPPORTED / TOO_LARGE (row offsets beyond 32 bits): planar kernels + conversions
-            _NATIVE.check(st, 'ts_qshift_forward_nhwc')
+        # TS_ERR_TOO_LARGE: row offsets beyond 32 bits; both take the planar kernels and conversions
+        if _served(st, 'ts_qshift_forward_nhwc', (TS_ERR_UNSUPPORTED, TS_ERR_TOO_LARGE)):
             return out_cl.permute(*to_nc)
         del out_cl
     x = input if input.is_contiguous() else input.contiguous()
@@ -478,7 +431,7 @@ def _forward_qcuda(dim, input, weights, borders, new_size, padding_mode, active_
     geo, _ = _geometry(dim, x, lb, rb)
     with _guard(input.device):
         st = _NATIVE.lib.ts_qshift_forward(ct.byref(geo), *args, x.data_ptr(), *wargs, out.data_ptr(), _stream(input.device))
-    _NATIVE.check(st, 'ts_qshift_forward')
+    _served(st, 'ts_qshift_forward')
     if x is not input and fmt is not None and input.is_contiguous(memory_format=fmt):
         out = out.contiguous(memory_format=fmt)
     return out
@@ -499,11 +452,11 @@ def _backward_meta(dim, grad, weights, input, borders, padding_mode, active_flag
 
 
 def _forward_cl_meta(dim, input, weights, borders, new_size, padding_mode, active_flag):
-    return torch.empty(list(new_size), dtype=input.dtype, device=input.device, memory_format=_CL_FORMATS[dim + 2])
+    return torch.empty(list(new_size), dtype=input.dtype, device=input.device, memory_format=CL_FORMATS[dim])
 
 
 def _backward_cl_meta(dim, grad, weights, input, borders, padding_mode, active_flag):
-    return (torch.empty(input.shape, dtype=input.dtype, device=input.device, memory_format=_CL_FORMATS[dim + 2]),
+    return (torch.empty(input.shape, dtype=input.dtype, device=input.device, memory_format=CL_FORMATS[dim]),
             weights.new_empty(weights.shape))
 
 
@@ -512,21 +465,22 @@ def _backward_cl_meta(dim, grad, weights, input, borders, padding_mode, active_f
 # borders; backward calls _shiftNd_backward and returns grads for input and weights only; the backward
 # op itself is not differentiable (:50-72).  Registered with torch.library.register_autograd (not an
 # Autograd-key kernel wrapping an autograd.Function) so that AOTAutograd / torch.compile can trace it.
-def _setup_forward_context(ctx, inputs, output):
-    input, weights, borders, new_size, padding_mode, active_flag = inputs
-    ctx.save_for_backward(input, weights, borders)
-    ctx.padding_mode, ctx.active_flag = padding_mode, active_flag
-    if _LAST_PLANAR[0] is not None:
-        _claim_planar(input)
+def _forward_autograd(backward_op, takes_new_size):
+    """-> (backward, setup_context) of a forward op: save input, weights and borders (and new_size when ``backward_op``
+    takes it), keep the planar copy the forward made, and call ``backward_op``."""
+    def setup_context(ctx, inputs, output):
+        input, weights, borders, new_size, padding_mode, active_flag = inputs
+        ctx.save_for_backward(input, weights, borders)
+        ctx.tail = (list(new_size), padding_mode, active_flag) if takes_new_size else (padding_mode, active_flag)
+        if _LAST_PLANAR[0] is not None:
+            _claim_planar(input)
 
-
-def _make_forward_backward(dim, suffix=''):
     def backward(ctx, grad_output):
         input, weights, borders = ctx.saved_tensors
-        op = getattr(torch.ops.torchshifts, f'_shift{dim}d_backward{suffix}')
-        grad_input, grad_weight = op(grad_output, weights, input, borders, ctx.padding_mode, ctx.active_flag)
+        op = getattr(torch.ops.torchshifts, backward_op)
+        grad_input, grad_weight = op(grad_output, weights, input, borders, *ctx.tail)
         return grad_input, grad_weight, None, None, None, None
-    return backward
+    return backward, setup_context
 
 
 def _setup_backward_context(ctx, inputs, output):
@@ -557,8 +511,7 @@ def _shift_composite(dim, input, weights, borders, padding_mode, active_flag):
     std_borders, new_size = check_borders(input, borders, dim)
     op = getattr(torch.ops.torchshifts, f'_shift{dim}d_forward')
     out = op(input, weights, std_borders, new_size, padding_mode, active_flag)
-    if not torch.compiler.is_compiling():
-        _LAST_PLANAR[0] = None      # a planar copy nobody claimed (no autograd): drop it now
+    drop_unclaimed_planar()
     return out
 
 
@@ -567,6 +520,12 @@ def _bind(fn, dim):
         return fn(dim, *args)
     bound.__name__ = f'{fn.__name__}_{dim}d'
     return bound
+
+
+_FORWARD = '(Tensor input, Tensor weights, Tensor borders, int[] new_size, int padding_mode, bool active_flag) -> Tensor'
+_BACKWARD = '(Tensor grad, Tensor weights, Tensor input, Tensor borders, int padding_mode, bool active_flag) -> (Tensor, Tensor)'
+_POOL_BACKWARD = ('(Tensor grad, Tensor weights, Tensor input, Tensor borders, int[] new_size, int padding_mode, '
+                  'bool active_flag) -> (Tensor, Tensor)')
 
 
 def register(native):
@@ -580,49 +539,32 @@ def register(native):
     lib.impl('_cuda_version', lambda: int(native.lib.ts_cuda_version()), 'CompositeExplicitAutograd')
     for dim in (1, 2, 3):
         lib.define(f'shift{dim}d(Tensor input, Tensor weights, Tensor borders, int padding_mode, bool active_flag) -> Tensor')
-        lib.define(f'_shift{dim}d_forward(Tensor input, Tensor weights, Tensor borders, int[] new_size, '
-                   f'int padding_mode, bool active_flag) -> Tensor')
-        lib.define(f'_shift{dim}d_backward(Tensor grad, Tensor weights, Tensor input, Tensor borders, '
-                   f'int padding_mode, bool active_flag) -> (Tensor, Tensor)')
         lib.impl(f'shift{dim}d', _bind(_shift_composite, dim), 'CompositeImplicitAutograd')
-        fwd, bwd = f'_shift{dim}d_forward', f'_shift{dim}d_backward'
-        lib.impl(fwd, _bind(_forward_cuda, dim), 'CUDA')
-        lib.impl(bwd, _bind(_backward_cuda, dim), 'CUDA')
-        lib.impl(fwd, _bind(_forward_qcuda, dim), 'QuantizedCUDA')
-        lib.impl(bwd, _bind(_backward_quantized, dim), 'QuantizedCUDA')
-        # fake (meta) implementations: `borders` is a host tensor next to device tensors, so the output
-        # device is stated here instead of being inferred from the arguments
-        torch.library.register_fake(f'torchshifts::{fwd}', _bind(_forward_meta, dim), lib=lib)
-        torch.library.register_fake(f'torchshifts::{bwd}', _bind(_backward_meta, dim), lib=lib)
-        torch.library.register_autograd(f'torchshifts::{fwd}', _make_forward_backward(dim), setup_context=_setup_forward_context, lib=lib)
-        torch.library.register_autograd(f'torchshifts::{bwd}', _double_backward, setup_context=_setup_backward_context, lib=lib)
-        for key in ('CPU', 'QuantizedCPU'):
-            lib.impl(fwd, _no_cpu, key)
-            lib.impl(bwd, _no_cpu, key)
+    # name -> (schema, CUDA kernel, fake kernel, QuantizedCUDA kernel or None).  Fake kernels: `borders` is a host tensor
+    # next to device tensors, so they state the output device instead of leaving it to be inferred from the arguments.
+    ops = {}
+    for dim in (1, 2, 3):
+        ops[f'_shift{dim}d_forward'] = (_FORWARD, _bind(_forward_cuda, dim), _bind(_forward_meta, dim), _bind(_forward_qcuda, dim))
+        ops[f'_shift{dim}d_backward'] = (_BACKWARD, _bind(_backward_cuda, dim), _bind(_backward_meta, dim),
+                                         _bind(_backward_quantized, dim))
     for dim in (2, 3):
-        fwd, bwd = f'_shift{dim}d_forward_cl', f'_shift{dim}d_backward_cl'
-        lib.define(f'{fwd}(Tensor input, Tensor weights, Tensor borders, int[] new_size, int padding_mode, bool active_flag) -> Tensor')
-        lib.define(f'{bwd}(Tensor grad, Tensor weights, Tensor input, Tensor borders, int padding_mode, bool active_flag) -> (Tensor, Tensor)')
-        lib.impl(fwd, _bind(_forward_cl_cuda, dim), 'CUDA')
-        lib.impl(bwd, _bind(_backward_cl_cuda, dim), 'CUDA')
-        lib.impl(fwd, _no_cpu, 'CPU')
-        lib.impl(bwd, _no_cpu, 'CPU')
-        torch.library.register_fake(f'torchshifts::{fwd}', _bind(_forward_cl_meta, dim), lib=lib)
-        torch.library.register_fake(f'torchshifts::{bwd}', _bind(_backward_cl_meta, dim), lib=lib)
-        torch.library.register_autograd(f'torchshifts::{fwd}', _make_forward_backward(dim, '_cl'), setup_context=_setup_forward_context, lib=lib)
-        torch.library.register_autograd(f'torchshifts::{bwd}', _double_backward, setup_context=_setup_backward_context, lib=lib)
+        ops[f'_shift{dim}d_forward_cl'] = (_FORWARD, _bind(_forward_cl_cuda, dim), _bind(_forward_cl_meta, dim), None)
+        ops[f'_shift{dim}d_backward_cl'] = (_BACKWARD, _bind(_backward_cl_cuda, dim), _bind(_backward_cl_meta, dim), None)
     # fused epilogue of the strided depth-wise-conv emulation (modules/shifts.py:85-89): shift + crop + avg_pool2d(2, 2, ceil)
-    pool = '_shift2d_avgpool2_forward'
-    lib.define(f'{pool}(Tensor input, Tensor weights, Tensor borders, int[] new_size, int padding_mode, bool active_flag) -> Tensor')
-    lib.impl(pool, _pool_forward_cuda, 'CUDA')
-    lib.impl(pool, _no_cpu, 'CPU')
-    torch.library.register_fake(f'torchshifts::{pool}', _pool_forward_meta, lib=lib)
-    torch.library.register_autograd(f'torchshifts::{pool}', _pool_backward, setup_context=_pool_setup_context, lib=lib)
-    poolb = '_shift2d_avgpool2_backward'
-    lib.define(f'{poolb}(Tensor grad, Tensor weights, Tensor input, Tensor borders, int[] new_size, int padding_mode, '
-               f'bool active_flag) -> (Tensor, Tensor)')
-    lib.impl(poolb, _pool_backward_cuda, 'CUDA')
-    lib.impl(poolb, _no_cpu, 'CPU')
-    torch.library.register_fake(f'torchshifts::{poolb}', _pool_backward_meta, lib=lib)
-    torch.library.register_autograd(f'torchshifts::{poolb}', _double_backward, setup_context=_setup_backward_context, lib=lib)
+    ops['_shift2d_avgpool2_forward'] = (_FORWARD, _pool_forward_cuda, _pool_forward_meta, None)
+    ops['_shift2d_avgpool2_backward'] = (_POOL_BACKWARD, _pool_backward_cuda, _pool_backward_meta, None)
+    for name, (schema, cuda, fake, qcuda) in ops.items():
+        lib.define(name + schema)
+        lib.impl(name, cuda, 'CUDA')
+        lib.impl(name, _no_cpu, 'CPU')
+        if qcuda is not None:
+            lib.impl(name, qcuda, 'QuantizedCUDA')
+            lib.impl(name, _no_cpu, 'QuantizedCPU')
+        torch.library.register_fake(f'torchshifts::{name}', fake, lib=lib)
+        if '_forward' in name:
+            backward_op = name.replace('_forward', '_backward')
+            backward, setup_context = _forward_autograd(backward_op, 'new_size' in ops[backward_op][0])
+        else:
+            backward, setup_context = _double_backward, _setup_backward_context
+        torch.library.register_autograd(f'torchshifts::{name}', backward, setup_context=setup_context, lib=lib)
     _LIB = lib

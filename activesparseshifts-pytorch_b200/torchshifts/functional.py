@@ -8,6 +8,7 @@ from typing import Optional
 
 import torch
 
+from ._ops import CL_FORMATS, drop_unclaimed_planar
 from .extension import _assert_has_ops
 
 Tensor = torch.Tensor
@@ -45,7 +46,15 @@ def _std_borders(vals):
     return torch.tensor(list(vals), dtype=torch.int32)
 
 
-_CL_FORMATS = {2: torch.channels_last, 3: torch.channels_last_3d}
+def _crop(dim: int, input: Tensor, borders: Optional[Tensor], border_ints):
+    """-> (std_borders, new_size) of the crop given by ``border_ints`` (the module's cached Python integers), else by
+    ``borders``' values; no crop when ``borders`` is None."""
+    if borders is None:
+        cuts = [[0, 0]] * dim
+    else:
+        cuts = border_ints if border_ints is not None else [[int(v) for v in row] for row in borders.tolist()]
+    lb, rb = _resolve_borders(dim, input.shape[2:], cuts)
+    return _std_borders((lb[0], rb[0], lb[1], rb[1], lb[2], rb[2])), list(input.shape[:2]) + [rb[a] - lb[a] for a in range(dim)]
 
 
 def _check_memory_format(memory_format) -> bool:
@@ -59,7 +68,7 @@ def _check_memory_format(memory_format) -> bool:
 
 def _keeps_channels_last(dim: int, input: Tensor) -> bool:
     """Dense channels-last (not also NCHW-contiguous) float input of a 2-D / 3-D shift."""
-    fmt = _CL_FORMATS.get(dim)
+    fmt = CL_FORMATS.get(dim)
     return (fmt is not None and not input.is_quantized and input.is_contiguous(memory_format=fmt)
             and not input.is_contiguous())
 
@@ -67,17 +76,9 @@ def _keeps_channels_last(dim: int, input: Tensor) -> bool:
 def _shift_cl(dim: int, input: Tensor, weights: Tensor, padding_mode: int, active_flag: bool,
               borders: Optional[Tensor], _border_ints) -> Tensor:
     """The channels-last operator ``_shift{dim}d_forward_cl``: output (and grad_input) dense channels-last."""
-    from . import _ops
-    if borders is None:
-        cuts = [[0, 0]] * dim
-    else:
-        cuts = _border_ints if _border_ints is not None else [[int(v) for v in row] for row in borders.tolist()]
-    lb, rb = _resolve_borders(dim, input.shape[2:], cuts)
-    std = _std_borders((lb[0], rb[0], lb[1], rb[1], lb[2], rb[2]))
-    new_size = [input.shape[0], input.shape[1]] + [rb[a] - lb[a] for a in range(dim)]
+    std, new_size = _crop(dim, input, borders, _border_ints)
     out = getattr(torch.ops.torchshifts, f'_shift{dim}d_forward_cl')(input, weights, std, new_size, padding_mode, active_flag)
-    if not torch.compiler.is_compiling():
-        _ops._LAST_PLANAR[0] = None      # a planar copy of the fallback path nobody claimed (no autograd): drop it now
+    drop_unclaimed_planar()
     return out
 
 
@@ -101,9 +102,7 @@ def _shift_func(dim: int, input: Tensor, weights: Tensor, padding_mode: int, act
         if _border_ints is not None and torch.compiler.is_compiling():
             # torch.compile: resolve the crop from Python integers (constants of the trace) and call the inner
             # operator, which has a fake kernel and a registered autograd formula
-            lb, rb = _resolve_borders(dim, input.shape[2:], _border_ints)
-            std = _std_borders((lb[0], rb[0], lb[1], rb[1], lb[2], rb[2]))
-            new_size = [input.shape[0], input.shape[1]] + [rb[a] - lb[a] for a in range(dim)]
+            std, new_size = _crop(dim, input, borders, _border_ints)
             return getattr(torch.ops.torchshifts, f'_shift{dim}d_forward')(input, weights, std, new_size, padding_mode, active_flag)
     else:
         borders = torch.Tensor()
@@ -156,15 +155,12 @@ def shift2d_avgpool2_func(input: Tensor, weights: Tensor, padding_mode: int, act
     assert weights.shape[-1] == 2, f'{name}(): expected [n_channels,2] tensor as weight, but it is shape is {weights.shape}'
     assert input.shape[1] == weights.shape[0], f'{name}(): expected that input and weight have equal number of channels'
     assert input.device == weights.device, f'{name}(): expected input and weights to be on same device'
-    if borders is None:
-        cuts = [[0, 0], [0, 0]]
-    else:
+    if borders is not None:
         assert tuple(borders.shape) == (2, 2), 'borders must have shape [2, 2]'
-        cuts = _border_ints if _border_ints is not None else [[int(v) for v in row] for row in borders.tolist()]
-    lb, rb = _resolve_borders(2, input.shape[2:], cuts)
-    std = _std_borders((lb[0], rb[0], lb[1], rb[1], lb[2], rb[2]))
-    new_size = [input.shape[0], input.shape[1], rb[0] - lb[0], rb[1] - lb[1]]
-    return torch.ops.torchshifts._shift2d_avgpool2_forward(input, weights, std, new_size, padding_mode, active_flag)
+    std, new_size = _crop(2, input, borders, _border_ints)
+    out = torch.ops.torchshifts._shift2d_avgpool2_forward(input, weights, std, new_size, padding_mode, active_flag)
+    drop_unclaimed_planar()
+    return out
 
 
 # BASELINE.json names these "functional.shift1d/2d/3d"; keep the real names and add the aliases.

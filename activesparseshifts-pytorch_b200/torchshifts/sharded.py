@@ -88,7 +88,7 @@ class FusedGradWeightAllReduce:
         with fused:                                                  # or fused.enable() / fused.disable()
             loss.backward()          # shift layers' weight.grad are global sums; do NOT all-reduce them again
 
-    Contract (checked where it can be, see ``_ops._backward_cuda``):
+    Contract (checked where it can be, see ``_ops._check_fused``):
 
     * every rank runs the same sequence of shift backward calls with the same ``C x dim`` while the mode
       is enabled (true for replicated models); a rank whose batch shard is EMPTY still takes part and

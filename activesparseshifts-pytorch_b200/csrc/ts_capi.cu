@@ -120,6 +120,20 @@ static int elem_size(int dtype) {
     return 0;
 }
 
+// Tuning knobs (ts_set_tuning): 0 = automatic, the planners pick per-mode defaults.
+Tuning& tuning() {
+    static Tuning t = [] {
+        Tuning d;
+        memset(&d, 0, sizeof(d));
+        d.warps = 15;
+        d.ctas_per_sm = 1;
+        d.use_tma = d.use_halo = d.use_flat = 1;
+        d.unit_order = 1;
+        return d;
+    }();
+    return t;
+}
+
 }  // namespace ts
 
 using namespace ts;
@@ -176,14 +190,8 @@ int ts_set_tuning(const char* spec) {
         else if (!strcmp(key, "halo")) t.halo = val;
         else if (!strcmp(key, "halo_stages")) t.halo_stages = val;
         else if (!strcmp(key, "halo_warps")) t.halo_warps = val;
-        else if (!strcmp(key, "halo_split")) t.halo_split = val != 0;
-        else if (!strcmp(key, "halo_compact")) t.halo_compact = val != 0;
-        else if (!strcmp(key, "halo_probe")) t.halo_probe = val;
         else if (!strcmp(key, "unit_order")) t.unit_order = val != 0;
-        else if (!strcmp(key, "no_table")) t.no_table = val != 0;
-        else if (!strcmp(key, "no_pdl")) t.no_pdl = val != 0;
         else if (!strcmp(key, "use_flat")) t.use_flat = val != 0;
-        else if (!strcmp(key, "flat_variant")) t.flat_variant = val;
         else if (!strcmp(key, "flat_ctas")) t.flat_ctas = val;
         else if (!strcmp(key, "flat_stage_kb")) t.flat_stage_kb = val;
         else if (!strcmp(key, "flat_stages")) t.flat_stages = val;

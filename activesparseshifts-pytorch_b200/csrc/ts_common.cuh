@@ -36,6 +36,9 @@ struct Geo {
     long long out_plane; // OS0*OS1*OS2
 };
 
+// Tensor axis of a LEVEL (0 slab, 1 row, 2 column) of a `dim`-dimensional geometry; negative: the level is absent.
+TS_HD int level_axis(int level, int dim) { return level - (3 - dim); }
+
 // ------------------------------------------------------------------------------------------
 // Index remap.
 TS_HD int pmod(int a, int b) { return (b + (a % b)) % b; }
@@ -334,10 +337,6 @@ cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t s
 
 // ------------------------------------------------------------------------------------------
 // Launch bookkeeping shared by the translation units.
-struct LaunchCtx {
-    cudaStream_t stream;
-    int sm_count;
-};
 void note_launch(int n = 1);
 void note_error(const char* text);  // text returned by ts_last_cuda_error() for non-CUDA-runtime failures
 int check_launch();               // cudaGetLastError -> ts_status

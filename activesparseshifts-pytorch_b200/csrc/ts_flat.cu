@@ -31,15 +31,8 @@ namespace {
 
 using namespace ptx;
 
-constexpr int SMEM_LIMIT = 232448;
 constexpr int GUARD = 32;
 constexpr int MAX_K = 32;          // planes per stage: one lane of a warp per plane
-
-TS_D void bulk_g2s(void* dst, const void* src, unsigned bytes, uint64_t* bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(dst)),
-                 "l"(src), "r"(bytes), "r"(smem_u32(bar))
-                 : "memory");
-}
 
 struct FArgs {
     Geo g;
@@ -55,7 +48,7 @@ struct FArgs {
     int K, stages, stage_stride, nw;
     int nstages;               // ceil(planes / K)
     int table;                 // per-channel (row shift, column shift in bytes) table in shared memory
-    FastDivU d_ipp, d_Lb, d_C;
+    FastDiv d_ipp, d_Lb, d_C;
 };
 
 // (row shift, column shift in bytes) of channel c; a size-1 axis ignores its shift (reduce_shift)
@@ -131,13 +124,13 @@ __global__ void __launch_bounds__(512, 1) k_flat_gather(const __grid_constant__ 
         for (int i0 = 0; i0 < total; i0 += nt) {       // warp-uniform trip count: the shuffles below need every lane
             const int i = i0 + tid;
             const bool live = i < total;
-            const int q = live ? (int)fdivu((unsigned)i, a.d_ipp) : 0;
+            const int q = live ? (int)fdiv((unsigned)i, a.d_ipp) : 0;
             const int sr = __shfl_sync(0xffffffffu, my_sr, q), scb = __shfl_sync(0xffffffffu, my_scb, q);
             if (!live) continue;
             const int m = i - q * a.ipp;
             const int delta = sr * Lb + scb;
             const int o = 16 * m;
-            const int r0 = (int)fdivu((unsigned)o, a.d_Lb), c0 = o - r0 * Lb;
+            const int r0 = (int)fdiv((unsigned)o, a.d_Lb), c0 = o - r0 * Lb;
             const int n0b = Lb - c0 < 16 ? Lb - c0 : 16;
             const int lo = scb > 0 ? scb : 0, hi = scb < 0 ? Lb + scb : Lb;          // valid byte columns of a row
             unsigned mask = 0u;
@@ -194,7 +187,7 @@ TS_D void plane_items(const FArgs& a, unsigned src_plane, unsigned char* dst, in
     const int base = (-delta) & ~15;                                            // so & ~15 = 16 m + base  (16 m is a multiple of 16)
     for (int m = lane; m < a.ipp; m += 32) {
         const int o = 16 * m;
-        const int r0 = (int)fdivu((unsigned)o, a.d_Lb), c0 = o - r0 * Lb;
+        const int r0 = (int)fdiv((unsigned)o, a.d_Lb), c0 = o - r0 * Lb;
         const int n0b = Lb - c0 < 16 ? Lb - c0 : 16;
         unsigned mask = 0u;
         if ((unsigned)(r0 - sr) < (unsigned)B) {
@@ -252,7 +245,7 @@ __global__ void __launch_bounds__(512, 1) k_flat_gather_wp(const __grid_constant
         const unsigned sbase = shared_addr(smem + (size_t)s * a.stage_stride + GUARD);
         unsigned char* dst0 = a.y + p0 * a.plane_bytes;
         int c0;                                  // channel of the stage's first plane
-        if (a.planes < 0x7fffffffLL) { const unsigned pu = (unsigned)p0; c0 = (int)(pu - fdivu(pu, a.d_C) * (unsigned)C); }
+        if (a.planes < 0x7fffffffLL) { const unsigned pu = (unsigned)p0; c0 = (int)(pu - fdiv(pu, a.d_C) * (unsigned)C); }
         else c0 = (int)(p0 % C);
         mbar_wait(&full[s], phase);
         for (int q = wid; q < np; q += a.nw) {
@@ -300,7 +293,7 @@ FlatPlan plan_flat(const Geo& g, int esize, bool dense_x, const void* x, const v
     // defaults from tools/knob_sweep.py cfg5 on B200: one CTA of 15 warps per SM, 4 stages of 48 KB (74 us; two CTAs of 8 warps
     // with 24 KB stages: 80 us; three with 16 KB: 77 us)
     const int ctas = t.flat_ctas > 0 ? t.flat_ctas : 1;
-    const bool wp = t.flat_variant != 1 && g.C <= 512;                 // warp-per-plane variant with the shift table
+    const bool wp = g.C <= TABLE_MAX_C;                // warp-per-plane variant with the shift table
     const long long table_bytes = wp ? g.C * 8 : 0;
     const long long budget = SMEM_LIMIT / ctas - 1024 - table_bytes;
     const long long target = (long long)(t.flat_stage_kb > 0 ? t.flat_stage_kb : (ctas == 1 ? 48 : 24)) * 1024;
@@ -346,10 +339,10 @@ int flat_gather(const Geo& g, const FlatPlan& p, int wk, const void* x, void* y,
     a.ipp = a.plane_bytes / 16;
     a.K = p.np; a.stages = p.stages; a.stage_stride = p.stage_stride; a.nw = p.warps;
     a.nstages = p.units;
-    a.d_ipp = make_fastdivu((unsigned)a.ipp);
-    a.d_Lb = make_fastdivu((unsigned)a.Lb);
+    a.d_ipp = make_fastdiv((unsigned)a.ipp);
+    a.d_Lb = make_fastdiv((unsigned)a.Lb);
     a.table = p.n_per_unit;
-    a.d_C = make_fastdivu((unsigned)g.C);
+    a.d_C = make_fastdiv((unsigned)g.C);
     if (a.table) {
         if (!ensure_dynamic_smem((const void*)k_flat_gather_wp, p.smem_bytes)) return check_launch();
         k_flat_gather_wp<<<p.grid, (p.warps + 1) * 32, p.smem_bytes, s>>>(a);

@@ -286,8 +286,8 @@ int launch_reduce_partials(const double* partials, int slots, int outputs, void*
             for (int p = 0; p < 8; ++p) pa.bufs[p] = (unsigned long long*)pg->bufs[p];
             pa.state = (unsigned*)pg->state;
             if (outputs > 32 * PEER_MAX_CTAS || outputs > pg->capacity) return TS_ERR_INVALID_ARGUMENT;
-            if (tuning().no_pdl || launch_pdl(k_reduce_partials_allreduce<ST>, dim3((outputs + 31) / 32), dim3(1024), 0, stream, partials, slots,
-                                              outputs, (ST*)gw, pa) != cudaSuccess) {
+            if (launch_pdl(k_reduce_partials_allreduce<ST>, dim3((outputs + 31) / 32), dim3(1024), 0, stream, partials, slots, outputs,
+                           (ST*)gw, pa) != cudaSuccess) {
                 (void)cudaGetLastError();
                 k_reduce_partials_allreduce<ST><<<(outputs + 31) / 32, 1024, 0, stream>>>(partials, slots, outputs, (ST*)gw, pa);
             }
@@ -297,8 +297,7 @@ int launch_reduce_partials(const double* partials, int slots, int outputs, void*
     }
     const int threads = 128;
     const int blocks = (outputs * 32 + threads - 1) / threads;
-    if (tuning().no_pdl || launch_pdl(k_reduce_partials<ST>, dim3(blocks), dim3(threads), 0, stream, partials, slots, outputs, (ST*)gw) !=
-                               cudaSuccess) {
+    if (launch_pdl(k_reduce_partials<ST>, dim3(blocks), dim3(threads), 0, stream, partials, slots, outputs, (ST*)gw) != cudaSuccess) {
         (void)cudaGetLastError();
         k_reduce_partials<ST><<<blocks, threads, 0, stream>>>(partials, slots, outputs, (ST*)gw);
     }

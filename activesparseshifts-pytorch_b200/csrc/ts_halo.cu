@@ -39,14 +39,7 @@ namespace {
 
 using namespace ptx;
 
-#ifdef TS_HALO_SPIN
-#define TS_HALO_WAIT mbar_wait
-#else
-#define TS_HALO_WAIT mbar_wait_parked
-#endif
-constexpr int SMEM_LIMIT = 232448;
 constexpr int MAXT = 512;
-constexpr int TABLE_MAX_C = 512;    // channels whose shift parameters are tabulated in shared memory (36 bytes each)
 constexpr int GUARD = 128;          // readable slack before / after the tiles of a stage (window pairs may start 16 bytes early)
 
 struct alignas(64) HArgs {
@@ -75,15 +68,11 @@ struct alignas(64) HArgs {
     long long out_plane_bytes;                // bytes of one (n, c) plane of the OUTPUT (pooled plane for the fused avg-pool epilogue)
     int pool;                                 // forward only: 2x2 / stride 2 / ceil_mode average pooling fused into the store
     int need_fix;                             // padding != zeros: a fixer warp patches the halo of every stage
-    int split;                                // 3-D interpolating backward: x-window warps and grad-window warps (two pairs per thread)
-    FastDivU d_GP, d_img, d_C, d_chunks, d_PW;
     int table;                                // per-channel shift table in shared memory (C <= TABLE_MAX_C)
-    int probe;                                // tuning knob halo_probe (measurement only)
+    FastDiv d_GP, d_img, d_C, d_chunks, d_PW;
     int nfix;                                 // fixer warps (1; 4 when they also expand the pooled gradient)
     int pool_bwd, PH, PW;                     // backward fused with the adjoint of avg_pool2d(2, 2, ceil_mode): pooled rows / columns
 };
-
-TS_D int level_axis(int level, int dim) { return level - (3 - dim); }
 
 struct UnitShift {
     int sx[3], sg[3];      // per level; absent levels 0
@@ -114,8 +103,8 @@ TS_D UnitShift compute_unit_shift(const HArgs& a, long long c) {
 // the single producer thread); a unit then costs one 36-byte read
 TS_D UnitShift unit_shift(const HArgs& a, const UnitShift* tbl, long long c) { return a.table ? tbl[c] : compute_unit_shift(a, c); }
 TS_D void decode_unit(const HArgs& a, int u, int& c, int& chunk) {
-    if (a.unit_order) { chunk = (int)fdivu((unsigned)u, a.d_C); c = u - chunk * (int)a.g.C; }
-    else { c = (int)fdivu((unsigned)u, a.d_chunks); chunk = u - c * a.chunks; }
+    if (a.unit_order) { chunk = (int)fdiv((unsigned)u, a.d_C); c = u - chunk * (int)a.g.C; }
+    else { c = (int)fdiv((unsigned)u, a.d_chunks); chunk = u - c * a.chunks; }
 }
 
 // Where a unit's windows sit inside the tiles, and whether they fit the halo.
@@ -317,7 +306,7 @@ TS_D void halo_apply_m(const unsigned* list, int n, float* tile, int lane, const
 // height; /4 and /2 are exact as multiplications).  pooled: dense [PH][PW]; tile: the grad tile, data at (hr, hc).
 TS_D void sts64(unsigned addr, float a, float b) { asm volatile("st.shared.v2.f32 [%0], {%1, %2};" ::"r"(addr), "f"(a), "f"(b) : "memory"); }
 TS_D void pool_expand(const float* pooled, float* tile, int PH, int PW, int OB, int pitch, int hr, int hc, int lane, int stride,
-                      const FastDivU& dPW) {
+                      const FastDiv& dPW) {
     // A few warps expand a plane between the copy engine and the arithmetic warps, so they must not crawl: shared-window
     // addresses (no generic stores), a flat index over the pooled cells, four independent cells in flight per thread
     // (lane: index among the `stride` expanding threads)
@@ -332,7 +321,7 @@ TS_D void pool_expand(const float* pooled, float* tile, int PH, int PW, int OB, 
             const int p = p0 + stride * i;
             on[i] = p < n;
             const int q = on[i] ? p : 0;
-            const int pr = (int)fdivu((unsigned)q, dPW), pc = q - pr * PW;
+            const int pr = (int)fdiv((unsigned)q, dPW), pc = q - pr * PW;
             two[i] = 2 * pr + 1 < OB;
             o[i] = dst + (unsigned)(2 * pr * pb + 8 * pc);
             v[i] = __uint_as_float(lds32(src + 4u * (unsigned)q)) * (two[i] ? 0.25f : 0.5f);
@@ -583,16 +572,9 @@ TS_D void producer(const HArgs& a, unsigned char* smem, uint64_t* full, uint64_t
                 const bool has_v = bwd && a.dim == 3 && k >= 1;
                 if (lane == 0) {
                     if (kk > 0) mbar_wait_parked(&empty[s], (unsigned)((kk - 1) & 1));
-#ifdef TS_HALO_PROBE
-                    if ((a.probe & 3) == 2) mbar_arrive(&full[s]);     // no copies, the consumers compute on whatever the stage holds
-                    else
-#endif
                     mbar_expect_tx(&full[s], (unsigned)npl * (unsigned)(a.box_x + (has_g ? (a.pool_bwd ? a.box_v : a.box_g) : 0) + (has_v ? a.box_v : 0)));
                 }
                 __syncwarp();                              // the slot is free and its byte count posted before any lane copies into it
-#ifdef TS_HALO_PROBE
-                if ((a.probe & 3) != 2)
-#endif
                 for (int job = lane; job < 3 * npl; job += 32) {
                     const int pl = job / 3, what = job - 3 * pl;
                     if (what == 0) tma_load_5d(st + (size_t)pl * a.tile_x, &a.map_x, -a.hc, -a.hr, xs, c, nb + pl, &full[s]);
@@ -651,9 +633,6 @@ TS_D void fixer(const HArgs& a, unsigned char* smem, uint64_t* full, uint64_t* r
                 for (int pl = 0; pl < npl; ++pl) {
                     float* tx = (float*)(st + (size_t)pl * a.tile_x);
                     float* tg = (float*)(st + a.off_g + (size_t)pl * a.tile_g);
-#ifdef TS_HALO_PROBE
-                    if (a.probe & 8) continue;
-#endif
                     if (use_list) {
                         halo_apply(list_x, nx, tx, lane);
                         if (has_g) halo_apply(list_g, ng, tg, lane);
@@ -662,9 +641,6 @@ TS_D void fixer(const HArgs& a, unsigned char* smem, uint64_t* full, uint64_t* r
                         if (has_g) halo_walk(nullptr, tg, a.pg, a.OB, a.OL, a.hr, a.hc, a.g.pad, hg, lane);
                     }
                 }
-#ifdef TS_HALO_PROBE
-                if (!(a.probe & 4))
-#endif
                 fence_proxy_async();             // the next TMA load of this stage must not overtake these generic-proxy writes
                 __syncwarp();
                 if (lane == 0) mbar_arrive(&ready[s]);
@@ -723,9 +699,6 @@ TS_D void fixer_pool(const HArgs& a, unsigned char* smem, uint64_t* full, uint64
                 unsigned char* st = smem + (size_t)s * a.stage_stride + GUARD;
                 const bool has_g = bwd && (a.dim == 2 || a.active || k >= 1);
                 mbar_wait_parked(&full[s], phase);
-#ifdef TS_HALO_PROBE
-                if (!(a.probe & 8)) {
-#endif
                 if (MULTI && a.pool_bwd) {
                     for (int pl = 0; pl < npl; ++pl)
                         pool_expand((const float*)(st + a.off_v + (size_t)pl * a.tile_v), (float*)(st + a.off_g + (size_t)pl * a.tile_g), a.PH, a.PW,
@@ -748,10 +721,6 @@ TS_D void fixer_pool(const HArgs& a, unsigned char* smem, uint64_t* full, uint64
                         if (has_g && fix_g) halo_walk_z(nullptr, tg, a.pg, a.OB, a.OL, a.hr, a.hc, a.g.pad, hg, lane, zero_g);
                     }
                 }
-#ifdef TS_HALO_PROBE
-                }
-                if (!(a.probe & 4))
-#endif
                 fence_proxy_async();             // the next TMA load of this stage must not overtake these generic-proxy writes
                 __syncwarp();
                 if (lane == 0) mbar_arrive(&ready[s]);
@@ -767,8 +736,8 @@ struct Pair { int pl, r, cg; };
 TS_D bool decode_pair(const HArgs& a, int p, Pair& q) {
     q.pl = 0;
     int rem = p;
-    if (a.np > 1) { q.pl = (int)fdivu((unsigned)p, a.d_img); rem = p - q.pl * a.img_pairs; }
-    const int rp = (int)fdivu((unsigned)rem, a.d_GP);
+    if (a.np > 1) { q.pl = (int)fdiv((unsigned)p, a.d_img); rem = p - q.pl * a.img_pairs; }
+    const int rp = (int)fdiv((unsigned)rem, a.d_GP);
     q.cg = rem - rp * a.GP;
     q.r = 2 * rp;
     return q.cg < a.IG;
@@ -821,12 +790,9 @@ struct Ring {
     unsigned phase;
 };
 
-// ROLE (3-D interpolating backward only): 0 = a thread does everything for ONE pair; 1 = grad_weight terms (x windows) of
-// TWO pairs; 2 = grad_input (grad windows + stores) of TWO pairs.  Splitting the two halves of the arithmetic over
-// different warps halves the window state a thread carries from slab to slab (30 instead of 60 registers).
 // CROP (backward only): the call has a border crop, so grad values outside the crop are masked element by element; without
 // one every mask is full and the mask code (48 of 510 instructions per slab step of the 3-D backward) is compiled out.
-template <int DIM, int MODE, bool ACTIVE, bool SPLIT, bool POOL, bool CROP>
+template <int DIM, int MODE, bool ACTIVE, bool POOL, bool CROP>
 struct Body {
     const HArgs& a;
     const int tid, nt, wid, lane;
@@ -950,7 +916,7 @@ struct Body {
     TS_D void run_images2(unsigned char* smem, Ring& ring, unsigned char* dst, int npl, const PairCtx& pc0, float* ts) const {
         unsigned char* st = smem + (size_t)ring.s * a.stage_stride + GUARD;
         const unsigned sb = shared_addr(st);
-        TS_HALO_WAIT(&wait_bar[ring.s], ring.phase);
+        mbar_wait_parked(&wait_bar[ring.s], ring.phase);
         const int total = npl * a.img_pairs;
         if (tid < total && pc0.rows) pair2<WSX, WSG, WSV>(sb, dst, pc0, ts);      // the thread's first pair: context cached per unit
         for (int p = tid + nt; p < total; p += nt) {
@@ -963,29 +929,17 @@ struct Body {
     }
 
     // ---------------------------------------------------------------------------------------------
-    // 3-D: a thread owns its pair(s) for the whole image; windows of the previous slab stay in registers
-    template <int ROLE>
+    // 3-D: a thread owns its pair for the whole image; windows of the previous slab stay in registers
     struct Carry {
-        float X[(MODE != 2 || ROLE != 2) ? 3 : 1][5];
-        float G[(MODE == 2 && ACTIVE && ROLE != 1) ? 3 : 1][5];
+        float X[3][5];
+        float G[(MODE == 2 && ACTIVE) ? 3 : 1][5];
     };
 
     // stage k of an image: combine the windows of slab k-1 (`prev`, registers) with this stage's (slab k), which are
     // loaded straight into `next`: the caller alternates two register sets, so nothing is copied from step to step
-    template <int WSX, int WSG, int WSV, int ROLE>
-    TS_D void step3(unsigned sb, unsigned char* dst_img, int k, const PairCtx& pc, const Carry<ROLE>& cy, Carry<ROLE>& nx, float* ts) const {
-        constexpr bool DOX = MODE != 2 || ROLE != 2;
-        constexpr bool DOG = MODE == 2 && ROLE != 1;
+    template <int WSX, int WSG, int WSV>
+    TS_D void step3(unsigned sb, unsigned char* dst_img, int k, const PairCtx& pc, const Carry& cy, Carry& nx, float* ts) const {
         if (pc.rows == 0) return;
-#ifdef TS_HALO_PROBE                   // measurement builds only (nvcc -DTS_HALO_PROBE; tuning knob halo_probe): results are WRONG when set
-        if ((a.probe & 3) == 1) {      // the stage hand-off, the copies and the stores without loads / arithmetic
-            if (k >= 1) {
-                unsigned char* o = dst_img + pc.out_off + (long long)(k - 1) * a.IB * (a.IG * 16);
-                for (int j = 0; j < pc.rows; ++j) __stcs((float4*)(o + j * a.IG * 16), make_float4(0.f, 0.f, 0.f, 0.f));
-            }
-            return;
-        }
-#endif
         const float d[3] = {us.d[0], us.d[1], us.d[2]};
         const int it = k - 1, orow = a.IG * 16;
         unsigned char* o = dst_img + pc.out_off + (long long)it * a.IB * orow;
@@ -993,15 +947,15 @@ struct Body {
         const unsigned cm = (k >= 1 && slab_pass) ? pc.cmask : 0u;
         const unsigned xa = sb + pc.xo, ga = sb + pc.go, va = sb + pc.vo;
         const int pxb = a.px * 4, pgb = a.pg * 4;
-        const bool gwin = DOG && ACTIVE && pc.cmask != 0u;
+        const bool gwin = MODE == 2 && ACTIVE && pc.cmask != 0u;
         float SL[2][5];
-        if (DOX) { load5<WSX>(xa, wsx, nx.X[0]); load5<WSX>(xa + pxb, wsx, nx.X[1]); }
+        load5<WSX>(xa, wsx, nx.X[0]); load5<WSX>(xa + pxb, wsx, nx.X[1]);
         if (gwin) { load5<WSG>(ga, wsg, nx.G[0]); load5<WSG>(ga + pgb, wsg, nx.G[1]); }
 #pragma unroll
         for (int j = 0; j < 2; ++j) {
             if (j >= pc.rows) continue;
             if (j == 1) {
-                if (DOX) load5<WSX>(xa + 2 * pxb, wsx, nx.X[2]);
+                load5<WSX>(xa + 2 * pxb, wsx, nx.X[2]);
                 if (gwin) load5<WSG>(ga + 2 * pgb, wsg, nx.G[2]);
             }
             if (k < 1) continue;
@@ -1024,47 +978,43 @@ struct Body {
                 const unsigned m = CROP ? (cm >> (4 * j)) & 15u : 15u;       // (no crop: k >= 1 and the row exists here)
                 float y[4] = {0.f, 0.f, 0.f, 0.f};
                 if (m) {
-                    if (DOX) {
-                        float gv[4];
-                        load4<WSV>(va + j * a.OL * 4, wsv, gv);
-                        if (CROP && m != 15u) {
+                    float gv[4];
+                    load4<WSV>(va + j * a.OL * 4, wsv, gv);
+                    if (CROP && m != 15u) {
 #pragma unroll
-                            for (int t = 0; t < 4; ++t) gv[t] = (m >> t) & 1u ? gv[t] : 0.f;
-                        }
-                        wp3(cy.X[j], nx.X[j], cy.X[j + 1], nx.X[j + 1], gv, d, ts);
+                        for (int t = 0; t < 4; ++t) gv[t] = (m >> t) & 1u ? gv[t] : 0.f;
                     }
-                    if (DOG) {
-                        if (ACTIVE) {
-                            float P[5];
+                    wp3(cy.X[j], nx.X[j], cy.X[j + 1], nx.X[j + 1], gv, d, ts);
+                    if (ACTIVE) {
+                        float P[5];
 #pragma unroll
-                            for (int t = 0; t < 5; ++t) P[t] = col3(cy.G[j][t], nx.G[j][t], cy.G[j + 1][t], nx.G[j + 1][t], d[0], d[1]);
+                        for (int t = 0; t < 5; ++t) P[t] = col3(cy.G[j][t], nx.G[j][t], cy.G[j + 1][t], nx.G[j + 1][t], d[0], d[1]);
 #pragma unroll
-                            for (int t = 0; t < 4; ++t) y[t] = lerp<float>(P[t], P[t + 1], d[2]);
-                        } else {
-                            load4<WSG>(ga + j * pgb, wsg, y);
-                        }
-                        if (CROP && m != 15u) {
+                        for (int t = 0; t < 4; ++t) y[t] = lerp<float>(P[t], P[t + 1], d[2]);
+                    } else {
+                        load4<WSG>(ga + j * pgb, wsg, y);
+                    }
+                    if (CROP && m != 15u) {
 #pragma unroll
-                            for (int t = 0; t < 4; ++t) y[t] = (m >> t) & 1u ? y[t] : 0.f;
-                        }
+                        for (int t = 0; t < 4; ++t) y[t] = (m >> t) & 1u ? y[t] : 0.f;
                     }
                 }
-                if (DOG) __stcs((float4*)(o + j * orow), make_float4(y[0], y[1], y[2], y[3]));
+                __stcs((float4*)(o + j * orow), make_float4(y[0], y[1], y[2], y[3]));
             }
         }
     }
 
-    template <int WSX, int WSG, int WSV, int ROLE>
+    // The pair's context and its backward steps sit in loops of ONE trip on purpose: the compiler's schedule of the 3-D
+    // kernels depends on that loop structure (straight-line code adds 36 bytes of spills per thread to the interpolating
+    // backward and reorders both interpolating kernels).
+    template <int WSX, int WSG, int WSV>
     TS_D void run_images3(unsigned char* smem, Ring& ring, unsigned char* dst_img, int npl, float* ts) const {
-        constexpr int NPT = ROLE == 0 ? 1 : 2;
-        const int half = nt >> 1;
-        PairCtx pc[NPT];
-        Carry<ROLE> ca[NPT], cb[NPT];          // the windows of two consecutive slabs, roles alternating from step to step
+        PairCtx pc[1];
+        Carry ca[1], cb[1];                    // the windows of two consecutive slabs, roles alternating from step to step
 #pragma unroll
-        for (int i = 0; i < NPT; ++i) {
-            const int p = ROLE == 0 ? tid : (tid < half ? tid : tid - half) + i * half;
+        for (int i = 0; i < 1; ++i) {
             Pair q;
-            const bool valid = p < npl * a.img_pairs && decode_pair(a, p, q);
+            const bool valid = tid < npl * a.img_pairs && decode_pair(a, tid, q);
             if (!valid) { q.pl = 0; q.r = 0; q.cg = 0; }
             pc[i] = pair_ctx<MODE, CROP>(a, ug, q, valid);
         }
@@ -1073,8 +1023,8 @@ struct Body {
             // new windows are copied into the carried set instead (15 moves per step)
             for (int k = 0; k <= a.IA; ++k) {
                 const unsigned sb = shared_addr(smem + (size_t)ring.s * a.stage_stride + GUARD);
-                TS_HALO_WAIT(&wait_bar[ring.s], ring.phase);
-                step3<WSX, WSG, WSV, ROLE>(sb, dst_img, k, pc[0], ca[0], cb[0], ts);
+                mbar_wait_parked(&wait_bar[ring.s], ring.phase);
+                step3<WSX, WSG, WSV>(sb, dst_img, k, pc[0], ca[0], cb[0], ts);
 #pragma unroll
                 for (int j = 0; j < 3; ++j)
 #pragma unroll
@@ -1086,16 +1036,16 @@ struct Body {
         for (int k = 0; k <= a.IA; k += 2) {
             {
                 const unsigned sb = shared_addr(smem + (size_t)ring.s * a.stage_stride + GUARD);
-                TS_HALO_WAIT(&wait_bar[ring.s], ring.phase);
+                mbar_wait_parked(&wait_bar[ring.s], ring.phase);
 #pragma unroll
-                for (int i = 0; i < NPT; ++i) step3<WSX, WSG, WSV, ROLE>(sb, dst_img, k, pc[i], cb[i], ca[i], ts);
+                for (int i = 0; i < 1; ++i) step3<WSX, WSG, WSV>(sb, dst_img, k, pc[i], cb[i], ca[i], ts);
                 release(ring);
             }
             if (k + 1 <= a.IA) {
                 const unsigned sb = shared_addr(smem + (size_t)ring.s * a.stage_stride + GUARD);
-                TS_HALO_WAIT(&wait_bar[ring.s], ring.phase);
+                mbar_wait_parked(&wait_bar[ring.s], ring.phase);
 #pragma unroll
-                for (int i = 0; i < NPT; ++i) step3<WSX, WSG, WSV, ROLE>(sb, dst_img, k + 1, pc[i], ca[i], cb[i], ts);
+                for (int i = 0; i < 1; ++i) step3<WSX, WSG, WSV>(sb, dst_img, k + 1, pc[i], ca[i], cb[i], ts);
                 release(ring);
             }
         }
@@ -1103,18 +1053,8 @@ struct Body {
 
     template <int WSX, int WSG, int WSV>
     TS_D void run_images(unsigned char* smem, Ring& ring, unsigned char* dst, int npl, const PairCtx& pc0, float* ts) const {
-        if constexpr (DIM == 2) {
-            run_images2<WSX, WSG, WSV>(smem, ring, dst, npl, pc0, ts);
-        } else if constexpr (MODE == 2 && ACTIVE) {
-if constexpr (SPLIT) {         // chosen at LAUNCH: both role layouts in one kernel cost 600 bytes of spills
-                if (tid < (nt >> 1)) run_images3<WSX, WSG, WSV, 1>(smem, ring, dst, npl, ts);
-                else run_images3<WSX, WSG, WSV, 2>(smem, ring, dst, npl, ts);
-            } else {
-                run_images3<WSX, WSG, WSV, 0>(smem, ring, dst, npl, ts);
-            }
-        } else {
-            run_images3<WSX, WSG, WSV, 0>(smem, ring, dst, npl, ts);
-        }
+        if constexpr (DIM == 2) run_images2<WSX, WSG, WSV>(smem, ring, dst, npl, pc0, ts);
+        else run_images3<WSX, WSG, WSV>(smem, ring, dst, npl, ts);
     }
 
     // CLS 0..3: every window misalignment is a compile-time constant (x window: CLS words; grad_input window: the same
@@ -1164,7 +1104,7 @@ if constexpr (SPLIT) {         // chosen at LAUNCH: both role layouts in one ker
     }
 };
 
-template <int DIM, int MODE, bool ACTIVE, bool SPLIT, bool POOL, bool CROP = false>
+template <int DIM, int MODE, bool ACTIVE, bool POOL, bool CROP = false>
 __global__ void __launch_bounds__(MAXT, 1) k_halo(const __grid_constant__ HArgs a) {
     extern __shared__ __align__(1024) unsigned char smem[];
     uint64_t* full = (uint64_t*)(smem + (size_t)a.stages * a.stage_stride);
@@ -1219,7 +1159,7 @@ __global__ void __launch_bounds__(MAXT, 1) k_halo(const __grid_constant__ HArgs 
         else fixer(a, smem, full, ready, lane, tbl, lists, uo);
         return;
     }
-    Body<DIM, MODE, ACTIVE, SPLIT, POOL, CROP> body(a, threadIdx.x, a.nt, wid, lane, a.need_fix ? ready : full, empty, tbl);
+    Body<DIM, MODE, ACTIVE, POOL, CROP> body(a, threadIdx.x, a.nt, wid, lane, a.need_fix ? ready : full, empty, tbl);
     Ring ring = {0, 0u};
     const UnitRange ur = unit_range(a.units, a.unit_order);
     int u = ur.u;
@@ -1269,10 +1209,9 @@ bool make_args(const Geo& g, const HaloPlan& p, int mode, int active, int pool, 
     a.n_per_unit = p.n_per_unit; a.units = p.units;
     a.chunks = (int)(p.units / (g.C > 0 ? g.C : 1));
     a.unit_order = tuning().unit_order;
-    a.d_C = make_fastdivu((unsigned)g.C);
-    a.d_chunks = make_fastdivu((unsigned)a.chunks);
+    a.d_C = make_fastdiv((unsigned)g.C);
+    a.d_chunks = make_fastdiv((unsigned)a.chunks);
     a.table = g.C <= TABLE_MAX_C ? 1 : 0;
-    a.probe = tuning().halo_probe;
     a.pool = pool;
     a.out_plane_bytes = pool ? (long long)((a.OB + 1) / 2) * (a.OL / 2) * 4 : (mode == 2 ? g.in_plane : g.out_plane) * 4;
     a.pool_bwd = pool_bwd ? 1 : 0;
@@ -1280,10 +1219,9 @@ bool make_args(const Geo& g, const HaloPlan& p, int mode, int active, int pool, 
     a.need_fix = g.pad != TS_PAD_ZEROS || pool_bwd;
     a.nfix = pool_bwd ? 4 : 1;
     if (pool_bwd) a.box_v = a.PW * a.PH * 4;
-    a.d_PW = make_fastdivu((unsigned)(a.PW > 0 ? a.PW : 1));
-    a.split = 0;      // (the role-split 3-D backward -- x-window warps and grad-window warps -- measured 1.7x slower and is no longer built)
-    a.d_GP = make_fastdivu((unsigned)a.GP);
-    a.d_img = make_fastdivu((unsigned)a.img_pairs);
+    a.d_PW = make_fastdiv((unsigned)(a.PW > 0 ? a.PW : 1));
+    a.d_GP = make_fastdiv((unsigned)a.GP);
+    a.d_img = make_fastdiv((unsigned)a.img_pairs);
     if (!make_tensor_map5(&a.map_x, x, 4, g.N, g.C, a.A, a.B, a.L, a.px, a.bpx, 1, 1)) return false;
     if (mode == 2 && pool_bwd) {
         if (!make_tensor_map5(&a.map_v, grad, 4, g.N, g.C, 1, a.PH, a.PW, a.PW, a.PH, 1, 1)) return false;
@@ -1335,7 +1273,6 @@ HaloPlan plan_halo(const Geo& g, int mode, int active, int dtype, bool dense_x, 
     const int IB = mode == 2 ? B : OB, IG = (mode == 2 ? L : OL) / 4;
     int GP = IG;
     if (IG % 8 != 0 && (double)IG / (double)((IG + 7) / 8 * 8) >= 0.85) GP = (IG + 7) / 8 * 8;
-    if (d == 3 && t.halo_compact && ((IB + 1) / 2 * IG + 31) / 32 < ((IB + 1) / 2 * GP + 31) / 32) GP = IG;   // one warp fewer
     const int img_pairs = (IB + 1) / 2 * GP;
     const int max_nt = MAXT - 64 - (pool_bwd ? 96 : 0);    // producer warp + fixer warp(s)
     const long long table_bytes = (g.C <= TABLE_MAX_C ? g.C * 36 : 0) + ((g.pad != TS_PAD_ZEROS || pool_bwd) ? 2 * FIXCAP * 4 : 0)      // + the fixer's cell lists
@@ -1366,7 +1303,6 @@ HaloPlan plan_halo(const Geo& g, int mode, int active, int dtype, bool dense_x, 
     int warps;
     if (d == 3) {
         warps = (int)((pairs + 31) / 32);
-        if (t.halo_split && mode == 2 && active && warps % 2 && warps < max_nt / 32) ++warps;      // x-window warps and grad-window warps
     } else {
         auto eff = [&](int w) {
             const long long nt = 32ll * w, passes = (pairs + nt - 1) / nt;
@@ -1400,7 +1336,7 @@ HaloPlan plan_halo(const Geo& g, int mode, int active, int dtype, bool dense_x, 
 int halo_active_forward(const Geo& g, const HaloPlan& p, const void* x, const void* w, void* y, cudaStream_t s) {
     HArgs a;
     if (!make_args(g, p, 1, 1, 0, x, nullptr, y, w, nullptr, &a)) return TS_ERR_UNSUPPORTED;
-    return g.dim == 3 ? launch(k_halo<3, 1, true, false, false>, a, p, s) : launch(k_halo<2, 1, true, false, false>, a, p, s);
+    return g.dim == 3 ? launch(k_halo<3, 1, true, false>, a, p, s) : launch(k_halo<2, 1, true, false>, a, p, s);
 }
 
 // 2-D forward (sparse or active) with the 2x2 / stride-2 / ceil_mode average pooling of modules/shifts.py:85-89 fused
@@ -1409,8 +1345,8 @@ int halo_forward2d(const Geo& g, const HaloPlan& p, int active, int pool, const 
     HArgs a;
     if (g.dim != 2) return TS_ERR_UNSUPPORTED;
     if (!make_args(g, p, active ? 1 : 0, active ? 1 : 0, pool, x, nullptr, y, w, nullptr, &a)) return TS_ERR_UNSUPPORTED;
-    if (active) return pool ? launch(k_halo<2, 1, true, false, true>, a, p, s) : launch(k_halo<2, 1, true, false, false>, a, p, s);
-    return pool ? launch(k_halo<2, 0, false, false, true>, a, p, s) : launch(k_halo<2, 0, false, false, false>, a, p, s);
+    if (active) return pool ? launch(k_halo<2, 1, true, true>, a, p, s) : launch(k_halo<2, 1, true, false>, a, p, s);
+    return pool ? launch(k_halo<2, 0, false, true>, a, p, s) : launch(k_halo<2, 0, false, false>, a, p, s);
 }
 
 int halo_backward(const Geo& g, const HaloPlan& p, int active, const void* grad, const void* x, const void* w, void* gi, void* gw,
@@ -1422,20 +1358,20 @@ int halo_backward(const Geo& g, const HaloPlan& p, int active, const void* grad,
     for (int ax = 0; ax < g.dim; ++ax) crop = crop || g.lb[ax] != 0 || g.OS[ax] != g.S[ax];
     if (pool_bwd) {
         if (g.dim != 2) return TS_ERR_UNSUPPORTED;
-        if (active) rc = crop ? launch(k_halo<2, 2, true, false, true, true>, a, p, s) : launch(k_halo<2, 2, true, false, true, false>, a, p, s);
-        else rc = crop ? launch(k_halo<2, 2, false, false, true, true>, a, p, s) : launch(k_halo<2, 2, false, false, true, false>, a, p, s);
+        if (active) rc = crop ? launch(k_halo<2, 2, true, true, true>, a, p, s) : launch(k_halo<2, 2, true, true, false>, a, p, s);
+        else rc = crop ? launch(k_halo<2, 2, false, true, true>, a, p, s) : launch(k_halo<2, 2, false, true, false>, a, p, s);
         if (rc != TS_OK) return rc;
         return launch_reduce_partials<float>(partials, p.slots, (int)(g.C * g.dim), gw, peers, s);
     }
     switch (g.dim * 2 + (active ? 1 : 0) + (crop ? 8 : 0)) {
-    case 4: rc = launch(k_halo<2, 2, false, false, false, false>, a, p, s); break;
-    case 5: rc = launch(k_halo<2, 2, true, false, false, false>, a, p, s); break;
-    case 6: rc = launch(k_halo<3, 2, false, false, false, false>, a, p, s); break;
-    case 7: rc = launch(k_halo<3, 2, true, false, false, false>, a, p, s); break;
-    case 12: rc = launch(k_halo<2, 2, false, false, false, true>, a, p, s); break;
-    case 13: rc = launch(k_halo<2, 2, true, false, false, true>, a, p, s); break;
-    case 14: rc = launch(k_halo<3, 2, false, false, false, true>, a, p, s); break;
-    default: rc = launch(k_halo<3, 2, true, false, false, true>, a, p, s); break;
+    case 4: rc = launch(k_halo<2, 2, false, false, false>, a, p, s); break;
+    case 5: rc = launch(k_halo<2, 2, true, false, false>, a, p, s); break;
+    case 6: rc = launch(k_halo<3, 2, false, false, false>, a, p, s); break;
+    case 7: rc = launch(k_halo<3, 2, true, false, false>, a, p, s); break;
+    case 12: rc = launch(k_halo<2, 2, false, false, true>, a, p, s); break;
+    case 13: rc = launch(k_halo<2, 2, true, false, true>, a, p, s); break;
+    case 14: rc = launch(k_halo<3, 2, false, false, true>, a, p, s); break;
+    default: rc = launch(k_halo<3, 2, true, false, true>, a, p, s); break;
     }
     if (rc != TS_OK) return rc;
     return launch_reduce_partials<float>(partials, p.slots, (int)(g.C * g.dim), gw, peers, s);

@@ -4,6 +4,9 @@
 
 namespace ts {
 
+constexpr int SMEM_LIMIT = 232448;   // 227 KB opt-in dynamic shared memory per CTA on sm_100
+constexpr int TABLE_MAX_C = 512;     // channels whose shift parameters a CTA tabulates in shared memory (TMA, staged, halo, flat)
+
 // How the integer shifts are obtained in the sparse/quantized gather kernels.
 enum { WK_F32 = 0, WK_F64 = 1, WK_F16 = 2, WK_BF16 = 3, WK_QUANT = 4 };
 
@@ -90,15 +93,9 @@ struct Tuning {
     int halo;          // halo rows / columns of the halo family (0 = 4)
     int halo_stages;   // ring depth of the halo family (0 = auto)
     int halo_warps;    // consumer warps of the 2-D halo kernels (0 = auto)
-    int halo_probe;    // measurement only (results are WRONG when set): 1 = 3-D consumers skip loads + arithmetic (pipeline rate), 2 = consumers do not wait for the data (compute rate)
-    int halo_compact;  // 3-D: 1 = pairs packed without padding the groups of a row to a multiple of 8 when that saves a consumer warp
-    int halo_split;    // 3-D interpolating backward: 0 (default) = one pair per thread, 1 = x-window warps + grad-window warps (two pairs per thread)
     int unit_order;    // 1 (default): units dealt round-robin over (chunk, channel); 0: contiguous channel-major ranges per CTA
                        // (measured on B200: 4 % faster for 32-image shards, 5 % slower for cfg3 at N=256)
-    int no_pdl;        // 1: plain launches instead of programmatic dependent launches (TMA family, pass 2)
-    int no_table;      // 1: do not tabulate the per-channel shift parameters in shared memory (A/B measurements)
     int use_flat;      // 0: the automatic path choice never picks the flat zero-padding gather
-    int flat_variant;  // 0 auto (a warp owns whole planes when C <= 512), 1 item-per-thread with shuffled shifts
     int flat_ctas, flat_stage_kb, flat_stages, flat_warps;   // flat gather: CTAs per SM (0 = 2), stage KiB (0 = 24), ring depth (0 = 4), consumer warps (0 = auto)
     int cl_ahead, cl_rows;   // channels-last float kernels: steps of copies in flight (0 = 2, at most 4), rows per step (0 = 2; 1, 2, 4, 8)
 };

@@ -300,7 +300,7 @@ TS_HD int ring_slot(const RingStep& st, int k, int row) {   // row in [st.lo, st
 
 TS_HD void copy16(uint8_t* dst_ring, const uint8_t* src_global) {
 #ifdef __CUDA_ARCH__
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(shared_addr(dst_ring)), "l"(src_global) : "memory");
+    ptx::cp_async16(shared_addr(dst_ring), src_global);
 #else
     for (int i = 0; i < 16; ++i) dst_ring[i] = src_global[i];
 #endif
@@ -761,10 +761,7 @@ __global__ void __launch_bounds__((ROWS_MAX_W + 1) * 32, 1) k_gather_nhwc_rows(G
             for (int row = sg.lo; row <= sg.hi; ++row, src += g.xs[2]) {
                 if (round > 0) mbar_wait_relaxed(&empty[slot], (unsigned)((round - 1) & 1), 64);
                 mbar_expect_tx(&full[slot], row_bytes);
-                asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                                 smem_u32(rsm + (size_t)slot * row_bytes)),
-                             "l"(src), "r"(row_bytes), "r"(smem_u32(&full[slot]))
-                             : "memory");
+                bulk_g2s(rsm + (size_t)slot * row_bytes, src, row_bytes, &full[slot]);
                 if (++slot == K) { slot = 0; ++round; }
             }
         }

@@ -25,10 +25,13 @@
 // into one fp64 partial slot per (image, segment) -- the layout launch_reduce_partials<ST> reads -- and that pass 2
 // (with its fused all-reduce) is reused unchanged.  Results are bit-identical from run to run.
 #include "ts_kernels.h"
+#include "ts_ptx.cuh"
 
 namespace ts {
 
 namespace {
+
+using namespace ptx;
 
 constexpr int CL_D = 2;            // default steps of copies in flight ahead of the gather (tuning knob cl_ahead: 1..4)
 constexpr int CL_G = 2;            // default rows per step (tuning knob cl_rows: 1, 2, 4 or 8)
@@ -65,11 +68,6 @@ template <typename ST> TS_D unsigned ldg_bits(const ST* p) {
     return (unsigned)__ldg(reinterpret_cast<const typename Bits<ST>::type*>(p));
 }
 
-TS_D void cp_async16(unsigned dst, const void* src) {
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(src) : "memory");
-}
-TS_D void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N> TS_D void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
 TS_D void cp_async_wait_n(int n) {      // wait_group takes an immediate
     switch (n) {
     case 1: cp_async_wait<1>(); break;

@@ -29,73 +29,16 @@
 #include <cstring>
 
 #include "ts_kernels.h"
+#include "ts_ptx.cuh"
 
 namespace ts {
 
-Tuning& tuning() {
-    static Tuning t = [] {
-        Tuning d;
-        memset(&d, 0, sizeof(d));          // 0 = automatic (per-mode defaults in the planners)
-        d.warps = 15;
-        d.ctas_per_sm = 1;
-        d.use_tma = d.use_halo = d.use_flat = 1;
-        d.unit_order = 1;
-        return d;
-    }();
-    return t;
-}
-
 namespace {
 
-constexpr int SMEM_LIMIT = 232448;   // 227 KB opt-in dynamic shared memory per CTA on sm_100
+using namespace ptx;
+
 constexpr int GUARD = 32;            // readable slack around the slabs of a stage (second group of a window pair)
 constexpr int MAXT_GATHER = 1024, MAXT_ARITH = 512;   // 512 threads -> 128 registers per thread
-
-// ---- exact division by a launch-invariant (n < 2^31) ------------------------------------------
-struct FastDiv { unsigned m, l, d; };
-FastDiv make_fastdiv(unsigned d) {
-    FastDiv f;
-    f.d = d ? d : 1;
-    unsigned l = 0;
-    while ((1ull << l) < f.d) ++l;
-    f.l = l;
-    f.m = (unsigned)(((((unsigned long long)1 << l) - f.d) << 32) / f.d + 1);
-    return f;
-}
-TS_D unsigned fdiv(unsigned n, const FastDiv& f) { return (__umulhi(n, f.m) + n) >> f.l; }
-
-// ---- PTX wrappers -----------------------------------------------------------------------------
-TS_D unsigned smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
-TS_D void mbar_init(uint64_t* bar, unsigned count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
-}
-TS_D void mbar_expect_tx(uint64_t* bar, unsigned bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-TS_D void mbar_arrive(uint64_t* bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-TS_D void mbar_wait(uint64_t* bar, unsigned parity) {
-    asm volatile(
-        "{\n\t"
-        ".reg .pred P1;\n\t"
-        "LAB_WAIT:\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 P1, [%0], %1;\n\t"
-        "@P1 bra DONE;\n\t"
-        "bra LAB_WAIT;\n\t"
-        "DONE:\n\t"
-        "}" ::"r"(smem_u32(bar)), "r"(parity) : "memory");
-}
-// 1-D bulk async copy global -> shared, completion reported to an mbarrier (SASS: UBLKCP)
-TS_D void bulk_g2s(void* dst, const void* src, unsigned bytes, uint64_t* bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(dst)),
-                 "l"(src), "r"(bytes), "r"(smem_u32(bar))
-                 : "memory");
-}
-TS_D void fence_barrier_init() {
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-}
 
 // ---- kernel arguments ---------------------------------------------------------------------------
 struct SArgs {
@@ -117,13 +60,11 @@ struct SArgs {
     int slab_x, slab_g;                       // bytes of one slab of x / of grad
     int np, stages, stage_stride, nw, n_per_unit, units, chunks, unit_order;
     int off_gv, off_gi;                       // byte offsets of the grad regions inside a stage (after GUARD)
-    int table;                                // per-channel shift parameters tabulated in shared memory (arithmetic kernels, C <= 512)
+    int table;                                // per-channel shift parameters tabulated in shared memory (arithmetic kernels, C <= TABLE_MAX_C)
     int img_items;                            // TA * IB * GP
     long long img_stride;                     // output bytes between consecutive images of one channel
     FastDiv d_img, d_GP, d_IB;
 };
-
-TS_D int level_axis(int level, int dim) { return level - (3 - dim); }
 
 // Per-unit shift parameters by LEVEL (0 slab, 1 row, 2 column).
 struct UnitShift {
@@ -1704,7 +1645,7 @@ StagedPlan plan_staged(const Geo& g, int mode, int active, int esize, int dtype,
     const long long IB = mode == 2 ? B : OB;
     const int ex = mode != 0 ? 1 : 0;                       // +1 neighbour slab for the arithmetic kernels
     const int ctas = (mode == 0 && t.ctas_per_sm > 1) ? t.ctas_per_sm : 1;     // byte mover only: several small pipelines per SM
-    const long long table_bytes = (mode != 0 && g.C <= 512 && !t.no_table) ? (g.C * 36 + 15) / 16 * 16 : 0;     // per-channel shift table
+    const long long table_bytes = (mode != 0 && g.C <= TABLE_MAX_C) ? (g.C * 36 + 15) / 16 * 16 : 0;     // per-channel shift table
     const long long budget = SMEM_LIMIT / ctas - 1024 - table_bytes;
     // bytes of one image's slots for a tile of `ta` slabs
     auto slots = [&](long long ta, int* xs, int* gvs, int* gis) {

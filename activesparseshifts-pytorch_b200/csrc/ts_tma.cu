@@ -30,27 +30,15 @@
 #include <cstdio>
 
 #include "ts_kernels.h"
+#include "ts_ptx.cuh"
 
 namespace ts {
 
 namespace {
 
-constexpr int SMEM_LIMIT = 232448;
-constexpr int MAXT_TMA_GATHER = 1024, MAXT_TMA_ARITH = 512;
-constexpr int TABLE_MAX_C = 512;      // channels whose shift parameters are tabulated in shared memory (24 bytes each)
+using namespace ptx;
 
-// ---- exact division by a launch-invariant (n < 2^31) ------------------------------------------
-struct FastDiv { unsigned m, l, d; };
-FastDiv make_fastdiv(unsigned d) {
-    FastDiv f;
-    f.d = d ? d : 1;
-    unsigned l = 0;
-    while ((1ull << l) < f.d) ++l;
-    f.l = l;
-    f.m = (unsigned)(((((unsigned long long)1 << l) - f.d) << 32) / f.d + 1);
-    return f;
-}
-TS_D unsigned fdiv(unsigned n, const FastDiv& f) { return (__umulhi(n, f.m) + n) >> f.l; }
+constexpr int MAXT_TMA_GATHER = 1024, MAXT_TMA_ARITH = 512;
 
 // ---- driver entry point (no libcuda link dependency) ------------------------------------------
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
@@ -116,42 +104,6 @@ bool make_map(CUtensorMap* map, const void* base, int es, long long N, long long
     return true;
 }
 
-// ---- PTX wrappers -----------------------------------------------------------------------------
-TS_D unsigned smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
-TS_D void mbar_init(uint64_t* bar, unsigned count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
-}
-TS_D void mbar_expect_tx(uint64_t* bar, unsigned bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-TS_D void mbar_arrive(uint64_t* bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-TS_D void mbar_wait(uint64_t* bar, unsigned parity) {
-    asm volatile(
-        "{\n\t"
-        ".reg .pred P1;\n\t"
-        "LAB_WAIT:\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 P1, [%0], %1;\n\t"
-        "@P1 bra DONE;\n\t"
-        "bra LAB_WAIT;\n\t"
-        "DONE:\n\t"
-        "}" ::"r"(smem_u32(bar)), "r"(parity) : "memory");
-}
-TS_D void fence_barrier_init() {
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-}
-// tiled 5-D TMA load global -> shared; coordinates innermost first; OOB elements arrive as zero.
-// c0 must be a multiple of 16 bytes worth of elements.
-TS_D void tma_load_5d(void* dst, const CUtensorMap* map, int c0, int c1, int c2, int c3, int c4, uint64_t* bar) {
-    asm volatile(
-        "cp.async.bulk.tensor.5d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4, %5, %6}], [%7];" ::"r"(
-            smem_u32(dst)),
-        "l"(map), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "r"(c4), "r"(smem_u32(bar))
-        : "memory");
-}
-
 // ---- arguments -------------------------------------------------------------------------------
 struct alignas(64) TArgs {
     CUtensorMap map_x;       // x,    box {(TG+1)*vec, xb, xa, 1, np}
@@ -182,7 +134,6 @@ struct alignas(64) TArgs {
     int table;               // per-channel shift table in shared memory (C <= TABLE_MAX_C): built once per CTA
 };
 
-TS_D int level_axis(int level, int dim) { return level - (3 - dim); }
 TS_D int floor_to(int v, int q) { return v & ~(q - 1); }      // q is a power of two (elements per 16 bytes)
 
 struct UnitShift {
@@ -250,7 +201,7 @@ TS_D Tile tile_of(const TArgs& a, int t) {
 // ---- producer ---------------------------------------------------------------------------------
 TS_D void producer(const TArgs& a, unsigned char* smem, uint64_t* full, uint64_t* empty, const UnitShift* tbl) {
     int s = 0, k = 0;
-    const long long C = a.g.C, N = a.g.N;
+    const long long N = a.g.N;
     const int dim = a.g.dim;
     const UnitRange ur = unit_range(a.units, a.unit_order);
     for (int u = ur.u; u < ur.end; u += ur.step) {
@@ -807,12 +758,8 @@ __global__ void __launch_bounds__(MAXT_TMA_ARITH, 1) k_tma_backward(const __grid
 template <class K>
 int launch(K kernel, const TArgs& a, const TmaPlan& p, cudaStream_t s) {
     if (!ensure_dynamic_smem((const void*)kernel, p.smem_bytes)) return check_launch();
-    if (!tuning().no_pdl) {
-        if (launch_pdl(kernel, dim3(p.grid), dim3((p.warps + 1) * 32), p.smem_bytes, s, a) != cudaSuccess) {
-            (void)cudaGetLastError();
-            kernel<<<p.grid, (p.warps + 1) * 32, p.smem_bytes, s>>>(a);
-        }
-    } else {
+    if (launch_pdl(kernel, dim3(p.grid), dim3((p.warps + 1) * 32), p.smem_bytes, s, a) != cudaSuccess) {
+        (void)cudaGetLastError();
         kernel<<<p.grid, (p.warps + 1) * 32, p.smem_bytes, s>>>(a);
     }
     note_launch();
@@ -854,7 +801,7 @@ bool make_args(const Geo& g, const TmaPlan& p, int mode, int active, int es, TAr
     a.unit_order = tuning().unit_order;
     a.d_C = make_fastdiv((unsigned)g.C);
     a.d_chunks = make_fastdiv((unsigned)a.chunks);
-    a.table = (g.C <= TABLE_MAX_C && !tuning().no_table) ? 1 : 0;
+    a.table = g.C <= TABLE_MAX_C ? 1 : 0;
     a.GP = p.gp;
     a.img_items = a.TA * a.TB * a.GP;
     a.img_stride16 = (int)(g.C * (mode == 2 ? g.in_plane : g.out_plane) * es / 16);

@@ -127,6 +127,12 @@ def test_geometry_validation(native):
     assert lib.ts_shift_forward(ct.byref(g), 0, 0, 0, None, None, None, None) in (1, 6, 7)   # null pointers / no device
     assert lib.ts_shift_backward_workspace_bytes(ct.byref(g), 0) >= 16
     assert lib.ts_set_tuning(b"stages=3,warps=8") == 0 and lib.ts_set_tuning(b"bogus=1") == 1
+    # retired measurement-only knobs are rejected like unknown keys; one kept key of each family still parses
+    for key in (b"halo_split", b"halo_probe", b"halo_compact", b"no_table", b"no_pdl", b"flat_variant"):
+        assert lib.ts_set_tuning(key + b"=1") == 1, key
+    for spec in (b"tma_stages=0", b"halo_stages=0", b"flat_stages=0", b"cl_rows=0", b"nhwc_variant=0"):
+        assert lib.ts_set_tuning(spec) == 0, spec
+    assert lib.ts_set_tuning(b"stages=0,warps=15") == 0          # back to the defaults for later tests
     assert lib.ts_set_kernel_path(0) in (0, 1, 2)
 
 

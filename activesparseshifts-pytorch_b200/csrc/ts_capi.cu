@@ -1,5 +1,5 @@
 // ts_capi.cu -- the C ABI of include/torchshifts_b200.h: argument validation, host-side border
-// logic, path selection (staged vs generic) and launch bookkeeping.  No torch types, no
+// logic, kernel-family routing, the backward's pass 2 and launch bookkeeping.  No torch types, no
 // allocation, no synchronisation; every entry point only enqueues kernels on the caller's stream.
 #include <atomic>
 #include <mutex>
@@ -134,6 +134,80 @@ Tuning& tuning() {
     return t;
 }
 
+// ---- kernel-family routing of the planar entry points -----------------------------------------
+// One call as the planners see it.
+struct Call {
+    int mode;                   // 0 sparse / quantized forward, 1 active forward, 2 backward
+    int active, esize, dtype;   // dtype -1: quantized (esize bytes per element)
+    unsigned long long fill;    // quantized: the bit pattern of the zero point
+    const void *x, *out, *grad; // out: y or grad_input; grad: null in a forward
+};
+
+struct Route {
+    int path;                   // TS_PATH_* of the family that serves the call, with its plan
+    TmaPlan tma;
+    HaloPlan halo;
+    FlatPlan flat;
+    StagedPlan staged;
+    GenericBwdPlan generic;
+    int slots;                  // backward: partial slots pass 1 fills
+};
+
+// The families each operation tries, in order of preference.  3-D interpolating backward, automatic choice: the
+// slab-streaming halo kernel (every slab staged once, windows of the previous slab in registers) beats the TMA family's
+// tile kernel under zeros padding as well (cfg4: 0.50 against 0.55 ms).
+static const int GATHER[] = {TS_PATH_TMA, TS_PATH_FLAT, TS_PATH_STAGED, TS_PATH_GENERIC};        // sparse and quantized forward
+static const int ARITHMETIC[] = {TS_PATH_TMA, TS_PATH_HALO, TS_PATH_STAGED, TS_PATH_GENERIC};    // active forward, backward
+static const int HALO_FIRST[] = {TS_PATH_HALO, TS_PATH_TMA, TS_PATH_STAGED, TS_PATH_GENERIC};
+
+// Plans family `path` for `c`: false when it declines (the generic family never does).  forced: plan_halo / plan_flat take
+// small planes too; pool: the pooled halo backward of ts_shift2d_avgpool2_backward.
+static bool plan(int path, const Geo& g, const Call& c, bool dense_x, int sms, bool forced, bool pool, Route* r) {
+    r->slots = 0;
+    switch (path) {
+    case TS_PATH_TMA:
+        r->tma = plan_tma(g, c.mode, c.active, c.esize, c.dtype, dense_x, c.fill, c.x, c.out, c.grad, sms);
+        r->slots = r->tma.slots;
+        return r->tma.ok;
+    case TS_PATH_HALO:
+        r->halo = plan_halo(g, c.mode, c.active, c.dtype, dense_x, c.x, c.out, c.grad, sms, forced, pool);
+        r->slots = r->halo.slots;
+        return r->halo.ok;
+    case TS_PATH_FLAT:
+        r->flat = plan_flat(g, c.esize, dense_x, c.x, c.out, sms, forced);
+        return r->flat.ok;
+    case TS_PATH_STAGED:
+        r->staged = plan_staged(g, c.mode, c.active, c.esize, c.dtype, dense_x, c.x, c.out, c.grad, sms);
+        r->slots = r->staged.slots;
+        return r->staged.ok;
+    }
+    if (c.mode == 2) {
+        r->generic = plan_generic_backward(g);
+        r->slots = r->generic.units;
+    }
+    return true;
+}
+
+// Automatic choice: the first family of the list whose use_* knob is on and whose plan is ok.  Under ts_set_kernel_path
+// only the forced family is planned: TS_ERR_UNSUPPORTED when it is not in the list or declines.
+static int route(const Geo& g, const Call& c, int sms, Route* r) {
+    const int forced = g_forced_path.load();
+    const int* list = c.mode == 0 ? GATHER : c.mode == 2 && c.active && g.dim == 3 && forced == TS_PATH_NONE ? HALO_FIRST : ARITHMETIC;
+    const Tuning& t = tuning();
+    const bool dense_x = x_is_dense(g);
+    for (int i = 0; i < 4; ++i) {
+        const int path = list[i];
+        const bool on = path == TS_PATH_TMA ? t.use_tma : path == TS_PATH_HALO ? t.use_halo : path == TS_PATH_FLAT ? t.use_flat : true;
+        if (forced == TS_PATH_NONE ? !on : path != forced) continue;
+        if (plan(path, g, c, dense_x, sms, forced == path, false, r)) {
+            r->path = path;
+            return TS_OK;
+        }
+        if (forced != TS_PATH_NONE) break;
+    }
+    return TS_ERR_UNSUPPORTED;
+}
+
 }  // namespace ts
 
 using namespace ts;
@@ -266,44 +340,20 @@ int ts_shift_forward(const ts_geometry* gin, int dtype, int padding, int active,
     if (!x || !weights || !y) return TS_ERR_INVALID_ARGUMENT;
     int sms = 0;
     if ((rc = sm_count(&sms)) != TS_OK) return rc;
+    Route r;
+    if ((rc = route(g, Call{active ? 1 : 0, active, es, dtype, 0ull, x, y, nullptr}, sms, &r)) != TS_OK) return rc;
+    t_last_path = r.path;
     cudaStream_t s = (cudaStream_t)stream;
-    const int forced = g_forced_path.load();
-    if ((forced == TS_PATH_NONE && tuning().use_tma) || forced == TS_PATH_TMA) {
-        const TmaPlan tp = plan_tma(g, active ? 1 : 0, active, es, dtype, x_is_dense(g), 0ull, x, y, nullptr, sms);
-        if (tp.ok) {
-            t_last_path = TS_PATH_TMA;
-            return active ? tma_active_forward(g, tp, x, weights, y, s) : tma_gather(g, tp, dtype, x, y, es, weights, 0, 0, s);
-        }
+    switch (r.path) {
+    case TS_PATH_TMA:
+        return active ? tma_active_forward(g, r.tma, x, weights, y, s) : tma_gather(g, r.tma, dtype, x, y, es, weights, 0, 0, s);
+    case TS_PATH_HALO: return halo_active_forward(g, r.halo, x, weights, y, s);
+    case TS_PATH_FLAT: return flat_gather(g, r.flat, dtype, x, y, 0ull, es, weights, 0, 0, s);
+    case TS_PATH_STAGED:
+        return active ? staged_active_forward(g, r.staged, dtype, x, weights, y, s)
+                      : staged_gather(g, r.staged, dtype, x, y, 0ull, es, weights, 0, 0, s);
     }
-    if (forced == TS_PATH_TMA) return TS_ERR_UNSUPPORTED;
-    if (active && ((forced == TS_PATH_NONE && tuning().use_halo) || forced == TS_PATH_HALO)) {
-        const HaloPlan hp = plan_halo(g, 1, 1, dtype, x_is_dense(g), x, y, nullptr, sms, forced == TS_PATH_HALO);
-        if (hp.ok) {
-            t_last_path = TS_PATH_HALO;
-            return halo_active_forward(g, hp, x, weights, y, s);
-        }
-    }
-    if (forced == TS_PATH_HALO) return TS_ERR_UNSUPPORTED;
-    if (!active && ((forced == TS_PATH_NONE && tuning().use_flat) || forced == TS_PATH_FLAT)) {
-        const FlatPlan fp = plan_flat(g, es, x_is_dense(g), x, y, sms, forced == TS_PATH_FLAT);
-        if (fp.ok) {
-            t_last_path = TS_PATH_FLAT;
-            return flat_gather(g, fp, dtype, x, y, 0ull, es, weights, 0, 0, s);
-        }
-    }
-    if (forced == TS_PATH_FLAT) return TS_ERR_UNSUPPORTED;
-    StagedPlan plan;
-    plan.ok = false;
-    if (forced != TS_PATH_GENERIC) plan = plan_staged(g, active ? 1 : 0, active, es, dtype, x_is_dense(g), x, y, nullptr, sms);
-    if (forced == TS_PATH_STAGED && !plan.ok) return TS_ERR_UNSUPPORTED;
-    if (plan.ok) {
-        t_last_path = TS_PATH_STAGED;
-        return active ? staged_active_forward(g, plan, dtype, x, weights, y, s)
-                      : staged_gather(g, plan, dtype, x, y, 0ull, es, weights, 0, 0, s);
-    }
-    t_last_path = TS_PATH_GENERIC;
-    return active ? generic_active_forward(g, dtype, x, weights, y, s)
-                  : generic_gather(g, dtype, x, y, 0ull, es, weights, 0, 0, s);
+    return active ? generic_active_forward(g, dtype, x, weights, y, s) : generic_gather(g, dtype, x, y, 0ull, es, weights, 0, 0, s);
 }
 
 int ts_shift2d_avgpool2_forward(const ts_geometry* gin, int dtype, int padding, int active, const void* x, const void* weights,
@@ -337,28 +387,21 @@ size_t ts_shift_backward_workspace_bytes(const ts_geometry* gin, int dtype) {
     if (g.N * g.C != 0) {
         int sms = 148;
         sm_count(&sms);
-        const GenericBwdPlan gp = plan_generic_backward(g);
-        size_t slots = (size_t)gp.units;
-        // assume the staged / TMA paths may apply (pointer alignment is unknown here)
-        for (int active = 0; active < 2; ++active) {
-            const StagedPlan sp = plan_staged(g, 2, active, elem_size(dtype), dtype, true, nullptr, nullptr, nullptr, sms);
-            if (sp.ok && (size_t)sp.slots > slots) slots = (size_t)sp.slots;
-        }
-        Geo gz = g;
-        gz.pad = TS_PAD_ZEROS;
-        for (int active = 0; active < 2; ++active) {
-            const TmaPlan tp = plan_tma(gz, 2, active, elem_size(dtype), dtype, true, 0ull, nullptr, nullptr, nullptr, sms);
-            if (tp.ok && (size_t)tp.slots > slots) slots = (size_t)tp.slots;
-        }
+        // every plan the backward may pick: pointers are unknown here (assume dense, aligned x), the padding is zeros or
+        // another one, the halo plans are forced and include the pooled kernel (ts_shift2d_avgpool2_backward shares this query)
+        int slots = 0;
         for (int pad = 0; pad < 2; ++pad)
             for (int active = 0; active < 2; ++active)
-                for (int pool = 0; pool < 2; ++pool) {      // (pool: ts_shift2d_avgpool2_backward shares this query)
-                    Geo gh = g;
-                    gh.pad = pad;
-                    const HaloPlan hp = plan_halo(gh, 2, active, dtype, true, nullptr, nullptr, nullptr, sms, true, pool != 0);
-                    if (hp.ok && (size_t)hp.slots > slots) slots = (size_t)hp.slots;
-                }
-        bytes = slots * (size_t)(g.C * g.dim) * sizeof(double) + 16;
+                for (const int path : ARITHMETIC)
+                    for (int pool = 0; pool < (path == TS_PATH_HALO ? 2 : 1); ++pool) {
+                        Geo gp = g;
+                        gp.pad = pad;
+                        Route r;
+                        if (plan(path, gp, Call{2, active, elem_size(dtype), dtype, 0ull, nullptr, nullptr, nullptr}, true, sms, true,
+                                 pool != 0, &r) && r.slots > slots)
+                            slots = r.slots;
+                    }
+        bytes = (size_t)slots * (size_t)(g.C * g.dim) * sizeof(double) + 16;
     }
     last_geo = *gin; last_dtype = dtype; last_epoch = epoch; last_bytes = bytes;
     return bytes;
@@ -376,14 +419,8 @@ static int backward_impl(const ts_geometry* gin, int dtype, int padding, int act
     if (g.C * g.dim == 0) return TS_OK;
     if (!grad_weight) return TS_ERR_INVALID_ARGUMENT;
     if (g.N == 0 || g.in_plane == 0) {
-        if (peers) {      // an empty shard still takes part in the exchange: it contributes zeros
-            const int outputs = (int)(g.C * g.dim);
-            switch (dtype) {
-            case TS_F32: return launch_reduce_partials<float>(nullptr, 0, outputs, grad_weight, peers, s);
-            case TS_F16: return launch_reduce_partials<__half>(nullptr, 0, outputs, grad_weight, peers, s);
-            default: return launch_reduce_partials<__nv_bfloat16>(nullptr, 0, outputs, grad_weight, peers, s);
-            }
-        }
+        // an empty shard still takes part in the exchange: it contributes zeros
+        if (peers) return reduce_partials(g, dtype, nullptr, 0, grad_weight, peers, s);
         const cudaError_t e = cudaMemsetAsync(grad_weight, 0, (size_t)(g.C * g.dim) * es, s);
         return e == cudaSuccess ? TS_OK : cuda_fail(e);
     }
@@ -392,42 +429,17 @@ static int backward_impl(const ts_geometry* gin, int dtype, int padding, int act
         return TS_ERR_WORKSPACE;
     int sms = 0;
     if ((rc = sm_count(&sms)) != TS_OK) return rc;
-    const int forced = g_forced_path.load();
-    // 3-D interpolating backward: the slab-streaming halo kernel (every slab staged once, windows of the previous slab in
-    // registers) beats the TMA family's tile kernel under zeros padding as well (cfg4: 0.50 against 0.55 ms)
-    if (forced == TS_PATH_NONE && tuning().use_halo && g.dim == 3 && active) {
-        const HaloPlan hp = plan_halo(g, 2, active, dtype, x_is_dense(g), x, grad_input, grad, sms, false);
-        if (hp.ok) {
-            t_last_path = TS_PATH_HALO;
-            return halo_backward(g, hp, active, grad, x, weights, grad_input, grad_weight, (double*)workspace, peers, s);
-        }
+    Route r;
+    if ((rc = route(g, Call{2, active, es, dtype, 0ull, x, grad_input, grad}, sms, &r)) != TS_OK) return rc;
+    t_last_path = r.path;
+    double* partials = (double*)workspace;
+    switch (r.path) {
+    case TS_PATH_TMA: rc = tma_backward(g, r.tma, active, grad, x, weights, grad_input, partials, s); break;
+    case TS_PATH_HALO: rc = halo_backward(g, r.halo, active, grad, x, weights, grad_input, partials, s); break;
+    case TS_PATH_STAGED: rc = staged_backward(g, r.staged, dtype, active, grad, x, weights, grad_input, partials, s); break;
+    default: rc = generic_backward(g, r.generic, dtype, active, grad, x, weights, grad_input, partials, s); break;
     }
-    if ((forced == TS_PATH_NONE && tuning().use_tma) || forced == TS_PATH_TMA) {
-        const TmaPlan tp = plan_tma(g, 2, active, es, dtype, x_is_dense(g), 0ull, x, grad_input, grad, sms);
-        if (tp.ok) {
-            t_last_path = TS_PATH_TMA;
-            return tma_backward(g, tp, active, grad, x, weights, grad_input, grad_weight, (double*)workspace, peers, s);
-        }
-    }
-    if (forced == TS_PATH_TMA) return TS_ERR_UNSUPPORTED;
-    if ((forced == TS_PATH_NONE && tuning().use_halo) || forced == TS_PATH_HALO) {
-        const HaloPlan hp = plan_halo(g, 2, active, dtype, x_is_dense(g), x, grad_input, grad, sms, forced == TS_PATH_HALO);
-        if (hp.ok) {
-            t_last_path = TS_PATH_HALO;
-            return halo_backward(g, hp, active, grad, x, weights, grad_input, grad_weight, (double*)workspace, peers, s);
-        }
-    }
-    if (forced == TS_PATH_HALO || forced == TS_PATH_FLAT) return TS_ERR_UNSUPPORTED;
-    StagedPlan plan;
-    plan.ok = false;
-    if (forced != TS_PATH_GENERIC) plan = plan_staged(g, 2, active, es, dtype, x_is_dense(g), x, grad_input, grad, sms);
-    if (forced == TS_PATH_STAGED && !plan.ok) return TS_ERR_UNSUPPORTED;
-    if (plan.ok) {
-        t_last_path = TS_PATH_STAGED;
-        return staged_backward(g, plan, dtype, active, grad, x, weights, grad_input, grad_weight, (double*)workspace, peers, s);
-    }
-    t_last_path = TS_PATH_GENERIC;
-    return generic_backward(g, dtype, active, grad, x, weights, grad_input, grad_weight, (double*)workspace, peers, s);
+    return rc != TS_OK ? rc : reduce_partials(g, dtype, partials, r.slots, grad_weight, peers, s);
 }
 
 int ts_shift2d_avgpool2_backward(const ts_geometry* gin, int dtype, int padding, int active, const void* grad_pooled, const void* x,
@@ -446,8 +458,9 @@ int ts_shift2d_avgpool2_backward(const ts_geometry* gin, int dtype, int padding,
     const HaloPlan hp = plan_halo(g, 2, active, dtype, x_is_dense(g), x, grad_input, grad_pooled, sms, true, true);
     if (!hp.ok) return TS_ERR_UNSUPPORTED;
     t_last_path = TS_PATH_HALO;
-    return halo_backward(g, hp, active, grad_pooled, x, weights, grad_input, grad_weight, (double*)workspace, nullptr,
-                         (cudaStream_t)stream, true);
+    cudaStream_t s = (cudaStream_t)stream;
+    rc = halo_backward(g, hp, active, grad_pooled, x, weights, grad_input, (double*)workspace, s, true);
+    return rc != TS_OK ? rc : reduce_partials(g, dtype, (double*)workspace, hp.slots, grad_weight, nullptr, s);
 }
 
 int ts_shift_backward(const ts_geometry* gin, int dtype, int padding, int active, const void* grad, const void* x,
@@ -516,8 +529,10 @@ int ts_shift_backward_nhwc(const ts_geometry* gin, int dtype, int padding, int a
     if (!workspace || ((uintptr_t)workspace & 15)) return TS_ERR_WORKSPACE;
     int sms = 0;
     if ((rc = sm_count(&sms)) != TS_OK) return rc;
-    rc = cl_backward(g, dtype, active, grad, x, weights, grad_input, grad_weight, (double*)workspace, workspace_bytes, peers, sms,
-                     (cudaStream_t)stream);
+    cudaStream_t s = (cudaStream_t)stream;
+    int slots = 0;
+    rc = cl_backward(g, dtype, active, grad, x, weights, grad_input, (double*)workspace, workspace_bytes, sms, &slots, s);
+    if (rc == TS_OK) rc = reduce_partials(g, dtype, (double*)workspace, slots, grad_weight, peers, s);
     if (rc == TS_OK) t_last_path = TS_PATH_NHWC;
     return rc;
 }
@@ -543,34 +558,17 @@ int ts_qshift_forward(const ts_geometry* gin, int elem_bytes, int padding, int64
     if (!xq || !qweights || !yq) return TS_ERR_INVALID_ARGUMENT;
     int sms = 0;
     if ((rc = sm_count(&sms)) != TS_OK) return rc;
-    cudaStream_t s = (cudaStream_t)stream;
     const unsigned long long fill = qfill(elem_bytes, zero_point);
-    const int forced = g_forced_path.load();
-    if ((forced == TS_PATH_NONE && tuning().use_tma) || forced == TS_PATH_TMA) {
-        const TmaPlan tp = plan_tma(g, 0, 0, elem_bytes, -1, x_is_dense(g), fill, xq, yq, nullptr, sms);
-        if (tp.ok) {
-            t_last_path = TS_PATH_TMA;
-            return tma_gather(g, tp, WK_QUANT, xq, yq, elem_bytes, qweights, qweight_kind, weight_zero_point, s);
-        }
+    Route r;
+    if ((rc = route(g, Call{0, 0, elem_bytes, -1, fill, xq, yq, nullptr}, sms, &r)) != TS_OK) return rc;
+    t_last_path = r.path;
+    cudaStream_t s = (cudaStream_t)stream;
+    switch (r.path) {
+    case TS_PATH_TMA: return tma_gather(g, r.tma, WK_QUANT, xq, yq, elem_bytes, qweights, qweight_kind, weight_zero_point, s);
+    case TS_PATH_FLAT: return flat_gather(g, r.flat, WK_QUANT, xq, yq, fill, elem_bytes, qweights, qweight_kind, weight_zero_point, s);
+    case TS_PATH_STAGED:
+        return staged_gather(g, r.staged, WK_QUANT, xq, yq, fill, elem_bytes, qweights, qweight_kind, weight_zero_point, s);
     }
-    if (forced == TS_PATH_TMA || forced == TS_PATH_HALO) return TS_ERR_UNSUPPORTED;
-    if ((forced == TS_PATH_NONE && tuning().use_flat) || forced == TS_PATH_FLAT) {
-        const FlatPlan fp = plan_flat(g, elem_bytes, x_is_dense(g), xq, yq, sms, forced == TS_PATH_FLAT);
-        if (fp.ok) {
-            t_last_path = TS_PATH_FLAT;
-            return flat_gather(g, fp, WK_QUANT, xq, yq, fill, elem_bytes, qweights, qweight_kind, weight_zero_point, s);
-        }
-    }
-    if (forced == TS_PATH_FLAT) return TS_ERR_UNSUPPORTED;
-    StagedPlan plan;
-    plan.ok = false;
-    if (forced != TS_PATH_GENERIC) plan = plan_staged(g, 0, 0, elem_bytes, -1, x_is_dense(g), xq, yq, nullptr, sms);
-    if (forced == TS_PATH_STAGED && !plan.ok) return TS_ERR_UNSUPPORTED;
-    if (plan.ok) {
-        t_last_path = TS_PATH_STAGED;
-        return staged_gather(g, plan, WK_QUANT, xq, yq, fill, elem_bytes, qweights, qweight_kind, weight_zero_point, s);
-    }
-    t_last_path = TS_PATH_GENERIC;
     return generic_gather(g, WK_QUANT, xq, yq, fill, elem_bytes, qweights, qweight_kind, weight_zero_point, s);
 }
 

@@ -276,7 +276,7 @@ __global__ void __launch_bounds__(1024, 1) k_reduce_partials_allreduce(const dou
 }
 
 template <typename ST>
-int launch_reduce_partials(const double* partials, int slots, int outputs, void* gw, const ts_peer_group* pg, cudaStream_t stream) {
+static int launch_reduce_partials(const double* partials, int slots, int outputs, void* gw, const ts_peer_group* pg, cudaStream_t stream) {
     if (pg) {
         if constexpr (sizeof(ST) == 8) {
             return TS_ERR_UNSUPPORTED;
@@ -304,10 +304,16 @@ int launch_reduce_partials(const double* partials, int slots, int outputs, void*
     note_launch();
     return check_launch();
 }
-template int launch_reduce_partials<float>(const double*, int, int, void*, const ts_peer_group*, cudaStream_t);
-template int launch_reduce_partials<double>(const double*, int, int, void*, const ts_peer_group*, cudaStream_t);
-template int launch_reduce_partials<__half>(const double*, int, int, void*, const ts_peer_group*, cudaStream_t);
-template int launch_reduce_partials<__nv_bfloat16>(const double*, int, int, void*, const ts_peer_group*, cudaStream_t);
+
+int reduce_partials(const Geo& g, int dtype, const double* partials, int slots, void* gw, const ts_peer_group* peers, cudaStream_t s) {
+    const int outputs = (int)(g.C * g.dim);
+    switch (dtype) {
+    case TS_F32: return launch_reduce_partials<float>(partials, slots, outputs, gw, peers, s);
+    case TS_F64: return launch_reduce_partials<double>(partials, slots, outputs, gw, peers, s);
+    case TS_F16: return launch_reduce_partials<__half>(partials, slots, outputs, gw, peers, s);
+    default: return launch_reduce_partials<__nv_bfloat16>(partials, slots, outputs, gw, peers, s);
+    }
+}
 
 // ------------------------------------------------------------------------------------------
 // Host launchers.
@@ -413,21 +419,18 @@ static int bwd_dim(const Geo& g, const GenericBwdPlan& p, const void* grad, cons
 }
 
 template <typename ST>
-static int bwd_t(const Geo& g, int active, const void* grad, const void* x, const void* w, void* gi, void* gw,
-                 double* partials, const ts_peer_group* peers, cudaStream_t s) {
-    const GenericBwdPlan p = plan_generic_backward(g);
-    int rc = active ? bwd_dim<ST, true>(g, p, grad, x, w, gi, partials, s) : bwd_dim<ST, false>(g, p, grad, x, w, gi, partials, s);
-    if (rc != TS_OK) return rc;
-    return launch_reduce_partials<ST>(partials, p.units, (int)(g.C * g.dim), gw, peers, s);
+static int bwd_t(const Geo& g, const GenericBwdPlan& p, int active, const void* grad, const void* x, const void* w, void* gi,
+                 double* partials, cudaStream_t s) {
+    return active ? bwd_dim<ST, true>(g, p, grad, x, w, gi, partials, s) : bwd_dim<ST, false>(g, p, grad, x, w, gi, partials, s);
 }
 
-int generic_backward(const Geo& g, int dtype, int active, const void* grad, const void* x, const void* w, void* gi,
-                     void* gw, double* partials, const ts_peer_group* peers, cudaStream_t s) {
+int generic_backward(const Geo& g, const GenericBwdPlan& p, int dtype, int active, const void* grad, const void* x, const void* w,
+                     void* gi, double* partials, cudaStream_t s) {
     switch (dtype) {
-    case TS_F32: return bwd_t<float>(g, active, grad, x, w, gi, gw, partials, peers, s);
-    case TS_F64: return bwd_t<double>(g, active, grad, x, w, gi, gw, partials, peers, s);
-    case TS_F16: return bwd_t<__half>(g, active, grad, x, w, gi, gw, partials, peers, s);
-    case TS_BF16: return bwd_t<__nv_bfloat16>(g, active, grad, x, w, gi, gw, partials, peers, s);
+    case TS_F32: return bwd_t<float>(g, p, active, grad, x, w, gi, partials, s);
+    case TS_F64: return bwd_t<double>(g, p, active, grad, x, w, gi, partials, s);
+    case TS_F16: return bwd_t<__half>(g, p, active, grad, x, w, gi, partials, s);
+    case TS_BF16: return bwd_t<__nv_bfloat16>(g, p, active, grad, x, w, gi, partials, s);
     }
     return TS_ERR_INVALID_ARGUMENT;
 }

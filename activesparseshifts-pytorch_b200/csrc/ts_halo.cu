@@ -1349,32 +1349,27 @@ int halo_forward2d(const Geo& g, const HaloPlan& p, int active, int pool, const 
     return pool ? launch(k_halo<2, 0, false, true>, a, p, s) : launch(k_halo<2, 0, false, false>, a, p, s);
 }
 
-int halo_backward(const Geo& g, const HaloPlan& p, int active, const void* grad, const void* x, const void* w, void* gi, void* gw,
-                  double* partials, const ts_peer_group* peers, cudaStream_t s, bool pool_bwd) {
+int halo_backward(const Geo& g, const HaloPlan& p, int active, const void* grad, const void* x, const void* w, void* gi,
+                  double* partials, cudaStream_t s, bool pool_bwd) {
     HArgs a;
     if (!make_args(g, p, 2, active ? 1 : 0, 0, x, grad, gi, w, partials, &a, pool_bwd)) return TS_ERR_UNSUPPORTED;
-    int rc;
     bool crop = false;
     for (int ax = 0; ax < g.dim; ++ax) crop = crop || g.lb[ax] != 0 || g.OS[ax] != g.S[ax];
     if (pool_bwd) {
         if (g.dim != 2) return TS_ERR_UNSUPPORTED;
-        if (active) rc = crop ? launch(k_halo<2, 2, true, true, true>, a, p, s) : launch(k_halo<2, 2, true, true, false>, a, p, s);
-        else rc = crop ? launch(k_halo<2, 2, false, true, true>, a, p, s) : launch(k_halo<2, 2, false, true, false>, a, p, s);
-        if (rc != TS_OK) return rc;
-        return launch_reduce_partials<float>(partials, p.slots, (int)(g.C * g.dim), gw, peers, s);
+        if (active) return crop ? launch(k_halo<2, 2, true, true, true>, a, p, s) : launch(k_halo<2, 2, true, true, false>, a, p, s);
+        return crop ? launch(k_halo<2, 2, false, true, true>, a, p, s) : launch(k_halo<2, 2, false, true, false>, a, p, s);
     }
     switch (g.dim * 2 + (active ? 1 : 0) + (crop ? 8 : 0)) {
-    case 4: rc = launch(k_halo<2, 2, false, false, false>, a, p, s); break;
-    case 5: rc = launch(k_halo<2, 2, true, false, false>, a, p, s); break;
-    case 6: rc = launch(k_halo<3, 2, false, false, false>, a, p, s); break;
-    case 7: rc = launch(k_halo<3, 2, true, false, false>, a, p, s); break;
-    case 12: rc = launch(k_halo<2, 2, false, false, true>, a, p, s); break;
-    case 13: rc = launch(k_halo<2, 2, true, false, true>, a, p, s); break;
-    case 14: rc = launch(k_halo<3, 2, false, false, true>, a, p, s); break;
-    default: rc = launch(k_halo<3, 2, true, false, true>, a, p, s); break;
+    case 4: return launch(k_halo<2, 2, false, false, false>, a, p, s);
+    case 5: return launch(k_halo<2, 2, true, false, false>, a, p, s);
+    case 6: return launch(k_halo<3, 2, false, false, false>, a, p, s);
+    case 7: return launch(k_halo<3, 2, true, false, false>, a, p, s);
+    case 12: return launch(k_halo<2, 2, false, false, true>, a, p, s);
+    case 13: return launch(k_halo<2, 2, true, false, true>, a, p, s);
+    case 14: return launch(k_halo<3, 2, false, false, true>, a, p, s);
+    default: return launch(k_halo<3, 2, true, false, true>, a, p, s);
     }
-    if (rc != TS_OK) return rc;
-    return launch_reduce_partials<float>(partials, p.slots, (int)(g.C * g.dim), gw, peers, s);
 }
 
 }  // namespace ts

@@ -53,13 +53,14 @@ GenericBwdPlan plan_generic_backward(const Geo& g);
 int generic_gather(const Geo& g, int wk, const void* x, void* y, unsigned long long fill, int esize, const void* w,
                    int qkind, long long wzp, cudaStream_t s);
 int generic_active_forward(const Geo& g, int dtype, const void* x, const void* w, void* y, cudaStream_t s);
-int generic_backward(const Geo& g, int dtype, int active, const void* grad, const void* x, const void* w, void* gi,
-                     void* gw, double* partials, const ts_peer_group* peers, cudaStream_t s);
+int generic_backward(const Geo& g, const GenericBwdPlan& p, int dtype, int active, const void* grad, const void* x, const void* w,
+                     void* gi, double* partials, cudaStream_t s);
 
-// peers != nullptr: the pass-2 launch is the variant fused with the all-reduce over peer memory
+// Every backward runs in two passes.  Pass 1 (the family's *_backward launcher) writes grad_input and `slots` fp64
+// partial sums of each of the C x dim grad_weight values to `partials`; pass 2 (this) reduces them into gw, in a fixed
+// order.  peers != nullptr: the pass-2 kernel is the variant fused with the all-reduce over peer memory
 // (ts_shift_backward_allreduce); slots may be 0 (a rank with an empty shard contributes zeros).
-template <typename ST>
-int launch_reduce_partials(const double* partials, int slots, int outputs, void* gw, const ts_peer_group* peers, cudaStream_t stream);
+int reduce_partials(const Geo& g, int dtype, const double* partials, int slots, void* gw, const ts_peer_group* peers, cudaStream_t s);
 
 // ---- channels-last gather (ts_nhwc.cu): input and output keep the channel axis innermost -------
 int nhwc_gather(const Geo& g, const void* x, void* y, unsigned long long fill, int esize, const void* w, int qkind,
@@ -68,11 +69,12 @@ int nhwc_gather(const Geo& g, const void* x, void* y, unsigned long long fill, i
 int nhwc_to_planar(const void* x, void* y, long long N, long long C, long long P, int esize, cudaStream_t s);
 
 // ---- channels-last float forward / backward (ts_nhwc_float.cu): 2-D, fp32 / fp16 / bf16, dense NHWC, C % 32 == 0 ----
-// TS_ERR_UNSUPPORTED (nothing launched) for what they do not serve.  partials: cl_backward_workspace_bytes().
+// TS_ERR_UNSUPPORTED (nothing launched) for what they do not serve.  partials: cl_backward_workspace_bytes(); *slots: the
+// partial slots the backward filled.
 int cl_forward(const Geo& g, int dtype, int active, const void* x, const void* w, void* y, int sm_count, cudaStream_t s);
 size_t cl_backward_workspace_bytes(const Geo& g, int dtype, int sm_count);
-int cl_backward(const Geo& g, int dtype, int active, const void* grad, const void* x, const void* w, void* gi, void* gw, double* partials,
-                size_t workspace_bytes, const ts_peer_group* peers, int sm_count, cudaStream_t s);
+int cl_backward(const Geo& g, int dtype, int active, const void* grad, const void* x, const void* w, void* gi, double* partials,
+                size_t workspace_bytes, int sm_count, int* slots, cudaStream_t s);
 
 // ---- staged family (ts_staged.cu): bulk-async shared-memory staging ---------------------------
 struct Tuning {
@@ -120,7 +122,7 @@ int staged_gather(const Geo& g, const StagedPlan& p, int wk, const void* x, void
                   const void* w, int qkind, long long wzp, cudaStream_t s);
 int staged_active_forward(const Geo& g, const StagedPlan& p, int dtype, const void* x, const void* w, void* y, cudaStream_t s);
 int staged_backward(const Geo& g, const StagedPlan& p, int dtype, int active, const void* grad, const void* x, const void* w,
-                    void* gi, void* gw, double* partials, const ts_peer_group* peers, cudaStream_t s);
+                    void* gi, double* partials, cudaStream_t s);
 
 // ---- TMA-tensor family (ts_tma.cu): zeros padding done by the copy engine ----------------------
 struct TmaPlan {
@@ -138,8 +140,8 @@ TmaPlan plan_tma(const Geo& g, int mode, int active, int esize, int dtype, bool 
 int tma_gather(const Geo& g, const TmaPlan& p, int wk, const void* x, void* y, int esize, const void* w, int qkind, long long wzp,
                cudaStream_t s);
 int tma_active_forward(const Geo& g, const TmaPlan& p, const void* x, const void* w, void* y, cudaStream_t s);
-int tma_backward(const Geo& g, const TmaPlan& p, int active, const void* grad, const void* x, const void* w, void* gi, void* gw,
-                 double* partials, const ts_peer_group* peers, cudaStream_t s);
+int tma_backward(const Geo& g, const TmaPlan& p, int active, const void* grad, const void* x, const void* w, void* gi,
+                 double* partials, cudaStream_t s);
 
 // rank-5 tensor map over a dense [N][C][A][B][L] tensor, box {bl, bb, ba, 1, bn} (memoised per thread); `map` points to a
 // CUtensorMap (128 bytes, 64-byte aligned)
@@ -175,7 +177,7 @@ HaloPlan plan_halo(const Geo& g, int mode, int active, int dtype, bool dense_x, 
                    int sm_count, bool forced, bool pool_bwd = false);
 int halo_active_forward(const Geo& g, const HaloPlan& p, const void* x, const void* w, void* y, cudaStream_t s);
 int halo_forward2d(const Geo& g, const HaloPlan& p, int active, int pool, const void* x, const void* w, void* y, cudaStream_t s);
-int halo_backward(const Geo& g, const HaloPlan& p, int active, const void* grad, const void* x, const void* w, void* gi, void* gw,
-                  double* partials, const ts_peer_group* peers, cudaStream_t s, bool pool_bwd = false);
+int halo_backward(const Geo& g, const HaloPlan& p, int active, const void* grad, const void* x, const void* w, void* gi,
+                  double* partials, cudaStream_t s, bool pool_bwd = false);
 
 }  // namespace ts

@@ -414,16 +414,14 @@ int cl_forward_t(const Geo& g, const ClPlan& pl, int active, const void* x, cons
 }
 
 template <typename ST, int PAD>
-int cl_backward_t(const Geo& g, const ClPlan& pl, int active, const void* grad, const void* x, const void* w, void* gi, void* gw,
-                  double* partials, const ts_peer_group* peers, cudaStream_t s) {
+int cl_backward_t(const Geo& g, const ClPlan& pl, int active, const void* grad, const void* x, const void* w, void* gi,
+                  double* partials, cudaStream_t s) {
     auto k = active ? k_cl_backward<ST, PAD, true> : k_cl_backward<ST, PAD, false>;
     if (!ensure_dynamic_smem((const void*)k, pl.smem_bytes)) return check_launch();
     const dim3 grid((unsigned)(g.N * pl.segs), (unsigned)pl.slices, 1);
     k<<<grid, CL_BWD_THREADS, pl.smem_bytes, s>>>(g, pl, (const ST*)grad, (const ST*)x, (const ST*)w, (ST*)gi, partials);
     note_launch();
-    const int rc = check_launch();
-    if (rc != TS_OK) return rc;
-    return launch_reduce_partials<ST>(partials, (int)(g.N * pl.segs), (int)(g.C * 2), gw, peers, s);
+    return check_launch();
 }
 
 template <typename ST>
@@ -438,14 +436,14 @@ int cl_forward_pad(const Geo& g, const ClPlan& pl, int active, const void* x, co
 }
 
 template <typename ST>
-int cl_backward_pad(const Geo& g, const ClPlan& pl, int active, const void* grad, const void* x, const void* w, void* gi, void* gw,
-                    double* partials, const ts_peer_group* peers, cudaStream_t s) {
+int cl_backward_pad(const Geo& g, const ClPlan& pl, int active, const void* grad, const void* x, const void* w, void* gi,
+                    double* partials, cudaStream_t s) {
     switch (g.pad) {
-    case TS_PAD_BORDER: return cl_backward_t<ST, TS_PAD_BORDER>(g, pl, active, grad, x, w, gi, gw, partials, peers, s);
-    case TS_PAD_PERIODIC: return cl_backward_t<ST, TS_PAD_PERIODIC>(g, pl, active, grad, x, w, gi, gw, partials, peers, s);
-    case TS_PAD_REFLECT: return cl_backward_t<ST, TS_PAD_REFLECT>(g, pl, active, grad, x, w, gi, gw, partials, peers, s);
-    case TS_PAD_SYMMETRIC: return cl_backward_t<ST, TS_PAD_SYMMETRIC>(g, pl, active, grad, x, w, gi, gw, partials, peers, s);
-    default: return cl_backward_t<ST, TS_PAD_ZEROS>(g, pl, active, grad, x, w, gi, gw, partials, peers, s);
+    case TS_PAD_BORDER: return cl_backward_t<ST, TS_PAD_BORDER>(g, pl, active, grad, x, w, gi, partials, s);
+    case TS_PAD_PERIODIC: return cl_backward_t<ST, TS_PAD_PERIODIC>(g, pl, active, grad, x, w, gi, partials, s);
+    case TS_PAD_REFLECT: return cl_backward_t<ST, TS_PAD_REFLECT>(g, pl, active, grad, x, w, gi, partials, s);
+    case TS_PAD_SYMMETRIC: return cl_backward_t<ST, TS_PAD_SYMMETRIC>(g, pl, active, grad, x, w, gi, partials, s);
+    default: return cl_backward_t<ST, TS_PAD_ZEROS>(g, pl, active, grad, x, w, gi, partials, s);
     }
 }
 
@@ -467,16 +465,17 @@ int cl_forward(const Geo& g, int dtype, int active, const void* x, const void* w
     }
 }
 
-int cl_backward(const Geo& g, int dtype, int active, const void* grad, const void* x, const void* w, void* gi, void* gw, double* partials,
-                size_t workspace_bytes, const ts_peer_group* peers, int sm_count, cudaStream_t s) {
+int cl_backward(const Geo& g, int dtype, int active, const void* grad, const void* x, const void* w, void* gi, double* partials,
+                size_t workspace_bytes, int sm_count, int* slots, cudaStream_t s) {
     ClPlan pl;
     if (!plan_cl(g, dtype, true, sm_count, &pl) || ((uintptr_t)x & 15u) || ((uintptr_t)grad & 15u) || ((uintptr_t)gi & 15u))
         return TS_ERR_UNSUPPORTED;
     if (workspace_bytes < (size_t)(g.N * pl.segs) * (size_t)(g.C * 2) * sizeof(double)) return TS_ERR_WORKSPACE;
+    *slots = (int)(g.N * pl.segs);
     switch (dtype) {
-    case TS_F32: return cl_backward_pad<float>(g, pl, active, grad, x, w, gi, gw, partials, peers, s);
-    case TS_F16: return cl_backward_pad<__half>(g, pl, active, grad, x, w, gi, gw, partials, peers, s);
-    default: return cl_backward_pad<__nv_bfloat16>(g, pl, active, grad, x, w, gi, gw, partials, peers, s);
+    case TS_F32: return cl_backward_pad<float>(g, pl, active, grad, x, w, gi, partials, s);
+    case TS_F16: return cl_backward_pad<__half>(g, pl, active, grad, x, w, gi, partials, s);
+    default: return cl_backward_pad<__nv_bfloat16>(g, pl, active, grad, x, w, gi, partials, s);
     }
 }
 

@@ -1801,7 +1801,7 @@ static int backward_t(const Geo& g, const SArgs& a, const StagedPlan& p, int act
 }
 
 int staged_backward(const Geo& g, const StagedPlan& p, int dtype, int active, const void* grad, const void* x, const void* w,
-                    void* gi, void* gw, double* partials, const ts_peer_group* peers, cudaStream_t s) {
+                    void* gi, double* partials, cudaStream_t s) {
     SArgs a = make_args(g, p, 2, active ? 1 : 0, dtype == TS_F32 ? 4 : 2);
     a.x = (const unsigned char*)x;
     a.grad = (const unsigned char*)grad;
@@ -1809,18 +1809,10 @@ int staged_backward(const Geo& g, const StagedPlan& p, int dtype, int active, co
     a.w = w;
     a.wk = dtype == TS_F32 ? WK_F32 : dtype == TS_F16 ? WK_F16 : WK_BF16;
     a.partials = partials;
-    int rc;
     switch (dtype) {
-    case TS_F32: rc = backward_t<float>(g, a, p, active, s); break;
-    case TS_F16: rc = backward_t<__half>(g, a, p, active, s); break;
-    default: rc = backward_t<__nv_bfloat16>(g, a, p, active, s); break;
-    }
-    if (rc != TS_OK) return rc;
-    const int outputs = (int)(g.C * g.dim);
-    switch (dtype) {
-    case TS_F32: return launch_reduce_partials<float>(partials, p.slots, outputs, gw, peers, s);
-    case TS_F16: return launch_reduce_partials<__half>(partials, p.slots, outputs, gw, peers, s);
-    default: return launch_reduce_partials<__nv_bfloat16>(partials, p.slots, outputs, gw, peers, s);
+    case TS_F32: return backward_t<float>(g, a, p, active, s);
+    case TS_F16: return backward_t<__half>(g, a, p, active, s);
+    default: return backward_t<__nv_bfloat16>(g, a, p, active, s);
     }
 }
 

@@ -1007,8 +1007,8 @@ int tma_active_forward(const Geo& g, const TmaPlan& p, const void* x, const void
     }
 }
 
-int tma_backward(const Geo& g, const TmaPlan& p, int active, const void* grad, const void* x, const void* w, void* gi, void* gw,
-                 double* partials, const ts_peer_group* peers, cudaStream_t s) {
+int tma_backward(const Geo& g, const TmaPlan& p, int active, const void* grad, const void* x, const void* w, void* gi,
+                 double* partials, cudaStream_t s) {
     TArgs a;
     make_args(g, p, 2, active ? 1 : 0, 4, &a);
     const int d = g.dim;
@@ -1019,17 +1019,14 @@ int tma_backward(const Geo& g, const TmaPlan& p, int active, const void* grad, c
     if (!make_map(&a.map_x, x, 4, g.N, g.C, A, B, L, (a.TG + 1) * 4, a.xb, a.xa, a.np)) return TS_ERR_UNSUPPORTED;
     if (!make_map(&a.map_gs, grad, 4, g.N, g.C, A, B, L, (a.TG + 1) * 4, a.TB, a.TA, a.np)) return TS_ERR_UNSUPPORTED;
     if (active && !make_map(&a.map_gb, grad, 4, g.N, g.C, A, B, L, (a.TG + 1) * 4, a.xb, a.xa, a.np)) return TS_ERR_UNSUPPORTED;
-    int rc;
     switch (d * 2 + (active ? 1 : 0)) {
-    case 2: rc = launch(k_tma_backward<1, false>, a, p, s); break;
-    case 3: rc = launch(k_tma_backward<1, true>, a, p, s); break;
-    case 4: rc = launch(k_tma_backward<2, false>, a, p, s); break;
-    case 5: rc = launch(k_tma_backward<2, true>, a, p, s); break;
-    case 6: rc = launch(k_tma_backward<3, false>, a, p, s); break;
-    default: rc = launch(k_tma_backward<3, true>, a, p, s); break;
+    case 2: return launch(k_tma_backward<1, false>, a, p, s);
+    case 3: return launch(k_tma_backward<1, true>, a, p, s);
+    case 4: return launch(k_tma_backward<2, false>, a, p, s);
+    case 5: return launch(k_tma_backward<2, true>, a, p, s);
+    case 6: return launch(k_tma_backward<3, false>, a, p, s);
+    default: return launch(k_tma_backward<3, true>, a, p, s);
     }
-    if (rc != TS_OK) return rc;
-    return launch_reduce_partials<float>(partials, p.slots, (int)(g.C * g.dim), gw, peers, s);
 }
 
 }  // namespace ts

@@ -253,7 +253,6 @@ int ts_set_tuning(const char* spec) {
         else if (!strcmp(key, "ctas_per_sm")) t.ctas_per_sm = val;
         else if (!strcmp(key, "chunk_planes")) t.chunk_planes = val;
         else if (!strcmp(key, "tma_stages")) t.tma_stages = val;
-        else if (!strcmp(key, "tma_ctas_per_sm")) t.tma_ctas_per_sm = val;
         else if (!strcmp(key, "tma_warps")) t.tma_warps = val;
         else if (!strcmp(key, "use_tma")) t.use_tma = val != 0;
         else if (!strcmp(key, "tma_stage_kb")) t.tma_stage_kb = val;
@@ -278,7 +277,7 @@ int ts_set_tuning(const char* spec) {
     }
     if (t.stages < 0 || t.stages > 8 || t.stage_kb < 0 || t.stage_kb > 220 || t.warps < 1 || t.warps > 31 ||
         t.ctas_per_sm < 1 || t.ctas_per_sm > 8 || t.chunk_planes < 0 || t.tma_stages < 0 || t.tma_stages > 32 ||
-        t.tma_ctas_per_sm < 0 || t.tma_ctas_per_sm > 8 || t.tma_warps < 0 || t.tma_warps > 31 || t.tma_stage_kb < 0 ||
+        t.tma_warps < 0 || t.tma_warps > 31 || t.tma_stage_kb < 0 ||
         t.tma_stage_kb > 220 || t.nhwc_variant < 0 || t.nhwc_variant > 3 || t.nhwc_ring_rows < 0 || t.nhwc_rows_warps < 0 || t.nhwc_rows_warps > 12 || t.halo < 0 || t.halo > 16 ||
         t.halo_stages < 0 || t.halo_stages > 32 || t.halo_warps < 0 || t.halo_warps > 15 || t.flat_ctas < 0 || t.flat_ctas > 8 ||
         t.flat_stage_kb < 0 || t.flat_stage_kb > 100 || t.flat_stages < 0 || t.flat_stages > 16 || t.flat_warps < 0 || t.flat_warps > 15 ||

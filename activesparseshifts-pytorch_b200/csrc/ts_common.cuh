@@ -263,6 +263,28 @@ TS_HD void load_qshifts(const void* __restrict__ qw, int kind, long long wzp, lo
 }
 
 // ------------------------------------------------------------------------------------------
+// How the integer shifts are obtained in the sparse/quantized gather kernels.
+enum { WK_F32 = 0, WK_F64 = 1, WK_F16 = 2, WK_BF16 = 3, WK_QUANT = 4 };
+
+// Integer shift of weight `idx` = c * dim + axis for the sparse forward (rounded float weight) or the quantized forward
+// (raw weight minus its zero point).  The arguments are references into the kernel's parameters, so that each is read only
+// on the path that uses it.
+TS_D long long sparse_shift(const void* const& w, const int& wk, const int& qkind, const long long& wzp, long long idx) {
+    long long iw = 0;
+    switch (wk) {
+    case WK_F32: { float d; split_forward<float>(((const float*)w)[idx], false, iw, d); break; }
+    case WK_F64: { double d; split_forward<double>(((const double*)w)[idx], false, iw, d); break; }
+    case WK_F16: { float d; split_forward<float>(__half2float(((const __half*)w)[idx]), false, iw, d); break; }
+    case WK_BF16: { float d; split_forward<float>(__bfloat162float(((const __nv_bfloat16*)w)[idx]), false, iw, d); break; }
+    default:
+        if (qkind == TS_QW_U8) iw = (long long)((const uint8_t*)w)[idx] - wzp;
+        else if (qkind == TS_QW_I8) iw = (long long)((const int8_t*)w)[idx] - wzp;
+        else iw = (long long)((const int32_t*)w)[idx] - wzp;
+    }
+    return iw;
+}
+
+// ------------------------------------------------------------------------------------------
 // Shared-memory vector loads as opaque instructions.  Written as plain C++ (`*(const uint4*)p`) the
 // compiler narrows a 128-bit load to the words a misaligned window actually uses (LDS.32 + LDS.64 ...),
 // and those narrower loads are 16-byte strided across a warp: 4-way bank conflicts (measured with ncu:
@@ -343,5 +365,20 @@ int check_launch();               // cudaGetLastError -> ts_status
 // cudaFuncAttributeMaxDynamicSharedMemorySize >= bytes for `func` on the current device; the attribute call is
 // made only when a kernel needs more than it was last given (not on every launch)
 bool ensure_dynamic_smem(const void* func, size_t bytes);
+
+#ifdef __CUDACC__
+// One launch of a kernel with `smem` bytes of dynamic shared memory, counted and checked.  pdl: programmatic dependent
+// launch (a plain launch where that is refused) -- only for kernels that call pdl_wait() before touching global memory.
+template <typename... KArgs, typename... Args>
+int launch_persistent(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, bool pdl, Args... args) {
+    if (!ensure_dynamic_smem((const void*)kernel, smem)) return check_launch();
+    if (!pdl || launch_pdl(kernel, grid, block, smem, stream, args...) != cudaSuccess) {
+        if (pdl) (void)cudaGetLastError();
+        kernel<<<grid, block, smem, stream>>>(args...);
+    }
+    note_launch();
+    return check_launch();
+}
+#endif
 
 }  // namespace ts

@@ -58,19 +58,7 @@ TS_D void flat_shift(const FArgs& a, long long c, int& sr, int& scb) {
     for (int lev = 0; lev < 2; ++lev) {
         const int ax = lev - (2 - a.dim);
         if (ax < 0) continue;
-        const long long idx = c * a.dim + ax;
-        long long iw = 0;
-        switch (a.wk) {
-        case WK_F32: { float d; split_forward<float>(((const float*)a.w)[idx], false, iw, d); break; }
-        case WK_F64: { double d; split_forward<double>(((const double*)a.w)[idx], false, iw, d); break; }
-        case WK_F16: { float d; split_forward<float>(__half2float(((const __half*)a.w)[idx]), false, iw, d); break; }
-        case WK_BF16: { float d; split_forward<float>(__bfloat162float(((const __nv_bfloat16*)a.w)[idx]), false, iw, d); break; }
-        default:
-            if (a.qkind == TS_QW_U8) iw = (long long)((const uint8_t*)a.w)[idx] - a.wzp;
-            else if (a.qkind == TS_QW_I8) iw = (long long)((const int8_t*)a.w)[idx] - a.wzp;
-            else iw = (long long)((const int32_t*)a.w)[idx] - a.wzp;
-        }
-        s[lev] = reduce_shift(iw, a.g.S[ax], TS_PAD_ZEROS);      // |s| <= len + 1
+        s[lev] = reduce_shift(sparse_shift(a.w, a.wk, a.qkind, a.wzp, c * a.dim + ax), a.g.S[ax], TS_PAD_ZEROS);      // |s| <= len + 1
     }
     sr = s[0];
     scb = s[1] * a.es;
@@ -268,8 +256,6 @@ __global__ void __launch_bounds__(512, 1) k_flat_gather_wp(const __grid_constant
     }
 }
 
-long long round_up(long long v, long long q) { return (v + q - 1) / q * q; }
-
 }  // namespace
 
 FlatPlan plan_flat(const Geo& g, int esize, bool dense_x, const void* x, const void* y, int sm_count, bool forced) {
@@ -343,15 +329,7 @@ int flat_gather(const Geo& g, const FlatPlan& p, int wk, const void* x, void* y,
     a.d_Lb = make_fastdiv((unsigned)a.Lb);
     a.table = p.n_per_unit;
     a.d_C = make_fastdiv((unsigned)g.C);
-    if (a.table) {
-        if (!ensure_dynamic_smem((const void*)k_flat_gather_wp, p.smem_bytes)) return check_launch();
-        k_flat_gather_wp<<<p.grid, (p.warps + 1) * 32, p.smem_bytes, s>>>(a);
-    } else {
-        if (!ensure_dynamic_smem((const void*)k_flat_gather, p.smem_bytes)) return check_launch();
-        k_flat_gather<<<p.grid, (p.warps + 1) * 32, p.smem_bytes, s>>>(a);
-    }
-    note_launch();
-    return check_launch();
+    return launch_persistent(a.table ? k_flat_gather_wp : k_flat_gather, p.grid, (p.warps + 1) * 32, p.smem_bytes, s, false, a);
 }
 
 }  // namespace ts

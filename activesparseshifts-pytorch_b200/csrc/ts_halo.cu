@@ -102,10 +102,6 @@ TS_D UnitShift compute_unit_shift(const HArgs& a, long long c) {
 // computed once per CTA into shared memory (a few hundred dependent instructions per channel otherwise paid per unit by
 // the single producer thread); a unit then costs one 36-byte read
 TS_D UnitShift unit_shift(const HArgs& a, const UnitShift* tbl, long long c) { return a.table ? tbl[c] : compute_unit_shift(a, c); }
-TS_D void decode_unit(const HArgs& a, int u, int& c, int& chunk) {
-    if (a.unit_order) { chunk = (int)fdiv((unsigned)u, a.d_C); c = u - chunk * (int)a.g.C; }
-    else { c = (int)fdiv((unsigned)u, a.d_chunks); chunk = u - c * a.chunks; }
-}
 
 // Where a unit's windows sit inside the tiles, and whether they fit the halo.
 struct UnitGeom {
@@ -1170,14 +1166,8 @@ __global__ void __launch_bounds__(MAXT, 1) k_halo(const __grid_constant__ HArgs 
     body.template run_class<4>(smem, ring, uo, u, ur);
 }
 
-long long round_up(long long v, long long q) { return (v + q - 1) / q * q; }
-
-template <class K>
-int launch(K kernel, const HArgs& a, const HaloPlan& p, cudaStream_t s) {
-    if (!ensure_dynamic_smem((const void*)kernel, p.smem_bytes)) return check_launch();
-    kernel<<<p.grid, (p.warps + 1 + (a.need_fix ? a.nfix : 0)) * 32, p.smem_bytes, s>>>(a);
-    note_launch();
-    return check_launch();
+int launch(void (*kernel)(HArgs), const HArgs& a, const HaloPlan& p, cudaStream_t s) {
+    return launch_persistent(kernel, p.grid, (p.warps + 1 + (a.need_fix ? a.nfix : 0)) * 32, p.smem_bytes, s, false, a);
 }
 
 bool make_args(const Geo& g, const HaloPlan& p, int mode, int active, int pool, const void* x, const void* grad, void* out, const void* w,
@@ -1185,12 +1175,13 @@ bool make_args(const Geo& g, const HaloPlan& p, int mode, int active, int pool, 
     HArgs& a = *o;
     memset(&a, 0, sizeof(a));
     const int d = g.dim;
+    const Levels lv(g);
     a.g = g;
     a.x = (const float*)x; a.grad = (const float*)grad; a.out = (float*)out; a.w = (const float*)w; a.partials = partials;
     a.mode = mode; a.active = active; a.dim = d;
-    a.A = d == 3 ? g.S[0] : 1;   a.OA = d == 3 ? g.OS[0] : 1;   a.lbA = d == 3 ? g.lb[0] : 0;
-    a.B = g.S[d - 2];            a.OB = g.OS[d - 2];            a.lbB = g.lb[d - 2];
-    a.L = g.S[d - 1];            a.OL = g.OS[d - 1];            a.lbL = g.lb[d - 1];
+    a.A = lv.A;    a.OA = lv.OA;    a.lbA = lv.lbA;
+    a.B = lv.B;    a.OB = lv.OB;    a.lbB = lv.lbB;
+    a.L = lv.L;    a.OL = lv.OL;    a.lbL = lv.lbL;
     a.IA = mode == 2 ? a.A : a.OA;
     a.IB = mode == 2 ? a.B : a.OB;
     a.IG = (mode == 2 ? a.L : a.OL) / 4;
@@ -1247,8 +1238,8 @@ HaloPlan plan_halo(const Geo& g, int mode, int active, int dtype, bool dense_x, 
     if (g.N * g.C == 0 || g.in_plane == 0 || g.out_plane == 0) return p;
     for (int ax = 0; ax < d; ++ax)
         if (g.S[ax] < 2 || g.OS[ax] < 2) return p;        // a size-1 axis ignores its shift (shifts_kernels.h:40-50): other families
-    const int B = g.S[d - 2], L = g.S[d - 1];
-    const int OB = g.OS[d - 2], OL = g.OS[d - 1];
+    const Levels lv(g);
+    const int B = lv.B, L = lv.L, OB = lv.OB, OL = lv.OL;
     if (L % 4 || OL % 4) return p;
     if (pool_bwd && (mode != 2 || d != 2 || OL % 8)) return p;      // pooled rows of a multiple of 16 bytes (TMA)
     if (((uintptr_t)x & 15) || ((uintptr_t)out & 15) || ((uintptr_t)grad & 15)) return p;
@@ -1271,8 +1262,7 @@ HaloPlan plan_halo(const Geo& g, int mode, int active, int dtype, bool dense_x, 
     if (pool_bwd) p.tile_v = p.tile_p;
     const long long per_image = (long long)p.tile_x + p.tile_g + p.tile_v;
     const int IB = mode == 2 ? B : OB, IG = (mode == 2 ? L : OL) / 4;
-    int GP = IG;
-    if (IG % 8 != 0 && (double)IG / (double)((IG + 7) / 8 * 8) >= 0.85) GP = (IG + 7) / 8 * 8;
+    const int GP = padded_groups(IG);
     const int img_pairs = (IB + 1) / 2 * GP;
     const int max_nt = MAXT - 64 - (pool_bwd ? 96 : 0);    // producer warp + fixer warp(s)
     const long long table_bytes = (g.C <= TABLE_MAX_C ? g.C * 36 : 0) + ((g.pad != TS_PAD_ZEROS || pool_bwd) ? 2 * FIXCAP * 4 : 0)      // + the fixer's cell lists
@@ -1314,21 +1304,13 @@ HaloPlan plan_halo(const Geo& g, int mode, int active, int dtype, bool dense_x, 
     }
     if (t.halo_warps > 0 && d != 3) warps = t.halo_warps < max_nt / 32 ? t.halo_warps : max_nt / 32;
     if (warps < 1) warps = 1;
-    const long long planes = g.N * g.C;
-    long long npu = t.chunk_planes > 0 ? t.chunk_planes : pick_unit_images(g.N, g.C, np, sm_count, mode == 2 ? 0.4 : 0.1);
-    (void)planes;
-    npu = (npu / np) * np;
-    if (npu < np) npu = np;
-    if (npu > g.N) npu = g.N;
-    const long long chunks = (g.N + npu - 1) / npu;
-    const long long units = chunks * g.C;
-    if (units > 0x7fffffffLL || chunks * warps > 0x7fffffffLL) return p;
+    const UnitPlan up = plan_units(np, t.chunk_planes > 0 ? t.chunk_planes : pick_unit_images(g.N, g.C, np, sm_count, mode == 2 ? 0.4 : 0.1),
+                                   g.N, g.C, sm_count, warps);
+    if (!up.ok) return p;
     p.ok = true;
     p.np = (int)np; p.GP = GP; p.positions = (int)pairs; p.ncol = 1;
     p.stages = (int)stages; p.stage_stride = (int)stride_of(np); p.warps = warps;
-    p.n_per_unit = (int)npu; p.units = (int)units;
-    p.grid = (int)(units < sm_count ? units : sm_count);
-    p.slots = (int)(chunks * warps);
+    p.n_per_unit = up.n_per_unit; p.units = up.units; p.grid = up.grid; p.slots = up.slots;
     p.smem_bytes = (size_t)(stages * stride_of(np) + 24 * stages + 64 + table_bytes);
     return p;
 }

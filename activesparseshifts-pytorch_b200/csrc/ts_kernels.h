@@ -7,9 +7,6 @@ namespace ts {
 constexpr int SMEM_LIMIT = 232448;   // 227 KB opt-in dynamic shared memory per CTA on sm_100
 constexpr int TABLE_MAX_C = 512;     // channels whose shift parameters a CTA tabulates in shared memory (TMA, staged, halo, flat)
 
-// How the integer shifts are obtained in the sparse/quantized gather kernels.
-enum { WK_F32 = 0, WK_F64 = 1, WK_F16 = 2, WK_BF16 = 3, WK_QUANT = 4 };
-
 template <int WK> struct WType;
 template <> struct WType<WK_F32> { using type = float; };
 template <> struct WType<WK_F64> { using type = double; };
@@ -26,6 +23,45 @@ TS_D void load_int_shifts(const void* __restrict__ w, int qkind, long long wzp, 
 #pragma unroll
         for (int a = 0; a < DIM; ++a) sx[a] = p.sx[a];
     }
+}
+
+// ---- planning helpers of the persistent families (TMA, staged, halo, flat) ----------------------
+inline long long round_up(long long v, long long q) { return (v + q - 1) / q * q; }
+
+// Padded row length of an item index space with `n` 16-byte groups per row: a multiple of 8 keeps every quarter-warp inside
+// one row (conflict-free 128-bit shared-memory loads) -- used when it idles <= 15 % of the lanes.
+inline int padded_groups(int n) { return n % 8 != 0 && (double)n / (double)((n + 7) / 8 * 8) >= 0.85 ? (n + 7) / 8 * 8 : n; }
+
+// Extents per LEVEL (0 slab, 1 row, 2 column) of a geometry: input A, B, L, output OA, OB, OL and the crop origin
+// lbA, lbB, lbL.  Absent levels have extent 1 and origin 0.
+struct Levels {
+    int A, B, L, OA, OB, OL, lbA, lbB, lbL;
+    explicit Levels(const Geo& g) {
+        const int d = g.dim;
+        A = d == 3 ? g.S[0] : 1;        OA = d == 3 ? g.OS[0] : 1;      lbA = d == 3 ? g.lb[0] : 0;
+        B = d >= 2 ? g.S[d - 2] : 1;    OB = d >= 2 ? g.OS[d - 2] : 1;  lbB = d >= 2 ? g.lb[d - 2] : 0;
+        L = g.S[d - 1];                 OL = g.OS[d - 1];               lbL = g.lb[d - 1];
+    }
+};
+
+// Work units of a persistent kernel: (channel, chunk of `n_per_unit` images of the batch), dealt to `grid` CTAs; each of the
+// `warps` consumer warps writes one grad_weight partial per chunk (`slots`).  `npu` is the family's proposed images per unit,
+// rounded here to a multiple of the `np` images of one stage.  ok = false: a count overflows 32 bits.
+struct UnitPlan { bool ok; int n_per_unit, units, grid, slots; };
+inline UnitPlan plan_units(long long np, long long npu, long long N, long long C, long long grid_max, int warps) {
+    UnitPlan u = {false, 0, 0, 0, 0};
+    npu = (npu / np) * np;
+    if (npu < np) npu = np;
+    if (npu > N) npu = N;
+    const long long chunks = (N + npu - 1) / npu;
+    const long long units = chunks * C;
+    if (units > 0x7fffffffLL || chunks * warps > 0x7fffffffLL) return u;
+    u.ok = true;
+    u.n_per_unit = (int)npu;
+    u.units = (int)units;
+    u.grid = (int)(units < grid_max ? units : grid_max);
+    u.slots = (int)(chunks * warps);
+    return u;
 }
 
 // Images per work unit (a multiple of `np`, the images of one stage).  A unit has a fixed cost (parameter fetch, the
@@ -84,7 +120,6 @@ struct Tuning {
     int ctas_per_sm;   // persistent CTAs per SM
     int chunk_planes;  // planes of one channel per work unit (0 = auto)
     int tma_stages;    // ring depth of the TMA-tensor kernels (0 = auto)
-    int tma_ctas_per_sm;
     int tma_warps;     // consumer warps of the TMA-tensor arithmetic kernels
     int use_tma;       // 0: the automatic path choice never picks the TMA-tensor family
     int tma_stage_kb;  // target bytes per stage of the TMA-tensor kernels (0 = auto)

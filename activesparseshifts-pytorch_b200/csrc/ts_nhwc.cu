@@ -620,12 +620,8 @@ int ring_launch(const Geo& g, const RingPlan& pl, const void* x, void* y, uint8_
         ring_emulate<PAD>(g, pl, (const uint8_t*)x, (uint8_t*)y, fill, w, qkind, wzp);
         return TS_OK;
     }
-    // per launch, like the other families: the attribute belongs to the current device's copy of the kernel
-    if (cudaFuncSetAttribute(k_gather_nhwc_ring<PAD>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl.smem_bytes) != cudaSuccess)
-        return check_launch();
-    k_gather_nhwc_ring<PAD><<<pl.grid, RING_THREADS, pl.smem_bytes, s>>>(g, pl, (const uint8_t*)x, (uint8_t*)y, fill, w, qkind, wzp);
-    note_launch();
-    return check_launch();
+    return launch_persistent(k_gather_nhwc_ring<PAD>, pl.grid, RING_THREADS, pl.smem_bytes, s, false, g, pl, (const uint8_t*)x, (uint8_t*)y,
+                             fill, w, qkind, wzp);
 }
 
 int ring_run(const Geo& g, const RingPlan& pl, const void* x, void* y, uint8_t fill, const void* w, int qkind, long long wzp,
@@ -964,10 +960,8 @@ bool plan_rows(const Geo& g, int esize, const void* x, const void* y, int sm_cou
 template <int PAD, int CB>
 int rows_launch(const Geo& g, const RowsPlan& pl, const void* x, void* y, uint8_t fill, const void* w, int qkind, long long wzp,
                 cudaStream_t s) {
-    if (!ensure_dynamic_smem((const void*)k_gather_nhwc_rows<PAD, CB>, pl.smem_bytes)) return check_launch();
-    k_gather_nhwc_rows<PAD, CB><<<pl.grid, (pl.W + 1) * 32, pl.smem_bytes, s>>>(g, pl, (const uint8_t*)x, (uint8_t*)y, fill, w, qkind, wzp);
-    note_launch();
-    return check_launch();
+    return launch_persistent(k_gather_nhwc_rows<PAD, CB>, pl.grid, (pl.W + 1) * 32, pl.smem_bytes, s, false, g, pl, (const uint8_t*)x,
+                             (uint8_t*)y, fill, w, qkind, wzp);
 }
 template <int PAD>
 int rows_run_c(const Geo& g, const RowsPlan& pl, const void* x, void* y, uint8_t fill, const void* w, int qkind, long long wzp, cudaStream_t s) {

@@ -406,22 +406,17 @@ bool plan_cl(const Geo& g, int dtype, bool backward, int sm_count, ClPlan* out) 
 template <typename ST, int PAD>
 int cl_forward_t(const Geo& g, const ClPlan& pl, int active, const void* x, const void* w, void* y, cudaStream_t s) {
     auto k = active ? k_cl_forward<ST, PAD, true> : k_cl_forward<ST, PAD, false>;
-    if (!ensure_dynamic_smem((const void*)k, pl.smem_bytes)) return check_launch();
     const dim3 grid((unsigned)(g.N * pl.segs), (unsigned)pl.slices, 1);
-    k<<<grid, CL_FWD_THREADS, pl.smem_bytes, s>>>(g, pl, (const ST*)x, (const ST*)w, (ST*)y);
-    note_launch();
-    return check_launch();
+    return launch_persistent(k, grid, CL_FWD_THREADS, pl.smem_bytes, s, false, g, pl, (const ST*)x, (const ST*)w, (ST*)y);
 }
 
 template <typename ST, int PAD>
 int cl_backward_t(const Geo& g, const ClPlan& pl, int active, const void* grad, const void* x, const void* w, void* gi,
                   double* partials, cudaStream_t s) {
     auto k = active ? k_cl_backward<ST, PAD, true> : k_cl_backward<ST, PAD, false>;
-    if (!ensure_dynamic_smem((const void*)k, pl.smem_bytes)) return check_launch();
     const dim3 grid((unsigned)(g.N * pl.segs), (unsigned)pl.slices, 1);
-    k<<<grid, CL_BWD_THREADS, pl.smem_bytes, s>>>(g, pl, (const ST*)grad, (const ST*)x, (const ST*)w, (ST*)gi, partials);
-    note_launch();
-    return check_launch();
+    return launch_persistent(k, grid, CL_BWD_THREADS, pl.smem_bytes, s, false, g, pl, (const ST*)grad, (const ST*)x, (const ST*)w, (ST*)gi,
+                             partials);
 }
 
 template <typename ST>

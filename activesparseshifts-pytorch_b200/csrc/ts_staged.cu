@@ -85,16 +85,7 @@ TS_D UnitShift unit_shift(const SArgs& a, long long c) {
         const long long idx = c * dim + ax;
         long long iw = 0;
         if (a.mode == 0) {
-            switch (a.wk) {
-            case WK_F32: { float d; split_forward<float>(((const float*)a.w)[idx], false, iw, d); break; }
-            case WK_F64: { double d; split_forward<double>(((const double*)a.w)[idx], false, iw, d); break; }
-            case WK_F16: { float d; split_forward<float>(__half2float(((const __half*)a.w)[idx]), false, iw, d); break; }
-            case WK_BF16: { float d; split_forward<float>(__bfloat162float(((const __nv_bfloat16*)a.w)[idx]), false, iw, d); break; }
-            default:
-                if (a.qkind == TS_QW_U8) iw = (long long)((const uint8_t*)a.w)[idx] - a.wzp;
-                else if (a.qkind == TS_QW_I8) iw = (long long)((const int8_t*)a.w)[idx] - a.wzp;
-                else iw = (long long)((const int32_t*)a.w)[idx] - a.wzp;
-            }
+            iw = sparse_shift(a.w, a.wk, a.qkind, a.wzp, idx);
         } else {
             float wv;
             if (a.wk == WK_F16) wv = __half2float(((const __half*)a.w)[idx]);
@@ -1560,15 +1551,9 @@ __global__ void __launch_bounds__(MAXT_ARITH, 1) k_staged_backward(const __grid_
     consumer_loop(a, smem, full, empty, lane, body);
 }
 
-template <class K>
-int launch(K kernel, const SArgs& a, const StagedPlan& p, cudaStream_t s) {
-    if (!ensure_dynamic_smem((const void*)kernel, p.smem_bytes)) return check_launch();
-    kernel<<<p.grid, (p.warps + 1) * 32, p.smem_bytes, s>>>(a);
-    note_launch();
-    return check_launch();
+int launch(void (*kernel)(SArgs), const SArgs& a, const StagedPlan& p, cudaStream_t s) {
+    return launch_persistent(kernel, p.grid, (p.warps + 1) * 32, p.smem_bytes, s, false, a);
 }
-
-long long round_up(long long v, long long q) { return (v + q - 1) / q * q; }
 
 SArgs make_args(const Geo& g, const StagedPlan& p, int mode, int active, int es) {
     SArgs a;
@@ -1577,10 +1562,10 @@ SArgs make_args(const Geo& g, const StagedPlan& p, int mode, int active, int es)
     a.es = es;
     a.mode = mode;
     a.active = active;
-    const int d = g.dim;
-    a.A = d == 3 ? g.S[0] : 1;        a.OA = d == 3 ? g.OS[0] : 1;      a.lbA = d == 3 ? g.lb[0] : 0;
-    a.B = d >= 2 ? g.S[d - 2] : 1;    a.OB = d >= 2 ? g.OS[d - 2] : 1;  a.lbB = d >= 2 ? g.lb[d - 2] : 0;
-    a.L = g.S[d - 1];                 a.OL = g.OS[d - 1];               a.lbL = g.lb[d - 1];
+    const Levels lv(g);
+    a.A = lv.A;    a.OA = lv.OA;    a.lbA = lv.lbA;
+    a.B = lv.B;    a.OB = lv.OB;    a.lbB = lv.lbB;
+    a.L = lv.L;    a.OL = lv.OL;    a.lbL = lv.lbL;
     a.IA = mode == 2 ? a.A : a.OA;
     a.IB = mode == 2 ? a.B : a.OB;
     a.VB = p.vec_bytes;
@@ -1626,9 +1611,10 @@ StagedPlan plan_staged(const Geo& g, int mode, int active, int esize, int dtype,
     }
     if (g.N >= (1ll << 31) || g.C >= (1ll << 31)) return p;
     const int d = g.dim;
-    const int A = d == 3 ? g.S[0] : 1, OA = d == 3 ? g.OS[0] : 1;
-    const long long B = d >= 2 ? g.S[d - 2] : 1, OB = d >= 2 ? g.OS[d - 2] : 1;
-    const long long Lb = (long long)g.S[d - 1] * esize, OLb = (long long)g.OS[d - 1] * esize;
+    const Levels lv(g);
+    const int A = lv.A, OA = lv.OA;
+    const long long B = lv.B, OB = lv.OB;
+    const long long Lb = (long long)lv.L * esize, OLb = (long long)lv.OL * esize;
     int vb = 0;
     if (mode == 0) {
         for (int cand : {16, 8, 4})
@@ -1697,10 +1683,7 @@ StagedPlan plan_staged(const Geo& g, int mode, int active, int esize, int dtype,
     }
     if (np * per_image >= (1 << 20)) return p;                // mbarrier tx-count range
 
-    // padded row length of the item index space (see ts_tma.cu)
-    const int gpr = (int)((mode == 2 ? Lb : OLb) / vb);
-    int GP = gpr;
-    if (gpr % 8 != 0 && (double)gpr / (double)((gpr + 7) / 8 * 8) >= 0.85) GP = (gpr + 7) / 8 * 8;
+    const int GP = padded_groups((int)((mode == 2 ? Lb : OLb) / vb));
     const long long img_items = TA * IB * GP;
     if (np * img_items >= 0x7fffffffLL) return p;
     if ((long long)xs * slab_x * np >= 0x7fffffffLL) return p;
@@ -1714,15 +1697,11 @@ StagedPlan plan_staged(const Geo& g, int mode, int active, int esize, int dtype,
         if (npu < 4 * np) npu = 4 * np;
         while (npu > np && ((g.N + npu - 1) / npu) * g.C < 8 * grid_max) npu -= np;
     }
-    npu = (npu / np) * np;
-    if (npu < np) npu = np;
-    if (npu > g.N) npu = g.N;
-    const long long chunks = (g.N + npu - 1) / npu;
-    const long long units = chunks * g.C;
     int warps = t.warps;
     const int max_warps = ((mode == 0 ? MAXT_GATHER : MAXT_ARITH) / 32) / ctas - 1;
     if (warps > max_warps) warps = max_warps;
-    if (units > 0x7fffffffLL || chunks * warps > 0x7fffffffLL) return p;
+    const UnitPlan up = plan_units(np, npu, g.N, g.C, grid_max, warps);
+    if (!up.ok) return p;
 
     p.ok = true;
     p.vec_bytes = vb;
@@ -1730,10 +1709,10 @@ StagedPlan plan_staged(const Geo& g, int mode, int active, int esize, int dtype,
     p.stages = stages;
     p.stage_stride = (int)stride_of(np);
     p.warps = warps;
-    p.n_per_unit = (int)npu;
-    p.units = (int)units;
-    p.grid = (int)(units < grid_max ? units : grid_max);
-    p.slots = (int)(chunks * warps);
+    p.n_per_unit = up.n_per_unit;
+    p.units = up.units;
+    p.grid = up.grid;
+    p.slots = up.slots;
     p.ta = (int)TA;
     p.tiles = tiles;
     p.xs = xs; p.gvs = gvs; p.gis = gis;

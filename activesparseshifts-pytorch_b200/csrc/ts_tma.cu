@@ -152,16 +152,7 @@ TS_D UnitShift compute_unit_shift(const TArgs& a, long long c) {
         if (ax >= 0) {
             const long long idx = c * dim + ax;
             if (a.mode == 0) {
-                switch (a.wk) {
-                case WK_F32: { float d; split_forward<float>(((const float*)a.w)[idx], false, iw, d); break; }
-                case WK_F64: { double d; split_forward<double>(((const double*)a.w)[idx], false, iw, d); break; }
-                case WK_F16: { float d; split_forward<float>(__half2float(((const __half*)a.w)[idx]), false, iw, d); break; }
-                case WK_BF16: { float d; split_forward<float>(__bfloat162float(((const __nv_bfloat16*)a.w)[idx]), false, iw, d); break; }
-                default:
-                    if (a.qkind == TS_QW_U8) iw = (long long)((const uint8_t*)a.w)[idx] - a.wzp;
-                    else if (a.qkind == TS_QW_I8) iw = (long long)((const int8_t*)a.w)[idx] - a.wzp;
-                    else iw = (long long)((const int32_t*)a.w)[idx] - a.wzp;
-                }
+                iw = sparse_shift(a.w, a.wk, a.qkind, a.wzp, idx);
             } else {
                 float d;
                 if (a.mode == 1) split_forward<float>(((const float*)a.w)[idx], true, iw, d);
@@ -755,32 +746,24 @@ __global__ void __launch_bounds__(MAXT_TMA_ARITH, 1) k_tma_backward(const __grid
     consumer_loop(a, smem, full, empty, lane, body);
 }
 
-template <class K>
-int launch(K kernel, const TArgs& a, const TmaPlan& p, cudaStream_t s) {
-    if (!ensure_dynamic_smem((const void*)kernel, p.smem_bytes)) return check_launch();
-    if (launch_pdl(kernel, dim3(p.grid), dim3((p.warps + 1) * 32), p.smem_bytes, s, a) != cudaSuccess) {
-        (void)cudaGetLastError();
-        kernel<<<p.grid, (p.warps + 1) * 32, p.smem_bytes, s>>>(a);
-    }
-    note_launch();
-    return check_launch();
+// every TMA kernel calls pdl_wait() before it touches global memory
+int launch(void (*kernel)(TArgs), const TArgs& a, const TmaPlan& p, cudaStream_t s) {
+    return launch_persistent(kernel, p.grid, (p.warps + 1) * 32, p.smem_bytes, s, true, a);
 }
-
-long long round_up(long long v, long long q) { return (v + q - 1) / q * q; }
 
 // fills everything of TArgs that does not depend on pointers
 bool make_args(const Geo& g, const TmaPlan& p, int mode, int active, int es, TArgs* out) {
     TArgs& a = *out;
     memset(&a, 0, sizeof(a));
-    const int d = g.dim;
+    const Levels lv(g);
     a.g = g;
     a.es = es;
     a.vec = 16 / es;
     a.mode = mode;
     a.active = active;
-    a.OA = d == 3 ? g.OS[0] : 1;      a.lbA = d == 3 ? g.lb[0] : 0;
-    a.OB = d >= 2 ? g.OS[d - 2] : 1;  a.lbB = d >= 2 ? g.lb[d - 2] : 0;
-    a.OGR = g.OS[d - 1] / a.vec;      a.lbL = g.lb[d - 1];
+    a.OA = lv.OA;            a.lbA = lv.lbA;
+    a.OB = lv.OB;            a.lbB = lv.lbB;
+    a.OGR = lv.OL / a.vec;   a.lbL = lv.lbL;
     a.TA = p.ta; a.TB = p.tb; a.TG = p.tg;
     a.xa = p.xa; a.xb = p.xb;
     a.tiles_b = (a.OB + a.TB - 1) / a.TB;
@@ -851,8 +834,8 @@ TmaPlan plan_tma(const Geo& g, int mode, int active, int esize, int dtype, bool 
         for (int ax = 0; ax < d; ++ax)                   // itself (shifts_kernels.h:40-50), not the zero the copy engine would fill
             if (g.S[ax] == 1) return p;
     const int vec = 16 / esize;
-    const int L = g.S[d - 1], OL = g.OS[d - 1];
-    const int OB = d >= 2 ? g.OS[d - 2] : 1, OA = d == 3 ? g.OS[0] : 1;
+    const Levels lv(g);
+    const int L = lv.L, OL = lv.OL, OB = lv.OB, OA = lv.OA;
     if (((long long)L * esize) % 16 || ((long long)OL * esize) % 16) return p;   // global strides / output rows: 16-byte multiples
     if (((uintptr_t)x & 15) || ((uintptr_t)out & 15) || ((uintptr_t)grad & 15)) return p;
     if (g.N >= (1ll << 31) || g.C >= (1ll << 31)) return p;
@@ -919,21 +902,7 @@ TmaPlan plan_tma(const Geo& g, int mode, int active, int esize, int dtype, bool 
     if (stages < 2) return p;
     if (tx >= (1 << 20)) return p;                       // mbarrier tx-count range
 
-    const long long planes = g.N * g.C;
-    const long long grid_max = (long long)sm_count;
-    long long npu = t.chunk_planes > 0 ? t.chunk_planes : pick_unit_images(g.N, g.C, np, grid_max, mode == 2 ? 0.4 : 0.1);
-    npu = (npu / np) * np;
-    if (npu < np) npu = np;
-    if (npu > g.N) npu = g.N;
-    const long long chunks = (g.N + npu - 1) / npu;
-    const long long units = chunks * g.C;
-    if (units > 0x7fffffffLL) return p;
-    (void)planes;
-
-    // padded row length of the item index space: a multiple of 8 groups keeps every quarter-warp inside
-    // one box row (conflict-free 128-bit shared loads) -- used when it idles <= 15 % of the lanes
-    int GP = TG;
-    if (TG % 8 != 0 && (double)TG / (double)((TG + 7) / 8 * 8) >= 0.85) GP = (TG + 7) / 8 * 8;
+    const int GP = padded_groups(TG);
     const long long plane16 = g.C * (mode == 2 ? g.in_plane : g.out_plane) * esize / 16;
     if (np * plane16 >= 0x7fffffffLL || np * TA * TB * (long long)GP >= 0x7fffffffLL) return p;
     // consumer warps: fill the last pass over a stage's items as well as possible
@@ -956,7 +925,9 @@ TmaPlan plan_tma(const Geo& g, int mode, int active, int esize, int dtype, bool 
             if (eff(w) >= eff(best_all) - 1e-9) best_all = w;
         warps = eff(best) >= eff(best_all) - 0.08 ? best : best_all;
     }
-    if (chunks * warps > 0x7fffffffLL) return p;
+    const UnitPlan up = plan_units(np, t.chunk_planes > 0 ? t.chunk_planes : pick_unit_images(g.N, g.C, np, sm_count, mode == 2 ? 0.4 : 0.1),
+                                   g.N, g.C, sm_count, warps);
+    if (!up.ok) return p;
 
     p.ok = true;
     p.ta = (int)TA; p.tb = (int)TB; p.tg = TG; p.gp = GP;
@@ -967,11 +938,11 @@ TmaPlan plan_tma(const Geo& g, int mode, int active, int esize, int dtype, bool 
     p.tx_bytes = (int)tx;
     p.stages = (int)stages;
     p.stage_stride = (int)stride;
-    p.n_per_unit = (int)npu;
-    p.units = (int)units;
-    p.grid = (int)(units < grid_max ? units : grid_max);
+    p.n_per_unit = up.n_per_unit;
+    p.units = up.units;
+    p.grid = up.grid;
     p.warps = warps;
-    p.slots = (int)(chunks * warps);
+    p.slots = up.slots;
     p.smem_bytes = (size_t)(stages * stride + 16 * stages + 64 + table_bytes);
     return p;
 }
@@ -980,14 +951,13 @@ int tma_gather(const Geo& g, const TmaPlan& p, int wk, const void* x, void* y, i
                cudaStream_t s) {
     TArgs a;
     make_args(g, p, 0, 0, esize, &a);
-    const int d = g.dim;
+    const Levels lv(g);
     a.out = (unsigned char*)y;
     a.w = w;
     a.wk = wk;
     a.qkind = qkind;
     a.wzp = wzp;
-    if (!make_map(&a.map_x, x, esize, g.N, g.C, d == 3 ? g.S[0] : 1, d >= 2 ? g.S[d - 2] : 1, g.S[d - 1], (a.TG + 1) * a.vec, a.xb,
-                  a.xa, a.np))
+    if (!make_map(&a.map_x, x, esize, g.N, g.C, lv.A, lv.B, lv.L, (a.TG + 1) * a.vec, a.xb, a.xa, a.np))
         return TS_ERR_UNSUPPORTED;
     return a.TA > 1 ? launch(k_tma_gather<true>, a, p, s) : launch(k_tma_gather<false>, a, p, s);
 }
@@ -995,12 +965,11 @@ int tma_gather(const Geo& g, const TmaPlan& p, int wk, const void* x, void* y, i
 int tma_active_forward(const Geo& g, const TmaPlan& p, const void* x, const void* w, void* y, cudaStream_t s) {
     TArgs a;
     make_args(g, p, 1, 1, 4, &a);
-    const int d = g.dim;
+    const Levels lv(g);
     a.out = (unsigned char*)y;
     a.w = w;
-    if (!make_map(&a.map_x, x, 4, g.N, g.C, d == 3 ? g.S[0] : 1, d >= 2 ? g.S[d - 2] : 1, g.S[d - 1], (a.TG + 1) * 4, a.xb, a.xa, a.np))
-        return TS_ERR_UNSUPPORTED;
-    switch (d) {
+    if (!make_map(&a.map_x, x, 4, g.N, g.C, lv.A, lv.B, lv.L, (a.TG + 1) * 4, a.xb, a.xa, a.np)) return TS_ERR_UNSUPPORTED;
+    switch (g.dim) {
     case 1: return launch(k_tma_active_forward<1>, a, p, s);
     case 2: return launch(k_tma_active_forward<2>, a, p, s);
     default: return launch(k_tma_active_forward<3>, a, p, s);
@@ -1011,15 +980,15 @@ int tma_backward(const Geo& g, const TmaPlan& p, int active, const void* grad, c
                  double* partials, cudaStream_t s) {
     TArgs a;
     make_args(g, p, 2, active ? 1 : 0, 4, &a);
-    const int d = g.dim;
+    const Levels lv(g);
+    const int A = lv.A, B = lv.B, L = lv.L;
     a.out = (unsigned char*)gi;
     a.w = w;
     a.partials = partials;
-    const int A = d == 3 ? g.S[0] : 1, B = d >= 2 ? g.S[d - 2] : 1, L = g.S[d - 1];
     if (!make_map(&a.map_x, x, 4, g.N, g.C, A, B, L, (a.TG + 1) * 4, a.xb, a.xa, a.np)) return TS_ERR_UNSUPPORTED;
     if (!make_map(&a.map_gs, grad, 4, g.N, g.C, A, B, L, (a.TG + 1) * 4, a.TB, a.TA, a.np)) return TS_ERR_UNSUPPORTED;
     if (active && !make_map(&a.map_gb, grad, 4, g.N, g.C, A, B, L, (a.TG + 1) * 4, a.xb, a.xa, a.np)) return TS_ERR_UNSUPPORTED;
-    switch (d * 2 + (active ? 1 : 0)) {
+    switch (g.dim * 2 + (active ? 1 : 0)) {
     case 2: return launch(k_tma_backward<1, false>, a, p, s);
     case 3: return launch(k_tma_backward<1, true>, a, p, s);
     case 4: return launch(k_tma_backward<2, false>, a, p, s);

@@ -128,7 +128,7 @@ def test_geometry_validation(native):
     assert lib.ts_shift_backward_workspace_bytes(ct.byref(g), 0) >= 16
     assert lib.ts_set_tuning(b"stages=3,warps=8") == 0 and lib.ts_set_tuning(b"bogus=1") == 1
     # retired measurement-only knobs are rejected like unknown keys; one kept key of each family still parses
-    for key in (b"halo_split", b"halo_probe", b"halo_compact", b"no_table", b"no_pdl", b"flat_variant"):
+    for key in (b"halo_split", b"halo_probe", b"halo_compact", b"no_table", b"no_pdl", b"flat_variant", b"tma_ctas_per_sm"):
         assert lib.ts_set_tuning(key + b"=1") == 1, key
     for spec in (b"tma_stages=0", b"halo_stages=0", b"flat_stages=0", b"cl_rows=0", b"nhwc_variant=0"):
         assert lib.ts_set_tuning(spec) == 0, spec

@@ -77,6 +77,7 @@ static int make_geo(const ts_geometry* in, int padding, Geo* g) {
     if (in->N < 0 || in->C < 0) return TS_ERR_INVALID_ARGUMENT;
     g->dim = in->dim;
     g->pad = padding;
+    g->wf32 = 0;
     g->N = in->N;
     g->C = in->C;
     long long ip = 1, op = 1;
@@ -119,6 +120,19 @@ static int elem_size(int dtype) {
     }
     return 0;
 }
+
+// The dtype argument of the float entry points: the element type, possibly OR'd with TS_WEIGHTS_F32 (fp16 / bf16 x with fp32
+// weights and grad_weight; sets g->wf32).  -> the element type, or -1 for TS_WEIGHTS_F32 with any other element type.
+static int weights_f32(int dtype, Geo* g) {
+    if (!(dtype & TS_WEIGHTS_F32)) return dtype;
+    dtype &= ~TS_WEIGHTS_F32;
+    if (dtype != TS_F16 && dtype != TS_BF16) return -1;
+    g->wf32 = 1;
+    return dtype;
+}
+
+// grad_weight's type: the weights'
+static int gw_dtype(const Geo& g, int dtype) { return g.wf32 ? TS_F32 : dtype; }
 
 // Tuning knobs (ts_set_tuning): 0 = automatic, the planners pick per-mode defaults.
 Tuning& tuning() {
@@ -333,6 +347,7 @@ int ts_shift_forward(const ts_geometry* gin, int dtype, int padding, int active,
     Geo g;
     int rc = make_geo(gin, padding, &g);
     if (rc != TS_OK) return rc;
+    if ((dtype = weights_f32(dtype, &g)) < 0) return TS_ERR_INVALID_ARGUMENT;
     const int es = elem_size(dtype);
     if (!es) return TS_ERR_INVALID_ARGUMENT;
     if (g.N * g.C == 0 || g.out_plane == 0) return TS_OK;
@@ -343,14 +358,15 @@ int ts_shift_forward(const ts_geometry* gin, int dtype, int padding, int active,
     if ((rc = route(g, Call{active ? 1 : 0, active, es, dtype, 0ull, x, y, nullptr}, sms, &r)) != TS_OK) return rc;
     t_last_path = r.path;
     cudaStream_t s = (cudaStream_t)stream;
+    const int wk = g.wf32 ? WK_F32 : dtype;     // the weight kind of the gathers (the generic family reads g.wf32 itself)
     switch (r.path) {
     case TS_PATH_TMA:
-        return active ? tma_active_forward(g, r.tma, x, weights, y, s) : tma_gather(g, r.tma, dtype, x, y, es, weights, 0, 0, s);
+        return active ? tma_active_forward(g, r.tma, dtype, x, weights, y, s) : tma_gather(g, r.tma, wk, x, y, es, weights, 0, 0, s);
     case TS_PATH_HALO: return halo_active_forward(g, r.halo, x, weights, y, s);
-    case TS_PATH_FLAT: return flat_gather(g, r.flat, dtype, x, y, 0ull, es, weights, 0, 0, s);
+    case TS_PATH_FLAT: return flat_gather(g, r.flat, wk, x, y, 0ull, es, weights, 0, 0, s);
     case TS_PATH_STAGED:
         return active ? staged_active_forward(g, r.staged, dtype, x, weights, y, s)
-                      : staged_gather(g, r.staged, dtype, x, y, 0ull, es, weights, 0, 0, s);
+                      : staged_gather(g, r.staged, wk, x, y, 0ull, es, weights, 0, 0, s);
     }
     return active ? generic_active_forward(g, dtype, x, weights, y, s) : generic_gather(g, dtype, x, y, 0ull, es, weights, 0, 0, s);
 }
@@ -360,6 +376,7 @@ int ts_shift2d_avgpool2_forward(const ts_geometry* gin, int dtype, int padding, 
     Geo g;
     int rc = make_geo(gin, padding, &g);
     if (rc != TS_OK) return rc;
+    if ((dtype = weights_f32(dtype, &g)) < 0) return TS_ERR_INVALID_ARGUMENT;
     if (g.dim != 2 || dtype != TS_F32) return TS_ERR_UNSUPPORTED;
     if (g.N * g.C == 0 || g.out_plane == 0) return TS_OK;
     if (!x || !weights || !y_pooled) return TS_ERR_INVALID_ARGUMENT;
@@ -382,6 +399,8 @@ size_t ts_shift_backward_workspace_bytes(const ts_geometry* gin, int dtype) {
     if (last_dtype == dtype && last_epoch == epoch && !memcmp(&last_geo, gin, sizeof(ts_geometry))) return last_bytes;
     Geo g;
     if (make_geo(gin, 0, &g) != TS_OK) return 0;
+    const int et = weights_f32(dtype, &g);
+    if (et < 0) return 0;
     size_t bytes = 16;
     if (g.N * g.C != 0) {
         int sms = 148;
@@ -396,7 +415,7 @@ size_t ts_shift_backward_workspace_bytes(const ts_geometry* gin, int dtype) {
                         Geo gp = g;
                         gp.pad = pad;
                         Route r;
-                        if (plan(path, gp, Call{2, active, elem_size(dtype), dtype, 0ull, nullptr, nullptr, nullptr}, true, sms, true,
+                        if (plan(path, gp, Call{2, active, elem_size(et), et, 0ull, nullptr, nullptr, nullptr}, true, sms, true,
                                  pool != 0, &r) && r.slots > slots)
                             slots = r.slots;
                     }
@@ -406,12 +425,14 @@ size_t ts_shift_backward_workspace_bytes(const ts_geometry* gin, int dtype) {
     return bytes;
 }
 
-static int backward_impl(const ts_geometry* gin, int dtype, int padding, int active, const void* grad, const void* x,
+static int backward_impl(const ts_geometry* gin, const int dtype_arg, int padding, int active, const void* grad, const void* x,
                          const void* weights, void* grad_input, void* grad_weight, void* workspace, size_t workspace_bytes,
                          const ts_peer_group* peers, void* stream) {
     Geo g;
     int rc = make_geo(gin, padding, &g);
     if (rc != TS_OK) return rc;
+    const int dtype = weights_f32(dtype_arg, &g);
+    if (dtype < 0) return TS_ERR_INVALID_ARGUMENT;
     const int es = elem_size(dtype);
     if (!es) return TS_ERR_INVALID_ARGUMENT;
     cudaStream_t s = (cudaStream_t)stream;
@@ -419,12 +440,12 @@ static int backward_impl(const ts_geometry* gin, int dtype, int padding, int act
     if (!grad_weight) return TS_ERR_INVALID_ARGUMENT;
     if (g.N == 0 || g.in_plane == 0) {
         // an empty shard still takes part in the exchange: it contributes zeros
-        if (peers) return reduce_partials(g, dtype, nullptr, 0, grad_weight, peers, s);
-        const cudaError_t e = cudaMemsetAsync(grad_weight, 0, (size_t)(g.C * g.dim) * es, s);
+        if (peers) return reduce_partials(g, gw_dtype(g, dtype), nullptr, 0, grad_weight, peers, s);
+        const cudaError_t e = cudaMemsetAsync(grad_weight, 0, (size_t)(g.C * g.dim) * elem_size(gw_dtype(g, dtype)), s);
         return e == cudaSuccess ? TS_OK : cuda_fail(e);
     }
     if (!grad || !x || !weights || !grad_input) return TS_ERR_INVALID_ARGUMENT;
-    if (!workspace || ((uintptr_t)workspace & 15) || workspace_bytes < ts_shift_backward_workspace_bytes(gin, dtype))
+    if (!workspace || ((uintptr_t)workspace & 15) || workspace_bytes < ts_shift_backward_workspace_bytes(gin, dtype_arg))
         return TS_ERR_WORKSPACE;
     int sms = 0;
     if ((rc = sm_count(&sms)) != TS_OK) return rc;
@@ -433,12 +454,12 @@ static int backward_impl(const ts_geometry* gin, int dtype, int padding, int act
     t_last_path = r.path;
     double* partials = (double*)workspace;
     switch (r.path) {
-    case TS_PATH_TMA: rc = tma_backward(g, r.tma, active, grad, x, weights, grad_input, partials, s); break;
+    case TS_PATH_TMA: rc = tma_backward(g, r.tma, dtype, active, grad, x, weights, grad_input, partials, s); break;
     case TS_PATH_HALO: rc = halo_backward(g, r.halo, active, grad, x, weights, grad_input, partials, s); break;
     case TS_PATH_STAGED: rc = staged_backward(g, r.staged, dtype, active, grad, x, weights, grad_input, partials, s); break;
     default: rc = generic_backward(g, r.generic, dtype, active, grad, x, weights, grad_input, partials, s); break;
     }
-    return rc != TS_OK ? rc : reduce_partials(g, dtype, partials, r.slots, grad_weight, peers, s);
+    return rc != TS_OK ? rc : reduce_partials(g, gw_dtype(g, dtype), partials, r.slots, grad_weight, peers, s);
 }
 
 int ts_shift2d_avgpool2_backward(const ts_geometry* gin, int dtype, int padding, int active, const void* grad_pooled, const void* x,
@@ -447,7 +468,8 @@ int ts_shift2d_avgpool2_backward(const ts_geometry* gin, int dtype, int padding,
     Geo g;
     int rc = make_geo(gin, padding, &g);
     if (rc != TS_OK) return rc;
-    if (g.dim != 2 || dtype != TS_F32) return TS_ERR_UNSUPPORTED;
+    if (weights_f32(dtype, &g) < 0) return TS_ERR_INVALID_ARGUMENT;
+    if (g.dim != 2 || dtype != TS_F32) return TS_ERR_UNSUPPORTED;      // (fp32 only: a flagged dtype lands here too)
     if (g.N * g.C == 0 || g.in_plane == 0 || g.out_plane == 0) return TS_ERR_UNSUPPORTED;     // (empty tensors: the two-step path)
     if (!grad_pooled || !x || !weights || !grad_input || !grad_weight) return TS_ERR_INVALID_ARGUMENT;
     if (!workspace || ((uintptr_t)workspace & 15) || workspace_bytes < ts_shift_backward_workspace_bytes(gin, dtype))
@@ -484,7 +506,9 @@ int ts_shift_backward_allreduce(const ts_geometry* gin, int dtype, int padding, 
                                 const void* weights, void* grad_input, void* grad_weight, void* workspace, size_t workspace_bytes,
                                 const ts_peer_group* peers, void* stream) {
     if (!peers || !gin) return TS_ERR_INVALID_ARGUMENT;
-    const int rc = check_peers(gin, dtype, peers);
+    Geo flag;
+    if (weights_f32(dtype, &flag) < 0) return TS_ERR_INVALID_ARGUMENT;
+    const int rc = check_peers(gin, dtype & ~TS_WEIGHTS_F32, peers);
     if (rc != TS_OK) return rc;
     return backward_impl(gin, dtype, padding, active, grad, x, weights, grad_input, grad_weight, workspace, workspace_bytes, peers,
                          stream);
@@ -495,7 +519,7 @@ int ts_shift_forward_nhwc(const ts_geometry* gin, int dtype, int padding, int ac
     Geo g;
     int rc = make_geo(gin, padding, &g);
     if (rc != TS_OK) return rc;
-    if (!elem_size(dtype)) return TS_ERR_INVALID_ARGUMENT;
+    if ((dtype = weights_f32(dtype, &g)) < 0 || !elem_size(dtype)) return TS_ERR_INVALID_ARGUMENT;
     if (g_forced_path.load() != TS_PATH_NONE) return TS_ERR_UNSUPPORTED;      // a forced family: callers take the planar path
     if (g.N * g.C == 0 || g.out_plane == 0) return TS_ERR_UNSUPPORTED;
     if (!x || !weights || !y) return TS_ERR_INVALID_ARGUMENT;
@@ -508,7 +532,7 @@ int ts_shift_forward_nhwc(const ts_geometry* gin, int dtype, int padding, int ac
 
 size_t ts_shift_backward_nhwc_workspace_bytes(const ts_geometry* gin, int dtype) {
     Geo g;
-    if (make_geo(gin, 0, &g) != TS_OK) return 0;
+    if (make_geo(gin, 0, &g) != TS_OK || (dtype = weights_f32(dtype, &g)) < 0) return 0;
     int sms = 148;
     sm_count(&sms);
     return cl_backward_workspace_bytes(g, dtype, sms);
@@ -520,7 +544,7 @@ int ts_shift_backward_nhwc(const ts_geometry* gin, int dtype, int padding, int a
     Geo g;
     int rc = make_geo(gin, padding, &g);
     if (rc != TS_OK) return rc;
-    if (!elem_size(dtype)) return TS_ERR_INVALID_ARGUMENT;
+    if ((dtype = weights_f32(dtype, &g)) < 0 || !elem_size(dtype)) return TS_ERR_INVALID_ARGUMENT;
     if (peers && (rc = check_peers(gin, dtype, peers)) != TS_OK) return rc;
     if (g_forced_path.load() != TS_PATH_NONE) return TS_ERR_UNSUPPORTED;
     if (g.N * g.C == 0 || g.in_plane == 0) return TS_ERR_UNSUPPORTED;        // empty shards: the planar path (zeros / exchange)
@@ -531,7 +555,7 @@ int ts_shift_backward_nhwc(const ts_geometry* gin, int dtype, int padding, int a
     cudaStream_t s = (cudaStream_t)stream;
     int slots = 0;
     rc = cl_backward(g, dtype, active, grad, x, weights, grad_input, (double*)workspace, workspace_bytes, sms, &slots, s);
-    if (rc == TS_OK) rc = reduce_partials(g, dtype, (double*)workspace, slots, grad_weight, peers, s);
+    if (rc == TS_OK) rc = reduce_partials(g, gw_dtype(g, dtype), (double*)workspace, slots, grad_weight, peers, s);
     if (rc == TS_OK) t_last_path = TS_PATH_NHWC;
     return rc;
 }

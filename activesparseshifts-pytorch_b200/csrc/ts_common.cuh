@@ -27,6 +27,7 @@ namespace ts {
 // Geometry handed to kernels by value.
 struct Geo {
     int dim, pad;
+    int wf32;            // weights are fp32 whatever the element type (TS_WEIGHTS_F32 with fp16 / bf16 x)
     long long N, C;
     int S[3];            // input sizes
     int OS[3];           // output sizes (rb - lb)
@@ -230,6 +231,16 @@ template <typename CT, int DIM> struct ShiftParams {
     CT d[3];       // fractional parts (0 for the sparse forward)
 };
 
+// Weight `idx` of a layer with `ST` elements, in the compute type: a 16-bit layer may carry fp32 weights (g.wf32), which are
+// split as they are -- never rounded to 16 bits first.
+template <typename ST>
+TS_D typename Elem<ST>::CT load_weight(const ST* __restrict__ w, long long idx, const Geo& g) {
+    if constexpr (sizeof(ST) == 2) {
+        if (g.wf32) return reinterpret_cast<const float*>(w)[idx];
+    }
+    return Elem<ST>::ld(w[idx]);
+}
+
 template <typename ST, int DIM>
 TS_D ShiftParams<typename Elem<ST>::CT, DIM> load_params(const ST* __restrict__ w, long long c, const Geo& g,
                                                          bool active, bool backward) {
@@ -238,7 +249,7 @@ TS_D ShiftParams<typename Elem<ST>::CT, DIM> load_params(const ST* __restrict__ 
     p.d[0] = p.d[1] = p.d[2] = (CT)0;
 #pragma unroll
     for (int a = 0; a < DIM; ++a) {
-        const CT wv = Elem<ST>::ld(w[c * DIM + a]);
+        const CT wv = load_weight<ST>(w, c * DIM + a, g);
         long long iw; CT dw;
         if (backward) split_backward<CT>(wv, active, iw, dw); else split_forward<CT>(wv, active, iw, dw);
         p.sx[a] = reduce_shift(iw, g.S[a], g.pad);
@@ -306,6 +317,113 @@ TS_D unsigned lds32(unsigned addr) {
     unsigned v;
     asm volatile("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(addr));
     return v;
+}
+
+// ------------------------------------------------------------------------------------------
+// 16-byte windows of staged boxes, shared by the staged and TMA families.  16-bit element types keep fp32 arithmetic: a
+// window is resolved with a compile-time word select plus a half-word shift, and the store rounds once (Pack::pack).
+// NW 32-bit words starting WS words into the aligned 16-byte group at byte offset `off` of `base`
+// (off is a multiple of 16).  Loads the second group only when the window needs it.
+template <int WS, int NW>
+TS_D void load_words(unsigned base, int off, unsigned* w) {
+    const uint4 A = lds128(base + off);
+    unsigned W[8] = {A.x, A.y, A.z, A.w, 0u, 0u, 0u, 0u};
+    if (WS + NW > 4) {
+        const uint4 B = lds128(base + off + 16);
+        W[4] = B.x; W[5] = B.y; W[6] = B.z; W[7] = B.w;
+    }
+#pragma unroll
+    for (int t = 0; t < NW; ++t) w[t] = W[(t + WS) & 7];
+}
+
+// Element-type traits of the arithmetic kernels: V elements per 16-byte item; a window of NV
+// elements spans words(NV) 32-bit words (one more than NV/2 for 16-bit types: half-word shift).
+template <typename ST> struct Pack;
+template <> struct Pack<float> {
+    static constexpr int V = 4;
+    static __host__ __device__ constexpr int words(int nv) { return nv; }
+    template <int NV> static TS_D void unpack(const unsigned* w, int, float* out) {
+#pragma unroll
+        for (int t = 0; t < NV; ++t) out[t] = __uint_as_float(w[t]);
+    }
+    template <int NV, int HS> static TS_D void unpack_c(const unsigned* w, float* out) {
+#pragma unroll
+        for (int t = 0; t < NV; ++t) out[t] = __uint_as_float(w[t]);
+    }
+    static TS_D uint4 pack(const float* o) {
+        return make_uint4(__float_as_uint(o[0]), __float_as_uint(o[1]), __float_as_uint(o[2]), __float_as_uint(o[3]));
+    }
+};
+template <> struct Pack<__nv_bfloat16> {
+    static constexpr int V = 8;
+    static __host__ __device__ constexpr int words(int nv) { return nv / 2 + 1; }
+    template <int NV> static TS_D void unpack(const unsigned* w, int hs, float* out) {
+#pragma unroll
+        for (int k = 0; k < (NV + 1) / 2; ++k) {
+            const unsigned v = __funnelshift_r(w[k], w[k + 1], hs);
+            out[2 * k] = __uint_as_float(v << 16);
+            if (2 * k + 1 < NV) out[2 * k + 1] = __uint_as_float(v & 0xffff0000u);
+        }
+    }
+    // compile-time half-word phase HS (0 / 16 bits): no funnel shift, one conversion per element
+    template <int NV, int HS> static TS_D void unpack_c(const unsigned* w, float* out) {
+#pragma unroll
+        for (int t = 0; t < NV; ++t) {
+            const int h = t + (HS ? 1 : 0);
+            out[t] = __uint_as_float((h & 1) ? (w[h >> 1] & 0xffff0000u) : (w[h >> 1] << 16));
+        }
+    }
+    static TS_D uint4 pack(const float* o) {
+        unsigned r[4];
+#pragma unroll
+        for (int k = 0; k < 4; ++k) {
+            const __nv_bfloat162 v = __floats2bfloat162_rn(o[2 * k], o[2 * k + 1]);
+            r[k] = *(const unsigned*)&v;
+        }
+        return make_uint4(r[0], r[1], r[2], r[3]);
+    }
+};
+template <> struct Pack<__half> {
+    static constexpr int V = 8;
+    static __host__ __device__ constexpr int words(int nv) { return nv / 2 + 1; }
+    template <int NV> static TS_D void unpack(const unsigned* w, int hs, float* out) {
+#pragma unroll
+        for (int k = 0; k < (NV + 1) / 2; ++k) {
+            const unsigned v = __funnelshift_r(w[k], w[k + 1], hs);
+            const float2 f = __half22float2(*(const __half2*)&v);
+            out[2 * k] = f.x;
+            if (2 * k + 1 < NV) out[2 * k + 1] = f.y;
+        }
+    }
+    template <int NV, int HS> static TS_D void unpack_c(const unsigned* w, float* out) {
+#pragma unroll
+        for (int t = 0; t < NV; ++t) {
+            const int h = t + (HS ? 1 : 0);
+            const __half2 v = *(const __half2*)&w[h >> 1];
+            out[t] = (h & 1) ? __high2float(v) : __low2float(v);
+        }
+    }
+    static TS_D uint4 pack(const float* o) {
+        unsigned r[4];
+#pragma unroll
+        for (int k = 0; k < 4; ++k) {
+            const __half2 v = __floats2half2_rn(o[2 * k], o[2 * k + 1]);
+            r[k] = *(const unsigned*)&v;
+        }
+        return make_uint4(r[0], r[1], r[2], r[3]);
+    }
+};
+
+
+// window of NV elements whose first element sits PH bytes (compile-time, a multiple of sizeof(ST)) into the
+// 16-byte group at shared address `group`: exactly the words the window touches are loaded, no run-time realignment
+template <typename ST, int PH, int NV>
+TS_D void load_window_c(unsigned group, float* out) {
+    constexpr int WS = PH >> 2, HS = (PH & 2) * 8;
+    constexpr int NW = sizeof(ST) == 4 ? NV : (NV + (HS ? 1 : 0) + 1) / 2;
+    unsigned w[NW];
+    load_words<WS, NW>(group, 0, w);
+    Pack<ST>::template unpack_c<NV, HS>(w, out);
 }
 #endif
 

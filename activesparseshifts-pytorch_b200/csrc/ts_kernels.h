@@ -174,8 +174,9 @@ TmaPlan plan_tma(const Geo& g, int mode, int active, int esize, int dtype, bool 
                  const void* out, const void* grad, int sm_count);
 int tma_gather(const Geo& g, const TmaPlan& p, int wk, const void* x, void* y, int esize, const void* w, int qkind, long long wzp,
                cudaStream_t s);
-int tma_active_forward(const Geo& g, const TmaPlan& p, const void* x, const void* w, void* y, cudaStream_t s);
-int tma_backward(const Geo& g, const TmaPlan& p, int active, const void* grad, const void* x, const void* w, void* gi,
+// dtype: TS_F32, or (2-D, fp32 weights: g.wf32) TS_F16 / TS_BF16
+int tma_active_forward(const Geo& g, const TmaPlan& p, int dtype, const void* x, const void* w, void* y, cudaStream_t s);
+int tma_backward(const Geo& g, const TmaPlan& p, int dtype, int active, const void* grad, const void* x, const void* w, void* gi,
                  double* partials, cudaStream_t s);
 
 // rank-5 tensor map over a dense [N][C][A][B][L] tensor, box {bl, bb, ba, 1, bn} (memoised per thread); `map` points to a

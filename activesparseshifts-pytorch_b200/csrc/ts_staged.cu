@@ -355,19 +355,6 @@ TS_D void strip_plan(const Interior& in, int images_x_slabs, int nt, int& R, int
 }
 
 // ---- window loads -----------------------------------------------------------------------------
-// NW 32-bit words starting WS words into the aligned 16-byte group at byte offset `off` of `base`
-// (off is a multiple of 16).  Loads the second group only when the window needs it.
-template <int WS, int NW>
-TS_D void load_words(unsigned base, int off, unsigned* w) {
-    const uint4 A = lds128(base + off);
-    unsigned W[8] = {A.x, A.y, A.z, A.w, 0u, 0u, 0u, 0u};
-    if (WS + NW > 4) {
-        const uint4 B = lds128(base + off + 16);
-        W[4] = B.x; W[5] = B.y; W[6] = B.z; W[7] = B.w;
-    }
-#pragma unroll
-    for (int t = 0; t < NW; ++t) w[t] = W[(t + WS) & 7];
-}
 template <int NW>
 TS_D void load_words_rt(unsigned base, int off, int ws, unsigned* w) {
     switch (ws) {
@@ -377,84 +364,6 @@ TS_D void load_words_rt(unsigned base, int off, int ws, unsigned* w) {
     default: load_words<3, NW>(base, off, w); break;
     }
 }
-
-// Element-type traits of the arithmetic kernels: V elements per 16-byte item; a window of NV
-// elements spans words(NV) 32-bit words (one more than NV/2 for 16-bit types: half-word shift).
-template <typename ST> struct Pack;
-template <> struct Pack<float> {
-    static constexpr int V = 4;
-    static __host__ __device__ constexpr int words(int nv) { return nv; }
-    template <int NV> static TS_D void unpack(const unsigned* w, int, float* out) {
-#pragma unroll
-        for (int t = 0; t < NV; ++t) out[t] = __uint_as_float(w[t]);
-    }
-    template <int NV, int HS> static TS_D void unpack_c(const unsigned* w, float* out) {
-#pragma unroll
-        for (int t = 0; t < NV; ++t) out[t] = __uint_as_float(w[t]);
-    }
-    static TS_D uint4 pack(const float* o) {
-        return make_uint4(__float_as_uint(o[0]), __float_as_uint(o[1]), __float_as_uint(o[2]), __float_as_uint(o[3]));
-    }
-};
-template <> struct Pack<__nv_bfloat16> {
-    static constexpr int V = 8;
-    static __host__ __device__ constexpr int words(int nv) { return nv / 2 + 1; }
-    template <int NV> static TS_D void unpack(const unsigned* w, int hs, float* out) {
-#pragma unroll
-        for (int k = 0; k < (NV + 1) / 2; ++k) {
-            const unsigned v = __funnelshift_r(w[k], w[k + 1], hs);
-            out[2 * k] = __uint_as_float(v << 16);
-            if (2 * k + 1 < NV) out[2 * k + 1] = __uint_as_float(v & 0xffff0000u);
-        }
-    }
-    // compile-time half-word phase HS (0 / 16 bits): no funnel shift, one conversion per element
-    template <int NV, int HS> static TS_D void unpack_c(const unsigned* w, float* out) {
-#pragma unroll
-        for (int t = 0; t < NV; ++t) {
-            const int h = t + (HS ? 1 : 0);
-            out[t] = __uint_as_float((h & 1) ? (w[h >> 1] & 0xffff0000u) : (w[h >> 1] << 16));
-        }
-    }
-    static TS_D uint4 pack(const float* o) {
-        unsigned r[4];
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-            const __nv_bfloat162 v = __floats2bfloat162_rn(o[2 * k], o[2 * k + 1]);
-            r[k] = *(const unsigned*)&v;
-        }
-        return make_uint4(r[0], r[1], r[2], r[3]);
-    }
-};
-template <> struct Pack<__half> {
-    static constexpr int V = 8;
-    static __host__ __device__ constexpr int words(int nv) { return nv / 2 + 1; }
-    template <int NV> static TS_D void unpack(const unsigned* w, int hs, float* out) {
-#pragma unroll
-        for (int k = 0; k < (NV + 1) / 2; ++k) {
-            const unsigned v = __funnelshift_r(w[k], w[k + 1], hs);
-            const float2 f = __half22float2(*(const __half2*)&v);
-            out[2 * k] = f.x;
-            if (2 * k + 1 < NV) out[2 * k + 1] = f.y;
-        }
-    }
-    template <int NV, int HS> static TS_D void unpack_c(const unsigned* w, float* out) {
-#pragma unroll
-        for (int t = 0; t < NV; ++t) {
-            const int h = t + (HS ? 1 : 0);
-            const __half2 v = *(const __half2*)&w[h >> 1];
-            out[t] = (h & 1) ? __high2float(v) : __low2float(v);
-        }
-    }
-    static TS_D uint4 pack(const float* o) {
-        unsigned r[4];
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-            const __half2 v = __floats2half2_rn(o[2 * k], o[2 * k + 1]);
-            r[k] = *(const unsigned*)&v;
-        }
-        return make_uint4(r[0], r[1], r[2], r[3]);
-    }
-};
 
 // window of NV elements starting at element index `e0` (>= 0, window inside the region) of a staged region
 // (`region` = 32-bit shared-window address)
@@ -475,17 +384,6 @@ TS_D void load_window_rt(unsigned region, int e0, float* out) {
     load_words_rt<NW>(region, byte & ~15, (byte >> 2) & 3, w);
     w[NW] = 0u;
     Pack<ST>::template unpack<NV>(w, (byte & 2) * 8, out);
-}
-
-// window of NV elements whose first element sits PH bytes (compile-time, a multiple of sizeof(ST)) into the
-// 16-byte group at shared address `group`: exactly the words the window touches are loaded, no run-time realignment
-template <typename ST, int PH, int NV>
-TS_D void load_window_c(unsigned group, float* out) {
-    constexpr int WS = PH >> 2, HS = (PH & 2) * 8;
-    constexpr int NW = sizeof(ST) == 4 ? NV : (NV + (HS ? 1 : 0) + 1) / 2;
-    unsigned w[NW];
-    load_words<WS, NW>(group, 0, w);
-    Pack<ST>::template unpack_c<NV, HS>(w, out);
 }
 
 // 1-D tensors (an image is ONE row): per-unit stepping of the flat (image, interior group) loop of a thread
@@ -1759,7 +1657,7 @@ int staged_active_forward(const Geo& g, const StagedPlan& p, int dtype, const vo
     a.x = (const unsigned char*)x;
     a.out = (unsigned char*)y;
     a.w = w;
-    a.wk = dtype == TS_F32 ? WK_F32 : dtype == TS_F16 ? WK_F16 : WK_BF16;
+    a.wk = dtype == TS_F32 || g.wf32 ? WK_F32 : dtype == TS_F16 ? WK_F16 : WK_BF16;
     switch (dtype) {
     case TS_F32: return active_forward_t<float>(g, a, p, s);
     case TS_F16: return active_forward_t<__half>(g, a, p, s);
@@ -1786,7 +1684,7 @@ int staged_backward(const Geo& g, const StagedPlan& p, int dtype, int active, co
     a.grad = (const unsigned char*)grad;
     a.out = (unsigned char*)gi;
     a.w = w;
-    a.wk = dtype == TS_F32 ? WK_F32 : dtype == TS_F16 ? WK_F16 : WK_BF16;
+    a.wk = dtype == TS_F32 || g.wf32 ? WK_F32 : dtype == TS_F16 ? WK_F16 : WK_BF16;
     a.partials = partials;
     switch (dtype) {
     case TS_F32: return backward_t<float>(g, a, p, active, s);

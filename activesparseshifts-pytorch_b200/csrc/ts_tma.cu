@@ -8,7 +8,7 @@
 // gather (ops/kernels/shifts_kernels.h:10-54 with BIPadding::Zeros) done by hardware, so the
 // consumers have no index remapping, no validity masks and no edge cases at all: every item reads
 // aligned 16-byte groups from shared memory and only resolves the residual sub-16-byte column
-// misalignment (0..3 fp32 elements; the copy engine requires the innermost coordinate to be a
+// misalignment (0..3 fp32 or 0..7 16-bit elements; the copy engine requires the innermost coordinate to be a
 // multiple of 16 bytes -- measured: an unaligned inner coordinate raises "illegal instruction").
 // The box carries one extra 16-byte group per row (and one extra row / slab for the arithmetic
 // kernels) for the residual window and the +1 interpolation neighbours.
@@ -23,11 +23,13 @@
 // per-(unit, warp) in fp64, fixed shuffle tree, second pass in ts_generic.cu -> deterministic.
 //
 // Applicability (plan_tma): zeros padding, dense NCHW x, row bytes a multiple of 16, pad value 0,
-// fp32 for the arithmetic modes, no border crop for the backward.  Everything else runs on
-// ts_staged.cu / ts_generic.cu.
+// no border crop for the backward; the arithmetic modes take fp32, and 2-D fp16 / bf16 tensors whose weights are
+// fp32 (TS_WEIGHTS_F32: an item is then 8 elements, fp32 arithmetic, one rounding at the store).  Everything else runs
+// on the other families.
 #include <cuda.h>
 
 #include <cstdio>
+#include <type_traits>
 
 #include "ts_kernels.h"
 #include "ts_ptx.cuh"
@@ -61,18 +63,19 @@ EncodeTiledFn encode_tiled() {
 struct MapKey {
     const void* base;
     long long N, C;
-    int es, A, B, L, bl, bb, ba, bn;
+    int es, dtype, A, B, L, bl, bb, ba, bn;
 };
 struct MapSlot { MapKey key; CUtensorMap map; bool used; };
 constexpr int MAP_CACHE = 32;
 
+// dtype: TS_F16 / TS_BF16 name the 16-bit element type of the arithmetic kernels' maps; anything else copies raw words.
 bool make_map(CUtensorMap* map, const void* base, int es, long long N, long long C, int A, int B, int L, int bl, int bb, int ba,
-              int bn) {
+              int bn, int dtype = -1) {
     static thread_local MapSlot cache[MAP_CACHE];
     static thread_local int next_victim = 0;
     MapKey key;
     memset(&key, 0, sizeof(key));
-    key.base = base; key.N = N; key.C = C; key.es = es; key.A = A; key.B = B; key.L = L; key.bl = bl; key.bb = bb; key.ba = ba; key.bn = bn;
+    key.base = base; key.N = N; key.C = C; key.es = es; key.dtype = dtype; key.A = A; key.B = B; key.L = L; key.bl = bl; key.bb = bb; key.ba = ba; key.bn = bn;
     for (int i = 0; i < MAP_CACHE; ++i)
         if (cache[i].used && !memcmp(&cache[i].key, &key, sizeof(key))) { *map = cache[i].map; return true; }
     EncodeTiledFn enc = encode_tiled();
@@ -82,7 +85,9 @@ bool make_map(CUtensorMap* map, const void* base, int es, long long N, long long
     // its first backward) has none yet (CUDA_ERROR_INVALID_CONTEXT); cudaFree(0) binds it.
     static thread_local bool ctx_bound = false;
     if (!ctx_bound) { (void)cudaFree(nullptr); ctx_bound = true; }
-    const CUtensorMapDataType dt = es == 1 ? CU_TENSOR_MAP_DATA_TYPE_UINT8 : es == 2 ? CU_TENSOR_MAP_DATA_TYPE_UINT16
+    const CUtensorMapDataType dt = es == 2 && dtype == TS_BF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16
+                                 : es == 2 && dtype == TS_F16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16
+                                 : es == 1 ? CU_TENSOR_MAP_DATA_TYPE_UINT8 : es == 2 ? CU_TENSOR_MAP_DATA_TYPE_UINT16
                                  : es == 4 ? CU_TENSOR_MAP_DATA_TYPE_UINT32 : CU_TENSOR_MAP_DATA_TYPE_UINT64;
     cuuint64_t dims[5] = {(cuuint64_t)L, (cuuint64_t)B, (cuuint64_t)A, (cuuint64_t)C, (cuuint64_t)N};
     const cuuint64_t row = (cuuint64_t)L * es;
@@ -153,7 +158,7 @@ TS_D UnitShift compute_unit_shift(const TArgs& a, long long c) {
             const long long idx = c * dim + ax;
             if (a.mode == 0) {
                 iw = sparse_shift(a.w, a.wk, a.qkind, a.wzp, idx);
-            } else {
+            } else {             // fp32 weights: fp32 layers, and 16-bit layers under TS_WEIGHTS_F32 (the only ones planned)
                 float d;
                 if (a.mode == 1) split_forward<float>(((const float*)a.w)[idx], true, iw, d);
                 else split_backward<float>(((const float*)a.w)[idx], a.active != 0, iw, d);
@@ -357,18 +362,12 @@ struct GatherBody {
 };
 
 // ================================================================================================
-// fp32 arithmetic bodies.  A window of NV consecutive elements starting M elements into the
-// aligned group `ch` of a staged box.
-template <int M, int NV>
+// Arithmetic bodies, fp32 arithmetic on ST elements (fp32, or fp16 / bf16 rounded once at the store).  An item is one
+// 16-byte group: V = 4 or 8 elements.  A window of NV consecutive elements starting M elements into the aligned group
+// `ch` of a staged box (compile-time word select, plus a half-word shift for 16-bit elements).
+template <typename ST, int M, int NV>
 TS_D void load_win(unsigned box, int ch, float* out) {
-    const uint4 A = lds128(box + ch * 16);
-    float W[8] = {__uint_as_float(A.x), __uint_as_float(A.y), __uint_as_float(A.z), __uint_as_float(A.w), 0.f, 0.f, 0.f, 0.f};
-    if (M + NV > 4) {
-        const uint4 B = lds128(box + ch * 16 + 16);
-        W[4] = __uint_as_float(B.x); W[5] = __uint_as_float(B.y); W[6] = __uint_as_float(B.z); W[7] = __uint_as_float(B.w);
-    }
-#pragma unroll
-    for (int t = 0; t < NV; ++t) out[t] = W[t + M];
+    load_window_c<ST, M * (int)sizeof(ST), NV>(box + ch * 16, out);
 }
 
 // group offset of the +1 neighbour rows inside a box with `rows` rows per slab, `pitch` groups per row
@@ -379,8 +378,8 @@ TS_D int neighbour_row_offset(int rv, int rows, int pitch) {
     return ((rv & 1) * rows + ((rv >> 1) & 1)) * pitch;
 }
 
-template <int DIM>
-TS_D void neighbours_from_rows(const float (*X)[5], int t, float* v) {
+template <int DIM, int NVW>
+TS_D void neighbours_from_rows(const float (*X)[NVW], int t, float* v) {
     constexpr int NR = 1 << (DIM - 1);
 #pragma unroll
     for (int q = 0; q < (1 << DIM); ++q) v[q] = X[q & (NR - 1)][t + (q >> (DIM - 1))];
@@ -408,8 +407,29 @@ TS_D void weight_partials_fast(const float* v, const float* d, float* g) {
     g[2] = fmaf(d[1], i3 - i2, i2) - fmaf(d[1], i1 - i0, i0);
 }
 
-template <int DIM>
+// f(integral_constant<M>) for the run-time window phase m in [0, V): the bodies are instantiated per phase
+template <int V, class F>
+TS_D void with_phase(int m, F&& f) {
+    using std::integral_constant;
+    if constexpr (V == 8) {
+        switch (m) {
+        case 4: f(integral_constant<int, 4>()); return;
+        case 5: f(integral_constant<int, 5>()); return;
+        case 6: f(integral_constant<int, 6>()); return;
+        case 7: f(integral_constant<int, 7>()); return;
+        }
+    }
+    switch (m) {
+    case 0: f(integral_constant<int, 0>()); return;
+    case 1: f(integral_constant<int, 1>()); return;
+    case 2: f(integral_constant<int, 2>()); return;
+    default: f(integral_constant<int, 3>()); return;
+    }
+}
+
+template <typename ST, int DIM>
 struct ActiveFwdBody {
+    static constexpr int V = Pack<ST>::V, NVW = V + 1;   // elements per item, window with the +1 neighbour
     const TArgs& a;
     const int tid, nt;
     UnitShift us;
@@ -419,7 +439,7 @@ struct ActiveFwdBody {
     TS_D ActiveFwdBody(const TArgs& a_, int tid_, int nt_, const UnitShift* tbl_) : a(a_), tid(tid_), nt(nt_), m(0), tbl(tbl_) {}
     TS_D void begin_unit(int c) {
         us = unit_shift(a, tbl, c);
-        m = pmod(a.lbL - us.sh[2], 4);
+        m = pmod(a.lbL - us.sh[2], V);
     }
     TS_D void end_unit(int, int) {}
 
@@ -433,17 +453,17 @@ struct ActiveFwdBody {
             Item p;
             if (!decode_item<DIM == 3>(a, sg, item, p)) continue;
             const int base = p.pl * ximg + (p.a * xb + p.b) * pitch + p.cg;
-            float X[NR][5];
+            float X[NR][NVW];
 #pragma unroll
-            for (int rv = 0; rv < NR; ++rv) load_win<M, 5>(box, base + neighbour_row_offset<DIM>(rv, xb, pitch), X[rv]);
-            float o[4];
+            for (int rv = 0; rv < NR; ++rv) load_win<ST, M, NVW>(box, base + neighbour_row_offset<DIM>(rv, xb, pitch), X[rv]);
+            float o[V];
 #pragma unroll
-            for (int t = 0; t < 4; ++t) {
+            for (int t = 0; t < V; ++t) {
                 float v[8];
                 neighbours_from_rows<DIM>(X, t, v);
                 o[t] = interpolate<float, DIM>(v, d);
             }
-            __stcs((float4*)item_dst(a, sg, p), make_float4(o[0], o[1], o[2], o[3]));
+            __stcs((uint4*)item_dst(a, sg, p), Pack<ST>::pack(o));
         }
     }
     // strip-mined variant, used for 3-D (see BackwardBody::run_strip)
@@ -470,29 +490,29 @@ struct ActiveFwdBody {
             p.pl = pl; p.a = ia; p.b = b0; p.cg = cg;
             int xch = pl * ximg + (ia * xb + b0) * pitch + cg;
             unsigned char* dst = item_dst(a, sg, p);
-            float Xlo[S][5];
+            float Xlo[S][NVW];
 #pragma unroll
-            for (int q = 0; q < S; ++q) load_win<M, 5>(box, xch + q * xslab, Xlo[q]);
+            for (int q = 0; q < S; ++q) load_win<ST, M, NVW>(box, xch + q * xslab, Xlo[q]);
             for (int b = b0; b < bend; ++b) {
-                float X[NR][5];
+                float X[NR][NVW];
 #pragma unroll
                 for (int q = 0; q < S; ++q) {
-                    load_win<M, 5>(box, xch + pitch + q * xslab, X[S + q]);
+                    load_win<ST, M, NVW>(box, xch + pitch + q * xslab, X[S + q]);
 #pragma unroll
-                    for (int t = 0; t < 5; ++t) X[q][t] = Xlo[q][t];
+                    for (int t = 0; t < NVW; ++t) X[q][t] = Xlo[q][t];
                 }
-                float o[4];
+                float o[V];
 #pragma unroll
-                for (int t = 0; t < 4; ++t) {
+                for (int t = 0; t < V; ++t) {
                     float v[8];
                     neighbours_from_rows<DIM>(X, t, v);
                     o[t] = interpolate<float, DIM>(v, d);
                 }
-                __stcs((float4*)dst, make_float4(o[0], o[1], o[2], o[3]));
+                __stcs((uint4*)dst, Pack<ST>::pack(o));
 #pragma unroll
                 for (int q = 0; q < S; ++q)
 #pragma unroll
-                    for (int t = 0; t < 5; ++t) Xlo[q][t] = X[S + q][t];
+                    for (int t = 0; t < NVW; ++t) Xlo[q][t] = X[S + q][t];
                 xch += pitch; dst += orow;
             }
         }
@@ -503,17 +523,13 @@ struct ActiveFwdBody {
                                                                      // padded index space is measurably faster there
     }
     TS_D void step(const Stage& sg) const {
-        switch (m) {
-        case 0: run_any<0>(sg); break;
-        case 1: run_any<1>(sg); break;
-        case 2: run_any<2>(sg); break;
-        default: run_any<3>(sg); break;
-        }
+        with_phase<V>(m, [&](auto M) { this->template run_any<decltype(M)::value>(sg); });
     }
 };
 
-template <int DIM, bool ACTIVE>
+template <typename ST, int DIM, bool ACTIVE>
 struct BackwardBody {
+    static constexpr int V = Pack<ST>::V, NVW = V + 1;
     const TArgs& a;
     const int tid, nt, wid, lane;
     UnitShift us;
@@ -525,7 +541,7 @@ struct BackwardBody {
         : a(a_), tid(tid_), nt(nt_), wid(wid_), lane(lane_), m(0), tbl(tbl_) {}
     TS_D void begin_unit(int c) {
         us = unit_shift(a, tbl, c);
-        m = pmod(-us.sh[2], 4);
+        m = pmod(-us.sh[2], V);
 #pragma unroll
         for (int d = 0; d < DIM; ++d) acc[d] = 0.0;
     }
@@ -543,7 +559,7 @@ struct BackwardBody {
     template <int M>
     TS_D void run(const Stage& sg) {
         constexpr int NR = 1 << (DIM - 1);
-        constexpr int MG = ACTIVE ? M : ((4 - M) & 3);      // misalignment of the grad window used for grad_input
+        constexpr int MG = ACTIVE ? M : ((V - M) & (V - 1));      // misalignment of the grad window used for grad_input
         const unsigned xbox = shared_addr(sg.st);
         const unsigned gv_box = xbox + a.off_gv;
         const unsigned g2_box = xbox + a.off_g2;
@@ -557,14 +573,14 @@ struct BackwardBody {
             if (!decode_item<DIM == 3>(a, sg, item, p)) continue;
             const int gch = p.pl * gimg + (p.a * tb + p.b) * pitch + p.cg;
             const int xch = p.pl * ximg + (p.a * xb + p.b) * pitch + p.cg;
-            float gv[4];
-            load_win<0, 4>(gv_box, gch, gv);
+            float gv[V];
+            load_win<ST, 0, V>(gv_box, gch, gv);
             // ---- grad_weight terms ----
-            float X[NR][5];
+            float X[NR][NVW];
 #pragma unroll
-            for (int rv = 0; rv < NR; ++rv) load_win<M, 5>(xbox, xch + neighbour_row_offset<DIM>(rv, xb, pitch), X[rv]);
+            for (int rv = 0; rv < NR; ++rv) load_win<ST, M, NVW>(xbox, xch + neighbour_row_offset<DIM>(rv, xb, pitch), X[rv]);
 #pragma unroll
-            for (int t = 0; t < 4; ++t) {
+            for (int t = 0; t < V; ++t) {
                 float v[8], wg[3];
                 neighbours_from_rows<DIM>(X, t, v);
                 weight_partials_fast<DIM>(v, d, wg);
@@ -572,21 +588,21 @@ struct BackwardBody {
                 for (int k = 0; k < DIM; ++k) ts[k] = fmaf(gv[t], wg[k], ts[k]);
             }
             // ---- grad_input ----
-            float o[4];
+            float o[V];
             if (ACTIVE) {
-                float G[NR][5];
+                float G[NR][NVW];
 #pragma unroll
-                for (int rv = 0; rv < NR; ++rv) load_win<MG, 5>(g2_box, xch + neighbour_row_offset<DIM>(rv, xb, pitch), G[rv]);
+                for (int rv = 0; rv < NR; ++rv) load_win<ST, MG, NVW>(g2_box, xch + neighbour_row_offset<DIM>(rv, xb, pitch), G[rv]);
 #pragma unroll
-                for (int t = 0; t < 4; ++t) {
+                for (int t = 0; t < V; ++t) {
                     float v[8];
                     neighbours_from_rows<DIM>(G, t, v);
                     o[t] = interpolate<float, DIM>(v, d);
                 }
             } else {
-                load_win<MG, 4>(g2_box, gch, o);
+                load_win<ST, MG, V>(g2_box, gch, o);
             }
-            __stcs((float4*)item_dst(a, sg, p), make_float4(o[0], o[1], o[2], o[3]));
+            __stcs((uint4*)item_dst(a, sg, p), Pack<ST>::pack(o));
         }
 #pragma unroll
         for (int k = 0; k < DIM; ++k) acc[k] += (double)ts[k];   // fp32 inside a stage, fp64 across stages
@@ -597,7 +613,7 @@ struct BackwardBody {
     TS_D void run_strip(const Stage& sg) {
         constexpr int NR = 1 << (DIM - 1);
         constexpr int S = DIM == 3 ? 2 : 1;
-        constexpr int MG = ACTIVE ? M : ((4 - M) & 3);
+        constexpr int MG = ACTIVE ? M : ((V - M) & (V - 1));
         const unsigned xbox = shared_addr(sg.st);
         const unsigned gv_box = xbox + a.off_gv;
         const unsigned g2_box = xbox + a.off_g2;
@@ -623,42 +639,42 @@ struct BackwardBody {
             int gch = pl * gimg + (ia * tb + b0) * pitch + cg;
             int xch = pl * ximg + (ia * xb + b0) * pitch + cg;
             unsigned char* dst = item_dst(a, sg, p);
-            float Xlo[S][5], Glo[S][5];
+            float Xlo[S][NVW], Glo[S][NVW];
 #pragma unroll
-            for (int q = 0; q < S; ++q) load_win<M, 5>(xbox, xch + q * xslab, Xlo[q]);
+            for (int q = 0; q < S; ++q) load_win<ST, M, NVW>(xbox, xch + q * xslab, Xlo[q]);
             if (ACTIVE) {
 #pragma unroll
-                for (int q = 0; q < S; ++q) load_win<MG, 5>(g2_box, xch + q * xslab, Glo[q]);
+                for (int q = 0; q < S; ++q) load_win<ST, MG, NVW>(g2_box, xch + q * xslab, Glo[q]);
             }
             for (int b = b0; b < bend; ++b) {
-                float gv[4];
-                load_win<0, 4>(gv_box, gch, gv);
-                float X[NR][5];
+                float gv[V];
+                load_win<ST, 0, V>(gv_box, gch, gv);
+                float X[NR][NVW];
 #pragma unroll
                 for (int q = 0; q < S; ++q) {
-                    load_win<M, 5>(xbox, xch + pitch + q * xslab, X[S + q]);
+                    load_win<ST, M, NVW>(xbox, xch + pitch + q * xslab, X[S + q]);
 #pragma unroll
-                    for (int t = 0; t < 5; ++t) X[q][t] = Xlo[q][t];
+                    for (int t = 0; t < NVW; ++t) X[q][t] = Xlo[q][t];
                 }
 #pragma unroll
-                for (int t = 0; t < 4; ++t) {
+                for (int t = 0; t < V; ++t) {
                     float v[8], wg[3];
                     neighbours_from_rows<DIM>(X, t, v);
                     weight_partials_fast<DIM>(v, d, wg);
 #pragma unroll
                     for (int k = 0; k < DIM; ++k) ts[k] = fmaf(gv[t], wg[k], ts[k]);
                 }
-                float o[4];
+                float o[V];
                 if (ACTIVE) {
-                    float G[NR][5];
+                    float G[NR][NVW];
 #pragma unroll
                     for (int q = 0; q < S; ++q) {
-                        load_win<MG, 5>(g2_box, xch + pitch + q * xslab, G[S + q]);
+                        load_win<ST, MG, NVW>(g2_box, xch + pitch + q * xslab, G[S + q]);
 #pragma unroll
-                        for (int t = 0; t < 5; ++t) G[q][t] = Glo[q][t];
+                        for (int t = 0; t < NVW; ++t) G[q][t] = Glo[q][t];
                     }
 #pragma unroll
-                    for (int t = 0; t < 4; ++t) {
+                    for (int t = 0; t < V; ++t) {
                         float v[8];
                         neighbours_from_rows<DIM>(G, t, v);
                         o[t] = interpolate<float, DIM>(v, d);
@@ -666,15 +682,15 @@ struct BackwardBody {
 #pragma unroll
                     for (int q = 0; q < S; ++q)
 #pragma unroll
-                        for (int t = 0; t < 5; ++t) Glo[q][t] = G[S + q][t];
+                        for (int t = 0; t < NVW; ++t) Glo[q][t] = G[S + q][t];
                 } else {
-                    load_win<MG, 4>(g2_box, gch, o);
+                    load_win<ST, MG, V>(g2_box, gch, o);
                 }
-                __stcs((float4*)dst, make_float4(o[0], o[1], o[2], o[3]));
+                __stcs((uint4*)dst, Pack<ST>::pack(o));
 #pragma unroll
                 for (int q = 0; q < S; ++q)
 #pragma unroll
-                    for (int t = 0; t < 5; ++t) Xlo[q][t] = X[S + q][t];
+                    for (int t = 0; t < NVW; ++t) Xlo[q][t] = X[S + q][t];
                 xch += pitch; gch += pitch; dst += orow;
             }
         }
@@ -687,12 +703,7 @@ struct BackwardBody {
                                                                      // padded index space is measurably faster there
     }
     TS_D void step(const Stage& sg) {
-        switch (m) {
-        case 0: run_any<0>(sg); break;
-        case 1: run_any<1>(sg); break;
-        case 2: run_any<2>(sg); break;
-        default: run_any<3>(sg); break;
-        }
+        with_phase<V>(m, [&](auto M) { this->template run_any<decltype(M)::value>(sg); });
     }
 };
 
@@ -724,25 +735,25 @@ __global__ void __launch_bounds__(MAXT_TMA_GATHER, 1) k_tma_gather(const __grid_
     consumer_loop(a, smem, full, empty, lane, body);
 }
 
-template <int DIM>
+template <typename ST, int DIM>
 __global__ void __launch_bounds__(MAXT_TMA_ARITH, 1) k_tma_active_forward(const __grid_constant__ TArgs a) {
     extern __shared__ __align__(1024) unsigned char smem[];
     uint64_t *full, *empty;
     const UnitShift* tbl = setup_barriers(a, smem, full, empty);
     const int wid = threadIdx.x >> 5, lane = threadIdx.x & 31;
     if (wid == a.nw) { if (lane == 0) producer(a, smem, full, empty, tbl); return; }
-    ActiveFwdBody<DIM> body(a, threadIdx.x, a.nw * 32, tbl);
+    ActiveFwdBody<ST, DIM> body(a, threadIdx.x, a.nw * 32, tbl);
     consumer_loop(a, smem, full, empty, lane, body);
 }
 
-template <int DIM, bool ACTIVE>
+template <typename ST, int DIM, bool ACTIVE>
 __global__ void __launch_bounds__(MAXT_TMA_ARITH, 1) k_tma_backward(const __grid_constant__ TArgs a) {
     extern __shared__ __align__(1024) unsigned char smem[];
     uint64_t *full, *empty;
     const UnitShift* tbl = setup_barriers(a, smem, full, empty);
     const int wid = threadIdx.x >> 5, lane = threadIdx.x & 31;
     if (wid == a.nw) { if (lane == 0) producer(a, smem, full, empty, tbl); return; }
-    BackwardBody<DIM, ACTIVE> body(a, threadIdx.x, a.nw * 32, wid, lane, tbl);
+    BackwardBody<ST, DIM, ACTIVE> body(a, threadIdx.x, a.nw * 32, wid, lane, tbl);
     consumer_loop(a, smem, full, empty, lane, body);
 }
 
@@ -823,8 +834,10 @@ TmaPlan plan_tma(const Geo& g, int mode, int active, int esize, int dtype, bool 
     if (!encode_tiled()) return p;
     if (g.pad != TS_PAD_ZEROS || !dense_x || fill != 0ull) return p;
     if (g.N * g.C == 0 || g.in_plane == 0 || g.out_plane == 0) return p;
-    if (mode != 0 && dtype != TS_F32) return p;          // arithmetic kernels: fp32
-    if (mode != 0) esize = 4;
+    // arithmetic kernels: fp32, or 2-D fp16 / bf16 whose weights are fp32 (same-dtype 16-bit layers keep their families)
+    const bool arith16 = g.wf32 && g.dim == 2 && (dtype == TS_F16 || dtype == TS_BF16);
+    if (mode != 0 && dtype != TS_F32 && !arith16) return p;
+    if (mode != 0) esize = dtype == TS_F32 ? 4 : 2;
     if (esize != 1 && esize != 2 && esize != 4 && esize != 8) return p;
     const int d = g.dim;
     if (mode == 2)                                       // the backward tiles assume output space == input space
@@ -962,40 +975,61 @@ int tma_gather(const Geo& g, const TmaPlan& p, int wk, const void* x, void* y, i
     return a.TA > 1 ? launch(k_tma_gather<true>, a, p, s) : launch(k_tma_gather<false>, a, p, s);
 }
 
-int tma_active_forward(const Geo& g, const TmaPlan& p, const void* x, const void* w, void* y, cudaStream_t s) {
-    TArgs a;
-    make_args(g, p, 1, 1, 4, &a);
-    const Levels lv(g);
-    a.out = (unsigned char*)y;
-    a.w = w;
-    if (!make_map(&a.map_x, x, 4, g.N, g.C, lv.A, lv.B, lv.L, (a.TG + 1) * 4, a.xb, a.xa, a.np)) return TS_ERR_UNSUPPORTED;
+template <typename ST>
+static int active_forward_t(const Geo& g, const TArgs& a, const TmaPlan& p, cudaStream_t s) {
     switch (g.dim) {
-    case 1: return launch(k_tma_active_forward<1>, a, p, s);
-    case 2: return launch(k_tma_active_forward<2>, a, p, s);
-    default: return launch(k_tma_active_forward<3>, a, p, s);
+    case 1: return launch(k_tma_active_forward<ST, 1>, a, p, s);
+    case 2: return launch(k_tma_active_forward<ST, 2>, a, p, s);
+    default: return launch(k_tma_active_forward<ST, 3>, a, p, s);
     }
 }
 
-int tma_backward(const Geo& g, const TmaPlan& p, int active, const void* grad, const void* x, const void* w, void* gi,
+int tma_active_forward(const Geo& g, const TmaPlan& p, int dtype, const void* x, const void* w, void* y, cudaStream_t s) {
+    TArgs a;
+    const int es = dtype == TS_F32 ? 4 : 2;
+    make_args(g, p, 1, 1, es, &a);
+    const Levels lv(g);
+    a.out = (unsigned char*)y;
+    a.w = w;
+    if (!make_map(&a.map_x, x, es, g.N, g.C, lv.A, lv.B, lv.L, (a.TG + 1) * a.vec, a.xb, a.xa, a.np, dtype)) return TS_ERR_UNSUPPORTED;
+    switch (dtype) {      // 16-bit: planned for 2-D only
+    case TS_F16: return launch(k_tma_active_forward<__half, 2>, a, p, s);
+    case TS_BF16: return launch(k_tma_active_forward<__nv_bfloat16, 2>, a, p, s);
+    }
+    return active_forward_t<float>(g, a, p, s);
+}
+
+template <typename ST>
+static int backward_t(const Geo& g, const TArgs& a, const TmaPlan& p, int active, cudaStream_t s) {
+    switch (g.dim * 2 + (active ? 1 : 0)) {
+    case 2: return launch(k_tma_backward<ST, 1, false>, a, p, s);
+    case 3: return launch(k_tma_backward<ST, 1, true>, a, p, s);
+    case 4: return launch(k_tma_backward<ST, 2, false>, a, p, s);
+    case 5: return launch(k_tma_backward<ST, 2, true>, a, p, s);
+    case 6: return launch(k_tma_backward<ST, 3, false>, a, p, s);
+    default: return launch(k_tma_backward<ST, 3, true>, a, p, s);
+    }
+}
+
+int tma_backward(const Geo& g, const TmaPlan& p, int dtype, int active, const void* grad, const void* x, const void* w, void* gi,
                  double* partials, cudaStream_t s) {
     TArgs a;
-    make_args(g, p, 2, active ? 1 : 0, 4, &a);
+    const int es = dtype == TS_F32 ? 4 : 2;
+    make_args(g, p, 2, active ? 1 : 0, es, &a);
     const Levels lv(g);
-    const int A = lv.A, B = lv.B, L = lv.L;
+    const int A = lv.A, B = lv.B, L = lv.L, bl = (a.TG + 1) * a.vec;
     a.out = (unsigned char*)gi;
     a.w = w;
     a.partials = partials;
-    if (!make_map(&a.map_x, x, 4, g.N, g.C, A, B, L, (a.TG + 1) * 4, a.xb, a.xa, a.np)) return TS_ERR_UNSUPPORTED;
-    if (!make_map(&a.map_gs, grad, 4, g.N, g.C, A, B, L, (a.TG + 1) * 4, a.TB, a.TA, a.np)) return TS_ERR_UNSUPPORTED;
-    if (active && !make_map(&a.map_gb, grad, 4, g.N, g.C, A, B, L, (a.TG + 1) * 4, a.xb, a.xa, a.np)) return TS_ERR_UNSUPPORTED;
-    switch (g.dim * 2 + (active ? 1 : 0)) {
-    case 2: return launch(k_tma_backward<1, false>, a, p, s);
-    case 3: return launch(k_tma_backward<1, true>, a, p, s);
-    case 4: return launch(k_tma_backward<2, false>, a, p, s);
-    case 5: return launch(k_tma_backward<2, true>, a, p, s);
-    case 6: return launch(k_tma_backward<3, false>, a, p, s);
-    default: return launch(k_tma_backward<3, true>, a, p, s);
+    if (!make_map(&a.map_x, x, es, g.N, g.C, A, B, L, bl, a.xb, a.xa, a.np, dtype)) return TS_ERR_UNSUPPORTED;
+    if (!make_map(&a.map_gs, grad, es, g.N, g.C, A, B, L, bl, a.TB, a.TA, a.np, dtype)) return TS_ERR_UNSUPPORTED;
+    if (active && !make_map(&a.map_gb, grad, es, g.N, g.C, A, B, L, bl, a.xb, a.xa, a.np, dtype)) return TS_ERR_UNSUPPORTED;
+    switch (dtype) {      // 16-bit: planned for 2-D only
+    case TS_F16: return active ? launch(k_tma_backward<__half, 2, true>, a, p, s) : launch(k_tma_backward<__half, 2, false>, a, p, s);
+    case TS_BF16:
+        return active ? launch(k_tma_backward<__nv_bfloat16, 2, true>, a, p, s) : launch(k_tma_backward<__nv_bfloat16, 2, false>, a, p, s);
     }
+    return backward_t<float>(g, a, p, active, s);
 }
 
 }  // namespace ts

@@ -15,6 +15,7 @@ STATUS_NAMES = {0: 'TS_OK', 1: 'TS_ERR_INVALID_ARGUMENT', 2: 'TS_ERR_UNSUPPORTED
                 4: 'TS_ERR_TOO_LARGE', 5: 'TS_ERR_BORDERS', 6: 'TS_ERR_CUDA', 7: 'TS_ERR_NO_DEVICE'}
 PATH_NONE, PATH_GENERIC, PATH_STAGED, PATH_TMA, PATH_NHWC, PATH_HALO, PATH_FLAT = 0, 1, 2, 3, 4, 5, 6
 QW_U8, QW_I8, QW_I32 = 0, 1, 2
+TS_WEIGHTS_F32 = 0x100        # dtype flag: fp16 / bf16 x with fp32 weights and grad_weight
 
 
 class Geometry(ct.Structure):

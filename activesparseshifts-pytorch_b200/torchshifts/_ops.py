@@ -20,6 +20,11 @@ Extension over the reference (the functional layer routes channels-last inputs h
 same arguments and values as ``_shiftNd_forward/_backward``, but the output and ``grad_input`` are dense
 channels-last (``channels_last`` / ``channels_last_3d``).
 
+Mixed precision (an extension over the reference, whose type check raises): an fp16 / bf16 ``input`` (and ``grad``) may
+come with fp32 ``weights``.  The output and ``grad_input`` keep the input's dtype, ``grad_weight`` is fp32 like the
+weights, and the weights are split in fp32 -- never rounded to 16 bits.  No autocast kernel is registered: under
+``torch.autocast`` the operators take the activation dtype they receive and never cast the weights.
+
 Dispatch keys: ``shiftNd`` is CompositeImplicitAutograd (border validation, then ``_shiftNd_forward``);
 ``_shiftNd_forward/_backward`` carry the autograd wiring of csrc/ops/autograd/shifts_autograd.cpp
 (``torch.library.register_autograd``: saves input/weights/borders, double backward is an error),
@@ -33,7 +38,8 @@ import weakref
 
 import torch
 
-from ._cabi import QW_I8, QW_I32, QW_U8, TS_ERR_TOO_LARGE, TS_ERR_UNSUPPORTED, TS_ERR_WORKSPACE, TS_OK, make_geometry
+from ._cabi import (QW_I8, QW_I32, QW_U8, TS_ERR_TOO_LARGE, TS_ERR_UNSUPPORTED, TS_ERR_WORKSPACE, TS_OK, TS_WEIGHTS_F32,
+                    make_geometry)
 
 _LIB = None            # torch.library.Library handle (kept alive)
 _FUSED_ALLREDUCE = None   # torchshifts.sharded.FusedGradWeightAllReduce while enabled: grad_weight is summed over the ranks in-kernel
@@ -63,17 +69,31 @@ def _borders_lists(borders, dim):
     return [b[0], b[2], b[4]], [b[1], b[3], b[5]]
 
 
+_HALF = (torch.float16, torch.bfloat16)
+
+
+def _mixed(input, weights):
+    """fp16 / bf16 activations with fp32 (master) weights."""
+    return input.dtype in _HALF and weights.dtype == torch.float32
+
+
 def _same_device_and_type(fn, input, weights, grad=None):
-    # checkAllSameGPU / checkAllSameType of cuda/shifts_cuda.cu:213-214, :282-283
+    # checkAllSameGPU / checkAllSameType of cuda/shifts_cuda.cu:213-214, :282-283; in addition fp16 / bf16 input and grad
+    # may come with fp32 weights (mixed precision)
     if weights.device != input.device or (grad is not None and grad.device != input.device):
         raise RuntimeError(f'{fn}: expected input, weights' + (', grad' if grad is not None else '') +
                            f' to be on the same GPU, but got {input.device}, {weights.device}' +
                            (f', {grad.device}' if grad is not None else ''))
-    if weights.dtype != input.dtype or (grad is not None and grad.dtype != input.dtype):
+    if (weights.dtype != input.dtype and not _mixed(input, weights)) or (grad is not None and grad.dtype != input.dtype):
         raise RuntimeError(f'{fn}: expected scalar type {input.dtype} for every tensor but found '
                            f'weights {weights.dtype}' + (f', grad {grad.dtype}' if grad is not None else ''))
     if input.dtype not in _DTYPES:
         raise RuntimeError(f'{fn}: "shiftnd_cuda" not implemented for {input.dtype}')
+
+
+def _dtype_code(input, weights):
+    """The C ABI's dtype argument: the element type, with TS_WEIGHTS_F32 for fp32 weights of a 16-bit input."""
+    return _DTYPES[input.dtype] | (TS_WEIGHTS_F32 if _mixed(input, weights) else 0)
 
 
 _COPY_THRESHOLD = 1 << 16
@@ -165,7 +185,7 @@ def _guard(device):
 
 
 _GEO_CACHE = {}        # (dim, shape, strides, lb, rb) -> ts_geometry; shift layers see the same few shapes every step
-_WS_CACHE = {}         # (workspace query's name, geometry key, dtype code, device index) -> backward workspace bytes
+_WS_CACHE = {}         # (workspace query's name, geometry key, dtype code with its flags, device index) -> backward workspace bytes
 
 
 def _geometry(dim, input, lb, rb):
@@ -194,7 +214,7 @@ def _launch_backward(entry, query, geo, key, grad, input, weights, padding_mode,
     With a ``fallback`` (statuses as for ``_served``) returns None when the kernel does not serve the call: the launch
     returned such a status, or ``query`` answered 16 bytes (no partials), which is decided before ``grad`` is converted
     to ``fmt`` -- a conversion the caller's fallback path would do again."""
-    code = _DTYPES[input.dtype]
+    code = _dtype_code(input, weights)
     dev = input.device
     wkey = (query.__name__, key, code, dev.index)
     with _guard(dev):
@@ -240,7 +260,7 @@ def _forward_cuda(dim, input, weights, borders, new_size, padding_mode, active_f
     geo, _ = _geometry(dim, input, lb, rb)
     _check_size(fn, 'new_size', new_size, dim, input, lb, rb)
     with _guard(input.device):
-        st = _NATIVE.lib.ts_shift_forward(ct.byref(geo), _DTYPES[input.dtype], int(padding_mode), int(bool(active_flag)),
+        st = _NATIVE.lib.ts_shift_forward(ct.byref(geo), _dtype_code(input, w), int(padding_mode), int(bool(active_flag)),
                                           input.data_ptr(), w.data_ptr(), out.data_ptr(), _stream(input.device))
     _served(st, 'ts_shift_forward')
     return out
@@ -345,7 +365,7 @@ def _forward_cl_cuda(dim, input, weights, borders, new_size, padding_mode, activ
         w = weights.contiguous()
         geo, _ = _geometry(dim, input, lb, rb)
         with _guard(input.device):
-            st = _NATIVE.lib.ts_shift_forward_nhwc(ct.byref(geo), _DTYPES[input.dtype], int(padding_mode), int(bool(active_flag)),
+            st = _NATIVE.lib.ts_shift_forward_nhwc(ct.byref(geo), _dtype_code(input, w), int(padding_mode), int(bool(active_flag)),
                                                    input.data_ptr(), w.data_ptr(), out.data_ptr(), _stream(input.device))
         if _served(st, 'ts_shift_forward_nhwc', _FALLBACK):
             return out

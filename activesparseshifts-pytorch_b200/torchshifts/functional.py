@@ -120,6 +120,11 @@ def shift1d_func(input: Tensor, weights: Tensor, padding_mode: int, active_flag:
     quantized inputs); ``borders [1, 2]`` = (left_cut, right_cut) crops the output.
     ``memory_format`` (keyword only) is accepted for symmetry with the 2-D / 3-D layers and ignored: 3-D
     tensors have no channels-last format.
+
+    Mixed precision: an fp16 / bf16 ``input`` may come with fp32 ``weights`` (an extension over the reference, which
+    raises).  The output and ``grad_input`` keep ``input``'s dtype, ``grad_weight`` is fp32, and the shifts are taken from
+    the fp32 weights without rounding them to 16 bits.  No autocast rule is registered: under ``torch.autocast`` the shift
+    takes the activation dtype it receives and never casts the weights.
     """
     return _shift_func(1, input, weights, padding_mode, active_flag, borders, _border_ints, memory_format)
 
@@ -132,14 +137,19 @@ def shift2d_func(input: Tensor, weights: Tensor, padding_mode: int, active_flag:
     ``memory_format`` (keyword only): ``torch.contiguous_format`` (default) returns NCHW outputs and NCHW
     ``grad_input``, as the reference does; ``torch.preserve_format`` returns both dense ``channels_last`` when
     ``input`` is dense channels-last (and not also NCHW-contiguous), with the same values.  Other layouts give
-    the default result.  This is an extension over the reference."""
+    the default result.  This is an extension over the reference.
+
+    Mixed precision (fp16 / bf16 ``input``, fp32 ``weights``, fp32 ``grad_weight``; no autocast cast of the weights) as
+    for :func:`shift1d_func`."""
     return _shift_func(2, input, weights, padding_mode, active_flag, borders, _border_ints, memory_format)
 
 
 def shift3d_func(input: Tensor, weights: Tensor, padding_mode: int, active_flag: bool,
                  borders: Optional[Tensor] = None, _border_ints=None, *, memory_format=torch.contiguous_format) -> Tensor:
     """3-D version: ``input [N, C, H, W, D]``, ``weights [C, 3]``, ``borders [3, 2]``; the active
-    shift is trilinear.  ``memory_format`` as for :func:`shift2d_func`, with ``channels_last_3d``."""
+    shift is trilinear.  ``memory_format`` as for :func:`shift2d_func`, with ``channels_last_3d``.  Mixed precision
+    (fp16 / bf16 ``input``, fp32 ``weights``, fp32 ``grad_weight``; no autocast cast of the weights) as for
+    :func:`shift1d_func`."""
     return _shift_func(3, input, weights, padding_mode, active_flag, borders, _border_ints, memory_format)
 
 

@@ -88,6 +88,11 @@ class _Shiftnd(nn.Module):
         memory_format (torch.memory_format): ``torch.contiguous_format`` (default): NCHW outputs, as the
             reference; ``torch.preserve_format``: a dense channels-last input gives a channels-last output and
             ``grad_input`` (see :func:`torchshifts.functional.shift2d_func`).  Ignored by ``Shift1d``.
+
+    Mixed precision: ``weight`` stays an fp32 parameter while the layer takes fp16 / bf16 inputs, e.g. under
+    ``torch.autocast('cuda', dtype=torch.bfloat16)``.  The output keeps the input's dtype, ``weight.grad`` is fp32, and
+    the shifts come from the fp32 weights unrounded.  No autocast rule is registered and the weights are never cast; an
+    extension over the reference, which raises on the dtype mismatch.
     """
 
     @staticmethod
@@ -200,7 +205,9 @@ def _make_shift_class(dim, what):
     _Shift.__name__ = _Shift.__qualname__ = f'Shift{dim}d'
     _Shift.__doc__ = (f'Per-channel learnable shift of a {dim + 2}-D tensor ({what}).\n\n'
                       '    ``forward`` returns ``(output, loss)``; ``loss`` is ``sparsity_term * sum|weight|`` or ``None`` when\n'
-                      '    ``sparsity_term`` is 0.  See :class:`_Shiftnd` for the arguments.')
+                      '    ``sparsity_term`` is 0.  See :class:`_Shiftnd` for the arguments.\n\n'
+                      '    Mixed precision: fp16 / bf16 inputs with the fp32 ``weight`` (e.g. under ``torch.autocast``) give an output\n'
+                      '    in the input\'s dtype and an fp32 ``weight.grad``; the weights are never cast or rounded to 16 bits.')
     return _Shift
 
 

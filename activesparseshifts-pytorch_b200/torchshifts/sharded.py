@@ -42,11 +42,16 @@ def allreduce_grad_weights(module_or_params, group=None, average: bool = False) 
     """Sum (or average) ``weight.grad`` of every shift layer over the ranks with ONE collective.
 
     Returns the number of elements reduced.  Parameters without a gradient contribute zeros so
-    that all ranks issue the same collective."""
+    that all ranks issue the same collective.
+
+    The coalesced buffer has ONE dtype: fp32, which holds fp16 / bf16 / fp32 gradients exactly (mixed-precision layers
+    keep fp32 weights and gradients, all-16-bit layers bf16 or fp16 ones), or fp64 when some layer has fp64 weights.
+    Every piece returns to its own parameter's dtype after the sum."""
     params = [p for p in _shift_weights(module_or_params)]
     if not params:
         return 0
-    flat = torch.cat([(p.grad if p.grad is not None else torch.zeros_like(p)).reshape(-1).to(torch.float32) for p in params])
+    wide = torch.float64 if any(p.dtype == torch.float64 for p in params) else torch.float32
+    flat = torch.cat([(p.grad if p.grad is not None else torch.zeros_like(p)).reshape(-1).to(wide) for p in params])
     dist.all_reduce(flat, op=dist.ReduceOp.SUM, group=group)
     if average:
         flat /= dist.get_world_size(group)
@@ -93,6 +98,8 @@ class FusedGradWeightAllReduce:
     * every rank runs the same sequence of shift backward calls with the same ``C x dim`` while the mode
       is enabled (true for replicated models); a rank whose batch shard is EMPTY still takes part and
       contributes zeros (``shard_batch`` hands empty slices to ranks beyond a ragged last batch);
+    * mixed-precision layers (fp16 / bf16 activations, fp32 weights) take part like any other: every contribution
+      travels as fp32 and their ``grad_weight`` is fp32;
     * fp64 weights, more than ``capacity`` weight elements or tensors on another device raise instead of
       silently skipping the exchange (a rank-local skip would leave the peers waiting);
     * the call counter lives in device memory, so a step that contains the exchange can be captured in a

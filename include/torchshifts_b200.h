@@ -21,7 +21,8 @@
  * Semantics (identical to the reference CPU path, see DESIGN.md):
  *   - tensors are [N, C, S0(, S1(, S2))], last axis fastest; `x` may have arbitrary element
  *     strides, every output (y, grad_input, grad_weight) and `grad` is dense;
- *   - weights are [C, dim] dense, same dtype as x; the integer/fractional split
+ *   - weights are [C, dim] dense, same dtype as x -- or fp32 for an fp16 / bf16 x when the dtype argument carries
+ *     TS_WEIGHTS_F32 (mixed precision: grad_weight is then fp32 too); the integer/fractional split
  *     (round-half-even for the sparse shift, floor for the active shift; the backward variant of
  *     ops/cpu/shifts_cpu.cpp:242-244) happens inside the kernels;
  *   - padding modes 0 zeros, 1 border, 2 periodic, 3 reflect, 4 symmetric
@@ -54,6 +55,14 @@ typedef enum ts_status {
 typedef enum ts_dtype {            /* element type of x / y / grad / weights                      */
     TS_F32 = 0, TS_F64 = 1, TS_F16 = 2, TS_BF16 = 3
 } ts_dtype;
+
+/* Flag OR'd into the `dtype` argument of the float entry points (ts_shift_forward, ts_shift_backward,
+ * ts_shift_backward_allreduce, ts_shift_backward_workspace_bytes, ts_shift_forward_nhwc, ts_shift_backward_nhwc,
+ * ts_shift_backward_nhwc_workspace_bytes, ts_shift2d_avgpool2_forward / _backward): `weights` is fp32 [C, dim] and
+ * grad_weight is written fp32, while x / y / grad / grad_input stay TS_F16 or TS_BF16 (mixed-precision training with fp32
+ * master weights).  The weights are split in fp32, never rounded to 16 bits.  Only with TS_F16 or TS_BF16: any other
+ * combination is TS_ERR_INVALID_ARGUMENT (the workspace queries return 0). */
+#define TS_WEIGHTS_F32 0x100
 
 typedef enum ts_padding {
     TS_PAD_ZEROS = 0, TS_PAD_BORDER = 1, TS_PAD_PERIODIC = 2, TS_PAD_REFLECT = 3, TS_PAD_SYMMETRIC = 4
@@ -143,7 +152,7 @@ int ts_shift2d_avgpool2_backward(const ts_geometry* g, int dtype, int padding, i
                                  void* workspace, size_t workspace_bytes, void* stream);
 
 /* grad: dense [N,C,rb-lb]; grad_input: dense like x's logical shape; grad_weight: dense [C,dim]
- * in `dtype`, fully overwritten (deterministic two-pass reduction, no atomics).
+ * in the weights' type (`dtype`, or fp32 under TS_WEIGHTS_F32), fully overwritten (deterministic two-pass reduction, no atomics).
  * workspace: >= ts_shift_backward_workspace_bytes(), 16-byte aligned. */
 int ts_shift_backward(const ts_geometry* g, int dtype, int padding, int active,
                       const void* grad, const void* x, const void* weights,

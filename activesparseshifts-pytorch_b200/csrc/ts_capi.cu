@@ -633,4 +633,62 @@ int ts_debug_nhwc_emulate(const ts_geometry* gin, int elem_bytes, int padding, i
                        sm_count_, max_grid_x, variant, ring_rows, true, nullptr);
 }
 
+int ts_debug_route(const ts_geometry* gin, int op, int dtype, int elem_bytes, int padding, int active, int64_t* out, int n_out) {
+    if (op < 0 || op > 2 || !out || n_out < 13) return TS_ERR_INVALID_ARGUMENT;
+    Geo g;
+    int rc = make_geo(gin, padding, &g);
+    if (rc != TS_OK) return rc;
+    int es = 0;
+    if (dtype == -1) {
+        if (op != 0) return TS_ERR_INVALID_ARGUMENT;
+        if (elem_bytes != 1 && elem_bytes != 4) return TS_ERR_UNSUPPORTED;
+        es = elem_bytes;
+    } else if ((dtype = weights_f32(dtype, &g)) < 0 || !(es = elem_size(dtype))) {
+        return TS_ERR_INVALID_ARGUMENT;
+    }
+    int sms = 0;
+    if ((rc = sm_count(&sms)) != TS_OK) return rc;
+    const Call c{op, op == 1 ? 1 : op == 2 ? (active != 0) : 0, es, dtype, 0ull, (const void*)256, (const void*)512,
+                 op == 2 ? (const void*)768 : nullptr};
+    Route r;
+    if ((rc = route(g, c, sms, &r)) != TS_OK) return rc;
+    int64_t v[13] = {r.path};
+    const bool table = g.C <= TABLE_MAX_C;
+    switch (r.path) {
+    case TS_PATH_TMA: {
+        const TmaPlan& p = r.tma;
+        const Levels lv(g);
+        const int ogr = lv.OL * (op == 0 ? es : dtype == TS_F32 ? 4 : 2) / 16;
+        const int64_t rest[12] = {p.tiles_per_plane, (lv.OA + p.ta - 1) / p.ta, (lv.OB + p.tb - 1) / p.tb, (ogr + p.tg - 1) / p.tg,
+                                  p.np, p.n_per_unit, p.units, p.grid, p.stages, p.warps, p.slots, table};
+        memcpy(v + 1, rest, sizeof(rest));
+        break;
+    }
+    case TS_PATH_STAGED: {
+        const StagedPlan& p = r.staged;
+        const int64_t rest[12] = {p.tiles, p.tiles, 1, 1, p.planes_per_step, p.n_per_unit, p.units, p.grid, p.stages, p.warps, p.slots,
+                                  p.table};
+        memcpy(v + 1, rest, sizeof(rest));
+        break;
+    }
+    case TS_PATH_HALO: {
+        const HaloPlan& p = r.halo;
+        const int64_t rest[12] = {1, 1, 1, 1, p.np, p.n_per_unit, p.units, p.grid, p.stages, p.warps, p.slots, table};
+        memcpy(v + 1, rest, sizeof(rest));
+        break;
+    }
+    case TS_PATH_FLAT: {
+        const FlatPlan& p = r.flat;       // units are stages of np (n, c) planes; n_per_unit is the warp-per-plane (table) flag
+        const int64_t rest[12] = {1, 1, 1, 1, p.np, 0, p.units, p.grid, p.stages, p.warps, 0, p.n_per_unit};
+        memcpy(v + 1, rest, sizeof(rest));
+        break;
+    }
+    default:
+        v[7] = op == 2 ? r.generic.units : 0;
+        v[11] = r.slots;
+    }
+    for (int i = 0; i < n_out; ++i) out[i] = i < 13 ? v[i] : 0;
+    return TS_OK;
+}
+
 }  // extern "C"

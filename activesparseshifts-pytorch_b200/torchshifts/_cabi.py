@@ -50,6 +50,7 @@ SIGNATURES = {
     'ts_qshift_forward': (_i, [_geo, _i, _i, _i64, _vp, _vp, _i, _i64, _vp, _vp]),
     'ts_qshift_forward_nhwc': (_i, [_geo, _i, _i, _i64, _vp, _vp, _i, _i64, _vp, _vp]),
     'ts_debug_nhwc_emulate': (_i, [_geo, _i, _i, _i64, _vp, _vp, _i, _i64, _vp, _i, _i, _i, _i]),
+    'ts_debug_route': (_i, [_geo, _i, _i, _i, _i, _i, _i64p, _i]),
     'ts_nhwc_to_nchw': (_i, [_vp, _vp, _i64, _i64, _i64, _i, _vp]),
     'ts_shift_backward_allreduce': (_i, [_geo, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _peers, _vp]),
     'ts_shift_forward_nhwc': (_i, [_geo, _i, _i, _i, _vp, _vp, _vp, _vp]),

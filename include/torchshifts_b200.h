@@ -239,6 +239,15 @@ int ts_debug_nhwc_emulate(const ts_geometry* g, int elem_bytes, int padding, int
                           int64_t weight_zero_point, void* yq_host, int sm_count, int max_grid_x,
                           int variant, int ring_rows);
 
+/* Test aid: no GPU work.  Runs the planar entry points' own route() for a call -- current forced path and tuning knobs,
+ * this device's SM count, placeholder 256-byte-aligned pointers -- and writes what it chose:
+ * out[0] path, then the plan's tiles_per_plane, tiles per level (a, b, g), images per stage, images per unit, units, grid,
+ * stages, consumer warps, partial slots, table (0/1).  op: 0 sparse/quantized forward, 1 active forward, 2 backward.
+ * dtype as for ts_shift_forward (TS_WEIGHTS_F32 allowed), or -1 with elem_bytes for the quantized forward (zero point 0).
+ * n_out >= 13.  Fields a family does not have are 0 (the flat gather: images per stage counts (n, c) planes).
+ * Returns the status the entry point's routing would return. */
+int ts_debug_route(const ts_geometry* g, int op, int dtype, int elem_bytes, int padding, int active, int64_t* out, int n_out);
+
 #ifdef __cplusplus
 }
 #endif

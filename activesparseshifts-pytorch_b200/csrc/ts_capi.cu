@@ -480,7 +480,7 @@ int ts_shift2d_avgpool2_backward(const ts_geometry* gin, int dtype, int padding,
     if (!hp.ok) return TS_ERR_UNSUPPORTED;
     t_last_path = TS_PATH_HALO;
     cudaStream_t s = (cudaStream_t)stream;
-    rc = halo_backward(g, hp, active, grad_pooled, x, weights, grad_input, (double*)workspace, s, true);
+    rc = halo_backward(g, hp, active, grad_pooled, x, weights, grad_input, (double*)workspace, s);
     return rc != TS_OK ? rc : reduce_partials(g, dtype, (double*)workspace, hp.slots, grad_weight, nullptr, s);
 }
 
@@ -653,33 +653,29 @@ int ts_debug_route(const ts_geometry* gin, int op, int dtype, int elem_bytes, in
     Route r;
     if ((rc = route(g, c, sms, &r)) != TS_OK) return rc;
     int64_t v[13] = {r.path};
-    const bool table = g.C <= TABLE_MAX_C;
     switch (r.path) {
     case TS_PATH_TMA: {
-        const TmaPlan& p = r.tma;
-        const Levels lv(g);
-        const int ogr = lv.OL * (op == 0 ? es : dtype == TS_F32 ? 4 : 2) / 16;
-        const int64_t rest[12] = {p.tiles_per_plane, (lv.OA + p.ta - 1) / p.ta, (lv.OB + p.tb - 1) / p.tb, (ogr + p.tg - 1) / p.tg,
-                                  p.np, p.n_per_unit, p.units, p.grid, p.stages, p.warps, p.slots, table};
+        const TArgs& a = r.tma.a;
+        const int64_t rest[12] = {a.tiles, a.tiles / (a.tiles_b * a.tiles_g), a.tiles_b, a.tiles_g,
+                                  a.np, a.n_per_unit, a.units, r.tma.grid, a.stages, a.nw, r.slots, a.table};
         memcpy(v + 1, rest, sizeof(rest));
         break;
     }
     case TS_PATH_STAGED: {
-        const StagedPlan& p = r.staged;
-        const int64_t rest[12] = {p.tiles, p.tiles, 1, 1, p.planes_per_step, p.n_per_unit, p.units, p.grid, p.stages, p.warps, p.slots,
-                                  p.table};
+        const SArgs& a = r.staged.a;
+        const int64_t rest[12] = {a.tiles, a.tiles, 1, 1, a.np, a.n_per_unit, a.units, r.staged.grid, a.stages, a.nw, r.slots, a.table};
         memcpy(v + 1, rest, sizeof(rest));
         break;
     }
     case TS_PATH_HALO: {
-        const HaloPlan& p = r.halo;
-        const int64_t rest[12] = {1, 1, 1, 1, p.np, p.n_per_unit, p.units, p.grid, p.stages, p.warps, p.slots, table};
+        const HArgs& a = r.halo.a;
+        const int64_t rest[12] = {1, 1, 1, 1, a.np, a.n_per_unit, a.units, r.halo.grid, a.stages, a.nw, r.slots, a.table};
         memcpy(v + 1, rest, sizeof(rest));
         break;
     }
     case TS_PATH_FLAT: {
-        const FlatPlan& p = r.flat;       // units are stages of np (n, c) planes; n_per_unit is the warp-per-plane (table) flag
-        const int64_t rest[12] = {1, 1, 1, 1, p.np, 0, p.units, p.grid, p.stages, p.warps, 0, p.n_per_unit};
+        const FArgs& a = r.flat.a;        // units are stages of K (n, c) planes; the table flag selects the warp-per-plane variant
+        const int64_t rest[12] = {1, 1, 1, 1, a.K, 0, a.nstages, r.flat.grid, a.stages, a.nw, 0, a.table};
         memcpy(v + 1, rest, sizeof(rest));
         break;
     }

@@ -40,6 +40,18 @@ struct Geo {
 // Tensor axis of a LEVEL (0 slab, 1 row, 2 column) of a `dim`-dimensional geometry; negative: the level is absent.
 TS_HD int level_axis(int level, int dim) { return level - (3 - dim); }
 
+// Exact division by a launch-invariant (n < 2^31), set up on the host; the device side is fdiv (ts_ptx.cuh).
+struct FastDiv { unsigned m, l, d; };
+inline FastDiv make_fastdiv(unsigned d) {
+    FastDiv f;
+    f.d = d ? d : 1;
+    unsigned l = 0;
+    while ((1ull << l) < f.d) ++l;
+    f.l = l;
+    f.m = (unsigned)(((((unsigned long long)1 << l) - f.d) << 32) / f.d + 1);
+    return f;
+}
+
 // ------------------------------------------------------------------------------------------
 // Index remap.
 TS_HD int pmod(int a, int b) { return (b + (a % b)) % b; }

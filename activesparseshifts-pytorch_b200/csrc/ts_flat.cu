@@ -34,23 +34,6 @@ using namespace ptx;
 constexpr int GUARD = 32;
 constexpr int MAX_K = 32;          // planes per stage: one lane of a warp per plane
 
-struct FArgs {
-    Geo g;
-    const unsigned char* x;
-    unsigned char* y;
-    const void* w;
-    long long wzp;
-    long long planes;          // N * C
-    unsigned fillw;            // pad value replicated to 32 bits
-    int qkind, wk, es, dim;
-    int B, Lb;                 // rows per plane, bytes per row
-    int plane_bytes, ipp;      // bytes / 16-byte items of one plane
-    int K, stages, stage_stride, nw;
-    int nstages;               // ceil(planes / K)
-    int table;                 // per-channel (row shift, column shift in bytes) table in shared memory
-    FastDiv d_ipp, d_Lb, d_C;
-};
-
 // (row shift, column shift in bytes) of channel c; a size-1 axis ignores its shift (reduce_shift)
 TS_D void flat_shift(const FArgs& a, long long c, int& sr, int& scb) {
     int s[2] = {0, 0};
@@ -301,9 +284,21 @@ FlatPlan plan_flat(const Geo& g, int esize, bool dense_x, const void* x, const v
     const long long grid_max = (long long)sm_count * ctas;
     int warps = t.flat_warps > 0 ? t.flat_warps : (ctas >= 2 ? (wp ? 8 : 7) : 15);
     if (warps > 15) warps = 15;
+    FArgs& a = p.a;
+    a.g = g;
+    a.planes = g.N * g.C;
+    a.es = esize; a.dim = d;
+    a.B = (int)B;
+    a.Lb = (int)Lb;
+    a.plane_bytes = (int)plane;
+    a.ipp = a.plane_bytes / 16;
+    a.K = (int)K; a.stages = stages; a.stage_stride = (int)stride_of(K); a.nw = warps;
+    a.nstages = (int)nstages;
+    a.table = wp ? 1 : 0;
+    a.d_ipp = make_fastdiv((unsigned)a.ipp);
+    a.d_Lb = make_fastdiv((unsigned)a.Lb);
+    a.d_C = make_fastdiv((unsigned)g.C);
     p.ok = true;
-    p.np = (int)K; p.stages = stages; p.stage_stride = (int)stride_of(K); p.warps = warps;
-    p.n_per_unit = wp ? 1 : 0; p.units = (int)nstages;      // n_per_unit doubles as the variant flag
     p.grid = (int)(nstages < grid_max ? nstages : grid_max);
     p.smem_bytes = (size_t)(stages * stride_of(K) + 16 * stages + 64 + table_bytes);
     return p;
@@ -311,25 +306,11 @@ FlatPlan plan_flat(const Geo& g, int esize, bool dense_x, const void* x, const v
 
 int flat_gather(const Geo& g, const FlatPlan& p, int wk, const void* x, void* y, unsigned long long fill, int esize, const void* w,
                 int qkind, long long wzp, cudaStream_t s) {
-    FArgs a;
-    memset(&a, 0, sizeof(a));
-    const int d = g.dim;
-    a.g = g;
+    FArgs a = p.a;
     a.x = (const unsigned char*)x; a.y = (unsigned char*)y; a.w = w; a.wzp = wzp;
-    a.planes = g.N * g.C;
     a.fillw = esize == 1 ? 0x01010101u * (unsigned)(fill & 0xffu) : esize == 2 ? 0x00010001u * (unsigned)(fill & 0xffffu) : (unsigned)fill;
-    a.qkind = qkind; a.wk = wk; a.es = esize; a.dim = d;
-    a.B = d == 2 ? g.S[0] : 1;
-    a.Lb = g.S[d - 1] * esize;
-    a.plane_bytes = a.B * a.Lb;
-    a.ipp = a.plane_bytes / 16;
-    a.K = p.np; a.stages = p.stages; a.stage_stride = p.stage_stride; a.nw = p.warps;
-    a.nstages = p.units;
-    a.d_ipp = make_fastdiv((unsigned)a.ipp);
-    a.d_Lb = make_fastdiv((unsigned)a.Lb);
-    a.table = p.n_per_unit;
-    a.d_C = make_fastdiv((unsigned)g.C);
-    return launch_persistent(a.table ? k_flat_gather_wp : k_flat_gather, p.grid, (p.warps + 1) * 32, p.smem_bytes, s, false, a);
+    a.qkind = qkind; a.wk = wk;
+    return launch_persistent(a.table ? k_flat_gather_wp : k_flat_gather, p.grid, (a.nw + 1) * 32, p.smem_bytes, s, false, a);
 }
 
 }  // namespace ts

@@ -42,38 +42,6 @@ using namespace ptx;
 constexpr int MAXT = 512;
 constexpr int GUARD = 128;          // readable slack before / after the tiles of a stage (window pairs may start 16 bytes early)
 
-struct alignas(64) HArgs {
-    CUtensorMap map_x;       // x,    box {px, bpx, 1, 1, 1}
-    CUtensorMap map_g;       // grad, box {pg, bpg, 1, 1, 1}
-    CUtensorMap map_v;       // grad, box {OL, OB, 1, 1, 1}   (dense slab: unshifted grad of the 3-D backward)
-                             // fused avg-pool backward: the POOLED grad, box {PW, PH, 1, 1, 1}
-    Geo g;
-    const float* x;
-    const float* grad;
-    float* out;
-    const float* w;
-    double* partials;
-    int mode, active, dim;
-    int A, B, L, OA, OB, OL, lbA, lbB, lbL;   // per level (0 slab, 1 row, 2 column); 2-D: A = OA = 1
-    int IA, IB, IG, GP;                       // iteration space (output space forward, input space backward): slabs, rows, groups; padded groups
-    int RP;                                   // row pairs per slab = ceil(IB / 2)
-    int hr, hc;
-    int px, bpx, pg, bpg;
-    int tile_x, tile_g, tile_v;               // bytes between consecutive tiles (128-byte multiples)
-    int box_x, box_g, box_v;                  // bytes one TMA box delivers
-    int off_g, off_v;                         // byte offsets of the grad tiles / dense grad tiles inside a stage (after GUARD)
-    int stage_stride, stages, nw, nt, np;
-    int img_pairs, pairs;                     // RP * GP, np * RP * GP
-    int n_per_unit, units, chunks, unit_order;
-    long long out_plane_bytes;                // bytes of one (n, c) plane of the OUTPUT (pooled plane for the fused avg-pool epilogue)
-    int pool;                                 // forward only: 2x2 / stride 2 / ceil_mode average pooling fused into the store
-    int need_fix;                             // padding != zeros: a fixer warp patches the halo of every stage
-    int table;                                // per-channel shift table in shared memory (C <= TABLE_MAX_C)
-    FastDiv d_GP, d_img, d_C, d_chunks, d_PW;
-    int nfix;                                 // fixer warps (1; 4 when they also expand the pooled gradient)
-    int pool_bwd, PH, PW;                     // backward fused with the adjoint of avg_pool2d(2, 2, ceil_mode): pooled rows / columns
-};
-
 struct UnitShift {
     int sx[3], sg[3];      // per level; absent levels 0
     float d[3];            // per TENSOR axis
@@ -1167,58 +1135,19 @@ __global__ void __launch_bounds__(MAXT, 1) k_halo(const __grid_constant__ HArgs 
 }
 
 int launch(void (*kernel)(HArgs), const HArgs& a, const HaloPlan& p, cudaStream_t s) {
-    return launch_persistent(kernel, p.grid, (p.warps + 1 + (a.need_fix ? a.nfix : 0)) * 32, p.smem_bytes, s, false, a);
+    return launch_persistent(kernel, p.grid, (a.nw + 1 + (a.need_fix ? a.nfix : 0)) * 32, p.smem_bytes, s, false, a);
 }
 
-bool make_args(const Geo& g, const HaloPlan& p, int mode, int active, int pool, const void* x, const void* grad, void* out, const void* w,
-               double* partials, HArgs* o, bool pool_bwd = false) {
-    HArgs& a = *o;
-    memset(&a, 0, sizeof(a));
-    const int d = g.dim;
-    const Levels lv(g);
-    a.g = g;
+// The pointers and tensor maps of one launch; false: a map could not be encoded.
+bool bind(HArgs& a, const void* x, const void* grad, void* out, const void* w, double* partials) {
+    const Geo& g = a.g;
     a.x = (const float*)x; a.grad = (const float*)grad; a.out = (float*)out; a.w = (const float*)w; a.partials = partials;
-    a.mode = mode; a.active = active; a.dim = d;
-    a.A = lv.A;    a.OA = lv.OA;    a.lbA = lv.lbA;
-    a.B = lv.B;    a.OB = lv.OB;    a.lbB = lv.lbB;
-    a.L = lv.L;    a.OL = lv.OL;    a.lbL = lv.lbL;
-    a.IA = mode == 2 ? a.A : a.OA;
-    a.IB = mode == 2 ? a.B : a.OB;
-    a.IG = (mode == 2 ? a.L : a.OL) / 4;
-    a.GP = p.GP;
-    a.RP = (a.IB + 1) / 2;
-    a.hr = p.hr; a.hc = p.hc;
-    a.px = p.px; a.bpx = p.bpx; a.pg = p.pg; a.bpg = p.bpg;
-    a.tile_x = p.tile_x; a.tile_g = p.tile_g; a.tile_v = p.tile_v;
-    a.box_x = p.px * p.bpx * 4; a.box_g = p.pg * p.bpg * 4; a.box_v = a.OL * a.OB * 4;
-    a.np = p.np;
-    a.off_g = p.np * p.tile_x;
-    a.off_v = a.off_g + p.np * p.tile_g;
-    a.stage_stride = p.stage_stride; a.stages = p.stages; a.nw = p.warps; a.nt = p.warps * 32;
-    a.img_pairs = a.RP * a.GP;
-    a.pairs = a.np * a.img_pairs;
-    a.n_per_unit = p.n_per_unit; a.units = p.units;
-    a.chunks = (int)(p.units / (g.C > 0 ? g.C : 1));
-    a.unit_order = tuning().unit_order;
-    a.d_C = make_fastdiv((unsigned)g.C);
-    a.d_chunks = make_fastdiv((unsigned)a.chunks);
-    a.table = g.C <= TABLE_MAX_C ? 1 : 0;
-    a.pool = pool;
-    a.out_plane_bytes = pool ? (long long)((a.OB + 1) / 2) * (a.OL / 2) * 4 : (mode == 2 ? g.in_plane : g.out_plane) * 4;
-    a.pool_bwd = pool_bwd ? 1 : 0;
-    a.PH = (a.OB + 1) / 2; a.PW = a.OL / 2;
-    a.need_fix = g.pad != TS_PAD_ZEROS || pool_bwd;
-    a.nfix = pool_bwd ? 4 : 1;
-    if (pool_bwd) a.box_v = a.PW * a.PH * 4;
-    a.d_PW = make_fastdiv((unsigned)(a.PW > 0 ? a.PW : 1));
-    a.d_GP = make_fastdiv((unsigned)a.GP);
-    a.d_img = make_fastdiv((unsigned)a.img_pairs);
     if (!make_tensor_map5(&a.map_x, x, 4, g.N, g.C, a.A, a.B, a.L, a.px, a.bpx, 1, 1)) return false;
-    if (mode == 2 && pool_bwd) {
+    if (a.mode == 2 && a.pool_bwd) {
         if (!make_tensor_map5(&a.map_v, grad, 4, g.N, g.C, 1, a.PH, a.PW, a.PW, a.PH, 1, 1)) return false;
-    } else if (mode == 2) {
+    } else if (a.mode == 2) {
         if (!make_tensor_map5(&a.map_g, grad, 4, g.N, g.C, a.OA, a.OB, a.OL, a.pg, a.bpg, 1, 1)) return false;
-        if (d == 3 && !make_tensor_map5(&a.map_v, grad, 4, g.N, g.C, a.OA, a.OB, a.OL, a.OL, a.OB, 1, 1)) return false;
+        if (a.dim == 3 && !make_tensor_map5(&a.map_v, grad, 4, g.N, g.C, a.OA, a.OB, a.OL, a.OL, a.OB, 1, 1)) return false;
     }
     return true;
 }
@@ -1246,24 +1175,36 @@ HaloPlan plan_halo(const Geo& g, int mode, int active, int dtype, bool dense_x, 
     if (g.N >= (1ll << 31) || g.C >= (1ll << 31)) return p;
     if (g.in_plane * 4 >= (1ll << 40) / (g.C > 0 ? g.C : 1)) return p;
     const Tuning& t = tuning();
+    HArgs& a = p.a;
+    a.g = g;
+    a.mode = mode; a.active = active ? 1 : 0; a.dim = d;
+    a.A = lv.A;    a.OA = lv.OA;    a.lbA = lv.lbA;
+    a.B = B;       a.OB = OB;       a.lbB = lv.lbB;
+    a.L = L;       a.OL = OL;       a.lbL = lv.lbL;
     const int halo = t.halo > 0 ? t.halo : 4;
-    p.hr = halo;
-    p.hc = (halo + 3) / 4 * 4;
+    a.hr = halo;
+    a.hc = (halo + 3) / 4 * 4;
     // row pitch = 4 (mod 8) words: the fixer warp walks DOWN the rows of a halo column (4-way bank conflicts instead of 32-way)
-    p.px = L + 2 * p.hc;   p.bpx = B + 2 * p.hr;
-    p.pg = OL + 2 * p.hc;  p.bpg = OB + 2 * p.hr;
-    if (p.px % 8 == 0) p.px += 4;
-    if (p.pg % 8 == 0) p.pg += 4;
-    if (p.px > 256 || p.bpx > 256 || p.pg > 256 || p.bpg > 256) return p;           // TMA box extents
-    p.tile_x = (int)round_up((long long)p.px * p.bpx * 4, 128);
-    p.tile_g = mode == 2 ? (int)round_up((long long)p.pg * p.bpg * 4, 128) : 0;
-    p.tile_v = (mode == 2 && d == 3) ? (int)round_up((long long)OL * OB * 4, 128) : 0;
-    p.tile_p = pool_bwd ? (int)round_up((long long)((OB + 1) / 2) * (OL / 2) * 4, 128) : 0;
-    if (pool_bwd) p.tile_v = p.tile_p;
-    const long long per_image = (long long)p.tile_x + p.tile_g + p.tile_v;
-    const int IB = mode == 2 ? B : OB, IG = (mode == 2 ? L : OL) / 4;
-    const int GP = padded_groups(IG);
-    const int img_pairs = (IB + 1) / 2 * GP;
+    a.px = L + 2 * a.hc;   a.bpx = B + 2 * a.hr;
+    a.pg = OL + 2 * a.hc;  a.bpg = OB + 2 * a.hr;
+    if (a.px % 8 == 0) a.px += 4;
+    if (a.pg % 8 == 0) a.pg += 4;
+    if (a.px > 256 || a.bpx > 256 || a.pg > 256 || a.bpg > 256) return p;           // TMA box extents
+    a.PH = (OB + 1) / 2; a.PW = OL / 2;
+    a.pool_bwd = pool_bwd ? 1 : 0;
+    a.need_fix = g.pad != TS_PAD_ZEROS || pool_bwd;
+    a.nfix = pool_bwd ? 4 : 1;
+    a.tile_x = (int)round_up((long long)a.px * a.bpx * 4, 128);
+    a.tile_g = mode == 2 ? (int)round_up((long long)a.pg * a.bpg * 4, 128) : 0;
+    // the dense grad slab of the 3-D backward, or the pooled-gradient tile of the fused avg-pool backward
+    a.tile_v = pool_bwd ? (int)round_up((long long)a.PH * a.PW * 4, 128) : (mode == 2 && d == 3) ? (int)round_up((long long)OL * OB * 4, 128) : 0;
+    a.box_x = a.px * a.bpx * 4; a.box_g = a.pg * a.bpg * 4; a.box_v = pool_bwd ? a.PW * a.PH * 4 : OL * OB * 4;
+    const long long per_image = (long long)a.tile_x + a.tile_g + a.tile_v;
+    a.IA = mode == 2 ? a.A : a.OA;
+    const int IB = a.IB = mode == 2 ? B : OB, IG = a.IG = (mode == 2 ? L : OL) / 4;
+    const int GP = a.GP = padded_groups(IG);
+    a.RP = (IB + 1) / 2;
+    const int img_pairs = a.img_pairs = a.RP * GP;
     const int max_nt = MAXT - 64 - (pool_bwd ? 96 : 0);    // producer warp + fixer warp(s)
     const long long table_bytes = (g.C <= TABLE_MAX_C ? g.C * 36 : 0) + ((g.pad != TS_PAD_ZEROS || pool_bwd) ? 2 * FIXCAP * 4 : 0)      // + the fixer's cell lists
                                   + (2 * NCLS + 1) * 4 + (g.C <= TABLE_MAX_C ? g.C * 3 : 0) + 16;                             // + the class order
@@ -1277,7 +1218,7 @@ HaloPlan plan_halo(const Geo& g, int mode, int active, int dtype, bool dense_x, 
     }
     if (np < 1) np = 1;
     if (np > g.N) np = g.N;
-    const long long tail = 4ll * (p.px > p.pg ? p.px : p.pg) + 256;       // a masked row may be read one row past the last tile
+    const long long tail = 4ll * (a.px > a.pg ? a.px : a.pg) + 256;       // a masked row may be read one row past the last tile
     auto stride_of = [&](long long n) { return round_up(n * per_image + GUARD + tail, 1024); };
     const int min_stages = d == 3 ? 3 : 2;
     while (np > 1 && budget / (stride_of(np) + 24) < min_stages + 1) --np;
@@ -1307,37 +1248,49 @@ HaloPlan plan_halo(const Geo& g, int mode, int active, int dtype, bool dense_x, 
     const UnitPlan up = plan_units(np, t.chunk_planes > 0 ? t.chunk_planes : pick_unit_images(g.N, g.C, np, sm_count, mode == 2 ? 0.4 : 0.1),
                                    g.N, g.C, sm_count, warps);
     if (!up.ok) return p;
+    a.np = (int)np; a.pairs = (int)pairs;
+    a.off_g = a.np * a.tile_x;
+    a.off_v = a.off_g + a.np * a.tile_g;
+    a.stages = (int)stages; a.stage_stride = (int)stride_of(np); a.nw = warps; a.nt = warps * 32;
+    a.n_per_unit = up.n_per_unit; a.units = up.units; a.chunks = up.chunks; a.unit_order = t.unit_order;
+    a.table = g.C <= TABLE_MAX_C ? 1 : 0;
+    a.out_plane_bytes = (mode == 2 ? g.in_plane : g.out_plane) * 4;
+    a.d_GP = make_fastdiv((unsigned)GP);
+    a.d_img = make_fastdiv((unsigned)img_pairs);
+    a.d_C = make_fastdiv((unsigned)g.C);
+    a.d_chunks = make_fastdiv((unsigned)a.chunks);
+    a.d_PW = make_fastdiv((unsigned)(a.PW > 0 ? a.PW : 1));
     p.ok = true;
-    p.np = (int)np; p.GP = GP; p.positions = (int)pairs; p.ncol = 1;
-    p.stages = (int)stages; p.stage_stride = (int)stride_of(np); p.warps = warps;
-    p.n_per_unit = up.n_per_unit; p.units = up.units; p.grid = up.grid; p.slots = up.slots;
+    p.grid = up.grid; p.slots = up.slots;
     p.smem_bytes = (size_t)(stages * stride_of(np) + 24 * stages + 64 + table_bytes);
     return p;
 }
 
 int halo_active_forward(const Geo& g, const HaloPlan& p, const void* x, const void* w, void* y, cudaStream_t s) {
-    HArgs a;
-    if (!make_args(g, p, 1, 1, 0, x, nullptr, y, w, nullptr, &a)) return TS_ERR_UNSUPPORTED;
+    HArgs a = p.a;
+    if (!bind(a, x, nullptr, y, w, nullptr)) return TS_ERR_UNSUPPORTED;
     return g.dim == 3 ? launch(k_halo<3, 1, true, false>, a, p, s) : launch(k_halo<2, 1, true, false>, a, p, s);
 }
 
 // 2-D forward (sparse or active) with the 2x2 / stride-2 / ceil_mode average pooling of modules/shifts.py:85-89 fused
 // into the store: one read of x, one QUARTER-size write (pool == 0: the plain 2-D forward through the same kernels).
 int halo_forward2d(const Geo& g, const HaloPlan& p, int active, int pool, const void* x, const void* w, void* y, cudaStream_t s) {
-    HArgs a;
     if (g.dim != 2) return TS_ERR_UNSUPPORTED;
-    if (!make_args(g, p, active ? 1 : 0, active ? 1 : 0, pool, x, nullptr, y, w, nullptr, &a)) return TS_ERR_UNSUPPORTED;
+    HArgs a = p.a;
+    a.pool = pool;
+    if (pool) a.out_plane_bytes = (long long)a.PH * a.PW * 4;
+    if (!bind(a, x, nullptr, y, w, nullptr)) return TS_ERR_UNSUPPORTED;
     if (active) return pool ? launch(k_halo<2, 1, true, true>, a, p, s) : launch(k_halo<2, 1, true, false>, a, p, s);
     return pool ? launch(k_halo<2, 0, false, true>, a, p, s) : launch(k_halo<2, 0, false, false>, a, p, s);
 }
 
 int halo_backward(const Geo& g, const HaloPlan& p, int active, const void* grad, const void* x, const void* w, void* gi,
-                  double* partials, cudaStream_t s, bool pool_bwd) {
-    HArgs a;
-    if (!make_args(g, p, 2, active ? 1 : 0, 0, x, grad, gi, w, partials, &a, pool_bwd)) return TS_ERR_UNSUPPORTED;
+                  double* partials, cudaStream_t s) {
+    HArgs a = p.a;
+    if (!bind(a, x, grad, gi, w, partials)) return TS_ERR_UNSUPPORTED;
     bool crop = false;
     for (int ax = 0; ax < g.dim; ++ax) crop = crop || g.lb[ax] != 0 || g.OS[ax] != g.S[ax];
-    if (pool_bwd) {
+    if (a.pool_bwd) {
         if (g.dim != 2) return TS_ERR_UNSUPPORTED;
         if (active) return crop ? launch(k_halo<2, 2, true, true, true>, a, p, s) : launch(k_halo<2, 2, true, true, false>, a, p, s);
         return crop ? launch(k_halo<2, 2, false, true, true>, a, p, s) : launch(k_halo<2, 2, false, true, false>, a, p, s);

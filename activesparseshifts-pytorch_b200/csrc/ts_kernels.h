@@ -1,5 +1,11 @@
 // ts_kernels.h -- internal interface between the C ABI (ts_capi.cu) and the kernel families.
+//
+// A persistent family's plan (TmaPlan, StagedPlan, HaloPlan, FlatPlan) is the launch shape plus the argument block its
+// kernels receive: the planner fills every field that does not depend on a pointer, the launcher adds the pointers,
+// the weight kind, the quantized arguments and the tensor maps.
 #pragma once
+#include <cuda.h>
+
 #include "ts_common.cuh"
 
 namespace ts {
@@ -46,10 +52,10 @@ struct Levels {
 
 // Work units of a persistent kernel: (channel, chunk of `n_per_unit` images of the batch), dealt to `grid` CTAs; each of the
 // `warps` consumer warps writes one grad_weight partial per chunk (`slots`).  `npu` is the family's proposed images per unit,
-// rounded here to a multiple of the `np` images of one stage.  ok = false: a count overflows 32 bits.
-struct UnitPlan { bool ok; int n_per_unit, units, grid, slots; };
+// rounded here to a multiple of the `np` images of one stage; units = chunks * C.  ok = false: a count overflows 32 bits.
+struct UnitPlan { bool ok; int n_per_unit, chunks, units, grid, slots; };
 inline UnitPlan plan_units(long long np, long long npu, long long N, long long C, long long grid_max, int warps) {
-    UnitPlan u = {false, 0, 0, 0, 0};
+    UnitPlan u = {false, 0, 0, 0, 0, 0};
     npu = (npu / np) * np;
     if (npu < np) npu = np;
     if (npu > N) npu = N;
@@ -58,6 +64,7 @@ inline UnitPlan plan_units(long long np, long long npu, long long N, long long C
     if (units > 0x7fffffffLL || chunks * warps > 0x7fffffffLL) return u;
     u.ok = true;
     u.n_per_unit = (int)npu;
+    u.chunks = (int)chunks;
     u.units = (int)units;
     u.grid = (int)(units < grid_max ? units : grid_max);
     u.slots = (int)(chunks * warps);
@@ -138,16 +145,35 @@ struct Tuning {
 };
 Tuning& tuning();
 
+struct SArgs {
+    Geo g;
+    const unsigned char* x;
+    const unsigned char* grad;
+    unsigned char* out;
+    const void* w;
+    double* partials;
+    long long wzp;
+    unsigned long long fill;
+    int qkind, wk, es, mode, active;
+    int A, B, L, OA, OB, OL, lbA, lbB, lbL;   // sizes per level (0 slab, 1 row, 2 column); absent levels 1 / 0
+    int IA, IB;                               // iteration space: output space (forward) / input space (backward)
+    int VB, V;                                // bytes / elements per item
+    int gpr, GP;                              // items per iteration-space row; padded row length of the index space
+    int TA, tiles;                            // slabs per tile, tiles per image
+    int xs, gvs, gis;                         // slab slots per image: x, grad at the output position, grad for grad_input (0: shares gvs)
+    int slab_x, slab_g;                       // bytes of one slab of x / of grad
+    int np, stages, stage_stride, nw, n_per_unit, units, chunks, unit_order;
+    int off_gv, off_gi;                       // byte offsets of the grad regions inside a stage (after GUARD)
+    int table;                                // per-channel shift parameters tabulated in shared memory (arithmetic kernels, C <= TABLE_MAX_C)
+    int img_items;                            // TA * IB * GP
+    long long img_stride;                     // output bytes between consecutive images of one channel
+    FastDiv d_img, d_GP, d_IB;
+};
 struct StagedPlan {
     bool ok;           // staged path applicable
-    int vec_bytes;     // bytes per thread item (16 / 8 / 4)
-    int planes_per_step, stages, stage_stride, warps, grid, units, n_per_unit, slots;  // slots = partial slots (backward)
-    bool table;        // per-channel shift parameters tabulated in shared memory
-    int ta, tiles;     // slabs per tile (3-D volumes are tiled over their first axis), tiles per image
-    int xs, gvs, gis;  // slab slots per image: x, grad at the output position, grad for grad_input (0: shares gvs)
-    int gp;            // padded items per row of the item index space
-    int off_gv, off_gi;
+    int grid, slots;   // slots = partial slots (backward)
     size_t smem_bytes;
+    SArgs a;
 };
 // mode: 0 sparse/quantized forward (esize = element bytes), 1 active forward, 2 backward
 StagedPlan plan_staged(const Geo& g, int mode, int active, int esize, int dtype, bool dense_x, const void* x, const void* y_or_gi,
@@ -160,14 +186,39 @@ int staged_backward(const Geo& g, const StagedPlan& p, int dtype, int active, co
                     void* gi, double* partials, cudaStream_t s);
 
 // ---- TMA-tensor family (ts_tma.cu): zeros padding done by the copy engine ----------------------
+struct alignas(64) TArgs {
+    CUtensorMap map_x;       // x,    box {(TG+1)*vec, xb, xa, 1, np}
+    CUtensorMap map_gs;      // grad, box {(TG+1)*vec, TB, TA, 1, np}     (backward)
+    CUtensorMap map_gb;      // grad, box {(TG+1)*vec, xb, xa, 1, np}     (active backward)
+    Geo g;
+    unsigned char* out;
+    const void* w;
+    double* partials;
+    long long wzp;
+    int qkind, wk, es, vec;  // vec = elements per 16-byte group
+    int mode, active;
+    int OA, OB, OGR;         // output slabs, rows, 16-byte groups per row
+    int lbA, lbB, lbL;
+    int TA, TB, TG;          // tile extents (slabs, rows, groups)
+    int xa, xb;              // x box slabs / rows (TA or TA+1, TB or TB+1)
+    int tiles_b, tiles_g, tiles;
+    int np;                  // images per stage (1 unless a whole plane is one tile)
+    int x_img_chunks;        // 16-byte groups of one image's x box
+    int g_img_chunks;        // 16-byte groups of one image's small grad box
+    int off_gv, off_g2;      // byte offsets of the grad boxes inside a stage
+    int tx_bytes;            // bytes landing per stage
+    int stage_stride, stages, nw, n_per_unit, units, chunks, unit_order;
+    int GP, img_items;       // padded groups per row of the item index space; items per image = TA*TB*GP
+    int img_stride16;        // output distance between consecutive images of one channel, in 16-byte units
+    int R, nchunk;           // strip-mined arithmetic kernels: rows per strip, strips per tile column
+    FastDiv d_img, d_GP, d_TB, d_tg, d_tb, d_TG, d_nchunk, d_TA, d_C, d_chunks;
+    int table;               // per-channel shift table in shared memory (C <= TABLE_MAX_C): built once per CTA
+};
 struct TmaPlan {
     bool ok;
-    int ta, tb, tg, gp;        // tile extents: slabs, rows, 16-byte column groups; gp = padded groups per row (index space)
-    int xa, xb;                // x box slabs / rows (tile + the +1 neighbours of the arithmetic kernels)
-    int tiles_per_plane, np;   // np = images per stage
-    int off_gv, off_g2, tx_bytes;
-    int stages, stage_stride, n_per_unit, units, grid, warps, slots;
+    int grid, slots;
     size_t smem_bytes;
+    TArgs a;
 };
 // mode: 0 sparse/quantized forward, 1 active forward, 2 backward (active = interpolating backward)
 TmaPlan plan_tma(const Geo& g, int mode, int active, int esize, int dtype, bool dense_x, unsigned long long fill, const void* x,
@@ -185,35 +236,79 @@ bool tma_available();
 bool make_tensor_map5(void* map, const void* base, int es, long long N, long long C, int A, int B, int L, int bl, int bb, int ba, int bn);
 
 // ---- flat gather (ts_flat.cu): zeros padding, no crop -> a linear shifted copy of each dense slab + byte masks ----
+struct FArgs {
+    Geo g;
+    const unsigned char* x;
+    unsigned char* y;
+    const void* w;
+    long long wzp;
+    long long planes;          // N * C
+    unsigned fillw;            // pad value replicated to 32 bits
+    int qkind, wk, es, dim;
+    int B, Lb;                 // rows per plane, bytes per row
+    int plane_bytes, ipp;      // bytes / 16-byte items of one plane
+    int K, stages, stage_stride, nw;
+    int nstages;               // ceil(planes / K)
+    int table;                 // per-channel (row shift, column shift in bytes) table in shared memory
+    FastDiv d_ipp, d_Lb, d_C;
+};
 struct FlatPlan {
     bool ok;
-    int np, stages, stage_stride, warps, n_per_unit, units, grid;
+    int grid;
     size_t smem_bytes;
+    FArgs a;
 };
 FlatPlan plan_flat(const Geo& g, int esize, bool dense_x, const void* x, const void* y, int sm_count, bool forced);
 int flat_gather(const Geo& g, const FlatPlan& p, int wk, const void* x, void* y, unsigned long long fill, int esize, const void* w,
                 int qkind, long long wzp, cudaStream_t s);
 
 // ---- halo family (ts_halo.cu): whole slabs staged WITH a padded halo, every item is interior ----
+struct alignas(64) HArgs {
+    CUtensorMap map_x;       // x,    box {px, bpx, 1, 1, 1}
+    CUtensorMap map_g;       // grad, box {pg, bpg, 1, 1, 1}
+    CUtensorMap map_v;       // grad, box {OL, OB, 1, 1, 1}   (dense slab: unshifted grad of the 3-D backward)
+                             // fused avg-pool backward: the POOLED grad, box {PW, PH, 1, 1, 1}
+    Geo g;
+    const float* x;
+    const float* grad;
+    float* out;
+    const float* w;
+    double* partials;
+    int mode, active, dim;
+    int A, B, L, OA, OB, OL, lbA, lbB, lbL;   // per level (0 slab, 1 row, 2 column); 2-D: A = OA = 1
+    int IA, IB, IG, GP;                       // iteration space (output space forward, input space backward): slabs, rows, groups; padded groups
+    int RP;                                   // row pairs per slab = ceil(IB / 2)
+    int hr, hc;                               // halo rows / columns on each side of a staged slab
+    int px, bpx, pg, bpg;                     // row pitch (elements) and rows of the x / grad tiles in shared memory
+    int tile_x, tile_g, tile_v;               // bytes between consecutive tiles (128-byte multiples)
+    int box_x, box_g, box_v;                  // bytes one TMA box delivers
+    int off_g, off_v;                         // byte offsets of the grad tiles / dense grad tiles inside a stage (after GUARD)
+    int stage_stride, stages, nw, nt, np;
+    int img_pairs, pairs;                     // RP * GP, np * RP * GP
+    int n_per_unit, units, chunks, unit_order;
+    long long out_plane_bytes;                // bytes of one (n, c) plane of the OUTPUT (pooled plane for the fused avg-pool epilogue)
+    int pool;                                 // forward only: 2x2 / stride 2 / ceil_mode average pooling fused into the store
+    int need_fix;                             // padding != zeros: a fixer warp patches the halo of every stage
+    int table;                                // per-channel shift table in shared memory (C <= TABLE_MAX_C)
+    FastDiv d_GP, d_img, d_C, d_chunks, d_PW;
+    int nfix;                                 // fixer warps (1; 4 when they also expand the pooled gradient)
+    int pool_bwd, PH, PW;                     // backward fused with the adjoint of avg_pool2d(2, 2, ceil_mode): pooled rows / columns
+};
 struct HaloPlan {
     bool ok;
-    int hr, hc;                 // halo rows / columns on each side of a staged slab
-    int px, bpx, pg, bpg;       // row pitch (elements) and rows of the x / grad tiles in shared memory
-    int tile_x, tile_g, tile_v; // bytes per tile (128-byte multiples); tile_v: dense grad slab (3-D backward)
-    int tile_p;                 // pooled-gradient tile of the fused avg-pool backward (0 otherwise)
-    int np, GP, positions, ncol;
-    int stages, stage_stride, warps, n_per_unit, units, grid, slots;
+    int grid, slots;
     size_t smem_bytes;
+    HArgs a;
 };
 // mode: 0 sparse forward (2-D only), 1 active forward, 2 backward (active = interpolating backward).  fp32, dims 2 and 3,
 // every padding, border crops.
 // pool_bwd (mode 2, 2-D): `grad` is the gradient of the 2x2 / stride-2 / ceil_mode average pooling of the shift's output;
-// the kernel expands it while staging (ts_shift2d_avgpool2_backward).
+// the kernel expands it while staging (ts_shift2d_avgpool2_backward); halo_backward then launches the pooled kernels.
 HaloPlan plan_halo(const Geo& g, int mode, int active, int dtype, bool dense_x, const void* x, const void* out, const void* grad,
                    int sm_count, bool forced, bool pool_bwd = false);
 int halo_active_forward(const Geo& g, const HaloPlan& p, const void* x, const void* w, void* y, cudaStream_t s);
 int halo_forward2d(const Geo& g, const HaloPlan& p, int active, int pool, const void* x, const void* w, void* y, cudaStream_t s);
 int halo_backward(const Geo& g, const HaloPlan& p, int active, const void* grad, const void* x, const void* w, void* gi,
-                  double* partials, cudaStream_t s, bool pool_bwd = false);
+                  double* partials, cudaStream_t s);
 
 }  // namespace ts

@@ -96,17 +96,7 @@ TS_D void named_barrier(int id, int count) { asm volatile("bar.sync %0, %1;" ::"
 
 }  // namespace ptx
 
-// ---- exact division by a launch-invariant (n < 2^31) ------------------------------------------
-struct FastDiv { unsigned m, l, d; };
-inline FastDiv make_fastdiv(unsigned d) {
-    FastDiv f;
-    f.d = d ? d : 1;
-    unsigned l = 0;
-    while ((1ull << l) < f.d) ++l;
-    f.l = l;
-    f.m = (unsigned)(((((unsigned long long)1 << l) - f.d) << 32) / f.d + 1);
-    return f;
-}
+// ---- exact division by a launch-invariant (n < 2^31; FastDiv: ts_common.cuh) -------------------
 TS_D unsigned fdiv(unsigned n, const FastDiv& f) { return (__umulhi(n, f.m) + n) >> f.l; }
 
 }  // namespace ts

@@ -40,32 +40,6 @@ using namespace ptx;
 constexpr int GUARD = 32;            // readable slack around the slabs of a stage (second group of a window pair)
 constexpr int MAXT_GATHER = 1024, MAXT_ARITH = 512;   // 512 threads -> 128 registers per thread
 
-// ---- kernel arguments ---------------------------------------------------------------------------
-struct SArgs {
-    Geo g;
-    const unsigned char* x;
-    const unsigned char* grad;
-    unsigned char* out;
-    const void* w;
-    double* partials;
-    long long wzp;
-    unsigned long long fill;
-    int qkind, wk, es, mode, active;
-    int A, B, L, OA, OB, OL, lbA, lbB, lbL;   // sizes per level (0 slab, 1 row, 2 column); absent levels 1 / 0
-    int IA, IB;                               // iteration space: output space (forward) / input space (backward)
-    int VB, V;                                // bytes / elements per item
-    int gpr, GP;                              // items per iteration-space row; padded row length of the index space
-    int TA, tiles;                            // slabs per tile, tiles per image
-    int xs, gvs, gis;                         // slab slots per image: x, grad at the output position, grad for grad_input (0: shares gvs)
-    int slab_x, slab_g;                       // bytes of one slab of x / of grad
-    int np, stages, stage_stride, nw, n_per_unit, units, chunks, unit_order;
-    int off_gv, off_gi;                       // byte offsets of the grad regions inside a stage (after GUARD)
-    int table;                                // per-channel shift parameters tabulated in shared memory (arithmetic kernels, C <= TABLE_MAX_C)
-    int img_items;                            // TA * IB * GP
-    long long img_stride;                     // output bytes between consecutive images of one channel
-    FastDiv d_img, d_GP, d_IB;
-};
-
 // Per-unit shift parameters by LEVEL (0 slab, 1 row, 2 column).
 struct UnitShift {
     int sx[3];     // integer shift reduced against the input sizes
@@ -1450,48 +1424,7 @@ __global__ void __launch_bounds__(MAXT_ARITH, 1) k_staged_backward(const __grid_
 }
 
 int launch(void (*kernel)(SArgs), const SArgs& a, const StagedPlan& p, cudaStream_t s) {
-    return launch_persistent(kernel, p.grid, (p.warps + 1) * 32, p.smem_bytes, s, false, a);
-}
-
-SArgs make_args(const Geo& g, const StagedPlan& p, int mode, int active, int es) {
-    SArgs a;
-    memset(&a, 0, sizeof(a));
-    a.g = g;
-    a.es = es;
-    a.mode = mode;
-    a.active = active;
-    const Levels lv(g);
-    a.A = lv.A;    a.OA = lv.OA;    a.lbA = lv.lbA;
-    a.B = lv.B;    a.OB = lv.OB;    a.lbB = lv.lbB;
-    a.L = lv.L;    a.OL = lv.OL;    a.lbL = lv.lbL;
-    a.IA = mode == 2 ? a.A : a.OA;
-    a.IB = mode == 2 ? a.B : a.OB;
-    a.VB = p.vec_bytes;
-    a.V = p.vec_bytes / es;
-    a.gpr = (mode == 2 ? a.L : a.OL) / a.V;
-    a.GP = p.gp;
-    a.TA = p.ta;
-    a.tiles = p.tiles;
-    a.xs = p.xs; a.gvs = p.gvs; a.gis = p.gis;
-    a.slab_x = (int)((long long)a.B * a.L * es);
-    a.slab_g = (int)((long long)a.OB * a.OL * es);
-    a.np = p.planes_per_step;
-    a.stages = p.stages;
-    a.stage_stride = p.stage_stride;
-    a.nw = p.warps;
-    a.n_per_unit = p.n_per_unit;
-    a.units = p.units;
-    a.chunks = (int)(p.units / (g.C > 0 ? g.C : 1));
-    a.unit_order = tuning().unit_order;
-    a.off_gv = p.off_gv;
-    a.off_gi = p.off_gi;
-    a.table = p.table ? 1 : 0;
-    a.img_items = a.TA * a.IB * a.GP;
-    a.img_stride = g.C * (mode == 2 ? g.in_plane : g.out_plane) * es;
-    a.d_img = make_fastdiv((unsigned)a.img_items);
-    a.d_GP = make_fastdiv((unsigned)a.GP);
-    a.d_IB = make_fastdiv((unsigned)a.IB);
-    return a;
+    return launch_persistent(kernel, p.grid, (a.nw + 1) * 32, p.smem_bytes, s, false, a);
 }
 
 }  // namespace
@@ -1525,8 +1458,22 @@ StagedPlan plan_staged(const Geo& g, int mode, int active, int esize, int dtype,
     if (((uintptr_t)x & 15) || ((uintptr_t)grad & 15) || ((uintptr_t)y_or_gi & (uintptr_t)(vb - 1))) return p;
 
     const Tuning& t = tuning();
-    const int IA = mode == 2 ? A : OA;
+    SArgs& a = p.a;
+    a.g = g;
+    a.es = esize;
+    a.mode = mode;
+    a.active = active ? 1 : 0;
+    a.A = lv.A;    a.OA = lv.OA;    a.lbA = lv.lbA;
+    a.B = lv.B;    a.OB = lv.OB;    a.lbB = lv.lbB;
+    a.L = lv.L;    a.OL = lv.OL;    a.lbL = lv.lbL;
+    a.VB = vb;
+    a.V = vb / esize;
+    a.gpr = (mode == 2 ? a.L : a.OL) / a.V;
+    a.slab_x = (int)slab_x;
+    a.slab_g = (int)slab_g;
+    const int IA = a.IA = mode == 2 ? A : OA;
     const long long IB = mode == 2 ? B : OB;
+    a.IB = (int)IB;
     const int ex = mode != 0 ? 1 : 0;                       // +1 neighbour slab for the arithmetic kernels
     const int ctas = (mode == 0 && t.ctas_per_sm > 1) ? t.ctas_per_sm : 1;     // byte mover only: several small pipelines per SM
     const long long table_bytes = (mode != 0 && g.C <= TABLE_MAX_C) ? (g.C * 36 + 15) / 16 * 16 : 0;     // per-channel shift table
@@ -1561,16 +1508,16 @@ StagedPlan plan_staged(const Geo& g, int mode, int active, int esize, int dtype,
         if (TA > 1) TA = (TA + 1) / 2;
         else return p;                                        // not even one slab (+ neighbours) double-buffers: generic family
     }
-    const int tiles = (int)((IA + TA - 1) / TA);
-    int xs, gvs, gis;
-    const long long per_image = slots(TA, &xs, &gvs, &gis);
+    const int tiles = a.tiles = (int)((IA + TA - 1) / TA);
+    a.TA = (int)TA;
+    const long long per_image = slots(TA, &a.xs, &a.gvs, &a.gis);
+    a.img_stride = g.C * (mode == 2 ? g.in_plane : g.out_plane) * esize;
     long long np = 1;
     if (tiles == 1) {
         np = stage_target / per_image;
         if (np < 1) np = 1;
         if (np > g.N) np = g.N;
-        const long long img_stride = g.C * (mode == 2 ? g.in_plane : g.out_plane) * esize;
-        while (np > 1 && np * img_stride >= 0x7fffffffLL) --np;      // 32-bit offsets inside a stage's destination
+        while (np > 1 && np * a.img_stride >= 0x7fffffffLL) --np;      // 32-bit offsets inside a stage's destination
     }
     auto stride_of = [&](long long n) { return round_up(n * per_image + 2 * GUARD, 128); };
     for (;;) {
@@ -1580,11 +1527,17 @@ StagedPlan plan_staged(const Geo& g, int mode, int active, int esize, int dtype,
         else return p;
     }
     if (np * per_image >= (1 << 20)) return p;                // mbarrier tx-count range
+    a.np = (int)np;
+    a.stages = stages;
+    a.stage_stride = (int)stride_of(np);
+    a.off_gv = (int)(np * a.xs * slab_x);
+    a.off_gi = (int)(np * a.xs * slab_x + np * a.gvs * slab_g);
 
-    const int GP = padded_groups((int)((mode == 2 ? Lb : OLb) / vb));
+    const int GP = a.GP = padded_groups((int)((mode == 2 ? Lb : OLb) / vb));
     const long long img_items = TA * IB * GP;
     if (np * img_items >= 0x7fffffffLL) return p;
-    if ((long long)xs * slab_x * np >= 0x7fffffffLL) return p;
+    if ((long long)a.xs * slab_x * np >= 0x7fffffffLL) return p;
+    a.img_items = (int)img_items;
 
     const long long planes = g.N * g.C;
     const long long grid_max = (long long)sm_count * ctas;
@@ -1600,32 +1553,27 @@ StagedPlan plan_staged(const Geo& g, int mode, int active, int esize, int dtype,
     if (warps > max_warps) warps = max_warps;
     const UnitPlan up = plan_units(np, npu, g.N, g.C, grid_max, warps);
     if (!up.ok) return p;
+    a.nw = warps;
+    a.n_per_unit = up.n_per_unit;
+    a.units = up.units;
+    a.chunks = up.chunks;
+    a.unit_order = t.unit_order;
+    a.table = table_bytes != 0;
+    a.d_img = make_fastdiv((unsigned)a.img_items);
+    a.d_GP = make_fastdiv((unsigned)GP);
+    a.d_IB = make_fastdiv((unsigned)IB);
 
     p.ok = true;
-    p.vec_bytes = vb;
-    p.planes_per_step = (int)np;
-    p.stages = stages;
-    p.stage_stride = (int)stride_of(np);
-    p.warps = warps;
-    p.n_per_unit = up.n_per_unit;
-    p.units = up.units;
     p.grid = up.grid;
     p.slots = up.slots;
-    p.ta = (int)TA;
-    p.tiles = tiles;
-    p.xs = xs; p.gvs = gvs; p.gis = gis;
-    p.gp = GP;
-    p.off_gv = (int)(np * xs * slab_x);
-    p.off_gi = (int)(np * xs * slab_x + np * gvs * slab_g);
     p.smem_bytes = (size_t)(stages * stride_of(np) + 16 * stages + 64 + table_bytes);
-    p.table = table_bytes != 0;
     return p;
 }
 
 // ---- launchers ----------------------------------------------------------------------------------
 int staged_gather(const Geo& g, const StagedPlan& p, int wk, const void* x, void* y, unsigned long long fill, int esize,
                   const void* w, int qkind, long long wzp, cudaStream_t s) {
-    SArgs a = make_args(g, p, 0, 0, esize);
+    SArgs a = p.a;
     a.x = (const unsigned char*)x;
     a.out = (unsigned char*)y;
     a.w = w;
@@ -1633,7 +1581,7 @@ int staged_gather(const Geo& g, const StagedPlan& p, int wk, const void* x, void
     a.qkind = qkind;
     a.wzp = wzp;
     a.fill = fill;
-    const int G = p.vec_bytes / 4;
+    const int G = a.VB / 4;
 #define TS_GATHER(GG, EE) if (G == GG && esize == EE) return launch(k_staged_gather<GG, EE>, a, p, s);
     TS_GATHER(4, 1) TS_GATHER(2, 1) TS_GATHER(1, 1)
     TS_GATHER(4, 2) TS_GATHER(2, 2) TS_GATHER(1, 2)
@@ -1653,7 +1601,7 @@ static int active_forward_t(const Geo& g, const SArgs& a, const StagedPlan& p, c
 }
 
 int staged_active_forward(const Geo& g, const StagedPlan& p, int dtype, const void* x, const void* w, void* y, cudaStream_t s) {
-    SArgs a = make_args(g, p, 1, 1, dtype == TS_F32 ? 4 : 2);
+    SArgs a = p.a;
     a.x = (const unsigned char*)x;
     a.out = (unsigned char*)y;
     a.w = w;
@@ -1679,7 +1627,7 @@ static int backward_t(const Geo& g, const SArgs& a, const StagedPlan& p, int act
 
 int staged_backward(const Geo& g, const StagedPlan& p, int dtype, int active, const void* grad, const void* x, const void* w,
                     void* gi, double* partials, cudaStream_t s) {
-    SArgs a = make_args(g, p, 2, active ? 1 : 0, dtype == TS_F32 ? 4 : 2);
+    SArgs a = p.a;
     a.x = (const unsigned char*)x;
     a.grad = (const unsigned char*)grad;
     a.out = (unsigned char*)gi;

@@ -109,36 +109,6 @@ bool make_map(CUtensorMap* map, const void* base, int es, long long N, long long
     return true;
 }
 
-// ---- arguments -------------------------------------------------------------------------------
-struct alignas(64) TArgs {
-    CUtensorMap map_x;       // x,    box {(TG+1)*vec, xb, xa, 1, np}
-    CUtensorMap map_gs;      // grad, box {(TG+1)*vec, TB, TA, 1, np}     (backward)
-    CUtensorMap map_gb;      // grad, box {(TG+1)*vec, xb, xa, 1, np}     (active backward)
-    Geo g;
-    unsigned char* out;
-    const void* w;
-    double* partials;
-    long long wzp;
-    int qkind, wk, es, vec;  // vec = elements per 16-byte group
-    int mode, active;
-    int OA, OB, OGR;         // output slabs, rows, 16-byte groups per row
-    int lbA, lbB, lbL;
-    int TA, TB, TG;          // tile extents (slabs, rows, groups)
-    int xa, xb;              // x box slabs / rows (TA or TA+1, TB or TB+1)
-    int tiles_b, tiles_g, tiles;
-    int np;                  // images per stage (1 unless a whole plane is one tile)
-    int x_img_chunks;        // 16-byte groups of one image's x box
-    int g_img_chunks;        // 16-byte groups of one image's small grad box
-    int off_gv, off_g2;      // byte offsets of the grad boxes inside a stage
-    int tx_bytes;            // bytes landing per stage
-    int stage_stride, stages, nw, n_per_unit, units, chunks, unit_order;
-    int GP, img_items;       // padded groups per row of the item index space; items per image = TA*TB*GP
-    int img_stride16;        // output distance between consecutive images of one channel, in 16-byte units
-    int R, nchunk;           // strip-mined arithmetic kernels: rows per strip, strips per tile column
-    FastDiv d_img, d_GP, d_TB, d_tg, d_tb, d_TG, d_nchunk, d_TA, d_C, d_chunks;
-    int table;               // per-channel shift table in shared memory (C <= TABLE_MAX_C): built once per CTA
-};
-
 TS_D int floor_to(int v, int q) { return v & ~(q - 1); }      // q is a power of two (elements per 16 bytes)
 
 struct UnitShift {
@@ -759,63 +729,7 @@ __global__ void __launch_bounds__(MAXT_TMA_ARITH, 1) k_tma_backward(const __grid
 
 // every TMA kernel calls pdl_wait() before it touches global memory
 int launch(void (*kernel)(TArgs), const TArgs& a, const TmaPlan& p, cudaStream_t s) {
-    return launch_persistent(kernel, p.grid, (p.warps + 1) * 32, p.smem_bytes, s, true, a);
-}
-
-// fills everything of TArgs that does not depend on pointers
-bool make_args(const Geo& g, const TmaPlan& p, int mode, int active, int es, TArgs* out) {
-    TArgs& a = *out;
-    memset(&a, 0, sizeof(a));
-    const Levels lv(g);
-    a.g = g;
-    a.es = es;
-    a.vec = 16 / es;
-    a.mode = mode;
-    a.active = active;
-    a.OA = lv.OA;            a.lbA = lv.lbA;
-    a.OB = lv.OB;            a.lbB = lv.lbB;
-    a.OGR = lv.OL / a.vec;   a.lbL = lv.lbL;
-    a.TA = p.ta; a.TB = p.tb; a.TG = p.tg;
-    a.xa = p.xa; a.xb = p.xb;
-    a.tiles_b = (a.OB + a.TB - 1) / a.TB;
-    a.tiles_g = (a.OGR + a.TG - 1) / a.TG;
-    a.tiles = p.tiles_per_plane;
-    a.np = p.np;
-    a.x_img_chunks = a.xa * a.xb * (a.TG + 1);
-    a.g_img_chunks = a.TA * a.TB * (a.TG + 1);
-    a.off_gv = p.off_gv;
-    a.off_g2 = p.off_g2;
-    a.tx_bytes = p.tx_bytes;
-    a.stage_stride = p.stage_stride;
-    a.stages = p.stages;
-    a.nw = p.warps;
-    a.n_per_unit = p.n_per_unit;
-    a.units = p.units;
-    a.chunks = (int)(p.units / (g.C > 0 ? g.C : 1));
-    a.unit_order = tuning().unit_order;
-    a.d_C = make_fastdiv((unsigned)g.C);
-    a.d_chunks = make_fastdiv((unsigned)a.chunks);
-    a.table = g.C <= TABLE_MAX_C ? 1 : 0;
-    a.GP = p.gp;
-    a.img_items = a.TA * a.TB * a.GP;
-    a.img_stride16 = (int)(g.C * (mode == 2 ? g.in_plane : g.out_plane) * es / 16);
-    {   // strips: about three per thread and stage, at least two rows each (the row reuse is the point)
-        const long long items = (long long)a.np * a.TA * a.TB * a.TG, nt = 32ll * p.warps;
-        long long R = (items + 3 * nt - 1) / (3 * nt);
-        if (R < 2) R = 2;
-        if (R > a.TB) R = a.TB;
-        a.R = (int)R;
-        a.nchunk = (a.TB + a.R - 1) / a.R;
-    }
-    a.d_TG = make_fastdiv((unsigned)a.TG);
-    a.d_nchunk = make_fastdiv((unsigned)a.nchunk);
-    a.d_TA = make_fastdiv((unsigned)a.TA);
-    a.d_img = make_fastdiv((unsigned)a.img_items);
-    a.d_GP = make_fastdiv((unsigned)a.GP);
-    a.d_TB = make_fastdiv((unsigned)a.TB);
-    a.d_tg = make_fastdiv((unsigned)a.tiles_g);
-    a.d_tb = make_fastdiv((unsigned)a.tiles_b);
-    return true;
+    return launch_persistent(kernel, p.grid, (a.nw + 1) * 32, p.smem_bytes, s, true, a);
 }
 
 }  // namespace
@@ -855,10 +769,19 @@ TmaPlan plan_tma(const Geo& g, int mode, int active, int esize, int dtype, bool 
     if (g.in_plane * esize >= (1ll << 40) / (g.C > 0 ? g.C : 1)) return p;       // tensor-map strides < 2^40
 
     const Tuning& t = tuning();
-    const int OGR = OL / vec;
+    TArgs& a = p.a;
+    a.g = g;
+    a.es = esize;
+    a.vec = vec;
+    a.mode = mode;
+    a.active = active ? 1 : 0;
+    a.OA = OA;    a.lbA = lv.lbA;
+    a.OB = OB;    a.lbB = lv.lbB;
+    const int OGR = a.OGR = OL / vec;
+    a.lbL = lv.lbL;
     const int max_groups = 256 / vec - 1;               // box inner extent (TG+1)*vec <= 256 elements
-    const int tiles_g = (OGR + max_groups - 1) / max_groups;
-    const int TG = (OGR + tiles_g - 1) / tiles_g;
+    const int tiles_g = a.tiles_g = (OGR + max_groups - 1) / max_groups;
+    const int TG = a.TG = (OGR + tiles_g - 1) / tiles_g;
     const int ex = mode != 0 ? 1 : 0;                   // +1 neighbour row / slab in the arithmetic boxes
     const int exb = d >= 2 ? ex : 0, exa = d == 3 ? ex : 0;
     long long TB = OB < 256 - exb ? OB : 256 - exb;
@@ -887,9 +810,12 @@ TmaPlan plan_tma(const Geo& g, int mode, int active, int esize, int dtype, bool 
         else if (TB > 1) TB = (TB + 1) / 2;
         else return p;
     }
-    const int tiles_a = (int)((OA + TA - 1) / TA), tiles_b = (int)((OB + TB - 1) / TB);
+    a.TA = (int)TA; a.TB = (int)TB;
+    a.xa = (int)(TA + exa); a.xb = (int)(TB + exb);
+    const int tiles_a = (int)((OA + TA - 1) / TA), tiles_b = a.tiles_b = (int)((OB + TB - 1) / TB);
     const long long tiles = (long long)tiles_a * tiles_b * tiles_g;
     if (tiles > 0x7fffffffLL) return p;
+    a.tiles = (int)tiles;
     long long np = 1;
     if (tiles == 1) {
         // several images per stage only through a rank-5 box; the sub-box offsets then scale with np
@@ -898,12 +824,14 @@ TmaPlan plan_tma(const Geo& g, int mode, int active, int esize, int dtype, bool 
         if (np > 256) np = 256;
         if (np > g.N) np = g.N;
     }
-    int off_gv = 0, off_g2 = 0;
+    a.np = (int)np;
+    a.x_img_chunks = a.xa * a.xb * (TG + 1);
+    a.g_img_chunks = a.TA * a.TB * (TG + 1);
     // with np images the three regions are [np x-boxes][np gv-boxes][np g2-boxes]
     const long long xbytes1 = (TA + exa) * (TB + exb) * (TG + 1) * 16, gsbytes1 = TA * TB * (TG + 1) * 16;
     const long long xreg = round_up(np * xbytes1, 128), gsreg = round_up(np * gsbytes1, 128);
-    off_gv = (int)xreg;
-    off_g2 = (int)(xreg + gsreg);
+    a.off_gv = (int)xreg;
+    a.off_g2 = (int)(xreg + gsreg);
     long long stage_bytes = xreg, tx = np * xbytes1;
     if (mode == 2) {
         stage_bytes += gsreg + (active ? xreg : gsreg);
@@ -914,10 +842,15 @@ TmaPlan plan_tma(const Geo& g, int mode, int active, int esize, int dtype, bool 
     if (stages > want_stages) stages = want_stages;
     if (stages < 2) return p;
     if (tx >= (1 << 20)) return p;                       // mbarrier tx-count range
+    a.tx_bytes = (int)tx;
+    a.stages = (int)stages;
+    a.stage_stride = (int)stride;
 
-    const int GP = padded_groups(TG);
+    const int GP = a.GP = padded_groups(TG);
     const long long plane16 = g.C * (mode == 2 ? g.in_plane : g.out_plane) * esize / 16;
     if (np * plane16 >= 0x7fffffffLL || np * TA * TB * (long long)GP >= 0x7fffffffLL) return p;
+    a.img_items = a.TA * a.TB * GP;
+    a.img_stride16 = (int)plane16;
     // consumer warps: fill the last pass over a stage's items as well as possible
     const long long items = np * TA * TB * GP;
     const int max_warps = mode == 0 ? MAXT_TMA_GATHER / 32 - 1 : MAXT_TMA_ARITH / 32 - 1;
@@ -938,23 +871,36 @@ TmaPlan plan_tma(const Geo& g, int mode, int active, int esize, int dtype, bool 
             if (eff(w) >= eff(best_all) - 1e-9) best_all = w;
         warps = eff(best) >= eff(best_all) - 0.08 ? best : best_all;
     }
+    a.nw = warps;
+    {   // strips: about three per thread and stage, at least two rows each (the row reuse is the point)
+        const long long nt = 32ll * warps;
+        long long R = (np * TA * TB * TG + 3 * nt - 1) / (3 * nt);
+        if (R < 2) R = 2;
+        if (R > TB) R = TB;
+        a.R = (int)R;
+        a.nchunk = (a.TB + a.R - 1) / a.R;
+    }
     const UnitPlan up = plan_units(np, t.chunk_planes > 0 ? t.chunk_planes : pick_unit_images(g.N, g.C, np, sm_count, mode == 2 ? 0.4 : 0.1),
                                    g.N, g.C, sm_count, warps);
     if (!up.ok) return p;
+    a.n_per_unit = up.n_per_unit;
+    a.units = up.units;
+    a.chunks = up.chunks;
+    a.unit_order = t.unit_order;
+    a.table = g.C <= TABLE_MAX_C ? 1 : 0;
+    a.d_img = make_fastdiv((unsigned)a.img_items);
+    a.d_GP = make_fastdiv((unsigned)GP);
+    a.d_TB = make_fastdiv((unsigned)a.TB);
+    a.d_tg = make_fastdiv((unsigned)tiles_g);
+    a.d_tb = make_fastdiv((unsigned)tiles_b);
+    a.d_TG = make_fastdiv((unsigned)TG);
+    a.d_nchunk = make_fastdiv((unsigned)a.nchunk);
+    a.d_TA = make_fastdiv((unsigned)a.TA);
+    a.d_C = make_fastdiv((unsigned)g.C);
+    a.d_chunks = make_fastdiv((unsigned)a.chunks);
 
     p.ok = true;
-    p.ta = (int)TA; p.tb = (int)TB; p.tg = TG; p.gp = GP;
-    p.xa = (int)(TA + exa); p.xb = (int)(TB + exb);
-    p.tiles_per_plane = (int)tiles;
-    p.np = (int)np;
-    p.off_gv = off_gv; p.off_g2 = off_g2;
-    p.tx_bytes = (int)tx;
-    p.stages = (int)stages;
-    p.stage_stride = (int)stride;
-    p.n_per_unit = up.n_per_unit;
-    p.units = up.units;
     p.grid = up.grid;
-    p.warps = warps;
     p.slots = up.slots;
     p.smem_bytes = (size_t)(stages * stride + 16 * stages + 64 + table_bytes);
     return p;
@@ -962,8 +908,7 @@ TmaPlan plan_tma(const Geo& g, int mode, int active, int esize, int dtype, bool 
 
 int tma_gather(const Geo& g, const TmaPlan& p, int wk, const void* x, void* y, int esize, const void* w, int qkind, long long wzp,
                cudaStream_t s) {
-    TArgs a;
-    make_args(g, p, 0, 0, esize, &a);
+    TArgs a = p.a;
     const Levels lv(g);
     a.out = (unsigned char*)y;
     a.w = w;
@@ -985,13 +930,11 @@ static int active_forward_t(const Geo& g, const TArgs& a, const TmaPlan& p, cuda
 }
 
 int tma_active_forward(const Geo& g, const TmaPlan& p, int dtype, const void* x, const void* w, void* y, cudaStream_t s) {
-    TArgs a;
-    const int es = dtype == TS_F32 ? 4 : 2;
-    make_args(g, p, 1, 1, es, &a);
+    TArgs a = p.a;
     const Levels lv(g);
     a.out = (unsigned char*)y;
     a.w = w;
-    if (!make_map(&a.map_x, x, es, g.N, g.C, lv.A, lv.B, lv.L, (a.TG + 1) * a.vec, a.xb, a.xa, a.np, dtype)) return TS_ERR_UNSUPPORTED;
+    if (!make_map(&a.map_x, x, a.es, g.N, g.C, lv.A, lv.B, lv.L, (a.TG + 1) * a.vec, a.xb, a.xa, a.np, dtype)) return TS_ERR_UNSUPPORTED;
     switch (dtype) {      // 16-bit: planned for 2-D only
     case TS_F16: return launch(k_tma_active_forward<__half, 2>, a, p, s);
     case TS_BF16: return launch(k_tma_active_forward<__nv_bfloat16, 2>, a, p, s);
@@ -1013,11 +956,9 @@ static int backward_t(const Geo& g, const TArgs& a, const TmaPlan& p, int active
 
 int tma_backward(const Geo& g, const TmaPlan& p, int dtype, int active, const void* grad, const void* x, const void* w, void* gi,
                  double* partials, cudaStream_t s) {
-    TArgs a;
-    const int es = dtype == TS_F32 ? 4 : 2;
-    make_args(g, p, 2, active ? 1 : 0, es, &a);
+    TArgs a = p.a;
     const Levels lv(g);
-    const int A = lv.A, B = lv.B, L = lv.L, bl = (a.TG + 1) * a.vec;
+    const int A = lv.A, B = lv.B, L = lv.L, es = a.es, bl = (a.TG + 1) * a.vec;
     a.out = (unsigned char*)gi;
     a.w = w;
     a.partials = partials;

@@ -514,6 +514,88 @@ int ts_shift_backward_allreduce(const ts_geometry* gin, int dtype, int padding, 
                          stream);
 }
 
+// The pooling of the fused avg-pool entry points: -> TS_OK and the slab stride (3-D; 1 for 2-D), TS_ERR_INVALID_ARGUMENT for a
+// stride entry below 1, TS_ERR_UNSUPPORTED for a stride no kernel serves (2-D: (2, 2); 3-D: (1, 2, 2), (2, 2, 2)).
+static int pool_stride(int dim, const int32_t* stride, int* sa) {
+    for (int a = 0; a < dim; ++a)
+        if (stride[a] < 1) return TS_ERR_INVALID_ARGUMENT;
+    if (dim < 2 || stride[dim - 2] != 2 || stride[dim - 1] != 2) return TS_ERR_UNSUPPORTED;
+    if (dim == 3 && stride[0] != 1 && stride[0] != 2) return TS_ERR_UNSUPPORTED;
+    *sa = dim == 3 ? stride[0] : 1;
+    return TS_OK;
+}
+
+// The halo plan of a fused avg-pool call (the kernels that serve it are forced: small planes too).
+static HaloPlan pool_plan(const Geo& g, int mode, int active, int sa, const void* x, const void* out, const void* grad, int sms) {
+    return plan_halo(g, mode, active, TS_F32, x_is_dense(g), x, out, grad, sms, true, mode == 2, g.dim == 3 ? sa : 0);
+}
+
+int ts_shift_avgpool_forward(const ts_geometry* gin, int dtype, int padding, int active, const int32_t* stride, const void* x,
+                             const void* weights, void* y_pooled, void* stream) {
+    Geo g;
+    int rc = make_geo(gin, padding, &g);
+    if (rc != TS_OK) return rc;
+    if ((dtype = weights_f32(dtype, &g)) < 0 || !elem_size(dtype) || !stride) return TS_ERR_INVALID_ARGUMENT;
+    int sa = 1;
+    if ((rc = pool_stride(g.dim, stride, &sa)) != TS_OK) return rc;
+    if (dtype != TS_F32 || g.wf32) return TS_ERR_UNSUPPORTED;
+    if (g.N * g.C == 0 || g.out_plane == 0) return TS_OK;
+    if (!x || !weights || !y_pooled) return TS_ERR_INVALID_ARGUMENT;
+    int sms = 0;
+    if ((rc = sm_count(&sms)) != TS_OK) return rc;
+    const int mode = active ? 1 : 0;
+    const HaloPlan hp = pool_plan(g, mode, active, sa, x, y_pooled, nullptr, sms);
+    if (!hp.ok) return TS_ERR_UNSUPPORTED;
+    t_last_path = TS_PATH_HALO;
+    cudaStream_t s = (cudaStream_t)stream;
+    return g.dim == 3 ? halo_forward3d_pool(g, hp, active, x, weights, y_pooled, s) : halo_forward2d(g, hp, active, 1, x, weights, y_pooled, s);
+}
+
+size_t ts_shift_avgpool_backward_workspace_bytes(const ts_geometry* gin, int dtype) {
+    Geo g;
+    if (!gin || make_geo(gin, 0, &g) != TS_OK || weights_f32(dtype, &g) != TS_F32 || g.wf32) return 16;
+    if (g.N * g.C == 0 || (g.dim != 2 && g.dim != 3)) return 16;
+    int sms = 148;
+    sm_count(&sms);
+    // every plan the backward may pick: dense aligned x, zeros or another padding, sparse or active, every served stride
+    int slots = 0;
+    for (int pad = 0; pad < 2; ++pad)
+        for (int active = 0; active < 2; ++active)
+            for (int sa = 1; sa <= (g.dim == 3 ? 2 : 1); ++sa) {
+                Geo gp = g;
+                gp.pad = pad;
+                const HaloPlan hp = pool_plan(gp, 2, active, sa, nullptr, nullptr, nullptr, sms);
+                if (hp.ok && hp.slots > slots) slots = hp.slots;
+            }
+    return (size_t)slots * (size_t)(g.C * g.dim) * sizeof(double) + 16;
+}
+
+int ts_shift_avgpool_backward(const ts_geometry* gin, int dtype, int padding, int active, const int32_t* stride, const void* grad_pooled,
+                              const void* x, const void* weights, void* grad_input, void* grad_weight, void* workspace,
+                              size_t workspace_bytes, const ts_peer_group* peers, void* stream) {
+    Geo g;
+    int rc = make_geo(gin, padding, &g);
+    if (rc != TS_OK) return rc;
+    const int et = weights_f32(dtype, &g);
+    if (et < 0 || !elem_size(et) || !stride) return TS_ERR_INVALID_ARGUMENT;
+    int sa = 1;
+    if ((rc = pool_stride(g.dim, stride, &sa)) != TS_OK) return rc;
+    if (peers && (rc = check_peers(gin, et, peers)) != TS_OK) return rc;
+    if (et != TS_F32 || g.wf32) return TS_ERR_UNSUPPORTED;
+    if (g.N * g.C == 0 || g.in_plane == 0 || g.out_plane == 0) return TS_ERR_UNSUPPORTED;     // (empty shards: the two-step path)
+    if (!grad_pooled || !x || !weights || !grad_input || !grad_weight) return TS_ERR_INVALID_ARGUMENT;
+    if (!workspace || ((uintptr_t)workspace & 15)) return TS_ERR_WORKSPACE;
+    int sms = 0;
+    if ((rc = sm_count(&sms)) != TS_OK) return rc;
+    const HaloPlan hp = pool_plan(g, 2, active, sa, x, grad_input, grad_pooled, sms);
+    if (!hp.ok) return TS_ERR_UNSUPPORTED;
+    if (workspace_bytes < (size_t)hp.slots * (size_t)(g.C * g.dim) * sizeof(double)) return TS_ERR_WORKSPACE;
+    t_last_path = TS_PATH_HALO;
+    cudaStream_t s = (cudaStream_t)stream;
+    rc = halo_backward(g, hp, active, grad_pooled, x, weights, grad_input, (double*)workspace, s);
+    return rc != TS_OK ? rc : reduce_partials(g, TS_F32, (double*)workspace, hp.slots, grad_weight, peers, s);
+}
+
 int ts_shift_forward_nhwc(const ts_geometry* gin, int dtype, int padding, int active, const void* x, const void* weights, void* y,
                           void* stream) {
     Geo g;

@@ -411,6 +411,24 @@ TS_D void slow_forward(const HArgs& a, int c, int n0, int n1, const UnitShift& u
                     }
                 yp[e] = __fdiv_rn(sum, (float)cnt);
             }
+        } else if constexpr (POOL && DIM == 3) {
+            // avg_pool3d(kernel = stride = (sA, 2, 2), ceil_mode): one running sum in (slab, row, column) order, as ATen's kernel
+            const int PH = a.PH, PW = a.PW, sA = a.sA;
+            for (int e = tid; e < a.PA * PH * PW; e += nt) {
+                const int pa = e / (PH * PW), rem = e - pa * (PH * PW), ph = rem / PW, pw = rem - ph * PW;
+                float sum = 0.f;
+                int cnt = 0;
+                for (int s = 0; s < sA; ++s)
+                    for (int i = 0; i < 2; ++i)
+                        for (int j = 0; j < 2; ++j) {
+                            const int o[3] = {sA * pa + s, 2 * ph + i, 2 * pw + j};
+                            if (o[0] >= g.OS[0] || o[1] >= g.OS[1]) continue;
+                            const float v = slow_forward_value<DIM, ACTIVE>(g, xp, o, sx, d);
+                            sum = cnt ? __fadd_rn(sum, v) : v;
+                            ++cnt;
+                        }
+                yp[e] = __fdiv_rn(sum, (float)cnt);
+            }
         } else {
             const int plane = (int)g.out_plane;
             for (int e = tid; e < plane; e += nt) {
@@ -431,17 +449,29 @@ TS_D void slow_backward(const HArgs& a, int c, int n0, int n1, const UnitShift& 
     float d[3] = {us.d[0], us.d[1], us.d[2]};
 #pragma unroll
     for (int ax = 0; ax < DIM; ++ax) { sx[ax] = us.sx[ax + 3 - DIM]; sg[ax] = us.sg[ax + 3 - DIM]; }
-    constexpr bool pool = PBWD;                 // 2-D only: a.grad is the POOLED gradient, expanded on the fly
+    constexpr bool pool = PBWD;                 // a.grad is the POOLED gradient, expanded on the fly
     const int PW = a.PW, OL = a.OL, OB = a.OB;
     for (int n = n0; n < n1; ++n) {
         const float* xp = a.x + ((long long)n * g.C + c) * g.in_plane;
-        const float* gp = a.grad + ((long long)n * g.C + c) * (pool ? (long long)a.PH * a.PW : g.out_plane);
+        const float* gp = a.grad + ((long long)n * g.C + c) * (pool ? (DIM == 3 ? (long long)a.PA : 1ll) * a.PH * a.PW : g.out_plane);
         float* gip = a.out + ((long long)n * g.C + c) * g.in_plane;
         // gradient of the shift's output at linear offset `off` of the (cropped) output plane
         auto gld = [gp, PW, OL, OB](long long off) {
             if (!pool) return gp[off];
             const int r = (int)(off / OL), cc = (int)(off - (long long)r * OL), pr = r >> 1;
             return gp[pr * PW + (cc >> 1)] * (2 * pr + 1 < OB ? 0.25f : 0.5f);
+        };
+        // 3-D: grad / count of the (sA, 2, 2) window (a power of two: the product is the quotient)
+        const int PH = a.PH, OA = a.OA, sA = a.sA;
+        auto gld3 = [gp, PW, PH, OL, OB, OA, sA](long long off) {
+            const int plane = OB * OL, o0 = (int)(off / plane), rem = (int)(off - (long long)o0 * plane), r = rem / OL, cc = rem - r * OL;
+            const int pa = sA == 2 ? o0 >> 1 : o0, pr = r >> 1;
+            const float f = (sA == 2 && 2 * pa + 1 < OA ? 0.5f : 1.f) * (2 * pr + 1 < OB ? 0.25f : 0.5f);
+            return gp[((long long)pa * PH + pr) * PW + (cc >> 1)] * f;
+        };
+        auto gsel = [&](long long off) {
+            if constexpr (pool && DIM == 3) return gld3(off);
+            else return gld(off);
         };
         for (int e = tid; e < plane; e += nt) {
             int pos[DIM], rem = e, o[DIM];
@@ -457,7 +487,7 @@ TS_D void slow_backward(const HArgs& a, int c, int n0, int n1, const UnitShift& 
             }
             float r = 0.f;
             if (pass) {
-                const float gv = gld(goff);
+                const float gv = gsel(goff);
                 int idx[DIM];
 #pragma unroll
                 for (int ax = 0; ax < DIM; ++ax) idx[ax] = pos[ax] - sx[ax];
@@ -469,7 +499,7 @@ TS_D void slow_backward(const HArgs& a, int c, int n0, int n1, const UnitShift& 
                 if (ACTIVE) {
 #pragma unroll
                     for (int ax = 0; ax < DIM; ++ax) idx[ax] = o[ax] - sg[ax];
-                    fetch8f<DIM>(gld, idx, g.OS, g.pad, v);
+                    fetch8f<DIM>(gsel, idx, g.OS, g.pad, v);
                     r = interpolate<float, DIM>(v, d);
                 } else {
                     bool in = true;
@@ -480,7 +510,7 @@ TS_D void slow_backward(const HArgs& a, int c, int n0, int n1, const UnitShift& 
                         in = in && t >= 0;
                         off = off * g.OS[ax] + t;
                     }
-                    r = in ? gld(off) : 0.f;
+                    r = in ? gsel(off) : 0.f;
                 }
             }
             gip[e] = r;
@@ -503,6 +533,11 @@ TS_D int slab_coord(int idx, int len, int pad) {
 // out for step k once per unit (one elected thread evaluating the remaps every stage was near the critical path of the 3-D
 // pipeline: reflect / symmetric padding ran 8 % behind border padding for ~20 extra dependent instructions per stage), and the
 // (up to three) tensor copies of an image are issued by three different lanes.
+// POOL3 (3-D backward fused with avg_pool3d): both grad copies are slabs of the POOLED gradient, the one that feeds
+// grad_input lands in the second dense tile of the image (after the a.np tiles at off_v) and the fixer warp expands it.
+TS_D int pooled_slab(int s, int sA) { return s < 0 ? -1 : (sA == 2 ? s >> 1 : s); }
+
+template <bool POOL3>
 TS_D void producer(const HArgs& a, unsigned char* smem, uint64_t* full, uint64_t* empty, const UnitShift* tbl, const UnitOrder& uo, int lane) {
     int s = 0, kk = 0, cls = 0;
     const int N = (int)a.g.N;
@@ -527,6 +562,7 @@ TS_D void producer(const HArgs& a, unsigned char* smem, uint64_t* full, uint64_t
                         gs_l = a.active ? slab_coord(kl - a.lbA - us.sg[0], a.OA, a.g.pad) : slab_coord(kl - 1 - a.lbA + us.sg[0], a.OA, a.g.pad);
                         const int oa = kl - 1 - a.lbA;
                         vs_l = (oa >= 0 && oa < a.OA) ? oa : -1;
+                        if constexpr (POOL3) { gs_l = pooled_slab(gs_l, a.sA); vs_l = pooled_slab(vs_l, a.sA); }
                     }
                 }
                 const int xs = __shfl_sync(0xffffffffu, xs_l, k & 31), gs = __shfl_sync(0xffffffffu, gs_l, k & 31),
@@ -543,7 +579,9 @@ TS_D void producer(const HArgs& a, unsigned char* smem, uint64_t* full, uint64_t
                     const int pl = job / 3, what = job - 3 * pl;
                     if (what == 0) tma_load_5d(st + (size_t)pl * a.tile_x, &a.map_x, -a.hc, -a.hr, xs, c, nb + pl, &full[s]);
                     else if (what == 1) {
-                        if (has_g && a.pool_bwd) tma_load_5d(st + a.off_v + (size_t)pl * a.tile_v, &a.map_v, 0, 0, 0, c, nb + pl, &full[s]);   // pooled grad, dense
+                        if constexpr (POOL3) {
+                            if (has_g) tma_load_5d(st + a.off_v + (size_t)(a.np + pl) * a.tile_v, &a.map_v, 0, 0, gs, c, nb + pl, &full[s]);
+                        } else if (has_g && a.pool_bwd) tma_load_5d(st + a.off_v + (size_t)pl * a.tile_v, &a.map_v, 0, 0, 0, c, nb + pl, &full[s]);   // pooled grad, dense
                         else if (has_g) tma_load_5d(st + a.off_g + (size_t)pl * a.tile_g, &a.map_g, -a.hc, -a.hr, gs, c, nb + pl, &full[s]);
                     }
                     else if (has_v) tma_load_5d(st + a.off_v + (size_t)pl * a.tile_v, &a.map_v, 0, 0, vs, c, nb + pl, &full[s]);
@@ -683,6 +721,102 @@ TS_D void fixer_pool(const HArgs& a, unsigned char* smem, uint64_t* full, uint64
                     } else if (fw == 0) {
                         if (fix_x) halo_walk_z(nullptr, tx, a.px, a.B, a.L, a.hr, a.hc, a.g.pad, hx, lane);
                         if (has_g && fix_g) halo_walk_z(nullptr, tg, a.pg, a.OB, a.OL, a.hr, a.hc, a.g.pad, hg, lane, zero_g);
+                    }
+                }
+                fence_proxy_async();             // the next TMA load of this stage must not overtake these generic-proxy writes
+                __syncwarp();
+                if (lane == 0) mbar_arrive(&ready[s]);
+                if (++s == a.stages) { s = 0; phase ^= 1u; }
+            }
+        }
+    }
+}
+
+// 3-D backward fused with avg_pool3d (kernel = stride = (sA, 2, 2), ceil_mode): ONE fixer warp -- a cfg4 slab (28 row pairs x 16
+// groups) takes all 448 consumer threads the CTA has left, so the four expansion warps of the 2-D kernels do not fit.  It
+// expands the pooled slab that feeds grad_input into the padded grad tile (every element of a window receives grad / count,
+// as ATen's avg_pool3d_backward; the count is a power of two, so the product is the quotient) and then clears (zeros
+// padding) or patches the tile's reachable halo: the padding rule applies to the EXPANDED gradient.  The consumers read the
+// unshifted gradient for grad_weight straight from the image's other pooled tile.
+TS_D void sts128(unsigned addr, float a, float b, float c, float d) {
+    asm volatile("st.shared.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "f"(a), "f"(b), "f"(c), "f"(d) : "memory");
+}
+TS_D void pool_expand3(unsigned src, unsigned dst, int PH, int PW, int OB, int pitch, float fa, int lane, const FastDiv& dPW) {
+    // item: 4 pooled values of a row (16 bytes) -> 8 columns of one or two rows of the tile (dst: its element (hr, hc))
+    const int n = PH * PW, pb = pitch * 4;
+    for (int e = 4 * lane; e < n; e += 128) {
+        const int pr = (int)fdiv((unsigned)e, dPW), pc = e - pr * PW;
+        const uint4 v = lds128(src + 4u * (unsigned)e);
+        const bool two = 2 * pr + 1 < OB;
+        const float f = fa * (two ? 0.25f : 0.5f);
+        const float v0 = __uint_as_float(v.x) * f, v1 = __uint_as_float(v.y) * f, v2 = __uint_as_float(v.z) * f, v3 = __uint_as_float(v.w) * f;
+        const unsigned o = dst + (unsigned)(2 * pr * pb + 8 * pc);
+        sts128(o, v0, v0, v1, v1);
+        sts128(o + 16, v2, v2, v3, v3);
+        if (two) { sts128(o + pb, v0, v0, v1, v1); sts128(o + pb + 16, v2, v2, v3, v3); }
+    }
+}
+
+TS_D void fixer_pool3(const HArgs& a, unsigned char* smem, uint64_t* full, uint64_t* ready, int lane, const UnitShift* tbl, unsigned* lists,
+                      const UnitOrder& uo) {
+    int s = 0, cls = 0;
+    unsigned phase = 0;
+    const int N = (int)a.g.N;
+    const int steps = a.IA + 1;
+    unsigned* list_x = lists;
+    unsigned* list_g = lists + FIXCAP;
+    const bool listable = a.px * a.bpx < 65536 && a.pg * a.bpg < 65536;
+    const bool fix_x = a.g.pad != TS_PAD_ZEROS, zero_g = !fix_x;
+    const UnitRange ur = unit_range(a.units, a.unit_order);
+    for (int u = ur.u; u < ur.end; u += ur.step) {
+        int chunk, c;
+        uo.decode(u, cls, c, chunk, a.unit_order);
+        const int n0 = chunk * a.n_per_unit;
+        const int n1 = n0 + a.n_per_unit < N ? n0 + a.n_per_unit : N;
+        const UnitShift us = unit_shift(a, tbl, c);
+        if (!unit_geom(a, us).fits) continue;
+        const int xr_lo = -us.sx[1], xc_lo = -us.sx[2];
+        const int sgr = a.active ? -us.sg[1] : us.sg[1], sgc = a.active ? -us.sg[2] : us.sg[2], ex = a.active ? 1 : 0;
+        const HaloRange hx = {xr_lo, xr_lo + a.IB, xc_lo, xc_lo + 4 * a.IG};
+        const HaloRange hg = {sgr, a.OB - 1 + sgr + ex, sgc, a.OL - 1 + sgc + ex};
+        const int nx = halo_cells(hx, a.B, a.L), ng = halo_cells(hg, a.OB, a.OL);
+        const bool use_list = listable && nx <= FIXCAP && ng <= FIXCAP;
+        if (use_list) {
+            __syncwarp();                       // every lane is done with the previous unit's lists
+            if (fix_x) halo_walk_z(list_x, nullptr, a.px, a.B, a.L, a.hr, a.hc, a.g.pad, hx, lane);
+            halo_walk_z(list_g, nullptr, a.pg, a.OB, a.OL, a.hr, a.hc, a.g.pad, hg, lane, zero_g);
+            __syncwarp();
+        }
+        for (int nb = n0; nb < n1; nb += a.np) {
+            const int npl = n1 - nb < a.np ? n1 - nb : a.np;
+            int gs_l = 0;                                   // pooled grad slab of step (k & ~31) + lane, as the producer loads it
+            for (int k = 0; k < steps; ++k) {
+                if ((k & 31) == 0) {
+                    const int kl = k + lane;
+                    gs_l = pooled_slab(a.active ? slab_coord(kl - a.lbA - us.sg[0], a.OA, a.g.pad) : slab_coord(kl - 1 - a.lbA + us.sg[0], a.OA, a.g.pad),
+                                       a.sA);
+                }
+                const int gs = __shfl_sync(0xffffffffu, gs_l, k & 31);
+                unsigned char* st = smem + (size_t)s * a.stage_stride + GUARD;
+                const bool has_g = a.active || k >= 1;
+                mbar_wait_parked(&full[s], phase);
+                if (has_g) {
+                    const float fa = a.sA == 2 && 2 * gs + 1 < a.OA ? 0.5f : 1.f;      // slabs in the window (a zero tile for gs < 0)
+                    for (int pl = 0; pl < npl; ++pl)
+                        pool_expand3(shared_addr(st + a.off_v + (size_t)(a.np + pl) * a.tile_v),
+                                     shared_addr(st + a.off_g + (size_t)pl * a.tile_g) + (unsigned)((a.hr * a.pg + a.hc) * 4), a.PH, a.PW, a.OB, a.pg,
+                                     fa, lane, a.d_PW);
+                    __syncwarp();                    // the halo copies below read cells other lanes have just written
+                }
+                for (int pl = 0; pl < npl; ++pl) {
+                    float* tx = (float*)(st + (size_t)pl * a.tile_x);
+                    float* tg = (float*)(st + a.off_g + (size_t)pl * a.tile_g);
+                    if (use_list) {
+                        if (fix_x) halo_apply_m<false>(list_x, nx, tx, lane);
+                        if (has_g) { if (zero_g) halo_apply_m<true>(list_g, ng, tg, lane); else halo_apply_m<false>(list_g, ng, tg, lane); }
+                    } else {
+                        if (fix_x) halo_walk_z(nullptr, tx, a.px, a.B, a.L, a.hr, a.hc, a.g.pad, hx, lane);
+                        if (has_g) halo_walk_z(nullptr, tg, a.pg, a.OB, a.OL, a.hr, a.hc, a.g.pad, hg, lane, zero_g);
                     }
                 }
                 fence_proxy_async();             // the next TMA load of this stage must not overtake these generic-proxy writes
@@ -968,11 +1102,171 @@ struct Body {
         }
     }
 
+    // ---------------------------------------------------------------------------------------------
+    // 3-D fused with avg_pool3d (kernel = stride = (sA, 2, 2), ceil_mode).  Forward: the pair's 2 x 4 outputs of a slab step are
+    // pooled into two values -- every window's elements added in (slab, row, column) order into ONE running sum, as ATen's
+    // kernel; with sA = 2 the sum of an even slab step is carried in registers to the odd one -- and divided by the count.
+    template <int WSX>
+    TS_D void pool_step_fwd(unsigned sb, unsigned char* dst_img, int k, const PairCtx& pc, const Carry& cy, Carry& nx, float* run) const {
+        if (pc.rows == 0) return;
+        const float d[3] = {us.d[0], us.d[1], us.d[2]};
+        const unsigned xa = sb + pc.xo;
+        const int pxb = a.px * 4;
+        float y[2][4];
+        int it;
+        if constexpr (MODE == 0) {
+            // the gather: output slab k is this stage's x slab (the ring's last stage only drains)
+            if (k >= a.IA) return;
+            it = k;
+            load4<WSX>(xa, wsx, y[0]);
+            if (pc.rows == 2) load4<WSX>(xa + pxb, wsx, y[1]);
+        } else {
+            load5<WSX>(xa, wsx, nx.X[0]); load5<WSX>(xa + pxb, wsx, nx.X[1]);
+            if (pc.rows == 2) load5<WSX>(xa + 2 * pxb, wsx, nx.X[2]);
+            if (k < 1) return;
+            it = k - 1;
+#pragma unroll
+            for (int j = 0; j < 2; ++j) {
+                if (j >= pc.rows) continue;
+                float S0[5], S1[5], P[5];
+#pragma unroll
+                for (int t = 0; t < 5; ++t) { S0[t] = lerp<float>(cy.X[j][t], nx.X[j][t], d[0]); S1[t] = lerp<float>(cy.X[j + 1][t], nx.X[j + 1][t], d[0]); }
+#pragma unroll
+                for (int t = 0; t < 5; ++t) P[t] = lerp<float>(S0[t], S1[t], d[1]);
+#pragma unroll
+                for (int t = 0; t < 4; ++t) y[j][t] = lerp<float>(P[t], P[t + 1], d[2]);
+            }
+        }
+        const bool two = pc.rows == 2, odd = a.sA == 2 && (it & 1);
+        float s0 = odd ? __fadd_rn(run[0], y[0][0]) : y[0][0], s1 = odd ? __fadd_rn(run[1], y[0][2]) : y[0][2];
+        s0 = __fadd_rn(s0, y[0][1]);
+        s1 = __fadd_rn(s1, y[0][3]);
+        if (two) {
+            s0 = __fadd_rn(__fadd_rn(s0, y[1][0]), y[1][1]);
+            s1 = __fadd_rn(__fadd_rn(s1, y[1][2]), y[1][3]);
+        }
+        if (a.sA == 2 && !odd && it != a.IA - 1) { run[0] = s0; run[1] = s1; return; }
+        const float cnt = (float)((two ? 4 : 2) * (odd ? 2 : 1));
+        const int pa = a.sA == 2 ? it >> 1 : it;
+        __stcs((float2*)(dst_img + pc.out_off + (long long)pa * a.PH * a.PW * 4), make_float2(__fdiv_rn(s0, cnt), __fdiv_rn(s1, cnt)));
+    }
+
+    // Backward: step3's backward with the unshifted gradient read from the pooled tile (value x 1 / count of its window); the
+    // grad tile that feeds grad_input was expanded by the fixer warp.  q: the pair (crops: element-wise pooled indices).
+    template <int WSX, int WSG, int WSV>
+    TS_D void pool_step_bwd(unsigned sb, unsigned char* dst_img, int k, const PairCtx& pc, const Pair& q, const Carry& cy, Carry& nx,
+                            float* ts) const {
+        if (pc.rows == 0) return;
+        const float d[3] = {us.d[0], us.d[1], us.d[2]};
+        const int it = k - 1, oa = it - a.lbA, orow = a.IG * 16;
+        unsigned char* o = dst_img + pc.out_off + (long long)it * a.IB * orow;
+        const bool slab_pass = !CROP || (oa >= 0 && oa < a.OA);
+        const unsigned cm = (k >= 1 && slab_pass) ? pc.cmask : 0u;
+        const unsigned xa = sb + pc.xo, ga = sb + pc.go, va = sb + pc.vo;
+        const int pxb = a.px * 4, pgb = a.pg * 4;
+        const bool gwin = ACTIVE && pc.cmask != 0u;
+        const float fa = a.sA == 2 && (oa | 1) < a.OA ? 0.5f : 1.f;          // slabs in the window of output slab oa
+        float pv[2] = {0.f, 0.f};
+        load5<WSX>(xa, wsx, nx.X[0]); load5<WSX>(xa + pxb, wsx, nx.X[1]);
+        if (gwin) { load5<WSG>(ga, wsg, nx.G[0]); load5<WSG>(ga + pgb, wsg, nx.G[1]); }
+        if (!CROP && k >= 1) {
+            // no crop: both rows of the pair lie in one pooled row, the group's 4 columns in 2 pooled columns
+            const uint2 v = lds64(va);
+            const float f = fa * (pc.rows == 2 ? 0.25f : 0.5f);
+            pv[0] = __uint_as_float(v.x) * f; pv[1] = __uint_as_float(v.y) * f;
+        }
+#pragma unroll
+        for (int j = 0; j < 2; ++j) {
+            if (j >= pc.rows) continue;
+            if (j == 1) {
+                load5<WSX>(xa + 2 * pxb, wsx, nx.X[2]);
+                if (gwin) load5<WSG>(ga + 2 * pgb, wsg, nx.G[2]);
+            }
+            if (k < 1) continue;
+            const unsigned m = CROP ? (cm >> (4 * j)) & 15u : 15u;
+            float y[4] = {0.f, 0.f, 0.f, 0.f};
+            if (m) {
+                float gv[4];
+                if constexpr (CROP) {
+                    const int pr = (q.r + j - a.lbB) >> 1;
+                    const float f = fa * (2 * pr + 1 < a.OB ? 0.25f : 0.5f);
+#pragma unroll
+                    for (int t = 0; t < 4; ++t) {
+                        const int oj = 4 * q.cg + t - a.lbL;
+                        gv[t] = (m >> t) & 1u ? __uint_as_float(lds32(va + (unsigned)((pr * a.PW + (oj >> 1)) * 4))) * f : 0.f;
+                    }
+                } else {
+                    gv[0] = gv[1] = pv[0]; gv[2] = gv[3] = pv[1];
+                }
+                wp3(cy.X[j], nx.X[j], cy.X[j + 1], nx.X[j + 1], gv, d, ts);
+                if (ACTIVE) {
+                    float P[5];
+#pragma unroll
+                    for (int t = 0; t < 5; ++t) P[t] = col3(cy.G[j][t], nx.G[j][t], cy.G[j + 1][t], nx.G[j + 1][t], d[0], d[1]);
+#pragma unroll
+                    for (int t = 0; t < 4; ++t) y[t] = lerp<float>(P[t], P[t + 1], d[2]);
+                } else {
+                    load4<WSG>(ga + j * pgb, wsg, y);
+                }
+                if (CROP && m != 15u) {
+#pragma unroll
+                    for (int t = 0; t < 4; ++t) y[t] = (m >> t) & 1u ? y[t] : 0.f;
+                }
+            }
+            __stcs((float4*)(o + j * orow), make_float4(y[0], y[1], y[2], y[3]));
+        }
+    }
+
+    template <int WSX, int WSG, int WSV>
+    TS_D void run_images3_pool(unsigned char* smem, Ring& ring, unsigned char* dst_img, int npl, float* ts) const {
+        Pair q;
+        const bool valid = tid < npl * a.img_pairs && decode_pair(a, tid, q);
+        if (!valid) { q.pl = 0; q.r = 0; q.cg = 0; }
+        PairCtx pc = pair_ctx<MODE, CROP>(a, ug, q, valid);
+        // the pooled tile of the unshifted gradient (crops: its origin, indexed element by element)
+        if (MODE == 2) pc.vo = (unsigned)(a.off_v + q.pl * a.tile_v + (CROP ? 0 : ((q.r >> 1) * a.PW + 2 * q.cg) * 4));
+        Carry ca, cb;
+        if constexpr (MODE != 2) {
+            float run[2] = {0.f, 0.f};
+            for (int k = 0; k <= a.IA; ++k) {
+                const unsigned sb = shared_addr(smem + (size_t)ring.s * a.stage_stride + GUARD);
+                mbar_wait_parked(&wait_bar[ring.s], ring.phase);
+                pool_step_fwd<WSX>(sb, dst_img, k, pc, ca, cb, run);
+                if (MODE == 1) {
+#pragma unroll
+                    for (int j = 0; j < 3; ++j)
+#pragma unroll
+                        for (int t = 0; t < 5; ++t) ca.X[j][t] = cb.X[j][t];
+                }
+                release(ring);
+            }
+        } else {
+            for (int k = 0; k <= a.IA; k += 2) {
+                {
+                    const unsigned sb = shared_addr(smem + (size_t)ring.s * a.stage_stride + GUARD);
+                    mbar_wait_parked(&wait_bar[ring.s], ring.phase);
+                    pool_step_bwd<WSX, WSG, WSV>(sb, dst_img, k, pc, q, cb, ca, ts);
+                    release(ring);
+                }
+                if (k + 1 <= a.IA) {
+                    const unsigned sb = shared_addr(smem + (size_t)ring.s * a.stage_stride + GUARD);
+                    mbar_wait_parked(&wait_bar[ring.s], ring.phase);
+                    pool_step_bwd<WSX, WSG, WSV>(sb, dst_img, k + 1, pc, q, ca, cb, ts);
+                    release(ring);
+                }
+            }
+        }
+    }
+
     // The pair's context and its backward steps sit in loops of ONE trip on purpose: the compiler's schedule of the 3-D
     // kernels depends on that loop structure (straight-line code adds 36 bytes of spills per thread to the interpolating
     // backward and reorders both interpolating kernels).
     template <int WSX, int WSG, int WSV>
     TS_D void run_images3(unsigned char* smem, Ring& ring, unsigned char* dst_img, int npl, float* ts) const {
+        if constexpr (POOL) {
+            run_images3_pool<WSX, WSG, WSV>(smem, ring, dst_img, npl, ts);
+            return;
+        }
         PairCtx pc[1];
         Carry ca[1], cb[1];                    // the windows of two consecutive slabs, roles alternating from step to step
 #pragma unroll
@@ -1115,11 +1409,12 @@ __global__ void __launch_bounds__(MAXT, 1) k_halo(const __grid_constant__ HArgs 
     }
     __syncthreads();
     const UnitOrder uo = {a.table ? order : nullptr, cend, coff, a.chunks, C};
-    if (wid == a.nw) { producer(a, smem, full, empty, tbl, uo, lane); return; }
+    if (wid == a.nw) { producer<POOL && MODE == 2 && DIM == 3>(a, smem, full, empty, tbl, uo, lane); return; }
     if (wid > a.nw) {                                                         // launched only when the padding needs it
         // (the pooled-gradient expansion and its multi-warp fixer exist only in the POOL && MODE == 2 instantiations: the same
         // code merely PRESENT in the other kernels changed ptxas' schedule of their hot loops -- cfg4 forward 0.31 -> 0.37 ms)
-        if constexpr (POOL && MODE == 2) fixer_pool<true>(a, smem, full, ready, lane, wid - a.nw - 1, tbl, lists, uo);
+        if constexpr (POOL && MODE == 2 && DIM == 3) fixer_pool3(a, smem, full, ready, lane, tbl, lists, uo);
+        else if constexpr (POOL && MODE == 2) fixer_pool<true>(a, smem, full, ready, lane, wid - a.nw - 1, tbl, lists, uo);
         else fixer(a, smem, full, ready, lane, tbl, lists, uo);
         return;
     }
@@ -1144,7 +1439,7 @@ bool bind(HArgs& a, const void* x, const void* grad, void* out, const void* w, d
     a.x = (const float*)x; a.grad = (const float*)grad; a.out = (float*)out; a.w = (const float*)w; a.partials = partials;
     if (!make_tensor_map5(&a.map_x, x, 4, g.N, g.C, a.A, a.B, a.L, a.px, a.bpx, 1, 1)) return false;
     if (a.mode == 2 && a.pool_bwd) {
-        if (!make_tensor_map5(&a.map_v, grad, 4, g.N, g.C, 1, a.PH, a.PW, a.PW, a.PH, 1, 1)) return false;
+        if (!make_tensor_map5(&a.map_v, grad, 4, g.N, g.C, a.PA, a.PH, a.PW, a.PW, a.PH, 1, 1)) return false;
     } else if (a.mode == 2) {
         if (!make_tensor_map5(&a.map_g, grad, 4, g.N, g.C, a.OA, a.OB, a.OL, a.pg, a.bpg, 1, 1)) return false;
         if (a.dim == 3 && !make_tensor_map5(&a.map_v, grad, 4, g.N, g.C, a.OA, a.OB, a.OL, a.OL, a.OB, 1, 1)) return false;
@@ -1156,21 +1451,22 @@ bool bind(HArgs& a, const void* x, const void* grad, void* out, const void* w, d
 
 // ---- planning -----------------------------------------------------------------------------------
 HaloPlan plan_halo(const Geo& g, int mode, int active, int dtype, bool dense_x, const void* x, const void* out, const void* grad,
-                   int sm_count, bool forced, bool pool_bwd) {
+                   int sm_count, bool forced, bool pool_bwd, int pool_sa) {
     HaloPlan p;
     memset(&p, 0, sizeof(p));
     p.ok = false;
     if (!tma_available() || !dense_x || dtype != TS_F32 || mode < 0 || mode > 2) return p;
     const int d = g.dim;
     if (d != 2 && d != 3) return p;
-    if (mode == 0 && d != 2) return p;                     // sparse forward: 2-D only (the pooled epilogue); 3-D gathers stay on ts_staged.cu
+    const bool pool3 = d == 3 && (pool_sa == 1 || pool_sa == 2);
+    if (mode == 0 && d != 2 && !pool3) return p;          // sparse forward: the pooled epilogues only; other 3-D gathers stay on ts_staged.cu
     if (g.N * g.C == 0 || g.in_plane == 0 || g.out_plane == 0) return p;
     for (int ax = 0; ax < d; ++ax)
         if (g.S[ax] < 2 || g.OS[ax] < 2) return p;        // a size-1 axis ignores its shift (shifts_kernels.h:40-50): other families
     const Levels lv(g);
     const int B = lv.B, L = lv.L, OB = lv.OB, OL = lv.OL;
     if (L % 4 || OL % 4) return p;
-    if (pool_bwd && (mode != 2 || d != 2 || OL % 8)) return p;      // pooled rows of a multiple of 16 bytes (TMA)
+    if (pool_bwd && (mode != 2 || (d != 2 && !pool3) || OL % 8)) return p;      // pooled rows of a multiple of 16 bytes (TMA)
     if (((uintptr_t)x & 15) || ((uintptr_t)out & 15) || ((uintptr_t)grad & 15)) return p;
     if (g.N >= (1ll << 31) || g.C >= (1ll << 31)) return p;
     if (g.in_plane * 4 >= (1ll << 40) / (g.C > 0 ? g.C : 1)) return p;
@@ -1191,21 +1487,25 @@ HaloPlan plan_halo(const Geo& g, int mode, int active, int dtype, bool dense_x, 
     if (a.pg % 8 == 0) a.pg += 4;
     if (a.px > 256 || a.bpx > 256 || a.pg > 256 || a.bpg > 256) return p;           // TMA box extents
     a.PH = (OB + 1) / 2; a.PW = OL / 2;
+    a.sA = pool3 ? pool_sa : 1;
+    a.PA = pool3 ? (lv.OA + pool_sa - 1) / pool_sa : 1;
     a.pool_bwd = pool_bwd ? 1 : 0;
     a.need_fix = g.pad != TS_PAD_ZEROS || pool_bwd;
-    a.nfix = pool_bwd ? 4 : 1;
+    const bool expand_warps = pool_bwd && d == 2;          // 3-D: the one fixer warp expands the pooled gradient
+    a.nfix = expand_warps ? 4 : 1;
     a.tile_x = (int)round_up((long long)a.px * a.bpx * 4, 128);
     a.tile_g = mode == 2 ? (int)round_up((long long)a.pg * a.bpg * 4, 128) : 0;
     // the dense grad slab of the 3-D backward, or the pooled-gradient tile of the fused avg-pool backward
     a.tile_v = pool_bwd ? (int)round_up((long long)a.PH * a.PW * 4, 128) : (mode == 2 && d == 3) ? (int)round_up((long long)OL * OB * 4, 128) : 0;
     a.box_x = a.px * a.bpx * 4; a.box_g = a.pg * a.bpg * 4; a.box_v = pool_bwd ? a.PW * a.PH * 4 : OL * OB * 4;
-    const long long per_image = (long long)a.tile_x + a.tile_g + a.tile_v;
+    // (3-D pooled backward: two pooled tiles per image, the unshifted gradient's and the one expanded for grad_input)
+    const long long per_image = (long long)a.tile_x + a.tile_g + a.tile_v * (pool_bwd && pool3 ? 2 : 1);
     a.IA = mode == 2 ? a.A : a.OA;
     const int IB = a.IB = mode == 2 ? B : OB, IG = a.IG = (mode == 2 ? L : OL) / 4;
     const int GP = a.GP = padded_groups(IG);
     a.RP = (IB + 1) / 2;
     const int img_pairs = a.img_pairs = a.RP * GP;
-    const int max_nt = MAXT - 64 - (pool_bwd ? 96 : 0);    // producer warp + fixer warp(s)
+    const int max_nt = MAXT - 64 - (expand_warps ? 96 : 0);    // producer warp + fixer warp(s)
     const long long table_bytes = (g.C <= TABLE_MAX_C ? g.C * 36 : 0) + ((g.pad != TS_PAD_ZEROS || pool_bwd) ? 2 * FIXCAP * 4 : 0)      // + the fixer's cell lists
                                   + (2 * NCLS + 1) * 4 + (g.C <= TABLE_MAX_C ? g.C * 3 : 0) + 16;                             // + the class order
     const long long budget = SMEM_LIMIT - 1024 - table_bytes;
@@ -1284,12 +1584,27 @@ int halo_forward2d(const Geo& g, const HaloPlan& p, int active, int pool, const 
     return pool ? launch(k_halo<2, 0, false, true>, a, p, s) : launch(k_halo<2, 0, false, false>, a, p, s);
 }
 
+// 3-D forward (sparse or active) with avg_pool3d(kernel = stride = (sA, 2, 2), ceil_mode) fused into the store: one read of x,
+// one pooled write.
+int halo_forward3d_pool(const Geo& g, const HaloPlan& p, int active, const void* x, const void* w, void* y, cudaStream_t s) {
+    if (g.dim != 3) return TS_ERR_UNSUPPORTED;
+    HArgs a = p.a;
+    a.pool = 1;
+    a.out_plane_bytes = (long long)a.PA * a.PH * a.PW * 4;
+    if (!bind(a, x, nullptr, y, w, nullptr)) return TS_ERR_UNSUPPORTED;
+    return active ? launch(k_halo<3, 1, true, true>, a, p, s) : launch(k_halo<3, 0, false, true>, a, p, s);
+}
+
 int halo_backward(const Geo& g, const HaloPlan& p, int active, const void* grad, const void* x, const void* w, void* gi,
                   double* partials, cudaStream_t s) {
     HArgs a = p.a;
     if (!bind(a, x, grad, gi, w, partials)) return TS_ERR_UNSUPPORTED;
     bool crop = false;
     for (int ax = 0; ax < g.dim; ++ax) crop = crop || g.lb[ax] != 0 || g.OS[ax] != g.S[ax];
+    if (a.pool_bwd && g.dim == 3) {
+        if (active) return crop ? launch(k_halo<3, 2, true, true, true>, a, p, s) : launch(k_halo<3, 2, true, true, false>, a, p, s);
+        return crop ? launch(k_halo<3, 2, false, true, true>, a, p, s) : launch(k_halo<3, 2, false, true, false>, a, p, s);
+    }
     if (a.pool_bwd) {
         if (g.dim != 2) return TS_ERR_UNSUPPORTED;
         if (active) return crop ? launch(k_halo<2, 2, true, true, true>, a, p, s) : launch(k_halo<2, 2, true, true, false>, a, p, s);

@@ -293,6 +293,7 @@ struct alignas(64) HArgs {
     FastDiv d_GP, d_img, d_C, d_chunks, d_PW;
     int nfix;                                 // fixer warps (1; 4 when they also expand the pooled gradient)
     int pool_bwd, PH, PW;                     // backward fused with the adjoint of avg_pool2d(2, 2, ceil_mode): pooled rows / columns
+    int sA, PA;                               // 3-D fused avg-pool (forward and backward): slab stride (1 or 2), pooled slabs; 2-D: 1, 1
 };
 struct HaloPlan {
     bool ok;
@@ -304,10 +305,14 @@ struct HaloPlan {
 // every padding, border crops.
 // pool_bwd (mode 2, 2-D): `grad` is the gradient of the 2x2 / stride-2 / ceil_mode average pooling of the shift's output;
 // the kernel expands it while staging (ts_shift2d_avgpool2_backward); halo_backward then launches the pooled kernels.
+// pool_sa (3-D, mode 0..2): the plan of the kernels fused with avg_pool3d(kernel = stride = (pool_sa, 2, 2), ceil_mode);
+// 0: no 3-D pooling (a 3-D sparse forward is then declined: those gathers stay on the other families).
 HaloPlan plan_halo(const Geo& g, int mode, int active, int dtype, bool dense_x, const void* x, const void* out, const void* grad,
-                   int sm_count, bool forced, bool pool_bwd = false);
+                   int sm_count, bool forced, bool pool_bwd = false, int pool_sa = 0);
 int halo_active_forward(const Geo& g, const HaloPlan& p, const void* x, const void* w, void* y, cudaStream_t s);
 int halo_forward2d(const Geo& g, const HaloPlan& p, int active, int pool, const void* x, const void* w, void* y, cudaStream_t s);
+// 3-D forward of a pool_sa plan: y_pooled dense [N, C, ceil(O0 / pool_sa), ceil(O1 / 2), O2 / 2]
+int halo_forward3d_pool(const Geo& g, const HaloPlan& p, int active, const void* x, const void* w, void* y, cudaStream_t s);
 int halo_backward(const Geo& g, const HaloPlan& p, int active, const void* grad, const void* x, const void* w, void* gi,
                   double* partials, cudaStream_t s);
 

@@ -31,7 +31,7 @@ class PeerGroup(ct.Structure):
 
 
 _vp, _i, _i64, _sz = ct.c_void_p, ct.c_int, ct.c_int64, ct.c_size_t
-_geo, _peers, _i64p = ct.POINTER(Geometry), ct.POINTER(PeerGroup), ct.POINTER(ct.c_int64)
+_geo, _peers, _i64p, _i32p = ct.POINTER(Geometry), ct.POINTER(PeerGroup), ct.POINTER(ct.c_int64), ct.POINTER(ct.c_int32)
 # restype and argtypes of every symbol include/torchshifts_b200.h declares
 SIGNATURES = {
     'ts_abi_version': (_i, []), 'ts_cuda_version': (_i, []),
@@ -56,6 +56,9 @@ SIGNATURES = {
     'ts_shift_forward_nhwc': (_i, [_geo, _i, _i, _i, _vp, _vp, _vp, _vp]),
     'ts_shift_backward_nhwc_workspace_bytes': (_sz, [_geo, _i]),
     'ts_shift_backward_nhwc': (_i, [_geo, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _peers, _vp]),
+    'ts_shift_avgpool_forward': (_i, [_geo, _i, _i, _i, _i32p, _vp, _vp, _vp, _vp]),
+    'ts_shift_avgpool_backward_workspace_bytes': (_sz, [_geo, _i]),
+    'ts_shift_avgpool_backward': (_i, [_geo, _i, _i, _i, _i32p, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _peers, _vp]),
 }
 # tests check that the library exports all of them and that the header declares no others
 EXPORTED_SYMBOLS = tuple(SIGNATURES)

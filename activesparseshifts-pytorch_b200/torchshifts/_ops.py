@@ -207,9 +207,10 @@ def _check_size(fn, name, size, dim, input, lb, rb):
 
 
 def _launch_backward(entry, query, geo, key, grad, input, weights, padding_mode, active_flag, peers=(),
-                     fmt=torch.contiguous_format, fallback=()):
+                     fmt=torch.contiguous_format, fallback=(), lead=()):
     """Runs the backward entry point ``entry`` -> (grad_input in ``fmt``, grad_weight).  ``query`` is its workspace-size
-    function, cached per geometry; ``peers``: the trailing peer-group argument of the entry points that take one.
+    function, cached per geometry; ``peers``: the trailing peer-group argument of the entry points that take one;
+    ``lead``: arguments between ``active`` and ``grad`` (the pooling stride of the fused avg-pool backward).
 
     With a ``fallback`` (statuses as for ``_served``) returns None when the kernel does not serve the call: the launch
     returned such a status, or ``query`` answered 16 bytes (no partials), which is decided before ``grad`` is converted
@@ -231,7 +232,7 @@ def _launch_backward(entry, query, geo, key, grad, input, weights, padding_mode,
             grad_input = torch.empty(input.shape, dtype=input.dtype, device=dev, memory_format=fmt)
             grad_weight = torch.empty(w.shape, dtype=w.dtype, device=dev)
             workspace = torch.empty(max(nbytes, 16), dtype=torch.uint8, device=dev)
-            st = entry(ct.byref(geo), code, int(padding_mode), int(bool(active_flag)), grad.data_ptr(), input.data_ptr(),
+            st = entry(ct.byref(geo), code, int(padding_mode), int(bool(active_flag)), *lead, grad.data_ptr(), input.data_ptr(),
                        w.data_ptr(), grad_input.data_ptr(), grad_weight.data_ptr(), workspace.data_ptr(), nbytes, *peers,
                        _stream(dev))
             if st != TS_ERR_WORKSPACE:      # (nothing was launched): the tuning knobs changed since the size was cached
@@ -292,22 +293,37 @@ def _pool_forward_meta(input, weights, borders, new_size, padding_mode, active_f
     return input.new_empty([new_size[0], new_size[1], (new_size[2] + 1) // 2, (new_size[3] + 1) // 2])
 
 
+def _strides(values):
+    return (ct.c_int32 * len(values))(*[int(v) for v in values])
+
+
+def _pool_backward_fused(fn, dim, stride, grad_pooled, weights, input, lb, rb, padding_mode, active_flag):
+    """The fused avg-pool backward (ts_shift_avgpool_backward) -> (grad_input, grad_weight), or None where the kernels do not
+    serve the call.  Under FusedGradWeightAllReduce grad_weight is summed over the ranks in the same launch; a rank whose call
+    is not served takes the caller's two-step path, whose shift backward exchanges too."""
+    geo, key = _geometry(dim, input, lb, rb)
+    lib, fused = _NATIVE.lib, _FUSED_ALLREDUCE
+    peers = (ct.byref(fused.peer_group()) if fused is not None else None,)
+    return _launch_backward(lib.ts_shift_avgpool_backward, lib.ts_shift_avgpool_backward_workspace_bytes, geo, key, grad_pooled,
+                            input, weights, padding_mode, active_flag, peers, fallback=_FALLBACK, lead=(_strides(stride),))
+
+
 def _pool_backward_cuda(grad_pooled, weights, input, borders, new_size, padding_mode, active_flag):
-    """Backward of the fused shift + avg_pool2d(2, 2, ceil_mode): ONE kernel (ts_shift2d_avgpool2_backward) that expands the
+    """Backward of the fused shift + avg_pool2d(2, 2, ceil_mode): ONE kernel (ts_shift_avgpool_backward) that expands the
     pooled gradient while staging it -- the full-size gradient of the shift's output never exists in HBM.  Shapes the fused
     kernel does not serve take ATen's avg_pool2d_backward followed by the shift backward (same values)."""
     fn = 'shift2d_avgpool2_backward'
     _check_mode(padding_mode)
     _same_device_and_type(fn, input, weights, grad_pooled)
+    if _FUSED_ALLREDUCE is not None:
+        _check_fused(fn, _FUSED_ALLREDUCE, input.device, _DTYPES[input.dtype], weights.numel())
     lb, rb = _borders_lists(borders, 2)
     oh, ow = rb[0] - lb[0], rb[1] - lb[1]
     if list(grad_pooled.shape) != [input.shape[0], input.shape[1], (oh + 1) // 2, (ow + 1) // 2]:
         raise RuntimeError(f'{fn}: grad has shape {list(grad_pooled.shape)}, the pooled output is '
                            f'{[input.shape[0], input.shape[1], (oh + 1) // 2, (ow + 1) // 2]}')
     if input.dtype == torch.float32 and input.is_contiguous() and ow % 8 == 0 and input.dim() == 4 and input.numel() > 0:
-        geo, key = _geometry(2, input, lb, rb)
-        grads = _launch_backward(_NATIVE.lib.ts_shift2d_avgpool2_backward, _NATIVE.lib.ts_shift_backward_workspace_bytes, geo, key,
-                                 grad_pooled, input, weights, padding_mode, active_flag, fallback=_FALLBACK)
+        grads = _pool_backward_fused(fn, 2, (2, 2), grad_pooled, weights, input, lb, rb, padding_mode, active_flag)
         if grads is not None:
             return grads
     like = torch.empty(list(new_size), dtype=grad_pooled.dtype, device=grad_pooled.device)
@@ -316,6 +332,66 @@ def _pool_backward_cuda(grad_pooled, weights, input, borders, new_size, padding_
 
 
 def _pool_backward_meta(grad_pooled, weights, input, borders, new_size, padding_mode, active_flag):
+    return input.new_empty(input.shape), weights.new_empty(weights.shape)
+
+
+def _pooled_size(new_size, stride):
+    return list(new_size[:2]) + [-(-int(o) // int(s)) for o, s in zip(new_size[2:], stride)]
+
+
+def _pool3d_forward_cuda(input, weights, borders, new_size, stride, padding_mode, active_flag):
+    """Shift3d forward + avg_pool3d(kernel = stride, ceil_mode=True) for the strides (1, 2, 2) and (2, 2, 2) in ONE kernel
+    (ts_shift_avgpool_forward): one read of x, one pooled write.  Shapes the fused kernel does not serve (non-fp32, rows that
+    are not a multiple of 4 elements, strided inputs, slabs too large to stage) run the two steps separately -- same values."""
+    fn = 'shift3d_avgpool_forward'
+    _check_forward(fn, 3, input, weights, padding_mode)
+    lb, rb = _borders_lists(borders, 3)
+    _check_size(fn, 'new_size', new_size, 3, input, lb, rb)
+    if input.dtype == torch.float32 and weights.dtype == torch.float32 and input.is_contiguous():
+        out = torch.empty(_pooled_size(new_size, stride), dtype=input.dtype, device=input.device)
+        w = weights.contiguous()
+        geo, _ = _geometry(3, input, lb, rb)
+        with _guard(input.device):
+            st = _NATIVE.lib.ts_shift_avgpool_forward(ct.byref(geo), 0, int(padding_mode), int(bool(active_flag)), _strides(stride),
+                                                      input.data_ptr(), w.data_ptr(), out.data_ptr(), _stream(input.device))
+        if _served(st, 'ts_shift_avgpool_forward', _FALLBACK):
+            return out
+    y = _forward_cuda(3, input, weights, borders, new_size, padding_mode, active_flag)
+    return torch.nn.functional.avg_pool3d(y, kernel_size=list(stride), stride=list(stride), ceil_mode=True)
+
+
+def _pool3d_forward_meta(input, weights, borders, new_size, stride, padding_mode, active_flag):
+    return input.new_empty(_pooled_size(new_size, stride))
+
+
+def _pool3d_backward_cuda(grad_pooled, weights, input, borders, new_size, stride, padding_mode, active_flag):
+    """Backward of ``_shift3d_avgpool_forward``: ONE kernel (ts_shift_avgpool_backward) applies the pooling adjoint while the
+    pooled gradient is staged, plus the pass-2 reduction.  What the kernel does not serve (and empty shards) takes ATen's
+    avg_pool3d_backward followed by the shift backward -- same values, and the same grad_weight exchange."""
+    fn = 'shift3d_avgpool_backward'
+    _check_mode(padding_mode)
+    _same_device_and_type(fn, input, weights, grad_pooled)
+    if _FUSED_ALLREDUCE is not None:
+        _check_fused(fn, _FUSED_ALLREDUCE, input.device, _DTYPES[input.dtype], weights.numel())
+    lb, rb = _borders_lists(borders, 3)
+    _check_size(fn, 'new_size', new_size, 3, input, lb, rb)
+    if list(grad_pooled.shape) != _pooled_size(new_size, stride):
+        raise RuntimeError(f'{fn}: grad has shape {list(grad_pooled.shape)}, the pooled output is {_pooled_size(new_size, stride)}')
+    if (input.dtype == torch.float32 and weights.dtype == torch.float32 and input.is_contiguous() and new_size[4] % 8 == 0
+            and input.numel() > 0):
+        grads = _pool_backward_fused(fn, 3, stride, grad_pooled, weights, input, lb, rb, padding_mode, active_flag)
+        if grads is not None:
+            return grads
+    if grad_pooled.numel() == 0:
+        grad_y = grad_pooled.new_zeros(list(new_size))
+    else:
+        like = torch.empty(list(new_size), dtype=grad_pooled.dtype, device=grad_pooled.device)
+        grad_y = torch.ops.aten.avg_pool3d_backward(grad_pooled.contiguous(), like, list(stride), list(stride), [0, 0, 0], True, True,
+                                                    None)
+    return _backward_cuda(3, grad_y, weights, input, borders, padding_mode, active_flag)
+
+
+def _pool3d_backward_meta(grad_pooled, weights, input, borders, new_size, stride, padding_mode, active_flag):
     return input.new_empty(input.shape), weights.new_empty(weights.shape)
 
 
@@ -489,9 +565,10 @@ def _forward_autograd(backward_op, takes_new_size):
     """-> (backward, setup_context) of a forward op: save input, weights and borders (and new_size when ``backward_op``
     takes it), keep the planar copy the forward made, and call ``backward_op``."""
     def setup_context(ctx, inputs, output):
-        input, weights, borders, new_size, padding_mode, active_flag = inputs
+        input, weights, borders, new_size, *rest = inputs         # rest: (stride,) padding_mode, active_flag
         ctx.save_for_backward(input, weights, borders)
-        ctx.tail = (list(new_size), padding_mode, active_flag) if takes_new_size else (padding_mode, active_flag)
+        ctx.tail = (list(new_size), *rest) if takes_new_size else tuple(rest)
+        ctx.n_inputs = len(inputs)
         if _LAST_PLANAR[0] is not None:
             _claim_planar(input)
 
@@ -499,7 +576,7 @@ def _forward_autograd(backward_op, takes_new_size):
         input, weights, borders = ctx.saved_tensors
         op = getattr(torch.ops.torchshifts, backward_op)
         grad_input, grad_weight = op(grad_output, weights, input, borders, *ctx.tail)
-        return grad_input, grad_weight, None, None, None, None
+        return (grad_input, grad_weight) + (None,) * (ctx.n_inputs - 2)
     return backward, setup_context
 
 
@@ -547,6 +624,11 @@ _BACKWARD = '(Tensor grad, Tensor weights, Tensor input, Tensor borders, int pad
 _POOL_BACKWARD = ('(Tensor grad, Tensor weights, Tensor input, Tensor borders, int[] new_size, int padding_mode, '
                   'bool active_flag) -> (Tensor, Tensor)')
 
+_POOL3D_FORWARD = ('(Tensor input, Tensor weights, Tensor borders, int[] new_size, int[] stride, int padding_mode, '
+                   'bool active_flag) -> Tensor')
+_POOL3D_BACKWARD = ('(Tensor grad, Tensor weights, Tensor input, Tensor borders, int[] new_size, int[] stride, int padding_mode, '
+                    'bool active_flag) -> (Tensor, Tensor)')
+
 
 def register(native):
     """Define and implement the operators (idempotent)."""
@@ -573,6 +655,9 @@ def register(native):
     # fused epilogue of the strided depth-wise-conv emulation (modules/shifts.py:85-89): shift + crop + avg_pool2d(2, 2, ceil)
     ops['_shift2d_avgpool2_forward'] = (_FORWARD, _pool_forward_cuda, _pool_forward_meta, None)
     ops['_shift2d_avgpool2_backward'] = (_POOL_BACKWARD, _pool_backward_cuda, _pool_backward_meta, None)
+    # 3-D: shift + crop + avg_pool3d(kernel = stride, ceil_mode) for the strides (1, 2, 2) and (2, 2, 2)
+    ops['_shift3d_avgpool_forward'] = (_POOL3D_FORWARD, _pool3d_forward_cuda, _pool3d_forward_meta, None)
+    ops['_shift3d_avgpool_backward'] = (_POOL3D_BACKWARD, _pool3d_backward_cuda, _pool3d_backward_meta, None)
     for name, (schema, cuda, fake, qcuda) in ops.items():
         lib.define(name + schema)
         lib.impl(name, cuda, 'CUDA')

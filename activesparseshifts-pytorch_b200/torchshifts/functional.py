@@ -173,5 +173,36 @@ def shift2d_avgpool2_func(input: Tensor, weights: Tensor, padding_mode: int, act
     return out
 
 
+_POOL3D_STRIDES = ((1, 2, 2), (2, 2, 2))
+
+
+def shift3d_avgpool_func(input: Tensor, weights: Tensor, padding_mode: int, active_flag: bool, stride,
+                         borders: Optional[Tensor] = None, _border_ints=None) -> Tensor:
+    """``avg_pool3d(shift3d_func(...), kernel_size=stride, stride=stride, ceil_mode=True)`` in one kernel, for ``stride``
+    (1, 2, 2) -- the spatial downsampling of video networks -- or (2, 2, 2) (a scalar 2 is (2, 2, 2)): what a ``Shift3d``
+    built with ``emulate_dw={..., 'stride': stride}`` computes (reference ``modules/shifts.py:85-89``), with one read of the
+    input and one pooled write; the backward never materialises the full-size gradient.  Same values as the two steps (the
+    forward and ``grad_input`` bit for bit).  Same argument checks as :func:`shift3d_func`; any other stride raises
+    ``ValueError``.  fp32 CUDA tensors run the fused kernels, others the two steps inside the same operator."""
+    name = 'shift3d_avgpool_func'
+    _assert_has_ops()
+    st = tuple(int(v) for v in stride) if isinstance(stride, (tuple, list, torch.Size)) else (int(stride),) * 3
+    if st not in _POOL3D_STRIDES:
+        raise ValueError(f'{name}(): stride must be (1, 2, 2) or (2, 2, 2), got {stride!r}')
+    assert padding_mode in [0, 1, 2, 3, 4], f'{name}() expected padding_mode can be {_MODES}'
+    assert len(input.shape) == 5, f'{name}(): expected 5D tensor as input, but it is shape is {input.shape}'
+    assert weights.shape[-1] == 3, f'{name}(): expected [n_channels,3] tensor as weight, but it is shape is {weights.shape}'
+    assert input.shape[1] == weights.shape[0], (f'{name}(): expected that input and weight have equal number of channels, '
+                                                f'but input have {input.shape[1]} and weight have {weights.shape[0]} channels.')
+    assert input.device == weights.device, (f'{name}(): expected input and weights to be on same device, '
+                                            f'but input is  on {input.device} and weights is on {weights.device}')
+    if borders is not None:
+        assert tuple(borders.shape) == (3, 2), 'borders must have shape [3, 2]'
+    std, new_size = _crop(3, input, borders, _border_ints)
+    out = torch.ops.torchshifts._shift3d_avgpool_forward(input, weights, std, new_size, list(st), padding_mode, active_flag)
+    drop_unclaimed_planar()
+    return out
+
+
 # BASELINE.json names these "functional.shift1d/2d/3d"; keep the real names and add the aliases.
 shift1d, shift2d, shift3d = shift1d_func, shift2d_func, shift3d_func

@@ -19,7 +19,7 @@ import torch
 from torch import nn
 
 from torchshifts.functional import (_check_memory_format, _keeps_channels_last, shift1d_func, shift2d_avgpool2_func,
-                                    shift2d_func, shift3d_func)
+                                    shift2d_func, shift3d_avgpool_func, shift3d_func)
 
 paddings_dict = {'zeros': 0, 'border': 1, 'periodic': 2, 'reflect': 3, 'symmetric': 4}
 _SHIFT_FUNCS = {1: shift1d_func, 2: shift2d_func, 3: shift3d_func}
@@ -169,17 +169,23 @@ class _Shiftnd(nn.Module):
         return cached[1]
 
     def _pool_is_fused(self, input):
-        """The stride-2 average pooling of a 2-D depth-wise-conv emulation runs inside the shift kernel (one read, one
-        quarter-size write) for float32 CUDA tensors; everything else takes the shift followed by ``_reduction_fn``."""
-        return (self.dim == 2 and self._reduction_fn is not self._identity and input.is_cuda and input.dtype == torch.float32
-                and not input.is_quantized and self._stride_ints == [2, 2]
-                and not (self.memory_format is torch.preserve_format and _keeps_channels_last(2, input)))
+        """The average pooling of a depth-wise-conv emulation with stride (2, 2), or (1, 2, 2) / (2, 2, 2) in 3-D, runs inside
+        the shift kernel (one read, one pooled write) for float32 CUDA tensors; everything else takes the shift followed by
+        ``_reduction_fn``."""
+        fused = {2: ([2, 2],), 3: ([1, 2, 2], [2, 2, 2])}.get(self.dim, ())
+        return (self._reduction_fn is not self._identity and self._stride_ints in fused and input.is_cuda
+                and input.dtype == torch.float32 and not input.is_quantized
+                and not (self.memory_format is torch.preserve_format and _keeps_channels_last(self.dim, input)))
 
     def forward(self, input):
         loss = self._compute_weight_loss() if bool(self.sparsity_term) else None
         if self._pool_is_fused(input):
-            out = shift2d_avgpool2_func(input, self.weight, self.padding, self._active_flag, self.cut_borders,
-                                        _border_ints=self._border_ints())
+            if self.dim == 3:
+                out = shift3d_avgpool_func(input, self.weight, self.padding, self._active_flag, self._stride_ints, self.cut_borders,
+                                           _border_ints=self._border_ints())
+            else:
+                out = shift2d_avgpool2_func(input, self.weight, self.padding, self._active_flag, self.cut_borders,
+                                            _border_ints=self._border_ints())
             return out, loss
         if self.cut_borders is None:
             out = self._shift_func(input, self.weight, self.padding, self._active_flag, None, memory_format=self.memory_format)

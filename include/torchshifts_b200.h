@@ -189,6 +189,34 @@ int ts_shift_backward_allreduce(const ts_geometry* g, int dtype, int padding, in
                                 void* workspace, size_t workspace_bytes,
                                 const ts_peer_group* peers, void* stream);
 
+/* Shift forward fused with the average pooling of a strided depth-wise-conv emulation (modules/shifts.py:85-89:
+ * avg_poolNd(kernel_size=stride, stride=stride, ceil_mode=True) after the shift and the border crop), for the strides in
+ * `stride` (g->dim entries): dim 2: (2, 2), the kernels of ts_shift2d_avgpool2_forward; dim 3: (1, 2, 2) or (2, 2, 2).
+ * y_pooled is dense [N, C, ceil(O0/s0), ceil(O1/s1)(, ceil(O2/s2))]; every window's elements are added in (slab,) row,
+ * column order into one fp32 sum and divided by their count, like ATen's kernels (bit-identical).  One read of x, one
+ * pooled write.  fp32 (no TS_WEIGHTS_F32), dense x, input and output rows of a multiple of 4 elements, planes that fit a
+ * stage; any other stride or shape: TS_ERR_UNSUPPORTED, nothing launched (callers then shift and pool separately).  A
+ * stride entry below 1, a null pointer or a bad dtype: TS_ERR_INVALID_ARGUMENT. */
+int ts_shift_avgpool_forward(const ts_geometry* g, int dtype, int padding, int active, const int32_t* stride,
+                             const void* x, const void* weights, void* y_pooled, void* stream);
+
+/* Workspace of ts_shift_avgpool_backward: enough for every stride and padding it serves on this geometry (16 when it
+ * serves none). */
+size_t ts_shift_avgpool_backward_workspace_bytes(const ts_geometry* g, int dtype);
+
+/* Backward of ts_shift_avgpool_forward in ONE kernel plus the pass-2 reduction: grad_pooled is the gradient of the pooled
+ * output; the adjoint of the pooling (every element of a window receives grad / count, as ATen's avg_poolNd_backward; the
+ * count is a power of two, so this is exact) is applied while the gradient is staged in shared memory, so the full-size
+ * gradient of the shift's output never exists in HBM.  grad_input / grad_weight as for ts_shift_backward; workspace: at least
+ * ts_shift_avgpool_backward_workspace_bytes(), 16-byte aligned.  peers: NULL, or the peer group of an in-kernel grad_weight
+ * exchange, with the rules of ts_shift_backward_allreduce.  Besides the forward's conditions, pooled rows of a multiple of
+ * 16 bytes (O_last a multiple of 8); empty tensors: TS_ERR_UNSUPPORTED (callers take the two-step path, which zero-fills or
+ * exchanges). */
+int ts_shift_avgpool_backward(const ts_geometry* g, int dtype, int padding, int active, const int32_t* stride,
+                              const void* grad_pooled, const void* x, const void* weights,
+                              void* grad_input, void* grad_weight, void* workspace, size_t workspace_bytes,
+                              const ts_peer_group* peers, void* stream);
+
 /* Quantized forward on the raw integer representation.  elem_bytes: 1 (qint8/quint8) or
  * 4 (qint32).  zero_point: input zero point = pad value.  qweights: raw integer weights
  * [C,dim] of kind `qweight_kind`; effective shift = qweights - weight_zero_point. */
